@@ -21,6 +21,10 @@ send/recv while earlier blocks are being intersected and are adopted in place
 `--impl reference` times the reference's own CPU algorithm (oracle string-set port of
 FastaDistanceProcessor; the Java original cannot run here: no JVM, arithmetic in an un-vendored artifact)
 on a bounded sample.  That arm never loads the product library.
+
+`--dump-outputs DIR` writes what the last timed step returned (intersection counts and distances of the
+pairs) to DIR as float64 .npy files, so that two builds can be compared output for output on the same
+seeded inputs.
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ METRIC = "genome pairs/sec all-vs-all k-mer distance"
 UNIT = "pairs/s"
 SEED = 0x5EED0000
 RATES = [0.001, 0.01, 0.05, 0.2]
+DUMP_PAIRS = 2_000_000  # --dump-outputs: three float64 arrays of at most this length, 48 MB
 
 
 def parse_args():
@@ -62,7 +67,14 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--other-configs", action="store_true", default=os.environ.get("GKD_BENCH_OTHER", "0") == "1",
                     help="also run BASELINE configs 1, 3 and 5 at full size (N=1) and report them as other_configs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's results to DIR/{pair_index,intersections,"
+                         f"distances}}.npy (float64, pairs in row-major upper-triangle order; a fixed seeded sample "
+                         f"of {DUMP_PAIRS} pairs when there are more)")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
+    return a
 
 
 def genome_params(g: int, n_genomes: int, families: int):
@@ -254,6 +266,21 @@ def reference_main(a):
 # ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, inter, dist_out):
+    """write one step's per-pair results as float64 .npy files; pair_index holds each entry's row-major index in
+    the strict upper triangle (counts and indices stay exact in float64 below 2**53)"""
+    import numpy as np
+
+    total = inter.size
+    if total > DUMP_PAIRS:
+        idx = np.sort(np.random.default_rng(SEED).choice(total, DUMP_PAIRS, replace=False))
+    else:
+        idx = np.arange(total)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("pair_index", idx), ("intersections", inter[idx]), ("distances", dist_out[idx])):
+        np.save(os.path.join(out_dir, name + ".npy"), arr.astype(np.float64))
+
+
 def main():
     a = parse_args()
     if a.impl == "reference":
@@ -268,6 +295,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if a.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single process: at N>1 the pair results stay on their ranks")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a GPU: libgkd has no CPU fallback")
     torch.cuda.set_device(local)
@@ -361,6 +390,8 @@ def main():
         sampler.start()
     dev_s, wall_s, mets = timed(d_text, a.steps)
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs:  # before the e2e leg, which writes its results into the same arrays
+        dump_outputs(a.dump_outputs, inter, dist_out)
     launches = eng.metrics()["launches"] - launches0
     if world > 1:
         t = torch.tensor([float(launches), float(check["pairs"])], dtype=torch.float64, device=dev)

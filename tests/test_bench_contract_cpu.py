@@ -61,5 +61,32 @@ def test_bench_argument_surface():
     ast.parse(src)
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", "x"],
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and "--dump-outputs" in out.stderr
+
+
+def test_dump_outputs_samples_large_results_at_fixed_pairs(tmp_path, monkeypatch):
+    """more pairs than DUMP_PAIRS: the same seeded, sorted pair sample every time, values taken at those pairs"""
+    import numpy as np
+
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_PAIRS", 500)
+    total = 4950
+    inter = (np.arange(total, dtype=np.uint64) * 7919) % 100003
+    dist = 1.0 - np.arange(total) / total
+    got = []
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), inter, dist)
+        got.append({n: np.load(tmp_path / d / (n + ".npy")) for n in ("pair_index", "intersections", "distances")})
+    idx = got[0]["pair_index"]
+    assert all(x.dtype == np.float64 and x.shape == (500,) for x in got[0].values())
+    assert (np.diff(idx) > 0).all() and idx[0] >= 0 and idx[-1] < total
+    k = idx.astype(np.int64)
+    assert np.array_equal(got[0]["intersections"], inter[k].astype(np.float64))
+    assert np.array_equal(got[0]["distances"], dist[k])
+    for n in got[0]:
+        assert np.array_equal(got[0][n], got[1][n])
