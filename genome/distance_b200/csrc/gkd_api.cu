@@ -125,6 +125,7 @@ struct gkd_ctx {
     DevBuf msd_genomes, msd_bins32, msd_bins64, msd_gstat;
     DevBuf gr_reps, gr_flags;
     DevBuf join_rows, join_err;
+    DevBuf hit_a, hit_b, sel_cta;  // selection epilogues: hit ids / positions (nearest: ref_pos, n_found), tile offsets + total
     int isect_algo = 0;  // GKD_ISECT_ALGO: 0 = choose per call, 1 = bucket merge only, 2 = block join whenever it applies
     bool use_msd = true;  // GKD_SORT_ALGO=lsd pins the LSD path
     bool sets_dirty = true;
@@ -951,7 +952,143 @@ bool plan_join(gkd_ctx *c, const HostPairs &hp, uint64_t first, uint64_t count, 
     return true;
 }
 
-int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out) {
+// What a selection call wants instead of the dense outputs (run_pairs with sel == nullptr writes gkd_outputs).
+struct Selection {
+    bool within;          // true: pairs with dist <= max_dist (gkd_hits); false: k nearest per query row (RECT only)
+    double max_dist;
+    gkd_hits *hits;       // within: the caller's arrays; hits->n counts the hits so far and is the next write position
+    uint32_t a_base;      // within, RECT: position in the caller's q of the first query row of this call
+    uint32_t k;           // nearest
+    int exclude_self;
+    uint32_t *ref_pos;    // nearest: outputs of this call's first row (host or device memory)
+    uint64_t *inter;
+    double *dist;
+    uint32_t *n_found;
+};
+
+// GKD_AMBIG_LITERAL: the chunk's pairs were completed on the host (inter / dist of pairs done .. done+cnt), so the
+// selection runs here with the device kernels' rules
+void host_select(const HostPairs &hp, const Selection &sel, uint64_t done, uint64_t cnt, const uint64_t *inter, const double *dist) {
+    if (sel.within) {
+        gkd_hits &h = *sel.hits;
+        for (uint64_t t = 0; t < cnt; t++) {
+            if (!(dist[t] <= sel.max_dist)) continue;
+            const uint64_t at = h.n++;
+            if (at >= h.cap) continue;
+            uint32_t a, b;
+            if (hp.mode == PAIRS_RECT) a = sel.a_base + (uint32_t)((done + t) / hp.nb), b = (uint32_t)((done + t) % hp.nb);
+            else host_pair_ids(hp, done + t, a, b);
+            if (h.a) h.a[at] = a;
+            if (h.b) h.b[at] = b;
+            if (h.inter) h.inter[at] = inter[t];
+            if (h.dist) h.dist[at] = dist[t];
+        }
+        return;
+    }
+    std::vector<uint32_t> js;
+    for (uint32_t row = 0; row < hp.na; row++) {
+        const uint64_t r0 = (uint64_t)row * hp.nb;
+        js.clear();
+        for (uint32_t j = 0; j < hp.nb; j++)
+            if (dist[r0 + j] <= sel.max_dist && !(sel.exclude_self && hp.a[row] == hp.b[j])) js.push_back(j);
+        const size_t m = std::min<size_t>(js.size(), sel.k);
+        std::partial_sort(js.begin(), js.begin() + m, js.end(), [&](uint32_t x, uint32_t y) {
+            return dist[r0 + x] < dist[r0 + y] || (dist[r0 + x] == dist[r0 + y] && x < y);
+        });
+        for (uint32_t i = 0; i < sel.k; i++) {
+            const uint64_t o = (uint64_t)row * sel.k + i;
+            if (sel.ref_pos) sel.ref_pos[o] = i < m ? js[i] : 0xFFFFFFFFu;
+            if (sel.inter) sel.inter[o] = i < m ? inter[r0 + js[i]] : 0;
+            if (sel.dist) sel.dist[o] = i < m ? dist[r0 + js[i]] : -1.0;
+        }
+        if (sel.n_found) sel.n_found[row] = (uint32_t)m;
+    }
+}
+
+constexpr int SELECT_REDO = 1;  // select_chunk: a join table overflowed; nothing of the attempt was kept
+
+// The selection epilogue of one chunk whose kernel-4 launches are queued: launches the within or nearest selection,
+// then copies back only the hits (within: plus the chunk's 8-byte hit total) or the rows' best lists (nearest).
+// The hit total and the join overflow flag are read before anything is copied, so a chunk that has to be redone by
+// the merge kernel appends nothing.
+int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const Selection &sel, uint64_t cnt, bool need_pal,
+                 bool both, const uint32_t &join_err) {
+    const SetDesc *sets = (const SetDesc *)c->d_sets.p;
+    const uint32_t *counts = (const uint32_t *)c->counts.p, *pal = need_pal ? (const uint32_t *)c->pal_counts.p : nullptr;
+    int rc;
+    unsigned long long chunk_hits = 0;
+    uint64_t wcap = 0, nctas = 0;
+    if (sel.within) {
+        const gkd_hits &h = *sel.hits;
+        const bool any_out = h.a || h.b || h.inter || h.dist;
+        wcap = (any_out && h.n < h.cap) ? std::min<uint64_t>(cnt, h.cap - h.n) : 0;  // the device buffers hold at most this
+        nctas = select_within_ctas(cnt);
+        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
+        if (h.a && (rc = ensure(c, c->hit_a, wcap * 4))) return rc;
+        if (h.b && (rc = ensure(c, c->hit_b, wcap * 4))) return rc;
+        if (h.inter && (rc = ensure(c, c->d_inter, wcap * 8))) return rc;
+        if (h.dist && (rc = ensure(c, c->d_dist, wcap * 8))) return rc;
+        const HitsOut ho{h.a ? (uint32_t *)c->hit_a.p : nullptr, h.b ? (uint32_t *)c->hit_b.p : nullptr,
+                         h.inter ? (uint64_t *)c->d_inter.p : nullptr, h.dist ? (double *)c->d_dist.p : nullptr};
+        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
+        nvtxRangePushA("gkd kernel 5: within selection");
+        CK(launch_select_within(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.a_base, wcap, ho, cta, cta + nctas, c->stream));
+        nvtxRangePop();
+        c->m.launches += wcap ? 3 : 2;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
+    } else {
+        const uint64_t slots = (uint64_t)hp.na * sel.k;
+        if (sel.ref_pos && (rc = ensure(c, c->hit_a, slots * 4))) return rc;
+        if (sel.n_found && (rc = ensure(c, c->hit_b, (uint64_t)hp.na * 4))) return rc;
+        if (sel.inter && (rc = ensure(c, c->d_inter, slots * 8))) return rc;
+        if (sel.dist && (rc = ensure(c, c->d_dist, slots * 8))) return rc;
+        const NearestOut no{sel.ref_pos ? (uint32_t *)c->hit_a.p : nullptr, sel.inter ? (uint64_t *)c->d_inter.p : nullptr,
+                            sel.dist ? (double *)c->d_dist.p : nullptr, sel.n_found ? (uint32_t *)c->hit_b.p : nullptr};
+        nvtxRangePushA("gkd kernel 5: nearest selection");
+        CK(launch_select_nearest(sets, src, hp.na, counts, pal, both ? 1 : 0, sel.max_dist, sel.k, sel.exclude_self, no, c->stream));
+        nvtxRangePop();
+        c->m.launches++;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    if (join_err) return SELECT_REDO;
+    struct {
+        void *dst;
+        const void *src;
+        uint64_t bytes;
+    } copies[4];
+    if (sel.within) {
+        const gkd_hits &h = *sel.hits;
+        const uint64_t w = std::min<uint64_t>(chunk_hits, wcap);
+        copies[0] = {h.a ? h.a + h.n : nullptr, c->hit_a.p, w * 4};
+        copies[1] = {h.b ? h.b + h.n : nullptr, c->hit_b.p, w * 4};
+        copies[2] = {h.inter ? h.inter + h.n : nullptr, c->d_inter.p, w * 8};
+        copies[3] = {h.dist ? h.dist + h.n : nullptr, c->d_dist.p, w * 8};
+    } else {
+        const uint64_t slots = (uint64_t)hp.na * sel.k;
+        copies[0] = {sel.ref_pos, c->hit_a.p, slots * 4};
+        copies[1] = {sel.inter, c->d_inter.p, slots * 8};
+        copies[2] = {sel.dist, c->d_dist.p, slots * 8};
+        copies[3] = {sel.n_found, c->hit_b.p, (uint64_t)hp.na * 4};
+    }
+    uint64_t d2h = sel.within ? 8 : 0;
+    for (const auto &cp : copies) {
+        if (!cp.dst || !cp.bytes) continue;
+        CK(cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, cudaMemcpyDefault, c->stream));
+        d2h += cp.bytes;
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    if (sel.within) sel.hits->n += chunk_hits;
+    c->m.d2h_bytes += d2h;
+    const double ims = elapsed(c->ev[4], c->ev[5]);
+    c->m.intersect_ms += ims;
+    c->m.total_intersect_ms += ims;
+    c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+    return GKD_OK;
+}
+
+int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out, const Selection *sel = nullptr) {
     int rc = upload_sets(c);
     if (rc) return rc;
     const bool nuc = c->cfg.alphabet != GKD_PROT;
@@ -1059,6 +1196,8 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out) {
     if ((rc = ensure(c, c->work_counter, 8))) return rc;
 
     bool join_banned = false;  // set when a join table overflowed: the chunk is redone by the merge kernel
+    std::vector<uint64_t> lit_inter;  // selection on a GKD_AMBIG_LITERAL context: the chunk's completed pairs
+    std::vector<double> lit_dist;
     JoinPlan jplan{};
     std::vector<uint32_t> jrows;
     for (uint64_t done = 0; done < hp.count;) {
@@ -1086,12 +1225,24 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out) {
             if ((rc = ensure(c, c->pal_counts, cnt * 4))) return rc;
             CK(cudaMemsetAsync(c->pal_counts.p, 0, cnt * 4, c->stream));
         }
-        // with literal side lists the pairs are completed on the host, which needs the counts
-        const bool want_inter = out.inter || any_lit;
-        if (want_inter && (rc = ensure(c, c->d_inter, cnt * 8))) return rc;
-        if (out.dist && (rc = ensure(c, c->d_dist, cnt * 8))) return rc;
-        if (out.contain_a && (rc = ensure(c, c->d_ca, cnt * 8))) return rc;
-        if (out.contain_b && (rc = ensure(c, c->d_cb, cnt * 8))) return rc;
+        // with literal side lists the pairs are completed on the host, which needs the counts; a selection on such a
+        // context runs the dense epilogue into host scratch and selects after the completion (host_select)
+        const bool dev_sel = sel && !any_lit;
+        gkd_outputs o = out;
+        uint64_t at = done;  // where this chunk's dense outputs go in o
+        if (sel && any_lit) {
+            lit_inter.resize(cnt);
+            lit_dist.resize(cnt);
+            o = gkd_outputs{lit_inter.data(), lit_dist.data(), nullptr, nullptr};
+            at = 0;
+        }
+        const bool want_inter = o.inter || any_lit;
+        if (!dev_sel) {
+            if (want_inter && (rc = ensure(c, c->d_inter, cnt * 8))) return rc;
+            if (o.dist && (rc = ensure(c, c->d_dist, cnt * 8))) return rc;
+            if (o.contain_a && (rc = ensure(c, c->d_ca, cnt * 8))) return rc;
+            if (o.contain_b && (rc = ensure(c, c->d_cb, cnt * 8))) return rc;
+        }
 
         if (use_join) {
             if ((rc = ensure(c, c->join_rows, jrows.size() * 4))) return rc;
@@ -1130,8 +1281,18 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out) {
             c->m.launches++;
         }
         CK(cudaEventRecord(c->ev[6], c->stream));
-        EpilogueOut eo{want_inter ? (uint64_t *)c->d_inter.p : nullptr, out.dist ? (double *)c->d_dist.p : nullptr,
-                       out.contain_a ? (double *)c->d_ca.p : nullptr, out.contain_b ? (double *)c->d_cb.p : nullptr};
+        if (dev_sel) {
+            rc = select_chunk(c, hp, src, *sel, cnt, need_pal, both, join_err);
+            if (rc == SELECT_REDO) {
+                join_banned = true;
+                continue;
+            }
+            if (rc) return rc;
+            done += PAIR_CHUNK;
+            continue;
+        }
+        EpilogueOut eo{want_inter ? (uint64_t *)c->d_inter.p : nullptr, o.dist ? (double *)c->d_dist.p : nullptr,
+                       o.contain_a ? (double *)c->d_ca.p : nullptr, o.contain_b ? (double *)c->d_cb.p : nullptr};
         nvtxRangePushA("gkd kernel 5: distance epilogue");
         CK(launch_epilogue((const SetDesc *)c->d_sets.p, src, (const uint32_t *)c->counts.p,
                            need_pal ? (const uint32_t *)c->pal_counts.p : nullptr, both ? 1 : 0, eo, c->stream));
@@ -1139,7 +1300,7 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out) {
         c->m.launches++;
         CK(cudaEventRecord(c->ev[7], c->stream));
         std::vector<uint64_t> tmp_inter;
-        uint64_t *h_inter = out.inter ? out.inter + done : nullptr;
+        uint64_t *h_inter = o.inter ? o.inter + at : nullptr;
         if (any_lit && !h_inter) {
             tmp_inter.resize(cnt);
             h_inter = tmp_inter.data();
@@ -1148,9 +1309,9 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out) {
         const struct {
             void *dst;
             const void *src;
-        } copies[4] = {{h_inter, c->d_inter.p}, {out.dist ? out.dist + done : nullptr, c->d_dist.p},
-                       {out.contain_a ? out.contain_a + done : nullptr, c->d_ca.p},
-                       {out.contain_b ? out.contain_b + done : nullptr, c->d_cb.p}};
+        } copies[4] = {{h_inter, c->d_inter.p}, {o.dist ? o.dist + at : nullptr, c->d_dist.p},
+                       {o.contain_a ? o.contain_a + at : nullptr, c->d_ca.p},
+                       {o.contain_b ? o.contain_b + at : nullptr, c->d_cb.p}};
         for (const auto &cp : copies) {
             if (!cp.dst) continue;
             CK(cudaMemcpyAsync(cp.dst, cp.src, cnt * 8, cudaMemcpyDefault, c->stream));
@@ -1176,11 +1337,12 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out) {
                 if (ga.lit.empty() && gb.lit.empty()) continue;
                 const uint64_t I = h_inter[t] + literal_intersection(ga.lit, gb.lit);
                 const uint64_t sa = both_size(c, ga), sb = both_size(c, gb);
-                if (out.inter) out.inter[done + t] = I;
-                if (out.dist) out.dist[done + t] = host_distance(I, sa, sb);
-                if (out.contain_a) out.contain_a[done + t] = sa ? (double)I / (double)sa : 0.0;
-                if (out.contain_b) out.contain_b[done + t] = sb ? (double)I / (double)sb : 0.0;
+                if (o.inter) o.inter[at + t] = I;
+                if (o.dist) o.dist[at + t] = host_distance(I, sa, sb);
+                if (o.contain_a) o.contain_a[at + t] = sa ? (double)I / (double)sa : 0.0;
+                if (o.contain_b) o.contain_b[at + t] = sb ? (double)I / (double)sb : 0.0;
             }
+            if (sel) host_select(hp, *sel, done, cnt, lit_inter.data(), lit_dist.data());
         }
         done += PAIR_CHUNK;
     }
@@ -1374,7 +1536,7 @@ int gkd_destroy(gkd_ctx *c) {
                       &c->set_build, &c->d_sets, &c->counts, &c->pal_counts, &c->d_inter, &c->d_dist, &c->d_ca,
                       &c->d_cb, &c->ids_a, &c->ids_b, &c->work_counter, &c->sk_cand, &c->sk_misc, &c->sk_sig,
                       &c->sk_len, &c->sk_out, &c->msd_genomes, &c->msd_bins32, &c->msd_bins64, &c->msd_gstat,
-                      &c->gr_reps, &c->gr_flags, &c->join_rows, &c->join_err};
+                      &c->gr_reps, &c->gr_flags, &c->join_rows, &c->join_err, &c->hit_a, &c->hit_b, &c->sel_cta};
     for (DevBuf *b : bufs)
         if (b->p) cudaFreeAsync(b->p, c->stream);
     cudaStreamSynchronize(c->stream);
@@ -1954,6 +2116,127 @@ int gkd_pair(gkd_ctx *c, uint32_t a, uint32_t b, uint64_t *inter, uint64_t *uni,
         *uni = sa + sb - I;
     }
     return GKD_OK;
+}
+
+// ---- selections ---------------------------------------------------------------------------------------------
+// The arguments are checked before the context is touched, so a bad k or a NaN threshold is GKD_EINVAL even
+// without a usable device.
+static int hits_host_ok(gkd_ctx *c, const void *const *ps, int n) {
+    // literal side lists are completed and selected on the host, so the outputs must be host memory in that mode
+    if (c->cfg.ambig_policy != GKD_AMBIG_LITERAL) return GKD_OK;
+    for (int i = 0; i < n; i++)
+        if (ps[i] && classify(ps[i]) == MEM_DEVICE) return fail(c, GKD_EINVAL, "GKD_AMBIG_LITERAL needs host output buffers");
+    return GKD_OK;
+}
+
+// a query x reference selection, split by query rows like gkd_query_vs_ref_ex (every row is complete in one launch)
+static int rect_selection(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, const Selection &sel) {
+    const uint32_t rows_per = (uint32_t)std::max<uint64_t>(1, PAIR_CHUNK / nr);
+    uint64_t pairs = 0, bytes = 0;
+    double ims = 0, ems = 0;
+    for (uint32_t q0 = 0; q0 < nq; q0 += rows_per) {
+        const uint32_t rows = std::min(rows_per, nq - q0);
+        HostPairs hp{PAIRS_RECT, nr, 0, (uint64_t)rows * nr, q + q0, r, rows, nr};
+        Selection s = sel;
+        s.a_base = q0;
+        const uint64_t at = (uint64_t)q0 * sel.k;
+        if (s.ref_pos) s.ref_pos += at;
+        if (s.inter) s.inter += at;
+        if (s.dist) s.dist += at;
+        if (s.n_found) s.n_found += q0;
+        const int rc = run_pairs(c, hp, gkd_outputs{}, &s);
+        if (rc) return rc;
+        pairs += c->m.pairs;
+        bytes += c->m.intersect_bytes;
+        ims += c->m.intersect_ms;
+        ems += c->m.epilogue_ms;
+    }
+    c->m.pairs = pairs;
+    c->m.intersect_bytes = bytes;
+    c->m.intersect_ms = ims;
+    c->m.epilogue_ms = ems;
+    return GKD_OK;
+}
+
+int gkd_all_vs_all_range_within(gkd_ctx *c, uint32_t n, uint64_t first, uint64_t count, double max_dist, gkd_hits *out) {
+    if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_range_within: null hits");
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_range_within: max_dist is NaN");
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "range over %u sets but only %zu exist", n, c->genomes.size());
+    uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
+    if (first > total || count > total - first) return fail(c, GKD_EINVAL, "pair range [%llu, +%llu) outside 0..%llu", (unsigned long long)first, (unsigned long long)count, (unsigned long long)total);
+    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
+    int rc = hits_host_ok(c, ps, 4);
+    if (rc) return rc;
+    out->n = 0;
+    ABI_GUARD_BEGIN
+    HostPairs hp{PAIRS_UPPER, n, first, count, nullptr, nullptr, 0, 0};
+    Selection sel{};
+    sel.within = true;
+    sel.max_dist = max_dist;
+    sel.hits = out;
+    return run_pairs(c, hp, gkd_outputs{}, &sel);
+    ABI_GUARD_END(c)
+}
+
+int gkd_query_vs_ref_within(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, double max_dist,
+                            gkd_hits *out) {
+    if (!out) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_within: null hits");
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_within: max_dist is NaN");
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_within: null id array");
+    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
+    int rc = hits_host_ok(c, ps, 4);
+    if (rc) return rc;
+    out->n = 0;
+    if (nq == 0 || nr == 0) {
+        c->m.pairs = 0;
+        return GKD_OK;
+    }
+    ABI_GUARD_BEGIN
+    Selection sel{};
+    sel.within = true;
+    sel.max_dist = max_dist;
+    sel.hits = out;
+    return rect_selection(c, q, nq, r, nr, sel);
+    ABI_GUARD_END(c)
+}
+
+int gkd_query_vs_ref_nearest(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
+                             double max_dist, int exclude_self, uint32_t *ref_pos, uint64_t *inter, double *dist,
+                             uint32_t *n_found) {
+    if (k < 1 || k > NEAREST_MAX_K) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_nearest: k = %u is outside 1..%u", k, NEAREST_MAX_K);
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_nearest: max_dist is NaN");
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_nearest: null id array");
+    const void *ps[4] = {ref_pos, inter, dist, n_found};
+    int rc = hits_host_ok(c, ps, 4);
+    if (rc) return rc;
+    c->m.pairs = 0;
+    if (nq == 0) return GKD_OK;
+    ABI_GUARD_BEGIN
+    if (nr == 0) {  // no reference: every row is empty
+        const uint64_t slots = (uint64_t)nq * k;
+        if (ref_pos) CK(cudaMemcpy(ref_pos, std::vector<uint32_t>(slots, 0xFFFFFFFFu).data(), slots * 4, cudaMemcpyDefault));
+        if (inter) CK(cudaMemcpy(inter, std::vector<uint64_t>(slots, 0).data(), slots * 8, cudaMemcpyDefault));
+        if (dist) CK(cudaMemcpy(dist, std::vector<double>(slots, -1.0).data(), slots * 8, cudaMemcpyDefault));
+        if (n_found) CK(cudaMemcpy(n_found, std::vector<uint32_t>(nq, 0).data(), (uint64_t)nq * 4, cudaMemcpyDefault));
+        return GKD_OK;
+    }
+    Selection sel{};
+    sel.within = false;
+    sel.max_dist = max_dist;
+    sel.k = k;
+    sel.exclude_self = exclude_self ? 1 : 0;
+    sel.ref_pos = ref_pos;
+    sel.inter = inter;
+    sel.dist = dist;
+    sel.n_found = n_found;
+    return rect_selection(c, q, nq, r, nr, sel);
+    ABI_GUARD_END(c)
 }
 
 // ---- MinHash sketches ---------------------------------------------------------------------------------------

@@ -137,19 +137,33 @@ inline uint64_t row_start(uint64_t i, uint64_t n) { return i * (2 * n - i - 1) /
         }                                                     \
     } while (0)
 
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist);
+// gkd_group_all_vs_all_within: a member's hits in global ids (a < b); no dense result exists on this path
+struct GroupHit {
+    uint32_t a, b;
+    uint64_t inter;
+    double dist;
+};
+struct WithinSink {
+    double max_dist;
+    std::vector<GroupHit> hits;
+};
+// first capacity a member offers a within call; a call with more hits is repeated with the exact total
+constexpr uint64_t WITHIN_FIRST_CAP = 4ull << 20;
 
-// the ring of one member (runs on its own host thread; no exception may leave the thread)
-void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist) {
+void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within);
+
+// the ring of one member (runs on its own host thread; no exception may leave the thread).  With `within` the
+// member selects on its device and collects its hits there instead of scattering dense blocks into inter / dist.
+void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within) {
     try {
-        member_ring(g, x, inter, dist);
+        member_ring(g, x, inter, dist, within);
     } catch (const std::exception &ex) {
         g->members[x].rc = GKD_ENOMEM;
         g->members[x].err = ex.what();
     }
 }
 
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist) {
+void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within) {
     Member &M = g->members[x];
     const uint32_t R = (uint32_t)g->members.size();
     const uint64_t N = g->n_genomes;
@@ -157,6 +171,23 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist) {
     MCK(cudaSetDevice(M.device));
     std::vector<uint64_t> bi;
     std::vector<double> bd;
+    std::vector<uint32_t> ha, hb;  // within: hit positions of one call
+    uint64_t nh = 0;
+    auto fetch = [&](uint64_t pairs, auto call) -> int {  // one within call, repeated once with cap = n if it was short
+        uint64_t cap = std::min(pairs, WITHIN_FIRST_CAP);
+        for (;;) {
+            ha.resize(cap);
+            hb.resize(cap);
+            bi.resize(cap);
+            bd.resize(cap);
+            gkd_hits h{ha.data(), hb.data(), bi.data(), bd.data(), cap, 0};
+            const int rc = call(h);
+            if (rc != GKD_OK) return rc;
+            nh = h.n;
+            if (h.n <= cap) return GKD_OK;
+            cap = h.n;
+        }
+    };
     auto put = [&](uint32_t ga, uint32_t gb, uint64_t I, double d) {
         if (ga > gb) std::swap(ga, gb);
         const uint64_t t = row_start(ga, N) + (gb - ga - 1);
@@ -226,7 +257,11 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist) {
     if (M.rc) return;
 
     // diagonal block (runs while the first group is in flight)
-    if (m >= 2) {
+    if (m >= 2 && within) {
+        const uint64_t cnt = (uint64_t)m * (m - 1) / 2;
+        MGK(fetch(cnt, [&](gkd_hits &h) { return gkd_all_vs_all_range_within(M.ctx, m, 0, cnt, within->max_dist, &h); }));
+        for (uint64_t t = 0; t < nh; t++) within->hits.push_back({M.global_ids[ha[t]], M.global_ids[hb[t]], bi[t], bd[t]});
+    } else if (m >= 2) {
         const uint64_t cnt = (uint64_t)m * (m - 1) / 2;
         bi.resize(cnt);
         bd.resize(cnt);
@@ -235,7 +270,7 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist) {
         for (uint32_t i = 0; i < m; i++)
             for (uint32_t j = i + 1; j < m; j++, t++) put(M.global_ids[i], M.global_ids[j], bi[t], bd[t]);
     }
-    std::vector<uint32_t> rows, cols;
+    std::vector<uint32_t> rows, cols, col_gid;  // col_gid: global id of every column of the call
     for (size_t gi = 0; gi < groups.size(); gi++) {
         if (gi + 1 < groups.size()) {
             // buffer (gi+1)&1 was last used by group gi-1, whose sets were dropped (and the stream drained) below
@@ -248,12 +283,28 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist) {
         const Slot &S0 = slots[G.s0];
         rows.clear();
         cols.clear();
+        col_gid.clear();
         for (uint32_t r = S0.row0; r < S0.row1; r++) rows.push_back(r);
         for (size_t k = G.s0; k < G.s1; k++) {
             const Slot &S = slots[k];
             uint32_t first = 0;
             MGK(gkd_adopt_sets(M.ctx, (char *)M.recv[b] + G.off[k - G.s0], S.p.end - S.p.begin, S.p.table.data(), S.p.count, &first));
-            for (uint32_t c = 0; c < S.p.count; c++) cols.push_back(first + c);
+            for (uint32_t c = 0; c < S.p.count; c++) {
+                cols.push_back(first + c);
+                col_gid.push_back(g->members[S.src].global_ids[S.p.first + c]);
+            }
+        }
+        if (within) {
+            MGK(fetch((uint64_t)rows.size() * cols.size(), [&](gkd_hits &h) {
+                return gkd_query_vs_ref_within(M.ctx, rows.data(), (uint32_t)rows.size(), cols.data(), (uint32_t)cols.size(),
+                                               within->max_dist, &h);
+            }));
+            for (uint64_t t = 0; t < nh; t++) {
+                const uint32_t ga = M.global_ids[rows[ha[t]]], gb = col_gid[hb[t]];
+                within->hits.push_back({std::min(ga, gb), std::max(ga, gb), bi[t], bd[t]});
+            }
+            MGK(gkd_truncate(M.ctx, m));
+            continue;
         }
         bi.resize((size_t)rows.size() * cols.size());
         bd.resize(bi.size());
@@ -465,7 +516,7 @@ int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist) {
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, inter, dist);
+            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -473,6 +524,44 @@ int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist) {
         return GKD_OK;
     } catch (const std::exception &ex) {
         return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all: %s", ex.what());
+    }
+}
+
+int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
+    if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_within: null hits");
+    if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_within: max_dist is NaN");
+    if (!g) return GKD_EINVAL;
+    try {
+        for (auto &M : g->members)
+            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
+        out->n = 0;
+        std::vector<WithinSink> sinks(g->members.size(), WithinSink{max_dist, {}});
+        std::vector<std::thread> threads;
+        for (uint32_t x = 0; x < g->members.size(); x++) {
+            g->members[x].rc = GKD_OK;
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x]);
+        }
+        for (auto &t : threads) t.join();
+        for (size_t i = 0; i < g->members.size(); i++)
+            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        // the members own disjoint pairs: one sort by (a, b) gives the order of one context's row-major triangle
+        std::vector<GroupHit> all;
+        for (auto &s : sinks) {
+            all.insert(all.end(), s.hits.begin(), s.hits.end());
+            std::vector<GroupHit>().swap(s.hits);
+        }
+        std::sort(all.begin(), all.end(), [](const GroupHit &p, const GroupHit &q) { return p.a < q.a || (p.a == q.a && p.b < q.b); });
+        out->n = all.size();
+        const uint64_t w = std::min<uint64_t>(all.size(), out->cap);
+        for (uint64_t t = 0; t < w; t++) {
+            if (out->a) out->a[t] = all[t].a;
+            if (out->b) out->b[t] = all[t].b;
+            if (out->inter) out->inter[t] = all[t].inter;
+            if (out->dist) out->dist[t] = all[t].dist;
+        }
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_within: %s", ex.what());
     }
 }
 

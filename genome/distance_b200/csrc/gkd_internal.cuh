@@ -283,6 +283,28 @@ struct EpilogueOut {
 };
 cudaError_t launch_epilogue(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
                             int both_strands, EpilogueOut out, cudaStream_t s);
+// kernel 5, selection forms (replace launch_epilogue for the within / nearest calls)
+struct HitsOut {         // any member may be nullptr
+    uint32_t *a, *b;     // UPPER / LIST: set ids; RECT: a_base + query row, reference position
+    uint64_t *inter;
+    double *dist;
+};
+constexpr uint32_t NEAREST_MAX_K = 256;
+struct NearestOut {      // rows * k row-major, n_found per row; any member may be nullptr
+    uint32_t *ref_pos;
+    uint64_t *inter;
+    double *dist;
+    uint32_t *n_found;
+};
+uint64_t select_within_ctas(uint64_t count);  // entries of the `cta` scratch array of launch_select_within
+// pairs with dist <= max_dist compacted in enumeration order into out[0 .. min(hits, cap)); *total = hits of the launch
+cudaError_t launch_select_within(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
+                                 int both_strands, double max_dist, uint32_t a_base, uint64_t cap, HitsOut out,
+                                 unsigned long long *cta, unsigned long long *total, cudaStream_t s);
+// PAIRS_RECT only: per query row the <= k (<= NEAREST_MAX_K) nearest references within max_dist, ties by position
+cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t rows, const uint32_t *counts,
+                                  const uint32_t *pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
+                                  NearestOut out, cudaStream_t s);
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless
 // some representative is within max_dist; clears the counts it consumed
 cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *n_reps, uint32_t cand, uint32_t visit,

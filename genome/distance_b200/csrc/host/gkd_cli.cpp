@@ -20,6 +20,7 @@
 #include <fstream>
 #include <iostream>
 #include <map>
+#include <memory>
 #include <set>
 #include <sstream>
 
@@ -133,34 +134,49 @@ const std::vector<OptSpec> FASTA_OPTS = {
     {{"--gpus"}, true, "number of GPUs to shard the pair matrix over (additive option; default 1; needs --input)"},
     {{"--devices"}, true, "explicit comma-separated device ordinals for the group, e.g. 0,1,2,3 (an ordinal may repeat)"},
     {{"--metrics"}, true, "write one JSON line of engine metrics to this file (additive option)"},
+    {{"--maxDist"}, true, "report only the pairs with distance <= this (additive option; selected on the GPU)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
+
+// one report line of fastaDist (:188-192)
+template <class LabelFn, class CommentFn>
+void writePairLine(std::ostream &writer, std::string &line, size_t i, size_t j, double dist, LabelFn label, CommentFn comment) {
+    line.clear();
+    line += label(i);
+    line += '\t';
+    line += comment(i);
+    line += '\t';
+    line += label(j);
+    line += '\t';
+    line += comment(j);
+    line += '\t';
+    line += javaDouble(dist);
+    line += '\n';
+    writer << line;
+}
 
 // the report lines of fastaDist (:188-192), in list order
 template <class LabelFn, class CommentFn>
 size_t writePairs(std::ostream &writer, size_t n, const std::vector<double> &dist, LabelFn label, CommentFn comment) {
     size_t t = 0;
     std::string line;
-    for (size_t i = 0; i < n; i++) {
-        for (size_t j = i + 1; j < n; j++, t++) {
-            line.clear();
-            line += label(i);
-            line += '\t';
-            line += comment(i);
-            line += '\t';
-            line += label(j);
-            line += '\t';
-            line += comment(j);
-            line += '\t';
-            line += javaDouble(dist[t]);
-            line += '\n';
-            writer << line;
-        }
-    }
+    for (size_t i = 0; i < n; i++)
+        for (size_t j = i + 1; j < n; j++, t++) writePairLine(writer, line, i, j, dist[t], label, comment);
     writer.flush();
     return t;
 }
+
+// the lines of the full report whose distance is <= maxDist, in the same order: hits of gkd_*_within (a < b)
+template <class LabelFn, class CommentFn>
+void writeHits(std::ostream &writer, const uint32_t *a, const uint32_t *b, const double *dist, uint64_t n, LabelFn label,
+               CommentFn comment) {
+    std::string line;
+    for (uint64_t t = 0; t < n; t++) writePairLine(writer, line, a[t], b[t], dist[t], label, comment);
+}
+
+// pairs per gkd_all_vs_all_range_within call of `fastaDist --maxDist`: host memory stays O(range), not O(n^2)
+constexpr uint64_t WITHIN_RANGE = 64ull << 20;
 
 void writeMetrics(const std::string &path, const std::string &command, gkd_ctx *ctx, size_t pairs, int gpus) {
     if (path.empty()) return;
@@ -197,6 +213,9 @@ int fastaDist(const std::vector<std::string> &args) {
     if (kmerSize == 0) kmerSize = kmerTypeDefaultK(seqType);
     if (kmerSize < 2) throw ParseFailureException("Kmer size must be at least 2.");
     if (batchSize < 1) throw ParseFailureException("Batch size must be at least 1.");
+    const bool within = p.values.count("--maxDist") > 0;
+    const double maxDist = within ? toDouble("--maxDist", p.values["--maxDist"]) : 1.0;
+    if (!(maxDist > 0.0 && maxDist <= 1.0)) throw ParseFailureException("Maximum distance must be > 0 and <= 1.");
     const char *typeName = seqType == KmerType::DNA ? "DNA" : (seqType == KmerType::RNA ? "RNA" : "PROT");
     if (inFile.empty()) logInfo(std::string("Reading ") + typeName + " sequences from the standard input.");
     else if (!readable(inFile)) throw IOException("Input file " + inFile + " is not found or unreadable.");
@@ -250,6 +269,30 @@ int fastaDist(const std::vector<std::string> &args) {
         writer << "seq1\tname1\tseq2\tname2\tdistance\n";
         gcheck(gkd_group_build(grp));
         logInfo(std::to_string(n) + " sequences cached on " + std::to_string(gpus) + " GPUs. Computing distances.");
+        const uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
+        if (within) {
+            // every member selects on its device; one call, repeated with the exact capacity if the first was short
+            uint64_t cap = std::min<uint64_t>(total, WITHIN_RANGE);
+            std::vector<uint32_t> a, b;
+            std::vector<double> d;
+            gkd_hits h{};
+            for (;;) {
+                a.resize(cap);
+                b.resize(cap);
+                d.resize(cap);
+                h = gkd_hits{a.data(), b.data(), nullptr, d.data(), cap, 0};
+                gcheck(gkd_group_all_vs_all_within(grp, maxDist, &h));
+                if (h.n <= cap) break;
+                cap = h.n;
+            }
+            writeHits(writer, a.data(), b.data(), d.data(), h.n, [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
+                      [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
+            writer.flush();
+            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(h.n) + " within distance " +
+                    javaDouble(maxDist) + ".");
+            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
+            return 0;
+        }
         std::vector<double> dist((size_t)n * (n > 0 ? n - 1 : 0) / 2);
         gcheck(gkd_group_all_vs_all(grp, nullptr, dist.data()));
         size_t t = writePairs(writer, n, dist, [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
@@ -266,6 +309,26 @@ int fastaDist(const std::vector<std::string> &args) {
     writer << "seq1\tname1\tseq2\tname2\tdistance\n";
     engine.build();
     logInfo(std::to_string(seqs.size()) + " sequences cached. Computing distances.");
+    if (within) {
+        // the triangle in ranges of <= WITHIN_RANGE pairs; only the pairs within maxDist leave the GPU
+        const uint64_t n = seqs.size(), total = n < 2 ? 0 : n * (n - 1) / 2, room = std::min(total, WITHIN_RANGE);
+        std::unique_ptr<uint32_t[]> a(new uint32_t[room + 1]), b(new uint32_t[room + 1]);
+        std::unique_ptr<double[]> d(new double[room + 1]);
+        uint64_t hits = 0;
+        for (uint64_t first = 0; first < total; first += WITHIN_RANGE) {
+            const uint64_t cnt = std::min(WITHIN_RANGE, total - first);
+            gkd_hits h{a.get(), b.get(), nullptr, d.get(), cnt, 0};
+            engine.check(gkd_all_vs_all_range_within(engine.raw(), (uint32_t)n, first, cnt, maxDist, &h));
+            writeHits(writer, a.get(), b.get(), d.get(), h.n, [&](size_t i) { return seqs[i].getGenomeId(); },
+                      [&](size_t i) { return seqs[i].getGenomeName(); });
+            hits += h.n;
+        }
+        writer.flush();
+        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(hits) + " within distance " +
+                javaDouble(maxDist) + ".");
+        writeMetrics(metricsFile, "fastaDist", engine.raw(), total, 1);
+        return 0;
+    }
     std::vector<double> dist;
     engine.allVsAll(nullptr, dist);
     size_t t = writePairs(writer, seqs.size(), dist, [&](size_t i) { return seqs[i].getGenomeId(); },
@@ -569,6 +632,7 @@ const std::vector<OptSpec> GENOME_OPTS = {
     {{"--type", "-t"}, true, "genome source type (DIR = directory of GTO files; FASTA = directory of FASTA files)"},
     {{"--output", "-o"}, true, "output file for report (if not STDOUT)"},
     {{"--device"}, true, "CUDA device ordinal (additive option; default 0)"},
+    {{"--nearest"}, true, "report only the N nearest base genomes of each genome within --maxDist (additive option; 1..256)"},
     {{"--help", "-h"}, false, "display usage information"},
     {{"--verbose", "-v"}, false, "show more detail on the log"},
 };
@@ -592,6 +656,9 @@ int genomes(const std::vector<std::string> &args) {
     if (kmerSize < 4) throw ParseFailureException("Kmer size cannot be less than 4.");
     logInfo("Chosen kmer size is " + std::to_string(kmerSize) + ".");
     if (maxDist <= 0.0 || maxDist > 1.0) throw ParseFailureException("Maximum distance must be > 0 and <= 1.");
+    const int nearest = p.values.count("--nearest") ? toInt("--nearest", p.values["--nearest"]) : 0;
+    if (p.values.count("--nearest") && (nearest < 1 || nearest > 256))
+        throw ParseFailureException("Number of neighbors must be between 1 and 256.");
     const std::string baseDir = p.positional[0];
     if (!exists(baseDir)) throw IOException("Main genome source \"" + baseDir + "\" is not found.");
     for (size_t i = 1; i < p.positional.size(); i++)
@@ -611,7 +678,8 @@ int genomes(const std::vector<std::string> &args) {
         for (auto &g : base) mainKmers.push_back(engine.genomeKmers(g.contigs, g.id, g.name));
     }
     // runReporter (:119-150): every genome of the other sources against all base genomes; the
-    // maxDist option is validated but, as in the reference, never applied to the output (:143-146)
+    // maxDist option is validated but, as in the reference, never applied to the output (:143-146) -- unless
+    // --nearest asks for each genome's N nearest base genomes within maxDist
     writer << "genome1\tgenome2\tdistance\n";
     std::vector<SequenceKmers> queries;
     for (size_t i = 1; i < p.positional.size(); i++) {
@@ -622,9 +690,24 @@ int genomes(const std::vector<std::string> &args) {
     std::vector<uint32_t> q, r;
     for (auto &s : queries) q.push_back(s.handle());
     for (auto &s : mainKmers) r.push_back(s.handle());
+    size_t compares = 0;
+    if (nearest) {
+        // selected on the GPU: ascending distance, ties in base load order; only the kept neighbours come back
+        const uint64_t k = (uint64_t)nearest;
+        std::vector<uint32_t> pos(q.size() * k), found(q.size());
+        std::vector<double> nd(q.size() * k);
+        engine.check(gkd_query_vs_ref_nearest(engine.raw(), q.data(), (uint32_t)q.size(), r.data(), (uint32_t)r.size(), (uint32_t)k,
+                                              maxDist, 0, pos.data(), nullptr, nd.data(), found.data()));
+        for (size_t qi = 0; qi < queries.size(); qi++)
+            for (uint32_t i = 0; i < found[qi]; i++, compares++)
+                writer << queries[qi].getGenomeId() << '\t' << mainKmers[pos[qi * k + i]].getGenomeId() << '\t'
+                       << javaDouble(nd[qi * k + i]) << '\n';
+        writer.flush();
+        logInfo(std::to_string(compares) + " comparisons output.");
+        return 0;
+    }
     std::vector<double> dist;
     engine.queryVsRef(q, r, dist);
-    size_t compares = 0;
     for (size_t qi = 0; qi < queries.size(); qi++)
         for (size_t ri = 0; ri < mainKmers.size(); ri++, compares++)
             writer << queries[qi].getGenomeId() << '\t' << mainKmers[ri].getGenomeId() << '\t'
@@ -724,21 +807,24 @@ int distReps(const std::vector<std::string> &args) {
             qIdx.push_back(i);
         }
     for (size_t x : reps) r.push_back(all[x].handle());
-    std::vector<double> block;
-    if (!q.empty()) engine.queryVsRef(q, r, block);
+    // the nearest representative of every genome is selected on the GPU (k = 1, ties by representative order); only
+    // one distance per genome comes back
+    std::vector<uint32_t> nearPos(q.size()), nearFound(q.size());
+    std::vector<double> nearDist(q.size());
+    if (!q.empty())
+        engine.check(gkd_query_vs_ref_nearest(engine.raw(), q.data(), (uint32_t)q.size(), r.data(), (uint32_t)r.size(), 1, 1.0, 0,
+                                              nearPos.data(), nullptr, nearDist.data(), nearFound.data()));
     std::vector<size_t> bestRep(all.size());
     std::vector<double> bestDist(all.size(), 0.0);
     for (size_t i = 0; i < all.size(); i++) bestRep[i] = i;
     for (size_t qi = 0; qi < qIdx.size(); qi++) {
-        // reduce(NULL_RESULT, merge): start from distance 1.0 and replace only on a strictly smaller distance
+        // reduce(NULL_RESULT, merge): start from distance 1.0 and replace only on a strictly smaller distance, so the
+        // result is the first representative at the smallest distance when that is below 1.0
         double best = 1.0;
         size_t arg = reps[0];  // only kept if no distance is below 1.0, which pass 1 rules out
-        for (size_t ri = 0; ri < reps.size(); ri++) {
-            const double d = block[qi * reps.size() + ri];
-            if (d < best) {
-                best = d;
-                arg = reps[ri];
-            }
+        if (nearFound[qi] && nearDist[qi] < best) {
+            best = nearDist[qi];
+            arg = reps[nearPos[qi]];
         }
         bestRep[qIdx[qi]] = arg;
         bestDist[qIdx[qi]] = best;

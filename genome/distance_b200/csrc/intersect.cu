@@ -518,6 +518,222 @@ __global__ void __launch_bounds__(256)
     if (out.contain_b) out.contain_b[t] = sb ? (double)I / (double)sb : 0.0;
 }
 
+// ---- kernel 5, selection forms: only the chosen pairs leave the device ------------------------------------------
+// Both compute every pair with decode_pair + pair_result, so a selected pair's inter and dist are the dense call's.
+//
+// Within: pairs with dist <= max_dist, compacted in enumeration order.  A CTA owns a tile of SEL_TILE consecutive
+// pairs; pass 1 counts its hits, one CTA scans the tile totals (exclusive offsets + the launch total), and pass 2
+// recomputes the tile and writes each hit at tile offset + ballot/popc rank.  No atomics, so the order and the
+// output are deterministic.  Hits at positions >= cap are counted but not written.
+constexpr int SEL_THREADS = 256, SEL_ITEMS = 8;
+constexpr uint64_t SEL_TILE = (uint64_t)SEL_THREADS * SEL_ITEMS;
+
+uint64_t select_within_ctas(uint64_t count) { return (count + SEL_TILE - 1) / SEL_TILE; }
+
+template <bool WRITE>
+__global__ void __launch_bounds__(SEL_THREADS)
+    k_select_within(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
+                    const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t a_base, uint64_t cap,
+                    HitsOut out, unsigned long long *__restrict__ cta) {
+    __shared__ uint32_t s_warp[SEL_THREADS / 32];
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint64_t tile0 = (uint64_t)blockIdx.x * SEL_TILE;
+    unsigned long long base = WRITE ? cta[blockIdx.x] : 0ull;
+    uint32_t mine = 0;
+    for (int it = 0; it < SEL_ITEMS; it++) {
+        const uint64_t t = tile0 + (uint64_t)it * SEL_THREADS + threadIdx.x;
+        bool hit = false;
+        uint32_t ida = 0, idb = 0;
+        uint64_t I = 0;
+        double d = 1.0;
+        if (t < src.count) {
+            decode_pair(src, t, ida, idb);
+            uint64_t sa, sb;
+            pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+            hit = d <= max_dist;
+        }
+        if (!WRITE) {
+            mine += hit ? 1u : 0u;
+            continue;
+        }
+        const uint32_t bal = __ballot_sync(0xffffffffu, hit);
+        if (lane == 0) s_warp[warp] = __popc(bal);
+        __syncthreads();
+        uint32_t before = 0, total = 0;
+#pragma unroll
+        for (int w = 0; w < SEL_THREADS / 32; w++) {
+            const uint32_t v = s_warp[w];
+            before += w < (int)warp ? v : 0u;
+            total += v;
+        }
+        __syncthreads();  // s_warp is rewritten by the next item
+        if (hit) {
+            const unsigned long long at = base + before + __popc(bal & ((1u << lane) - 1u));
+            if (at < cap) {
+                const bool rect = src.mode == PAIRS_RECT;
+                if (out.a) out.a[at] = rect ? a_base + (uint32_t)(t / src.n) : ida;
+                if (out.b) out.b[at] = rect ? (uint32_t)(t % src.n) : idb;
+                if (out.inter) out.inter[at] = I;
+                if (out.dist) out.dist[at] = d;
+            }
+        }
+        base += total;
+    }
+    if (!WRITE) {
+        mine = __reduce_add_sync(0xffffffffu, mine);
+        if (lane == 0) s_warp[warp] = mine;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            uint32_t sum = 0;
+            for (int w = 0; w < SEL_THREADS / 32; w++) sum += s_warp[w];
+            cta[blockIdx.x] = sum;
+        }
+    }
+}
+
+// tile hit counts -> exclusive offsets in place, and the launch total (one CTA; thread x owns a contiguous run of tiles)
+__global__ void __launch_bounds__(1024) k_select_scan(unsigned long long *__restrict__ cta, uint64_t n, unsigned long long *__restrict__ total) {
+    __shared__ unsigned long long s_w[32];
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint64_t per = (n + 1023) / 1024;
+    const uint64_t lo = min(n, (uint64_t)threadIdx.x * per), hi = min(n, lo + per);
+    unsigned long long sum = 0;
+    for (uint64_t i = lo; i < hi; i++) sum += cta[i];
+    unsigned long long x = sum;  // inclusive scan over the warp
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned long long y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= (uint32_t)o) x += y;
+    }
+    if (lane == 31) s_w[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+        unsigned long long v = s_w[lane];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long y = __shfl_up_sync(0xffffffffu, v, o);
+            if (lane >= (uint32_t)o) v += y;
+        }
+        s_w[lane] = v;
+    }
+    __syncthreads();
+    unsigned long long run = x - sum + (warp ? s_w[warp - 1] : 0ull);
+    for (uint64_t i = lo; i < hi; i++) {
+        const unsigned long long v = cta[i];
+        cta[i] = run;
+        run += v;
+    }
+    if (threadIdx.x == 1023) *total = run;
+}
+
+cudaError_t launch_select_within(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
+                                 int both_strands, double max_dist, uint32_t a_base, uint64_t cap, HitsOut out,
+                                 unsigned long long *cta, unsigned long long *total, cudaStream_t s) {
+    if (src.count == 0) return cudaMemsetAsync(total, 0, sizeof(unsigned long long), s);
+    const uint64_t blocks = select_within_ctas(src.count);
+    k_select_within<false><<<(unsigned)blocks, SEL_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, a_base,
+                                                                   cap, out, cta);
+    k_select_scan<<<1, 1024, 0, s>>>(cta, blocks, total);
+    if (cap)
+        k_select_within<true><<<(unsigned)blocks, SEL_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist,
+                                                                      a_base, cap, out, cta);
+    return cudaGetLastError();
+}
+
+// Nearest: one CTA per query row of a PAIRS_RECT launch.  Slots [0, 256) of shared memory hold the row's best list
+// (sorted by (distance bits, reference position); distances are non-negative, so their IEEE bits order like the
+// values), slots [256, 512) the candidates of one round of 256 references: a reference is a candidate when it is
+// within max_dist and beats the current k-th best.  A round with candidates ends with a bitonic sort of all 512
+// slots, after which slots >= k are cleared.  Nothing leaves the CTA until the row is done.
+constexpr int NEAR_THREADS = 256, NEAR_SLOTS = 512;
+constexpr unsigned long long NEAR_NONE = ~0ull;  // sorts after every distance
+
+__global__ void __launch_bounds__(NEAR_THREADS)
+    k_select_nearest(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
+                     const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
+                     NearestOut out) {
+    __shared__ unsigned long long s_key[NEAR_SLOTS];
+    __shared__ unsigned long long s_inter[NEAR_SLOTS];
+    __shared__ uint32_t s_pos[NEAR_SLOTS];
+    __shared__ uint32_t s_n;
+    const uint32_t tid = threadIdx.x, row = blockIdx.x, nr = src.n;
+    for (uint32_t i = tid; i < NEAR_SLOTS; i += NEAR_THREADS) {
+        s_key[i] = NEAR_NONE;
+        s_inter[i] = 0;
+        s_pos[i] = 0xFFFFFFFFu;
+    }
+    if (tid == 0) s_n = 0;
+    __syncthreads();
+    unsigned long long thr = NEAR_NONE;  // distance bits of the k-th best so far
+    for (uint32_t j0 = 0; j0 < nr; j0 += NEAR_THREADS) {
+        const uint32_t j = j0 + tid;
+        if (j < nr) {
+            const uint64_t t = (uint64_t)row * nr + j;
+            uint32_t ida, idb;
+            decode_pair(src, t, ida, idb);
+            if (!(exclude_self && ida == idb)) {
+                uint64_t I, sa, sb;
+                double d;
+                pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+                const unsigned long long key = (unsigned long long)__double_as_longlong(d);
+                // a later reference with the k-th best distance loses the tie: strictly smaller only
+                if (d <= max_dist && key < thr) {
+                    const uint32_t slot = NEAR_THREADS + atomicAdd(&s_n, 1u);
+                    s_key[slot] = key;
+                    s_inter[slot] = I;
+                    s_pos[slot] = j;
+                }
+            }
+        }
+        __syncthreads();
+        const uint32_t n_cand = s_n;
+        __syncthreads();  // everyone has read s_n before it is reset
+        if (n_cand == 0) continue;
+        for (uint32_t size = 2; size <= NEAR_SLOTS; size <<= 1) {
+            for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
+                const uint32_t i = (tid / stride) * 2u * stride + (tid % stride), l = i + stride;
+                const bool up = (i & size) == 0;
+                const unsigned long long ki = s_key[i], kl = s_key[l];
+                const uint32_t pi = s_pos[i], pl = s_pos[l];
+                const bool gt = ki > kl || (ki == kl && pi > pl);
+                if (gt == up) {
+                    s_key[i] = kl, s_key[l] = ki;
+                    s_pos[i] = pl, s_pos[l] = pi;
+                    const unsigned long long t2 = s_inter[i];
+                    s_inter[i] = s_inter[l], s_inter[l] = t2;
+                }
+                __syncthreads();
+            }
+        }
+        for (uint32_t i = k + tid; i < NEAR_SLOTS; i += NEAR_THREADS) {
+            s_key[i] = NEAR_NONE;
+            s_inter[i] = 0;
+            s_pos[i] = 0xFFFFFFFFu;
+        }
+        if (tid == 0) s_n = 0;
+        __syncthreads();
+        thr = s_key[k - 1];
+    }
+    // k <= NEAR_THREADS: thread i writes slot i
+    const bool valid = tid < k && s_pos[tid] != 0xFFFFFFFFu;
+    if (tid < k) {
+        const uint64_t o = (uint64_t)row * k + tid;
+        if (out.ref_pos) out.ref_pos[o] = s_pos[tid];
+        if (out.inter) out.inter[o] = valid ? s_inter[tid] : 0ull;
+        if (out.dist) out.dist[o] = valid ? __longlong_as_double((long long)s_key[tid]) : -1.0;
+    }
+    const int found = __syncthreads_count(valid);
+    if (tid == 0 && out.n_found) out.n_found[row] = (uint32_t)found;
+}
+
+cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t rows, const uint32_t *counts,
+                                  const uint32_t *pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
+                                  NearestOut out, cudaStream_t s) {
+    if (rows == 0) return cudaSuccess;
+    k_select_nearest<<<rows, NEAR_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, k, exclude_self, out);
+    return cudaGetLastError();
+}
+
 // Greedy representative pass (DistanceRepsProcessor.java:185-201, FastaDistanceRepsProcessor.java:124-146): the
 // candidate was intersected with every current representative (counts[t] for reps[t]); it joins the list unless
 // one of them is within max_dist.  The list and its length live on the device, so the host queues the launches

@@ -8,12 +8,32 @@ from typing import List, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import (AMBIG_LITERAL, AMBIG_SKIP, DNA, PROT, RNA, STRAND_BOTH, STRAND_CANONICAL, GkdConfig, GkdMetrics,
-                   GkdOutputs, GkdPackedSet)
+from ._lib import (AMBIG_LITERAL, AMBIG_SKIP, DNA, PROT, RNA, STRAND_BOTH, STRAND_CANONICAL, GkdConfig, GkdHits,
+                   GkdMetrics, GkdOutputs, GkdPackedSet)
 
 PACKED_DTYPE = np.dtype([("offs_off", "<u8"), ("lows_off", "<u8"), ("pal_offs_off", "<u8"), ("pal_lows_off", "<u8"),
                          ("n", "<u4"), ("n_pal", "<u4"), ("level", "<u4"), ("pal_level", "<u4")])
 assert PACKED_DTYPE.itemsize == C.sizeof(GkdPackedSet)
+
+
+# Selections (gkd_hits) are sized by count-then-fetch: the first call offers room for min(pairs, FIRST_HITS_CAP) hits;
+# when the call reports more (n > cap) it is made once more with cap = n.  A selection that keeps few pairs -- the
+# use it exists for -- costs one call and host memory for its hits only.
+FIRST_HITS_CAP = 1 << 20
+
+
+def _select(call, pairs: int):
+    """(a, b, inter, dist) numpy arrays of a gkd_hits call `call(hits)` (count-then-fetch, see FIRST_HITS_CAP)"""
+    cap = min(pairs, FIRST_HITS_CAP)
+    while True:
+        a, b = np.empty(cap, dtype=np.uint32), np.empty(cap, dtype=np.uint32)
+        inter, dist = np.empty(cap, dtype=np.uint64), np.empty(cap, dtype=np.float64)
+        h = GkdHits(a.ctypes.data, b.ctypes.data, inter.ctypes.data, dist.ctypes.data, cap, 0)
+        call(h)
+        if h.n <= cap:
+            n = h.n
+            return a[:n], b[:n], inter[:n], dist[:n]
+        cap = h.n
 
 
 class GkdError(RuntimeError):
@@ -252,6 +272,38 @@ class Engine:
         self._ck(self._L.gkd_query_vs_ref(self._h, qa.ctypes.data, qa.size, ra.ctypes.data, ra.size, pi, pd))
         return inter.reshape(qa.size, ra.size), dist.reshape(qa.size, ra.size)
 
+    # -- selections: only the chosen pairs leave the device ----------------------------------------------------------
+    def all_vs_all_range_within(self, n: int, first: int, count: int, max_dist: float):
+        """(a, b, inter, dist) of the pairs [first, first+count) of the triangle over the first n sets whose distance is
+        <= max_dist, in enumeration order (a < b are set ids); each entry equals the dense call's"""
+        return _select(lambda h: self._ck(self._L.gkd_all_vs_all_range_within(self._h, n, first, count, float(max_dist),
+                                                                               C.byref(h))), count)
+
+    def all_vs_all_within(self, max_dist: float):
+        n = len(self)
+        return self.all_vs_all_range_within(n, 0, n * (n - 1) // 2, max_dist)
+
+    def query_vs_ref_within(self, q: Sequence[int], r: Sequence[int], max_dist: float):
+        """(a, b, inter, dist) of the query x reference pairs within max_dist in row-major order; a and b are positions
+        in q and r"""
+        qa, ra = np.ascontiguousarray(q, dtype=np.uint32), np.ascontiguousarray(r, dtype=np.uint32)
+        return _select(lambda h: self._ck(self._L.gkd_query_vs_ref_within(self._h, qa.ctypes.data, qa.size, ra.ctypes.data,
+                                                                           ra.size, float(max_dist), C.byref(h))),
+                       qa.size * ra.size)
+
+    def query_vs_ref_nearest(self, q: Sequence[int], r: Sequence[int], k: int, max_dist: float, exclude_self: bool = False):
+        """(ref_pos, inter, dist, n_found): every query's <= k nearest references within max_dist, as (len(q), k)
+        arrays in ascending distance, ties by position in r; unused slots hold ref_pos 2**32-1, inter 0, dist -1.0"""
+        qa, ra = np.ascontiguousarray(q, dtype=np.uint32), np.ascontiguousarray(r, dtype=np.uint32)
+        slots = qa.size * max(int(k), 0)
+        pos, inter = np.empty(slots, dtype=np.uint32), np.empty(slots, dtype=np.uint64)
+        dist, found = np.empty(slots, dtype=np.float64), np.empty(qa.size, dtype=np.uint32)
+        self._ck(self._L.gkd_query_vs_ref_nearest(self._h, qa.ctypes.data, qa.size, ra.ctypes.data, ra.size, int(k),
+                                                  float(max_dist), 1 if exclude_self else 0, pos.ctypes.data,
+                                                  inter.ctypes.data, dist.ctypes.data, found.ctypes.data))
+        shape = (qa.size, max(int(k), 0))
+        return pos.reshape(shape), inter.reshape(shape), dist.reshape(shape), found
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -415,3 +467,10 @@ class Group:
         inter, dist = np.empty(npairs, dtype=np.uint64), np.empty(npairs, dtype=np.float64)
         self._ck(self._L.gkd_group_all_vs_all(self._h, inter.ctypes.data, dist.ctypes.data))
         return inter, dist
+
+    def all_vs_all_within(self, max_dist: float):
+        """(a, b, inter, dist) of the pairs within max_dist over all global ids, ordered by (a, b): the single-context
+        Engine.all_vs_all_within result"""
+        n = len(self)
+        return _select(lambda h: self._ck(self._L.gkd_group_all_vs_all_within(self._h, float(max_dist), C.byref(h))),
+                       n * (n - 1) // 2)

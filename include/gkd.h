@@ -219,6 +219,36 @@ int gkd_greedy_reps(gkd_ctx *ctx, const uint32_t *order, uint32_t n, double max_
  * FastaDistanceRepsProcessor.java:128); uni = |A|+|B|-I */
 int gkd_pair(gkd_ctx *ctx, uint32_t a, uint32_t b, uint64_t *inter, uint64_t *uni, double *dist);
 
+/* ---- selections: only the chosen pairs leave the device (kernel 5 replaced by a selection epilogue) ----------
+ * Pairs whose distance is <= max_dist (the comparison gkd_greedy_reps uses), in the enumeration order of the call.
+ * Any array may be NULL; pointers may be host or device memory, like gkd_outputs (host memory only for a
+ * GKD_AMBIG_LITERAL context, whose pairs are completed and selected on the host). */
+typedef struct gkd_hits {
+    uint32_t *a;      /* all-vs-all: id i (i < j);  query_vs_ref: position of the query in q */
+    uint32_t *b;      /* all-vs-all: id j;          query_vs_ref: position of the reference in r */
+    uint64_t *inter;  /* similarity(), as gkd_all_vs_all */
+    double *dist;     /* bit-identical to the dense call's double for the same pair */
+    uint64_t cap;     /* entries each non-NULL array can hold */
+    uint64_t n;       /* out: number of qualifying pairs in the call; only the first min(n, cap) are written */
+} gkd_hits;
+/* The pairs of gkd_all_vs_all_range within max_dist: dereplication, clustering and relatives over one FASTA file
+ * (FastaDistanceProcessor.runReporter :141-194 followed by a distance filter; DistanceRepsProcessor.java:185-201 applies
+ * the same <= test one candidate at a time).  A cap smaller than the number of hits is not an error: n is the total,
+ * so a caller that got n > cap can call again with cap = n. */
+int gkd_all_vs_all_range_within(gkd_ctx *ctx, uint32_t n, uint64_t first, uint64_t count, double max_dist, gkd_hits *out);
+/* The pairs of gkd_query_vs_ref within max_dist (GenomeProcessor.runReporter :129-147 with its -m/--maxDist applied). */
+int gkd_query_vs_ref_within(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr,
+                            double max_dist, gkd_hits *out);
+/* For every query, its <= k nearest references with distance <= max_dist: ascending distance, ties broken by the
+ * smaller position in r (the left-biased merge of DistanceRepsProcessor :120-122).  Outputs are nq*k row-major;
+ * n_found[i] <= k; unused slots hold ref_pos = UINT32_MAX, inter = 0, dist = -1.0.  1 <= k <= 256.
+ * exclude_self != 0 skips pairs whose two ids are equal (q == r == all sets gives each set's neighbours).
+ * Pass 2 of DistanceRepsProcessor (:220-262, closest representative: k = 1, max_dist = 1.0) and classification
+ * against a reference panel.  Any output may be NULL; pointers may be host or device memory as for gkd_hits. */
+int gkd_query_vs_ref_nearest(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr,
+                             uint32_t k, double max_dist, int exclude_self,
+                             uint32_t *ref_pos, uint64_t *inter, double *dist, uint32_t *n_found);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -245,6 +275,9 @@ const char *gkd_group_comment(const gkd_group *g, uint32_t global_id);
 int gkd_group_build(gkd_group *g);  /* kernels 1-3 on every member concurrently */
 /* all pairs i < j over global ids, row-major strict upper triangle (either output may be NULL) */
 int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist);
+/* the group form of gkd_all_vs_all_range_within over all global ids: hits ordered by (a, b), equal to one context's.
+ * Every member selects on its own device; only the hits reach the host.  The arrays of out are host memory. */
+int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

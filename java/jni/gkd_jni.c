@@ -162,3 +162,58 @@ JNIEXPORT jint JNICALL FN(setSize)(JNIEnv *env, jclass c, jlong h, jint id, jlon
     (*env)->SetLongArrayRegion(env, out, 0, 1, &v);
     return GKD_OK;
 }
+
+/* fills a/b/dist (each at least `cap` long, cap = the shortest of the three) with the first hits of the pairs
+ * [first, first+count) within maxDist; returns the total number of hits (may exceed cap) or a negative status */
+JNIEXPORT jlong JNICALL FN(allVsAllRangeWithin)(JNIEnv *env, jclass c, jlong h, jint n, jlong first, jlong count, jdouble maxDist,
+                                               jintArray a, jintArray b, jdoubleArray dist) {
+    (void)c;
+    if (n < 0 || first < 0 || count < 0 || !a || !b || !dist) return GKD_EINVAL;
+    jlong cap = (*env)->GetArrayLength(env, a);
+    if ((jlong)(*env)->GetArrayLength(env, b) < cap) cap = (*env)->GetArrayLength(env, b);
+    if ((jlong)(*env)->GetArrayLength(env, dist) < cap) cap = (*env)->GetArrayLength(env, dist);
+    uint32_t *ha = (uint32_t *)malloc((size_t)cap * 4 + 4), *hb = (uint32_t *)malloc((size_t)cap * 4 + 4);
+    double *hd = (double *)malloc((size_t)cap * 8 + 8);
+    int rc = (ha && hb && hd) ? GKD_OK : GKD_ENOMEM;
+    gkd_hits hits = {ha, hb, NULL, hd, (uint64_t)cap, 0};
+    if (rc == GKD_OK) rc = gkd_all_vs_all_range_within(CTX(h), (uint32_t)n, (uint64_t)first, (uint64_t)count, maxDist, &hits);
+    if (rc == GKD_OK) {
+        /* the native call wrote min(n, cap) entries: exactly what the Java arrays receive */
+        const jsize w = (jsize)((jlong)hits.n < cap ? (jlong)hits.n : cap);
+        (*env)->SetIntArrayRegion(env, a, 0, w, (const jint *)ha);
+        (*env)->SetIntArrayRegion(env, b, 0, w, (const jint *)hb);
+        (*env)->SetDoubleArrayRegion(env, dist, 0, w, hd);
+    }
+    free(ha);
+    free(hb);
+    free(hd);
+    return rc == GKD_OK ? (jlong)hits.n : (jlong)rc;
+}
+
+/* every query's k nearest references within maxDist: refPos / dist hold q.length * k entries, nFound q.length */
+JNIEXPORT jint JNICALL FN(queryVsRefNearest)(JNIEnv *env, jclass c, jlong h, jintArray q, jintArray r, jint k, jdouble maxDist,
+                                             jboolean excludeSelf, jintArray refPos, jdoubleArray dist, jintArray nFound) {
+    (void)c;
+    if (!q || !r || !refPos || !dist || !nFound || k < 1) return GKD_EINVAL;
+    jsize nq = (*env)->GetArrayLength(env, q), nr = (*env)->GetArrayLength(env, r);
+    const jlong slots = (jlong)nq * (jlong)k;
+    if ((jlong)(*env)->GetArrayLength(env, refPos) < slots || (jlong)(*env)->GetArrayLength(env, dist) < slots ||
+        (*env)->GetArrayLength(env, nFound) < nq)
+        return GKD_EINVAL;
+    jint *qa = (*env)->GetIntArrayElements(env, q, NULL);
+    jint *ra = (*env)->GetIntArrayElements(env, r, NULL);
+    jint *pos = (*env)->GetIntArrayElements(env, refPos, NULL);
+    jint *found = (*env)->GetIntArrayElements(env, nFound, NULL);
+    jdouble *d = (*env)->GetDoubleArrayElements(env, dist, NULL);
+    int rc = (qa && ra && pos && found && d)
+                 ? gkd_query_vs_ref_nearest(CTX(h), (const uint32_t *)qa, (uint32_t)nq, (const uint32_t *)ra, (uint32_t)nr,
+                                            (uint32_t)k, maxDist, excludeSelf ? 1 : 0, (uint32_t *)pos, NULL, d,
+                                            (uint32_t *)found)
+                 : GKD_ENOMEM;
+    if (d) (*env)->ReleaseDoubleArrayElements(env, dist, d, 0);
+    if (found) (*env)->ReleaseIntArrayElements(env, nFound, found, 0);
+    if (pos) (*env)->ReleaseIntArrayElements(env, refPos, pos, 0);
+    if (ra) (*env)->ReleaseIntArrayElements(env, r, ra, JNI_ABORT);
+    if (qa) (*env)->ReleaseIntArrayElements(env, q, qa, JNI_ABORT);
+    return rc;
+}

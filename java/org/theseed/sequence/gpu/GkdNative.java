@@ -34,6 +34,15 @@ final class GkdNative {
     static native int allVsAllRange(long ctx, int n, long first, long count, double[] dist);
     /** fills dist (length q.length * r.length, row-major) */
     static native int queryVsRef(long ctx, int[] q, int[] r, double[] dist);
+    /** pairs [first, first+count) of the same enumeration whose distance is &lt;= maxDist, in order: the first
+     *  min(total, cap) go to a, b (set ids, a &lt; b) and dist, cap being the shortest of the three arrays; returns the
+     *  total number of such pairs (which may exceed cap) or a negative status */
+    static native long allVsAllRangeWithin(long ctx, int n, long first, long count, double maxDist, int[] a, int[] b,
+                                           double[] dist);
+    /** every query's &lt;= k nearest references within maxDist, ascending distance, ties by position in r: refPos and
+     *  dist (length q.length * k, row-major; unused slots -1 and -1.0), nFound (length q.length) */
+    static native int queryVsRefNearest(long ctx, int[] q, int[] r, int k, double maxDist, boolean excludeSelf,
+                                        int[] refPos, double[] dist, int[] nFound);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

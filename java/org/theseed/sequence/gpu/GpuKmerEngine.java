@@ -124,6 +124,56 @@ public class GpuKmerEngine implements AutoCloseable {
         return dist;
     }
 
+    /** pairs i &lt; j of the first n sets within maxDist, in list order: {a, b} ids and their distances.  The triangle
+     *  is read in ranges of at most rangePairs pairs; each range is selected on the GPU and only its hits come back. */
+    public synchronized Within allVsAllWithin(double maxDist, int rangePairs) {
+        this.build();
+        long n = this.size();
+        long pairs = n * (n - 1) / 2;
+        Within out = new Within();
+        int room = (int) Math.min(pairs, (long) rangePairs);
+        int[] a = new int[room], b = new int[room];
+        double[] dist = new double[room];
+        for (long first = 0; first < pairs; first += rangePairs) {
+            long count = Math.min((long) rangePairs, pairs - first);
+            long hits = GkdNative.allVsAllRangeWithin(this.ctx, (int) n, first, count, maxDist, a, b, dist);
+            if (hits < 0)
+                check((int) hits);
+            out.append(a, b, dist, (int) hits);  // hits <= count <= room: everything was written
+        }
+        return out;
+    }
+
+    /** the selected pairs of {@link #allVsAllWithin} */
+    public static final class Within {
+        public int[] a = new int[0], b = new int[0];
+        public double[] dist = new double[0];
+        public int size;
+
+        void append(int[] xa, int[] xb, double[] xd, int n) {
+            if (this.size + n > this.a.length) {
+                int cap = Math.max(this.size + n, 2 * this.a.length);
+                this.a = java.util.Arrays.copyOf(this.a, cap);
+                this.b = java.util.Arrays.copyOf(this.b, cap);
+                this.dist = java.util.Arrays.copyOf(this.dist, cap);
+            }
+            System.arraycopy(xa, 0, this.a, this.size, n);
+            System.arraycopy(xb, 0, this.b, this.size, n);
+            System.arraycopy(xd, 0, this.dist, this.size, n);
+            this.size += n;
+        }
+    }
+
+    /** every query's k nearest references within maxDist (ascending distance, ties by position in refs): refPos[i*k+j]
+     *  is a position in refs, -1 in unused slots; returns the number found per query.  dist receives q.length * k values. */
+    public synchronized int[] queryVsRefNearest(int[] queries, int[] refs, int k, double maxDist, boolean excludeSelf,
+                                                int[] refPos, double[] dist) {
+        this.build();
+        int[] found = new int[queries.length];
+        check(GkdNative.queryVsRefNearest(this.ctx, queries, refs, k, maxDist, excludeSelf, refPos, dist, found));
+        return found;
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
