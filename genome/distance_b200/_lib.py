@@ -37,6 +37,10 @@ class GkdHits(C.Structure):
                 ("n", C.c_uint64)]
 
 
+class GkdNeighbors(C.Structure):
+    _fields_ = [("pos", C.c_void_p), ("inter", C.c_void_p), ("dist", C.c_void_p), ("n_found", C.c_void_p)]
+
+
 class GkdMetrics(C.Structure):
     _fields_ = [("pack_ms", C.c_double), ("encode_ms", C.c_double), ("sort_ms", C.c_double), ("unique_ms", C.c_double),
                 ("intersect_ms", C.c_double), ("epilogue_ms", C.c_double), ("h2d_ms", C.c_double), ("d2h_ms", C.c_double),
@@ -77,6 +81,7 @@ SYMBOLS = {
     "gkd_group_build": (_i32, [_vp]),
     "gkd_group_all_vs_all": (_i32, [_vp, _vp, _vp]),
     "gkd_group_all_vs_all_within": (_i32, [_vp, _dbl, C.POINTER(GkdHits)]),
+    "gkd_group_all_vs_all_nearest": (_i32, [_vp, _u32, _dbl, C.POINTER(GkdNeighbors)]),
     "gkd_build_sets": (_i32, [_vp]),
     "gkd_set_size": (_i32, [_vp, _u32, _pu64, _pu64, _pu64]),
     "gkd_export_set": (_i32, [_vp, _u32, _vp, _u64, _pu64]),
@@ -100,6 +105,9 @@ SYMBOLS = {
     "gkd_all_vs_all_range_within": (_i32, [_vp, _u32, _u64, _u64, _dbl, C.POINTER(GkdHits)]),
     "gkd_query_vs_ref_within": (_i32, [_vp, _vp, _u32, _vp, _u32, _dbl, C.POINTER(GkdHits)]),
     "gkd_query_vs_ref_nearest": (_i32, [_vp, _vp, _u32, _vp, _u32, _u32, _dbl, _i32, _vp, _vp, _vp, _vp]),
+    "gkd_query_vs_ref_nearest_ex": (_i32, [_vp, _vp, _u32, _vp, _u32, _u32, _dbl, _i32, C.POINTER(GkdNeighbors),
+                                           C.POINTER(GkdNeighbors)]),
+    "gkd_all_vs_all_nearest": (_i32, [_vp, _u32, _u32, _dbl, C.POINTER(GkdNeighbors)]),
     "gkd_hash_set": (_i32, [_vp, _u32, _u32, _i32, _vp, _pu32]),
     "gkd_sketch_distances": (_i32, [_vp, _u32, _i32, _vp, _vp, _u64, _vp]),
     "gkd_format_double": (_i32, [_dbl, C.c_char_p, C.c_size_t]),

@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
 #include <unordered_map>
@@ -126,6 +127,7 @@ struct gkd_ctx {
     DevBuf gr_reps, gr_flags;
     DevBuf join_rows, join_err;
     DevBuf hit_a, hit_b, sel_cta;  // selection epilogues: hit ids / positions (nearest: ref_pos, n_found), tile offsets + total
+    DevBuf nn_pos, nn_inter, nn_dist, nn_found;  // accumulating nearest selection: per-target lists of one call
     int isect_algo = 0;  // GKD_ISECT_ALGO: 0 = choose per call, 1 = bucket merge only, 2 = block join whenever it applies
     bool use_msd = true;  // GKD_SORT_ALGO=lsd pins the LSD path
     bool sets_dirty = true;
@@ -952,18 +954,56 @@ bool plan_join(gkd_ctx *c, const HostPairs &hp, uint64_t first, uint64_t count, 
     return true;
 }
 
+// GKD_AMBIG_LITERAL: the per-target lists of an accumulating nearest selection, kept on the host because the pairs
+// are completed there.  Same layout and unused entry as the device lists (c->nn_*); n[t] entries of target t are used.
+struct HostLists {
+    uint32_t k = 0;
+    std::vector<uint32_t> pos, n;
+    std::vector<uint64_t> inter;
+    std::vector<double> dist;
+    HostLists(uint32_t targets, uint32_t k_) : k(k_), pos((uint64_t)targets * k_, 0xFFFFFFFFu), n(targets, 0),
+                                               inter((uint64_t)targets * k_, 0), dist((uint64_t)targets * k_, -1.0) {}
+    // the admission rule of k_nearest_absorb: below the k-th entry in (distance bits, position)
+    void offer(uint32_t tg, uint32_t nb, uint64_t I, double d) {
+        const uint64_t base = (uint64_t)tg * k;
+        uint64_t key;
+        std::memcpy(&key, &d, 8);
+        auto below = [&](uint64_t s) {
+            uint64_t ks;
+            std::memcpy(&ks, &dist[s], 8);
+            return key < ks || (key == ks && nb < pos[s]);
+        };
+        uint32_t &m = n[tg];
+        if (m == k && !below(base + k - 1)) return;
+        uint32_t at = m == k ? k - 1 : m;
+        for (; at > 0 && below(base + at - 1); at--) {
+            pos[base + at] = pos[base + at - 1];
+            inter[base + at] = inter[base + at - 1];
+            dist[base + at] = dist[base + at - 1];
+        }
+        pos[base + at] = nb;
+        inter[base + at] = I;
+        dist[base + at] = d;
+        if (m < k) m++;
+    }
+};
+
 // What a selection call wants instead of the dense outputs (run_pairs with sel == nullptr writes gkd_outputs).
 struct Selection {
-    bool within;          // true: pairs with dist <= max_dist (gkd_hits); false: k nearest per query row (RECT only)
+    bool within;          // true: pairs with dist <= max_dist (gkd_hits); false: k nearest (rows and / or absorb)
     double max_dist;
     gkd_hits *hits;       // within: the caller's arrays; hits->n counts the hits so far and is the next write position
-    uint32_t a_base;      // within, RECT: position in the caller's q of the first query row of this call
+    uint32_t a_base;      // RECT: position in the caller's q of the first query row of this call
     uint32_t k;           // nearest
     int exclude_self;
-    uint32_t *ref_pos;    // nearest: outputs of this call's first row (host or device memory)
+    bool rows;            // nearest, RECT: each query row's list, complete in this call (k_select_nearest) ...
+    uint32_t *ref_pos;    // ... written to these outputs of the call's first row (host or device memory)
     uint64_t *inter;
     double *dist;
     uint32_t *n_found;
+    bool absorb;          // nearest: merge the call into the per-target lists c->nn_* (UPPER: both ends of every pair;
+                          // RECT: each reference's nearest queries), or into host_lists when the pairs are completed
+    HostLists *host_lists;  // on the host (GKD_AMBIG_LITERAL; nullptr otherwise)
 };
 
 // GKD_AMBIG_LITERAL: the chunk's pairs were completed on the host (inter / dist of pairs done .. done+cnt), so the
@@ -985,6 +1025,21 @@ void host_select(const HostPairs &hp, const Selection &sel, uint64_t done, uint6
         }
         return;
     }
+    if (sel.absorb) {
+        for (uint64_t t = 0; t < cnt; t++) {
+            if (!(dist[t] <= sel.max_dist)) continue;
+            if (hp.mode == PAIRS_RECT) {
+                const uint32_t row = (uint32_t)((done + t) / hp.nb), j = (uint32_t)((done + t) % hp.nb);
+                if (!(sel.exclude_self && hp.a[row] == hp.b[j])) sel.host_lists->offer(j, sel.a_base + row, inter[t], dist[t]);
+            } else {
+                uint32_t a, b;
+                host_pair_ids(hp, done + t, a, b);
+                sel.host_lists->offer(a, b, inter[t], dist[t]);
+                sel.host_lists->offer(b, a, inter[t], dist[t]);
+            }
+        }
+    }
+    if (!sel.rows) return;
     std::vector<uint32_t> js;
     for (uint32_t row = 0; row < hp.na; row++) {
         const uint64_t r0 = (uint64_t)row * hp.nb;
@@ -1008,11 +1063,12 @@ void host_select(const HostPairs &hp, const Selection &sel, uint64_t done, uint6
 constexpr int SELECT_REDO = 1;  // select_chunk: a join table overflowed; nothing of the attempt was kept
 
 // The selection epilogue of one chunk whose kernel-4 launches are queued: launches the within or nearest selection,
-// then copies back only the hits (within: plus the chunk's 8-byte hit total) or the rows' best lists (nearest).
+// then copies back only the hits (within: plus the chunk's 8-byte hit total) or the rows' best lists (nearest).  The
+// absorb form merges the chunk into the device lists instead, which are copied once by the caller (lists_finish).
 // The hit total and the join overflow flag are read before anything is copied, so a chunk that has to be redone by
 // the merge kernel appends nothing.
 int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const Selection &sel, uint64_t cnt, bool need_pal,
-                 bool both, const uint32_t &join_err) {
+                 bool both, const uint32_t &join_err, bool use_join) {
     const SetDesc *sets = (const SetDesc *)c->d_sets.p;
     const uint32_t *counts = (const uint32_t *)c->counts.p, *pal = need_pal ? (const uint32_t *)c->pal_counts.p : nullptr;
     int rc;
@@ -1037,7 +1093,7 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         c->m.launches += wcap ? 3 : 2;
         CK(cudaEventRecord(c->ev[7], c->stream));
         CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
-    } else {
+    } else if (sel.rows) {
         const uint64_t slots = (uint64_t)hp.na * sel.k;
         if (sel.ref_pos && (rc = ensure(c, c->hit_a, slots * 4))) return rc;
         if (sel.n_found && (rc = ensure(c, c->hit_b, (uint64_t)hp.na * 4))) return rc;
@@ -1049,15 +1105,24 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         CK(launch_select_nearest(sets, src, hp.na, counts, pal, both ? 1 : 0, sel.max_dist, sel.k, sel.exclude_self, no, c->stream));
         nvtxRangePop();
         c->m.launches++;
-        CK(cudaEventRecord(c->ev[7], c->stream));
     }
+    if (sel.absorb) {
+        // the lists outlive this chunk: the kernel itself skips a chunk whose join overflowed
+        const NearestOut st{(uint32_t *)c->nn_pos.p, (uint64_t *)c->nn_inter.p, (double *)c->nn_dist.p, (uint32_t *)c->nn_found.p};
+        nvtxRangePushA("gkd kernel 5: nearest absorb");
+        CK(launch_nearest_absorb(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.k, sel.exclude_self, sel.a_base,
+                                 use_join ? (const uint32_t *)c->join_err.p : nullptr, st, c->stream));
+        nvtxRangePop();
+        c->m.launches++;
+    }
+    if (!sel.within) CK(cudaEventRecord(c->ev[7], c->stream));
     CK(cudaStreamSynchronize(c->stream));
     if (join_err) return SELECT_REDO;
     struct {
         void *dst;
         const void *src;
         uint64_t bytes;
-    } copies[4];
+    } copies[4] = {};  // absorb only: nothing leaves the device before the end of the call
     if (sel.within) {
         const gkd_hits &h = *sel.hits;
         const uint64_t w = std::min<uint64_t>(chunk_hits, wcap);
@@ -1065,7 +1130,7 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         copies[1] = {h.b ? h.b + h.n : nullptr, c->hit_b.p, w * 4};
         copies[2] = {h.inter ? h.inter + h.n : nullptr, c->d_inter.p, w * 8};
         copies[3] = {h.dist ? h.dist + h.n : nullptr, c->d_dist.p, w * 8};
-    } else {
+    } else if (sel.rows) {
         const uint64_t slots = (uint64_t)hp.na * sel.k;
         copies[0] = {sel.ref_pos, c->hit_a.p, slots * 4};
         copies[1] = {sel.inter, c->d_inter.p, slots * 8};
@@ -1282,7 +1347,7 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out, const Sel
         }
         CK(cudaEventRecord(c->ev[6], c->stream));
         if (dev_sel) {
-            rc = select_chunk(c, hp, src, *sel, cnt, need_pal, both, join_err);
+            rc = select_chunk(c, hp, src, *sel, cnt, need_pal, both, join_err, use_join);
             if (rc == SELECT_REDO) {
                 join_banned = true;
                 continue;
@@ -1536,7 +1601,8 @@ int gkd_destroy(gkd_ctx *c) {
                       &c->set_build, &c->d_sets, &c->counts, &c->pal_counts, &c->d_inter, &c->d_dist, &c->d_ca,
                       &c->d_cb, &c->ids_a, &c->ids_b, &c->work_counter, &c->sk_cand, &c->sk_misc, &c->sk_sig,
                       &c->sk_len, &c->sk_out, &c->msd_genomes, &c->msd_bins32, &c->msd_bins64, &c->msd_gstat,
-                      &c->gr_reps, &c->gr_flags, &c->join_rows, &c->join_err, &c->hit_a, &c->hit_b, &c->sel_cta};
+                      &c->gr_reps, &c->gr_flags, &c->join_rows, &c->join_err, &c->hit_a, &c->hit_b, &c->sel_cta, &c->nn_pos, &c->nn_inter,
+                      &c->nn_dist, &c->nn_found};
     for (DevBuf *b : bufs)
         if (b->p) cudaFreeAsync(b->p, c->stream);
     cudaStreamSynchronize(c->stream);
@@ -2204,38 +2270,152 @@ int gkd_query_vs_ref_within(gkd_ctx *c, const uint32_t *q, uint32_t nq, const ui
     ABI_GUARD_END(c)
 }
 
-int gkd_query_vs_ref_nearest(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
-                             double max_dist, int exclude_self, uint32_t *ref_pos, uint64_t *inter, double *dist,
-                             uint32_t *n_found) {
-    if (k < 1 || k > NEAREST_MAX_K) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_nearest: k = %u is outside 1..%u", k, NEAREST_MAX_K);
-    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_nearest: max_dist is NaN");
+// rows * k unused entries (and n_found 0) in every member of out
+static int fill_none(gkd_ctx *c, uint32_t rows, uint32_t k, const gkd_neighbors *out) {
+    if (!out || rows == 0) return GKD_OK;
+    const uint64_t slots = (uint64_t)rows * k;
+    if (out->pos) CK(cudaMemcpy(out->pos, std::vector<uint32_t>(slots, 0xFFFFFFFFu).data(), slots * 4, cudaMemcpyDefault));
+    if (out->inter) CK(cudaMemcpy(out->inter, std::vector<uint64_t>(slots, 0).data(), slots * 8, cudaMemcpyDefault));
+    if (out->dist) CK(cudaMemcpy(out->dist, std::vector<double>(slots, -1.0).data(), slots * 8, cudaMemcpyDefault));
+    if (out->n_found) CK(cudaMemcpy(out->n_found, std::vector<uint32_t>(rows, 0).data(), (uint64_t)rows * 4, cudaMemcpyDefault));
+    return GKD_OK;
+}
+
+// the per-target lists of an accumulating nearest call (k_nearest_absorb), all unused
+static int lists_begin(gkd_ctx *c, uint32_t targets, uint32_t k) {
+    const uint64_t slots = (uint64_t)targets * k;
+    int rc;
+    if ((rc = ensure(c, c->nn_pos, slots * 4)) || (rc = ensure(c, c->nn_inter, slots * 8)) ||
+        (rc = ensure(c, c->nn_dist, slots * 8)) || (rc = ensure(c, c->nn_found, (uint64_t)targets * 4)))
+        return rc;
+    const double none = -1.0;
+    uint64_t none_bits;
+    std::memcpy(&none_bits, &none, 8);
+    CK(cudaMemsetAsync(c->nn_pos.p, 0xFF, slots * 4, c->stream));
+    CK(cudaMemsetAsync(c->nn_inter.p, 0, slots * 8, c->stream));
+    CK(cudaMemsetAsync(c->nn_found.p, 0, (uint64_t)targets * 4, c->stream));
+    CK(launch_fill_u64((uint64_t *)c->nn_dist.p, slots, none_bits, c->stream));
+    c->m.launches++;
+    return GKD_OK;
+}
+
+// the lists to the caller, once, at the end of the call.  With host_lists (GKD_AMBIG_LITERAL, host outputs) the
+// launches that ran on the device are merged into the host lists first.
+static int lists_finish(gkd_ctx *c, uint32_t targets, uint32_t k, HostLists *hl, const gkd_neighbors &out) {
+    const uint64_t slots = (uint64_t)targets * k;
+    const struct {
+        void *dst;
+        const void *src;
+        uint64_t bytes;
+    } copies[4] = {{out.pos, c->nn_pos.p, slots * 4}, {out.inter, c->nn_inter.p, slots * 8}, {out.dist, c->nn_dist.p, slots * 8},
+                   {out.n_found, c->nn_found.p, (uint64_t)targets * 4}};
+    if (!hl) {
+        for (const auto &cp : copies) {
+            if (!cp.dst) continue;
+            CK(cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, cudaMemcpyDefault, c->stream));
+            c->m.d2h_bytes += cp.bytes;
+        }
+        CK(cudaStreamSynchronize(c->stream));
+        return GKD_OK;
+    }
+    HostLists dev(targets, k);
+    CK(cudaMemcpyAsync(dev.pos.data(), c->nn_pos.p, slots * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(dev.inter.data(), c->nn_inter.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(dev.dist.data(), c->nn_dist.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    c->m.d2h_bytes += slots * 20;
+    for (uint32_t t = 0; t < targets; t++)
+        for (uint64_t s = (uint64_t)t * k; s < (uint64_t)(t + 1) * k && dev.pos[s] != 0xFFFFFFFFu; s++)
+            hl->offer(t, dev.pos[s], dev.inter[s], dev.dist[s]);
+    if (out.pos) std::memcpy(out.pos, hl->pos.data(), slots * 4);
+    if (out.inter) std::memcpy(out.inter, hl->inter.data(), slots * 8);
+    if (out.dist) std::memcpy(out.dist, hl->dist.data(), slots * 8);
+    if (out.n_found) std::memcpy(out.n_found, hl->n.data(), (uint64_t)targets * 4);
+    return GKD_OK;
+}
+
+static int nearest_args_ok(gkd_ctx *c, const char *fn, uint32_t k, double max_dist) {
+    if (k < 1 || k > NEAREST_MAX_K) return fail(c, GKD_EINVAL, "%s: k = %u is outside 1..%u", fn, k, NEAREST_MAX_K);
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "%s: max_dist is NaN", fn);
+    return GKD_OK;
+}
+
+// gkd_query_vs_ref_nearest(_ex): the q side by k_select_nearest (rows complete in every launch), the r side through
+// the per-target lists across the launches of rect_selection
+static int nearest_rect(gkd_ctx *c, const char *fn, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
+                        double max_dist, int exclude_self, const gkd_neighbors *qs, const gkd_neighbors *rs) {
+    int rc = nearest_args_ok(c, fn, k, max_dist);
+    if (rc) return rc;
+    if (!qs && !rs) return fail(c, GKD_EINVAL, "%s: both sides are NULL", fn);
     CHECK_CTX(c);
     CK(cudaSetDevice(c->cfg.device));
-    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_nearest: null id array");
-    const void *ps[4] = {ref_pos, inter, dist, n_found};
-    int rc = hits_host_ok(c, ps, 4);
-    if (rc) return rc;
+    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "%s: null id array", fn);
+    const gkd_neighbors none{};
+    const gkd_neighbors &a = qs ? *qs : none, &b = rs ? *rs : none;
+    const void *ps[8] = {a.pos, a.inter, a.dist, a.n_found, b.pos, b.inter, b.dist, b.n_found};
+    if ((rc = hits_host_ok(c, ps, 8))) return rc;
     c->m.pairs = 0;
-    if (nq == 0) return GKD_OK;
     ABI_GUARD_BEGIN
-    if (nr == 0) {  // no reference: every row is empty
-        const uint64_t slots = (uint64_t)nq * k;
-        if (ref_pos) CK(cudaMemcpy(ref_pos, std::vector<uint32_t>(slots, 0xFFFFFFFFu).data(), slots * 4, cudaMemcpyDefault));
-        if (inter) CK(cudaMemcpy(inter, std::vector<uint64_t>(slots, 0).data(), slots * 8, cudaMemcpyDefault));
-        if (dist) CK(cudaMemcpy(dist, std::vector<double>(slots, -1.0).data(), slots * 8, cudaMemcpyDefault));
-        if (n_found) CK(cudaMemcpy(n_found, std::vector<uint32_t>(nq, 0).data(), (uint64_t)nq * 4, cudaMemcpyDefault));
-        return GKD_OK;
+    if (nq == 0 || nr == 0) {  // no pair: every list is empty
+        if ((rc = fill_none(c, nq, k, qs))) return rc;
+        return fill_none(c, nr, k, rs);
     }
     Selection sel{};
     sel.within = false;
     sel.max_dist = max_dist;
     sel.k = k;
     sel.exclude_self = exclude_self ? 1 : 0;
-    sel.ref_pos = ref_pos;
-    sel.inter = inter;
-    sel.dist = dist;
-    sel.n_found = n_found;
-    return rect_selection(c, q, nq, r, nr, sel);
+    sel.rows = qs != nullptr;
+    sel.ref_pos = a.pos;
+    sel.inter = a.inter;
+    sel.dist = a.dist;
+    sel.n_found = a.n_found;
+    sel.absorb = rs != nullptr;
+    std::unique_ptr<HostLists> hl;
+    if (rs && c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hl.reset(new HostLists(nr, k));
+    sel.host_lists = hl.get();
+    if (rs && (rc = lists_begin(c, nr, k))) return rc;
+    if ((rc = rect_selection(c, q, nq, r, nr, sel))) return rc;
+    return rs ? lists_finish(c, nr, k, hl.get(), *rs) : GKD_OK;
+    ABI_GUARD_END(c)
+}
+
+int gkd_query_vs_ref_nearest(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
+                             double max_dist, int exclude_self, uint32_t *ref_pos, uint64_t *inter, double *dist,
+                             uint32_t *n_found) {
+    const gkd_neighbors qs{ref_pos, inter, dist, n_found};
+    return nearest_rect(c, "gkd_query_vs_ref_nearest", q, nq, r, nr, k, max_dist, exclude_self, &qs, nullptr);
+}
+
+int gkd_query_vs_ref_nearest_ex(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
+                                double max_dist, int exclude_self, const gkd_neighbors *q_side, const gkd_neighbors *r_side) {
+    return nearest_rect(c, "gkd_query_vs_ref_nearest_ex", q, nq, r, nr, k, max_dist, exclude_self, q_side, r_side);
+}
+
+int gkd_all_vs_all_nearest(gkd_ctx *c, uint32_t n, uint32_t k, double max_dist, const gkd_neighbors *out) {
+    int rc = nearest_args_ok(c, "gkd_all_vs_all_nearest", k, max_dist);
+    if (rc) return rc;
+    if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_nearest: null output");
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "nearest over %u sets but only %zu exist", n, c->genomes.size());
+    const void *ps[4] = {out->pos, out->inter, out->dist, out->n_found};
+    if ((rc = hits_host_ok(c, ps, 4))) return rc;
+    c->m.pairs = 0;
+    if (n == 0) return GKD_OK;
+    ABI_GUARD_BEGIN
+    Selection sel{};
+    sel.within = false;
+    sel.max_dist = max_dist;
+    sel.k = k;
+    sel.absorb = true;
+    std::unique_ptr<HostLists> hl;
+    if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hl.reset(new HostLists(n, k));
+    sel.host_lists = hl.get();
+    if ((rc = lists_begin(c, n, k))) return rc;
+    HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
+    if ((rc = run_pairs(c, hp, gkd_outputs{}, &sel))) return rc;
+    return lists_finish(c, n, k, hl.get(), *out);
     ABI_GUARD_END(c)
 }
 

@@ -150,20 +150,47 @@ struct WithinSink {
 // first capacity a member offers a within call; a call with more hits is repeated with the exact total
 constexpr uint64_t WITHIN_FIRST_CAP = 4ull << 20;
 
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within);
+// gkd_group_all_vs_all_nearest: a member's partial lists by global id.  A pair is computed once in the whole ring, so
+// the global top k of an id, by (distance bits, global id), is the top k of the union of its partial top-k lists.
+constexpr uint32_t NEAREST_MAX_K = 256;
+struct Neighbor {
+    uint64_t key;  // distance bits (distances are non-negative: the bits order like the values)
+    uint32_t id;
+    uint64_t inter;
+    bool operator<(const Neighbor &o) const { return key < o.key || (key == o.key && id < o.id); }
+};
+struct NearestSink {
+    uint32_t k;
+    double max_dist;
+    std::vector<std::vector<Neighbor>> lists;  // global id -> <= k entries after every call
+    void add(uint32_t target, uint32_t id, uint64_t inter, double d) {
+        uint64_t key;
+        memcpy(&key, &d, 8);
+        lists[target].push_back(Neighbor{key, id, inter});
+    }
+    void keep_best(uint32_t target) {
+        std::vector<Neighbor> &l = lists[target];
+        if (l.size() <= k) return;
+        std::partial_sort(l.begin(), l.begin() + k, l.end());
+        l.resize(k);
+    }
+};
+
+void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest);
 
 // the ring of one member (runs on its own host thread; no exception may leave the thread).  With `within` the
-// member selects on its device and collects its hits there instead of scattering dense blocks into inter / dist.
-void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within) {
+// member selects on its device and collects its hits there instead of scattering dense blocks into inter / dist;
+// with `nearest` it collects partial k-nearest lists.
+void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest) {
     try {
-        member_ring(g, x, inter, dist, within);
+        member_ring(g, x, inter, dist, within, nearest);
     } catch (const std::exception &ex) {
         g->members[x].rc = GKD_ENOMEM;
         g->members[x].err = ex.what();
     }
 }
 
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within) {
+void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest) {
     Member &M = g->members[x];
     const uint32_t R = (uint32_t)g->members.size();
     const uint64_t N = g->n_genomes;
@@ -256,8 +283,30 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
     if (!groups.empty()) post(0);
     if (M.rc) return;
 
+    // nearest: host lists of one call, per side
+    std::vector<uint32_t> qpos, qn, rpos, rn;
+    std::vector<uint64_t> qi, ri;
+    std::vector<double> qd, rd;
+    auto side = [&](size_t rows_, std::vector<uint32_t> &pos, std::vector<uint64_t> &in, std::vector<double> &d,
+                    std::vector<uint32_t> &nf) {
+        const size_t slots = rows_ * nearest->k;
+        pos.resize(slots);
+        in.resize(slots);
+        d.resize(slots);
+        nf.resize(rows_);
+        return gkd_neighbors{pos.data(), in.data(), d.data(), nf.data()};
+    };
     // diagonal block (runs while the first group is in flight)
-    if (m >= 2 && within) {
+    if (m >= 2 && nearest) {
+        const uint32_t k = nearest->k;
+        const gkd_neighbors nb = side(m, qpos, qi, qd, qn);
+        MGK(gkd_all_vs_all_nearest(M.ctx, m, k, nearest->max_dist, &nb));
+        for (uint32_t i = 0; i < m; i++)
+            for (uint32_t s = 0; s < qn[i]; s++) {
+                const uint64_t o = (uint64_t)i * k + s;
+                nearest->add(M.global_ids[i], M.global_ids[qpos[o]], qi[o], qd[o]);
+            }
+    } else if (m >= 2 && within) {
         const uint64_t cnt = (uint64_t)m * (m - 1) / 2;
         MGK(fetch(cnt, [&](gkd_hits &h) { return gkd_all_vs_all_range_within(M.ctx, m, 0, cnt, within->max_dist, &h); }));
         for (uint64_t t = 0; t < nh; t++) within->hits.push_back({M.global_ids[ha[t]], M.global_ids[hb[t]], bi[t], bd[t]});
@@ -271,6 +320,7 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
             for (uint32_t j = i + 1; j < m; j++, t++) put(M.global_ids[i], M.global_ids[j], bi[t], bd[t]);
     }
     std::vector<uint32_t> rows, cols, col_gid;  // col_gid: global id of every column of the call
+    std::vector<uint32_t> order;
     for (size_t gi = 0; gi < groups.size(); gi++) {
         if (gi + 1 < groups.size()) {
             // buffer (gi+1)&1 was last used by group gi-1, whose sets were dropped (and the stream drained) below
@@ -293,6 +343,37 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
                 cols.push_back(first + c);
                 col_gid.push_back(g->members[S.src].global_ids[S.p.first + c]);
             }
+        }
+        if (nearest) {
+            // The lists break ties by position in the call, and a group of panels may span peers (x+1)%R, (x+2)%R, ...,
+            // whose global ids are not ascending: order the columns by global id so that position order is id order.
+            // The rows are this member's own ids, ascending.
+            order.resize(cols.size());
+            for (uint32_t c = 0; c < order.size(); c++) order[c] = c;
+            std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return col_gid[a] < col_gid[b]; });
+            std::vector<uint32_t> scols(cols.size()), sgid(cols.size());
+            for (size_t c = 0; c < order.size(); c++) scols[c] = cols[order[c]], sgid[c] = col_gid[order[c]];
+            const uint32_t k = nearest->k;
+            const gkd_neighbors qs = side(rows.size(), qpos, qi, qd, qn), rs = side(cols.size(), rpos, ri, rd, rn);
+            MGK(gkd_query_vs_ref_nearest_ex(M.ctx, rows.data(), (uint32_t)rows.size(), scols.data(), (uint32_t)scols.size(), k,
+                                            nearest->max_dist, 0, &qs, &rs));
+            for (size_t r = 0; r < rows.size(); r++) {
+                const uint32_t target = M.global_ids[rows[r]];
+                for (uint32_t s = 0; s < qn[r]; s++) {
+                    const uint64_t o = (uint64_t)r * k + s;
+                    nearest->add(target, sgid[qpos[o]], qi[o], qd[o]);
+                }
+                nearest->keep_best(target);
+            }
+            for (size_t c = 0; c < scols.size(); c++) {
+                for (uint32_t s = 0; s < rn[c]; s++) {
+                    const uint64_t o = (uint64_t)c * k + s;
+                    nearest->add(sgid[c], M.global_ids[rows[rpos[o]]], ri[o], rd[o]);
+                }
+                nearest->keep_best(sgid[c]);
+            }
+            MGK(gkd_truncate(M.ctx, m));
+            continue;
         }
         if (within) {
             MGK(fetch((uint64_t)rows.size() * cols.size(), [&](gkd_hits &h) {
@@ -516,7 +597,7 @@ int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist) {
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr);
+            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr, nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -539,7 +620,7 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x]);
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x], nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -562,6 +643,49 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
         return GKD_OK;
     } catch (const std::exception &ex) {
         return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_within: %s", ex.what());
+    }
+}
+
+int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, const gkd_neighbors *out) {
+    if (k < 1 || k > NEAREST_MAX_K) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nearest: k = %u is outside 1..%u", k, NEAREST_MAX_K);
+    if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nearest: max_dist is NaN");
+    if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nearest: null output");
+    if (!g) return GKD_EINVAL;
+    try {
+        for (auto &M : g->members)
+            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
+        const uint32_t N = g->n_genomes;
+        std::vector<NearestSink> sinks(g->members.size(), NearestSink{k, max_dist, std::vector<std::vector<Neighbor>>(N)});
+        std::vector<std::thread> threads;
+        for (uint32_t x = 0; x < g->members.size(); x++) {
+            g->members[x].rc = GKD_OK;
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, &sinks[x]);
+        }
+        for (auto &t : threads) t.join();
+        for (size_t i = 0; i < g->members.size(); i++)
+            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        std::vector<Neighbor> all;
+        for (uint32_t t = 0; t < N; t++) {
+            all.clear();
+            for (auto &s : sinks) {
+                all.insert(all.end(), s.lists[t].begin(), s.lists[t].end());
+                std::vector<Neighbor>().swap(s.lists[t]);
+            }
+            const size_t m = std::min<size_t>(all.size(), k);
+            std::partial_sort(all.begin(), all.begin() + m, all.end());
+            for (uint32_t i = 0; i < k; i++) {
+                const uint64_t o = (uint64_t)t * k + i;
+                double d = -1.0;
+                if (i < m) memcpy(&d, &all[i].key, 8);
+                if (out->pos) out->pos[o] = i < m ? all[i].id : 0xFFFFFFFFu;
+                if (out->inter) out->inter[o] = i < m ? all[i].inter : 0;
+                if (out->dist) out->dist[o] = d;
+            }
+            if (out->n_found) out->n_found[t] = (uint32_t)m;
+        }
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_nearest: %s", ex.what());
     }
 }
 

@@ -305,6 +305,13 @@ cudaError_t launch_select_within(const SetDesc *sets, PairSource src, const uint
 cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t rows, const uint32_t *counts,
                                   const uint32_t *pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
                                   NearestOut out, cudaStream_t s);
+// PAIRS_UPPER or PAIRS_RECT: merge the launch into per-target lists that persist across launches (`state`, every member
+// set; targets * k slots, filled with the unused entry before the first launch).  UPPER: every pair (i, j) is offered
+// to target i (neighbour j) and target j (neighbour i); RECT: to reference column j, neighbour a_base + query row.
+// Writes nothing when join_err (may be nullptr) reads nonzero on the stream.
+cudaError_t launch_nearest_absorb(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
+                                  int both_strands, double max_dist, uint32_t k, int exclude_self, uint32_t a_base,
+                                  const uint32_t *join_err, NearestOut state, cudaStream_t s);
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless
 // some representative is within max_dist; clears the counts it consumed
 cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *n_reps, uint32_t cand, uint32_t visit,

@@ -135,6 +135,8 @@ const std::vector<OptSpec> FASTA_OPTS = {
     {{"--devices"}, true, "explicit comma-separated device ordinals for the group, e.g. 0,1,2,3 (an ordinal may repeat)"},
     {{"--metrics"}, true, "write one JSON line of engine metrics to this file (additive option)"},
     {{"--maxDist"}, true, "report only the pairs with distance <= this (additive option; selected on the GPU)"},
+    {{"--nearest"}, true, "report each record's N (1..256) nearest other records within --maxDist (default 1.0), in "
+                          "input order, nearest first; a pair can appear twice, once from each end (additive option)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
@@ -173,6 +175,20 @@ void writeHits(std::ostream &writer, const uint32_t *a, const uint32_t *b, const
                CommentFn comment) {
     std::string line;
     for (uint64_t t = 0; t < n; t++) writePairLine(writer, line, a[t], b[t], dist[t], label, comment);
+}
+
+// the lines of `fastaDist --nearest`: for each record in input order its neighbours (n*k lists of gkd_*_nearest), record
+// first, in ascending distance and then input order
+template <class LabelFn, class CommentFn>
+uint64_t writeNeighbors(std::ostream &writer, size_t n, uint32_t k, const uint32_t *pos, const double *dist,
+                        const uint32_t *found, LabelFn label, CommentFn comment) {
+    std::string line;
+    uint64_t lines = 0;
+    for (size_t i = 0; i < n; i++)
+        for (uint32_t s = 0; s < found[i]; s++, lines++)
+            writePairLine(writer, line, i, pos[i * k + s], dist[i * k + s], label, comment);
+    writer.flush();
+    return lines;
 }
 
 // pairs per gkd_all_vs_all_range_within call of `fastaDist --maxDist`: host memory stays O(range), not O(n^2)
@@ -216,6 +232,9 @@ int fastaDist(const std::vector<std::string> &args) {
     const bool within = p.values.count("--maxDist") > 0;
     const double maxDist = within ? toDouble("--maxDist", p.values["--maxDist"]) : 1.0;
     if (!(maxDist > 0.0 && maxDist <= 1.0)) throw ParseFailureException("Maximum distance must be > 0 and <= 1.");
+    const int nearest = p.values.count("--nearest") ? toInt("--nearest", p.values["--nearest"]) : 0;
+    if (p.values.count("--nearest") && (nearest < 1 || nearest > 256))
+        throw ParseFailureException("Number of neighbors must be between 1 and 256.");
     const char *typeName = seqType == KmerType::DNA ? "DNA" : (seqType == KmerType::RNA ? "RNA" : "PROT");
     if (inFile.empty()) logInfo(std::string("Reading ") + typeName + " sequences from the standard input.");
     else if (!readable(inFile)) throw IOException("Input file " + inFile + " is not found or unreadable.");
@@ -270,6 +289,19 @@ int fastaDist(const std::vector<std::string> &args) {
         gcheck(gkd_group_build(grp));
         logInfo(std::to_string(n) + " sequences cached on " + std::to_string(gpus) + " GPUs. Computing distances.");
         const uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
+        if (nearest) {
+            const uint32_t k = (uint32_t)nearest;
+            std::vector<uint32_t> pos((size_t)n * k), found(n);
+            std::vector<double> d((size_t)n * k);
+            const gkd_neighbors nb{pos.data(), nullptr, d.data(), found.data()};
+            gcheck(gkd_group_all_vs_all_nearest(grp, k, maxDist, &nb));
+            const uint64_t lines = writeNeighbors(writer, n, k, pos.data(), d.data(), found.data(),
+                                                  [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
+                                                  [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
+            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(lines) + " neighbor lines.");
+            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
+            return 0;
+        }
         if (within) {
             // every member selects on its device; one call, repeated with the exact capacity if the first was short
             uint64_t cap = std::min<uint64_t>(total, WITHIN_RANGE);
@@ -309,6 +341,22 @@ int fastaDist(const std::vector<std::string> &args) {
     writer << "seq1\tname1\tseq2\tname2\tdistance\n";
     engine.build();
     logInfo(std::to_string(seqs.size()) + " sequences cached. Computing distances.");
+    if (nearest) {
+        // each pair i < j is intersected once and offered to both rows; only the n*k lists leave the GPU
+        const uint32_t k = (uint32_t)nearest;
+        const size_t n = seqs.size();
+        std::vector<uint32_t> pos(n * k), found(n);
+        std::vector<double> d(n * k);
+        const gkd_neighbors nb{pos.data(), nullptr, d.data(), found.data()};
+        engine.check(gkd_all_vs_all_nearest(engine.raw(), (uint32_t)n, k, maxDist, &nb));
+        const uint64_t lines = writeNeighbors(writer, n, k, pos.data(), d.data(), found.data(),
+                                              [&](size_t i) { return seqs[i].getGenomeId(); },
+                                              [&](size_t i) { return seqs[i].getGenomeName(); });
+        logInfo(std::to_string(n < 2 ? 0 : n * (n - 1) / 2) + " pairs computed in 1 batches, " + std::to_string(lines) +
+                " neighbor lines.");
+        writeMetrics(metricsFile, "fastaDist", engine.raw(), n < 2 ? 0 : n * (n - 1) / 2, 1);
+        return 0;
+    }
     if (within) {
         // the triangle in ranges of <= WITHIN_RANGE pairs; only the pairs within maxDist leave the GPU
         const uint64_t n = seqs.size(), total = n < 2 ? 0 : n * (n - 1) / 2, room = std::min(total, WITHIN_RANGE);

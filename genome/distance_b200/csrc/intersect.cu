@@ -648,6 +648,47 @@ cudaError_t launch_select_within(const SetDesc *sets, PairSource src, const uint
 constexpr int NEAR_THREADS = 256, NEAR_SLOTS = 512;
 constexpr unsigned long long NEAR_NONE = ~0ull;  // sorts after every distance
 
+// bitonic sort of the 512 slots by (distance bits, position), then slots >= k are cleared; the caller synchronises
+// before it reads the list
+__device__ __forceinline__ void near_sort_keep(unsigned long long *s_key, unsigned long long *s_inter, uint32_t *s_pos,
+                                               uint32_t k, uint32_t tid) {
+    for (uint32_t size = 2; size <= NEAR_SLOTS; size <<= 1) {
+        for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
+            const uint32_t i = (tid / stride) * 2u * stride + (tid % stride), l = i + stride;
+            const bool up = (i & size) == 0;
+            const unsigned long long ki = s_key[i], kl = s_key[l];
+            const uint32_t pi = s_pos[i], pl = s_pos[l];
+            const bool gt = ki > kl || (ki == kl && pi > pl);
+            if (gt == up) {
+                s_key[i] = kl, s_key[l] = ki;
+                s_pos[i] = pl, s_pos[l] = pi;
+                const unsigned long long t2 = s_inter[i];
+                s_inter[i] = s_inter[l], s_inter[l] = t2;
+            }
+            __syncthreads();
+        }
+    }
+    for (uint32_t i = k + tid; i < NEAR_SLOTS; i += NEAR_THREADS) {
+        s_key[i] = NEAR_NONE;
+        s_inter[i] = 0;
+        s_pos[i] = 0xFFFFFFFFu;
+    }
+}
+
+// list slots [0, k) -> row `row` of out (k <= NEAR_THREADS: thread i writes slot i); unused slots as gkd.h documents
+__device__ __forceinline__ void near_write(const unsigned long long *s_key, const unsigned long long *s_inter,
+                                           const uint32_t *s_pos, uint32_t k, uint32_t tid, uint32_t row, NearestOut out) {
+    const bool valid = tid < k && s_pos[tid] != 0xFFFFFFFFu;
+    if (tid < k) {
+        const uint64_t o = (uint64_t)row * k + tid;
+        if (out.ref_pos) out.ref_pos[o] = s_pos[tid];
+        if (out.inter) out.inter[o] = valid ? s_inter[tid] : 0ull;
+        if (out.dist) out.dist[o] = valid ? __longlong_as_double((long long)s_key[tid]) : -1.0;
+    }
+    const int found = __syncthreads_count(valid);
+    if (tid == 0 && out.n_found) out.n_found[row] = (uint32_t)found;
+}
+
 __global__ void __launch_bounds__(NEAR_THREADS)
     k_select_nearest(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
                      const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
@@ -689,41 +730,12 @@ __global__ void __launch_bounds__(NEAR_THREADS)
         const uint32_t n_cand = s_n;
         __syncthreads();  // everyone has read s_n before it is reset
         if (n_cand == 0) continue;
-        for (uint32_t size = 2; size <= NEAR_SLOTS; size <<= 1) {
-            for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
-                const uint32_t i = (tid / stride) * 2u * stride + (tid % stride), l = i + stride;
-                const bool up = (i & size) == 0;
-                const unsigned long long ki = s_key[i], kl = s_key[l];
-                const uint32_t pi = s_pos[i], pl = s_pos[l];
-                const bool gt = ki > kl || (ki == kl && pi > pl);
-                if (gt == up) {
-                    s_key[i] = kl, s_key[l] = ki;
-                    s_pos[i] = pl, s_pos[l] = pi;
-                    const unsigned long long t2 = s_inter[i];
-                    s_inter[i] = s_inter[l], s_inter[l] = t2;
-                }
-                __syncthreads();
-            }
-        }
-        for (uint32_t i = k + tid; i < NEAR_SLOTS; i += NEAR_THREADS) {
-            s_key[i] = NEAR_NONE;
-            s_inter[i] = 0;
-            s_pos[i] = 0xFFFFFFFFu;
-        }
+        near_sort_keep(s_key, s_inter, s_pos, k, tid);
         if (tid == 0) s_n = 0;
         __syncthreads();
         thr = s_key[k - 1];
     }
-    // k <= NEAR_THREADS: thread i writes slot i
-    const bool valid = tid < k && s_pos[tid] != 0xFFFFFFFFu;
-    if (tid < k) {
-        const uint64_t o = (uint64_t)row * k + tid;
-        if (out.ref_pos) out.ref_pos[o] = s_pos[tid];
-        if (out.inter) out.inter[o] = valid ? s_inter[tid] : 0ull;
-        if (out.dist) out.dist[o] = valid ? __longlong_as_double((long long)s_key[tid]) : -1.0;
-    }
-    const int found = __syncthreads_count(valid);
-    if (tid == 0 && out.n_found) out.n_found[row] = (uint32_t)found;
+    near_write(s_key, s_inter, s_pos, k, tid, row, out);
 }
 
 cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t rows, const uint32_t *counts,
@@ -731,6 +743,124 @@ cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t 
                                   NearestOut out, cudaStream_t s) {
     if (rows == 0) return cudaSuccess;
     k_select_nearest<<<rows, NEAR_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, k, exclude_self, out);
+    return cudaGetLastError();
+}
+
+// Nearest, accumulating form: per-target lists of k slots that live in HBM (`state`, the layout of NearestOut) across
+// the chunks and launches of one call.  One CTA per target loads its list into the slots [0, 256) of the layout above,
+// gathers the target's pairs of this launch in rounds of 256 candidates and writes the list back if a round changed it.
+//   UPPER chunk [first, first+count) with rows i0..i1: target i takes its row segment (i, j), target j the column
+//     entries (i, j), i0 <= i < j, whose position is inside the chunk.  Targets are i0..n-1.
+//   RECT launch: target = reference column j; it takes counts[row * nr + j] of every query row, neighbour a_base + row.
+// A candidate enters when (distance bits, position) is below the k-th entry: unlike k_select_nearest, positions do not
+// arrive in ascending order (the column side of a later chunk may tie the k-th distance with a smaller position).
+// The lists outlive the launch, so a launch whose block join overflowed (it is redone by the merge kernel) must not
+// touch them: the flag is read here, on the stream after kernel 4, rather than on the host afterwards.
+__device__ __forceinline__ uint64_t upper_row_start(uint64_t i, uint64_t n) { return i * (2 * n - i - 1) / 2; }
+
+__global__ void __launch_bounds__(NEAR_THREADS)
+    k_nearest_absorb(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
+                     const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
+                     uint32_t i0, uint32_t i1, uint32_t a_base, const uint32_t *__restrict__ join_err, NearestOut state) {
+    if (join_err && *join_err) return;
+    __shared__ unsigned long long s_key[NEAR_SLOTS];
+    __shared__ unsigned long long s_inter[NEAR_SLOTS];
+    __shared__ uint32_t s_pos[NEAR_SLOTS];
+    __shared__ uint32_t s_n;
+    const uint32_t tid = threadIdx.x;
+    const bool upper = src.mode == PAIRS_UPPER;
+    const uint32_t tg = (upper ? i0 : 0u) + blockIdx.x;
+    const uint64_t n = src.n, first = src.first, end = src.first + src.count;
+    uint64_t rs = 0, row_lo = 0;
+    uint32_t n_row = 0, n_col;
+    if (upper) {
+        rs = upper_row_start(tg, n);
+        if (tg <= i1) {
+            const uint64_t lo = max(rs, first), hi = min(rs + (n - tg - 1), end);
+            if (hi > lo) row_lo = lo, n_row = (uint32_t)(hi - lo);
+        }
+        n_col = tg > i0 ? min(i1, tg - 1) - i0 + 1 : 0u;
+    } else {
+        n_col = (uint32_t)(src.count / src.n);
+    }
+    const uint32_t total = n_row + n_col;
+    if (total == 0) return;
+
+    const uint64_t base = (uint64_t)tg * k;
+    for (uint32_t i = tid; i < NEAR_SLOTS; i += NEAR_THREADS) {
+        const uint32_t p = i < k ? state.ref_pos[base + i] : 0xFFFFFFFFu;
+        const bool used = p != 0xFFFFFFFFu;
+        s_key[i] = used ? (unsigned long long)__double_as_longlong(state.dist[base + i]) : NEAR_NONE;
+        s_inter[i] = used ? state.inter[base + i] : 0ull;
+        s_pos[i] = p;
+    }
+    if (tid == 0) s_n = 0;
+    __syncthreads();
+    unsigned long long thr = s_key[k - 1];
+    uint32_t thr_pos = s_pos[k - 1];
+    bool changed = false;
+    for (uint32_t u0 = 0; u0 < total; u0 += NEAR_THREADS) {
+        const uint32_t u = u0 + tid;
+        bool have = false;
+        uint64_t t = 0;
+        uint32_t ida = 0, idb = 0, nb = 0;
+        if (u < n_row) {  // (tg, j): the row segment is contiguous
+            const uint64_t p = row_lo + u;
+            t = p - first;
+            ida = tg, idb = tg + 1 + (uint32_t)(p - rs), nb = idb;
+            have = true;
+        } else if (u < total && upper) {  // (i, tg), i < tg: one entry per earlier row
+            const uint32_t i = i0 + (u - n_row);
+            const uint64_t p = upper_row_start(i, n) + (tg - i - 1);
+            if (p >= first && p < end) {
+                t = p - first;
+                ida = i, idb = tg, nb = i;
+                have = true;
+            }
+        } else if (u < total) {  // RECT: query row u against reference tg
+            t = (uint64_t)u * src.n + tg;
+            decode_pair(src, t, ida, idb);
+            nb = a_base + u;
+            have = !(exclude_self && ida == idb);
+        }
+        if (have) {
+            uint64_t I, sa, sb;
+            double d;
+            pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+            const unsigned long long key = (unsigned long long)__double_as_longlong(d);
+            if (d <= max_dist && (key < thr || (key == thr && nb < thr_pos))) {
+                const uint32_t slot = NEAR_THREADS + atomicAdd(&s_n, 1u);
+                s_key[slot] = key;
+                s_inter[slot] = I;
+                s_pos[slot] = nb;
+            }
+        }
+        __syncthreads();
+        const uint32_t n_cand = s_n;
+        __syncthreads();
+        if (n_cand == 0) continue;
+        near_sort_keep(s_key, s_inter, s_pos, k, tid);
+        if (tid == 0) s_n = 0;
+        __syncthreads();
+        thr = s_key[k - 1];
+        thr_pos = s_pos[k - 1];
+        changed = true;
+    }
+    if (changed) near_write(s_key, s_inter, s_pos, k, tid, tg, state);
+}
+
+cudaError_t launch_nearest_absorb(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
+                                  int both_strands, double max_dist, uint32_t k, int exclude_self, uint32_t a_base,
+                                  const uint32_t *join_err, NearestOut state, cudaStream_t s) {
+    if (src.count == 0) return cudaSuccess;
+    uint32_t i0 = 0, i1 = 0, j = 0, targets = src.n;
+    if (src.mode == PAIRS_UPPER) {
+        upper_pair(src.first, src.n, i0, j);
+        upper_pair(src.first + src.count - 1, src.n, i1, j);
+        targets = src.n - i0;
+    }
+    k_nearest_absorb<<<targets, NEAR_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, k, exclude_self,
+                                                      i0, i1, a_base, join_err, state);
     return cudaGetLastError();
 }
 

@@ -9,7 +9,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (AMBIG_LITERAL, AMBIG_SKIP, DNA, PROT, RNA, STRAND_BOTH, STRAND_CANONICAL, GkdConfig, GkdHits,
-                   GkdMetrics, GkdOutputs, GkdPackedSet)
+                   GkdMetrics, GkdNeighbors, GkdOutputs, GkdPackedSet)
 
 PACKED_DTYPE = np.dtype([("offs_off", "<u8"), ("lows_off", "<u8"), ("pal_offs_off", "<u8"), ("pal_lows_off", "<u8"),
                          ("n", "<u4"), ("n_pal", "<u4"), ("level", "<u4"), ("pal_level", "<u4")])
@@ -34,6 +34,14 @@ def _select(call, pairs: int):
             n = h.n
             return a[:n], b[:n], inter[:n], dist[:n]
         cap = h.n
+
+
+def _neighbors(rows: int, k: int):
+    """host arrays (pos, inter, dist, n_found) of `rows` k-nearest lists and the gkd_neighbors that points at them"""
+    k = max(int(k), 0)
+    pos, inter = np.empty((rows, k), dtype=np.uint32), np.empty((rows, k), dtype=np.uint64)
+    dist, found = np.empty((rows, k), dtype=np.float64), np.empty(rows, dtype=np.uint32)
+    return (pos, inter, dist, found), GkdNeighbors(pos.ctypes.data, inter.ctypes.data, dist.ctypes.data, found.ctypes.data)
 
 
 class GkdError(RuntimeError):
@@ -304,6 +312,27 @@ class Engine:
         shape = (qa.size, max(int(k), 0))
         return pos.reshape(shape), inter.reshape(shape), dist.reshape(shape), found
 
+    def query_vs_ref_nearest_ex(self, q: Sequence[int], r: Sequence[int], k: int, max_dist: float,
+                                exclude_self: bool = False):
+        """(q_side, r_side) of one query x reference pass: q_side is query_vs_ref_nearest(q, r, ...), r_side every
+        reference's <= k nearest queries (positions in q), equal to query_vs_ref_nearest(r, q, ...); each side is a
+        (pos, inter, dist, n_found) tuple"""
+        qa, ra = np.ascontiguousarray(q, dtype=np.uint32), np.ascontiguousarray(r, dtype=np.uint32)
+        q_side, qn = _neighbors(qa.size, k)
+        r_side, rn = _neighbors(ra.size, k)
+        self._ck(self._L.gkd_query_vs_ref_nearest_ex(self._h, qa.ctypes.data, qa.size, ra.ctypes.data, ra.size, int(k),
+                                                     float(max_dist), 1 if exclude_self else 0, C.byref(qn), C.byref(rn)))
+        return q_side, r_side
+
+    def all_vs_all_nearest(self, k: int, max_dist: float, n: int = None):
+        """(pos, inter, dist, n_found): each of the first n sets' (default: all) <= k nearest other sets within
+        max_dist, as (n, k) arrays in ascending distance, ties by the smaller id; every pair is intersected once.  Equal
+        to query_vs_ref_nearest(range(n), range(n), k, max_dist, exclude_self=True)"""
+        n = len(self) if n is None else int(n)
+        out, nb = _neighbors(n, k)
+        self._ck(self._L.gkd_all_vs_all_nearest(self._h, n, int(k), float(max_dist), C.byref(nb)))
+        return out
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -474,3 +503,9 @@ class Group:
         n = len(self)
         return _select(lambda h: self._ck(self._L.gkd_group_all_vs_all_within(self._h, float(max_dist), C.byref(h))),
                        n * (n - 1) // 2)
+
+    def all_vs_all_nearest(self, k: int, max_dist: float):
+        """(pos, inter, dist, n_found) over all global ids: the single-context Engine.all_vs_all_nearest result"""
+        out, nb = _neighbors(len(self), k)
+        self._ck(self._L.gkd_group_all_vs_all_nearest(self._h, int(k), float(max_dist), C.byref(nb)))
+        return out

@@ -249,6 +249,26 @@ int gkd_query_vs_ref_nearest(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const
                              uint32_t k, double max_dist, int exclude_self,
                              uint32_t *ref_pos, uint64_t *inter, double *dist, uint32_t *n_found);
 
+/* k-nearest-neighbour lists: rows*k row-major (n_found: rows).  Any member may be NULL; pointers may be host or device
+ * memory as for gkd_hits.  Unused slots hold pos = UINT32_MAX, inter = 0, dist = -1.0 (as gkd_query_vs_ref_nearest). */
+typedef struct gkd_neighbors {
+    uint32_t *pos;      /* neighbour: set id (all-vs-all) or position in the other list (query_vs_ref) */
+    uint64_t *inter;    /* similarity(), as gkd_all_vs_all */
+    double *dist;       /* bit-identical to the dense call's double for the same pair */
+    uint32_t *n_found;  /* entries used per row, <= k */
+} gkd_neighbors;
+/* The k-nearest-neighbour graph of one collection (the exact form of what MashProcessor.java:150, getClosest(kmers, n,
+ * maxDist), estimates): each of the first n sets gets its <= k nearest OTHER sets within max_dist, ascending distance,
+ * ties by the smaller id.  Every pair i < j is intersected once and offered to both of its rows, so this costs half the
+ * kernel-4 work of the rectangle and is equal, bit for bit, to gkd_query_vs_ref_nearest(q = r = 0..n-1, exclude_self = 1).
+ * 1 <= k <= 256; out may not be NULL. */
+int gkd_all_vs_all_nearest(gkd_ctx *ctx, uint32_t n, uint32_t k, double max_dist, const gkd_neighbors *out);
+/* One query x reference pass, both directions: q_side = gkd_query_vs_ref_nearest's result; r_side = each reference's
+ * <= k nearest queries (positions in q, ties by the smaller position), equal to gkd_query_vs_ref_nearest(r, q).
+ * Either side may be NULL, but not both. */
+int gkd_query_vs_ref_nearest_ex(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
+                                double max_dist, int exclude_self, const gkd_neighbors *q_side, const gkd_neighbors *r_side);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -278,6 +298,10 @@ int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist);
 /* the group form of gkd_all_vs_all_range_within over all global ids: hits ordered by (a, b), equal to one context's.
  * Every member selects on its own device; only the hits reach the host.  The arrays of out are host memory. */
 int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out);
+/* gkd_all_vs_all_nearest over all global ids (pos holds global ids), equal to one context's result.  Every member
+ * selects its diagonal block and both directions of its ring blocks on its own device; the host merges the partial
+ * lists of every id.  The arrays of out are host memory, N*k (n_found: N). */
+int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, const gkd_neighbors *out);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

@@ -217,3 +217,23 @@ JNIEXPORT jint JNICALL FN(queryVsRefNearest)(JNIEnv *env, jclass c, jlong h, jin
     if (qa) (*env)->ReleaseIntArrayElements(env, q, qa, JNI_ABORT);
     return rc;
 }
+
+/* each of the first n sets' k nearest other sets within maxDist: pos / dist hold n * k entries, nFound n */
+JNIEXPORT jint JNICALL FN(allVsAllNearest)(JNIEnv *env, jclass c, jlong h, jint n, jint k, jdouble maxDist, jintArray pos,
+                                           jdoubleArray dist, jintArray nFound) {
+    (void)c;
+    if (!pos || !dist || !nFound || n < 0 || k < 1) return GKD_EINVAL;
+    const jlong slots = (jlong)n * (jlong)k;
+    if ((jlong)(*env)->GetArrayLength(env, pos) < slots || (jlong)(*env)->GetArrayLength(env, dist) < slots ||
+        (*env)->GetArrayLength(env, nFound) < n)
+        return GKD_EINVAL;
+    jint *p = (*env)->GetIntArrayElements(env, pos, NULL);
+    jint *found = (*env)->GetIntArrayElements(env, nFound, NULL);
+    jdouble *d = (*env)->GetDoubleArrayElements(env, dist, NULL);
+    gkd_neighbors out = {(uint32_t *)p, NULL, d, (uint32_t *)found};
+    int rc = (p && found && d) ? gkd_all_vs_all_nearest(CTX(h), (uint32_t)n, (uint32_t)k, maxDist, &out) : GKD_ENOMEM;
+    if (d) (*env)->ReleaseDoubleArrayElements(env, dist, d, 0);
+    if (found) (*env)->ReleaseIntArrayElements(env, nFound, found, 0);
+    if (p) (*env)->ReleaseIntArrayElements(env, pos, p, 0);
+    return rc;
+}

@@ -43,6 +43,10 @@ final class GkdNative {
      *  dist (length q.length * k, row-major; unused slots -1 and -1.0), nFound (length q.length) */
     static native int queryVsRefNearest(long ctx, int[] q, int[] r, int k, double maxDist, boolean excludeSelf,
                                         int[] refPos, double[] dist, int[] nFound);
+    /** each of the first n sets' &lt;= k nearest other sets within maxDist, ascending distance, ties by the smaller id;
+     *  every pair is intersected once: pos and dist (length n * k, row-major; unused slots -1 and -1.0), nFound
+     *  (length n) */
+    static native int allVsAllNearest(long ctx, int n, int k, double maxDist, int[] pos, double[] dist, int[] nFound);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

@@ -174,6 +174,17 @@ public class GpuKmerEngine implements AutoCloseable {
         return found;
     }
 
+    /** the k-nearest-neighbour graph of every set (MashProcessor's getClosest, exact): pos[i*k+j] is the id of the
+     *  j-th nearest other set of set i within maxDist (ascending distance, ties by the smaller id), -1 in unused slots;
+     *  returns the number found per set.  pos and dist receive size() * k values. */
+    public synchronized int[] allVsAllNearest(int k, double maxDist, int[] pos, double[] dist) {
+        this.build();
+        int n = this.size();
+        int[] found = new int[n];
+        check(GkdNative.allVsAllNearest(this.ctx, n, k, maxDist, pos, dist, found));
+        return found;
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
