@@ -87,7 +87,7 @@ typedef struct gkd_metrics {
     uint64_t kmer_positions;    /* k-mer positions encoded by kernel 2 */
     uint64_t keys_sorted;       /* keys through the radix sort (kernel 3 input) */
     uint32_t sort_passes;       /* LSD passes per key */
-    uint32_t intersect_kernel;  /* kernel 4 variant of the last distance call: 3 = bucket merge on 32-bit low words, 4 = on 64-bit keys, 5 = block join (32 rows per shared-memory table) */
+    uint32_t intersect_kernel;  /* kernel 4 variant of the last distance call: 3 = bucket merge on 32-bit low words, 4 = on 64-bit keys, 5 = block join (32 or 64 rows per shared-memory table) */
     uint64_t keys_unique;       /* sum of |C| over the sets built */
     uint64_t pairs;             /* pairs intersected by the last distance call */
     uint64_t intersect_bytes;   /* ALGORITHMIC bytes of the last distance call: 8*(|C_A|+|C_B|) per pair */

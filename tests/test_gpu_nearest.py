@@ -6,9 +6,9 @@ numpy ranking of the dense matrix made symmetric: ascending distance, ties by th
 The same accumulator gives the reference side of gkd_query_vs_ref_nearest_ex, and the group form merges the members'
 partial lists by (distance, global id).
 
-Join-overflow redo: no supported switch makes a block-join table overflow (see tests/test_gpu_select.py), so the
-device-side guard of the absorb kernel (it reads the overflow flag on the stream and writes nothing when it is set) is
-not forced here.
+Join-overflow redo: the device-side guard of the absorb kernel (it reads the overflow flag on the stream and writes
+nothing when it is set) is forced in tests/test_gpu_join_redo.py, with coarse set tables and skewed imported key sets,
+including an overflow in the second chunk only.
 """
 import os
 import subprocess

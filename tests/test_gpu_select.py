@@ -6,12 +6,11 @@ GPU, and each one must be exactly the dense call's entry.
            protein 8, at D = 1.0, at an attained distance (the comparison is inclusive) and below every distance;
 * nearest: each query row = a stable sort of the dense row by (distance, position in r), filtered and cut to k.
 
-Join-overflow redo: a block-join table is flagged (and the chunk redone by the merge kernel) only when the rows of one
-key range fill more than 62.5 % of its slots, while GKD_JOIN_FILL, the only supported switch on the table load, is
-clamped to 45 % and every row's range count is chosen so that its expected share stays under that target.  No
-supported switch makes a table overflow, so the redo is not forced here; the within and nearest selections of a
-chunk are copied and counted only after its overflow flag has been read as clear (select_chunk in gkd_api.cu).
-The 45 % fill itself is covered below.
+Join-overflow redo: a block-join table is flagged (and the chunk redone by the merge kernel) when the rows of one key
+range fill more than 62.5 % of its slots.  With uniform keys that does not happen: GKD_JOIN_FILL is clamped to 45 % and
+every row's range count keeps its expected share under that target (the 45 % fill is covered below).  Coarse set
+tables and skewed imported key sets do overflow; tests/test_gpu_join_redo.py forces the redo that way and checks that
+the within and nearest selections of a redone chunk are copied and counted once (select_chunk in gkd_api.cu).
 """
 import ctypes as C
 import os
