@@ -128,6 +128,7 @@ struct gkd_ctx {
     DevBuf join_rows, join_err;
     DevBuf hit_a, hit_b, sel_cta;  // selection epilogues: hit ids / positions (nearest: ref_pos, n_found), tile offsets + total
     DevBuf nn_pos, nn_inter, nn_dist, nn_found;  // accumulating nearest selection: per-target lists of one call
+    DevBuf uf_parent;  // cluster selection: the union-find forest of one call and its root counter
     int isect_algo = 0;  // GKD_ISECT_ALGO: 0 = choose per call, 1 = bucket merge only, 2 = block join whenever it applies
     bool use_msd = true;  // GKD_SORT_ALGO=lsd pins the LSD path
     bool sets_dirty = true;
@@ -990,7 +991,7 @@ struct HostLists {
 
 // What a selection call wants instead of the dense outputs (run_pairs with sel == nullptr writes gkd_outputs).
 struct Selection {
-    bool within;          // true: pairs with dist <= max_dist (gkd_hits); false: k nearest (rows and / or absorb)
+    bool within;          // true: pairs with dist <= max_dist (gkd_hits); false: k nearest (rows and / or absorb) or clusters
     double max_dist;
     gkd_hits *hits;       // within: the caller's arrays; hits->n counts the hits so far and is the next write position
     uint32_t a_base;      // RECT: position in the caller's q of the first query row of this call
@@ -1004,6 +1005,9 @@ struct Selection {
     bool absorb;          // nearest: merge the call into the per-target lists c->nn_* (UPPER: both ends of every pair;
                           // RECT: each reference's nearest queries), or into host_lists when the pairs are completed
     HostLists *host_lists;  // on the host (GKD_AMBIG_LITERAL; nullptr otherwise)
+    bool cluster;         // link the pairs within max_dist in the forest c->uf_parent (RECT: reference column j is node
+    uint32_t b_base;      // b_base + j, query row r is node a_base + r), or in host_forest when the pairs are completed
+    HostForest *host_forest;  // on the host (GKD_AMBIG_LITERAL; nullptr otherwise)
 };
 
 // GKD_AMBIG_LITERAL: the chunk's pairs were completed on the host (inter / dist of pairs done .. done+cnt), so the
@@ -1022,6 +1026,19 @@ void host_select(const HostPairs &hp, const Selection &sel, uint64_t done, uint6
             if (h.b) h.b[at] = b;
             if (h.inter) h.inter[at] = inter[t];
             if (h.dist) h.dist[at] = dist[t];
+        }
+        return;
+    }
+    if (sel.cluster) {  // the rule of k_cluster_link
+        for (uint64_t t = 0; t < cnt; t++) {
+            if (!(dist[t] <= sel.max_dist)) continue;
+            if (hp.mode == PAIRS_RECT) {
+                sel.host_forest->link(sel.a_base + (uint32_t)((done + t) / hp.nb), sel.b_base + (uint32_t)((done + t) % hp.nb));
+            } else {
+                uint32_t a, b;
+                host_pair_ids(hp, done + t, a, b);
+                sel.host_forest->link(a, b);
+            }
         }
         return;
     }
@@ -1064,7 +1081,8 @@ constexpr int SELECT_REDO = 1;  // select_chunk: a join table overflowed; nothin
 
 // The selection epilogue of one chunk whose kernel-4 launches are queued: launches the within or nearest selection,
 // then copies back only the hits (within: plus the chunk's 8-byte hit total) or the rows' best lists (nearest).  The
-// absorb form merges the chunk into the device lists instead, which are copied once by the caller (lists_finish).
+// absorb form merges the chunk into the device lists instead, which are copied once by the caller (lists_finish), and
+// the cluster form links it into the device forest, copied once by forest_finish.
 // The hit total and the join overflow flag are read before anything is copied, so a chunk that has to be redone by
 // the merge kernel appends nothing.
 int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const Selection &sel, uint64_t cnt, bool need_pal,
@@ -1115,6 +1133,14 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         nvtxRangePop();
         c->m.launches++;
     }
+    if (sel.cluster) {
+        // like absorb: the forest outlives this chunk, so the kernel itself skips a chunk whose join overflowed
+        nvtxRangePushA("gkd kernel 5: cluster link");
+        CK(launch_cluster_link(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.a_base, sel.b_base,
+                               use_join ? (const uint32_t *)c->join_err.p : nullptr, (uint32_t *)c->uf_parent.p, c->stream));
+        nvtxRangePop();
+        c->m.launches++;
+    }
     if (!sel.within) CK(cudaEventRecord(c->ev[7], c->stream));
     CK(cudaStreamSynchronize(c->stream));
     if (join_err) return SELECT_REDO;
@@ -1122,7 +1148,7 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         void *dst;
         const void *src;
         uint64_t bytes;
-    } copies[4] = {};  // absorb only: nothing leaves the device before the end of the call
+    } copies[4] = {};  // absorb and cluster: nothing leaves the device before the end of the call
     if (sel.within) {
         const gkd_hits &h = *sel.hits;
         const uint64_t w = std::min<uint64_t>(chunk_hits, wcap);
@@ -1602,7 +1628,7 @@ int gkd_destroy(gkd_ctx *c) {
                       &c->d_cb, &c->ids_a, &c->ids_b, &c->work_counter, &c->sk_cand, &c->sk_misc, &c->sk_sig,
                       &c->sk_len, &c->sk_out, &c->msd_genomes, &c->msd_bins32, &c->msd_bins64, &c->msd_gstat,
                       &c->gr_reps, &c->gr_flags, &c->join_rows, &c->join_err, &c->hit_a, &c->hit_b, &c->sel_cta, &c->nn_pos, &c->nn_inter,
-                      &c->nn_dist, &c->nn_found};
+                      &c->nn_dist, &c->nn_found, &c->uf_parent};
     for (DevBuf *b : bufs)
         if (b->p) cudaFreeAsync(b->p, c->stream);
     cudaStreamSynchronize(c->stream);
@@ -2416,6 +2442,109 @@ int gkd_all_vs_all_nearest(gkd_ctx *c, uint32_t n, uint32_t k, double max_dist, 
     HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
     if ((rc = run_pairs(c, hp, gkd_outputs{}, &sel))) return rc;
     return lists_finish(c, n, k, hl.get(), *out);
+    ABI_GUARD_END(c)
+}
+
+// ---- single-linkage clusters ----------------------------------------------------------------------------------
+// the forest of one cluster call (k_cluster_link): every node its own root
+static int forest_begin(gkd_ctx *c, uint32_t nodes) {
+    const int rc = ensure(c, c->uf_parent, ((uint64_t)nodes + 1) * 4);
+    if (rc) return rc;
+    CK(launch_cluster_init((uint32_t *)c->uf_parent.p, nodes, c->stream));
+    c->m.launches++;
+    return GKD_OK;
+}
+
+// The labels to the caller, once, at the end of the call: nodes [0, na) to a_out and [na, nodes) to b_out (either may
+// be NULL).  With hf (GKD_AMBIG_LITERAL, host outputs) the launches that ran on the device are merged into the host
+// forest first: every node is linked to its device label, which carries all of the device links' connectivity.
+static int forest_finish(gkd_ctx *c, uint32_t nodes, HostForest *hf, uint32_t *a_out, uint32_t na, uint32_t *b_out,
+                         uint32_t *n_clusters) {
+    uint32_t *parent = (uint32_t *)c->uf_parent.p;
+    CK(cudaEventRecord(c->ev[6], c->stream));
+    CK(launch_cluster_flatten(parent, nodes, c->stream));
+    CK(cudaEventRecord(c->ev[7], c->stream));
+    c->m.launches++;
+    uint32_t roots = 0;
+    if (!hf) {
+        const uint32_t nb = nodes - na;
+        if (a_out && na) CK(cudaMemcpyAsync(a_out, parent, (uint64_t)na * 4, cudaMemcpyDefault, c->stream));
+        if (b_out && nb) CK(cudaMemcpyAsync(b_out, parent + na, (uint64_t)nb * 4, cudaMemcpyDefault, c->stream));
+        CK(cudaMemcpyAsync(&roots, parent + nodes, 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += (a_out ? (uint64_t)na * 4 : 0) + (b_out ? (uint64_t)nb * 4 : 0) + 4;
+    } else {
+        std::vector<uint32_t> dev(nodes);
+        CK(cudaMemcpyAsync(dev.data(), parent, (uint64_t)nodes * 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += (uint64_t)nodes * 4;
+        for (uint32_t x = 0; x < nodes; x++)
+            if (dev[x] != x) hf->link(x, dev[x]);
+        for (uint32_t x = 0; x < nodes; x++) {
+            const uint32_t r = hf->find(x);
+            roots += r == x ? 1u : 0u;
+            if (x < na && a_out) a_out[x] = r;
+            if (x >= na && b_out) b_out[x - na] = r;
+        }
+    }
+    c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+    if (n_clusters) *n_clusters = roots;
+    return GKD_OK;
+}
+
+int gkd_all_vs_all_clusters(gkd_ctx *c, uint32_t n, double max_dist, uint32_t *label, uint32_t *n_clusters) {
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_clusters: max_dist is NaN");
+    if (!label) return fail(c, GKD_EINVAL, "gkd_all_vs_all_clusters: null label");
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "clusters over %u sets but only %zu exist", n, c->genomes.size());
+    const void *ps[1] = {label};
+    int rc = hits_host_ok(c, ps, 1);
+    if (rc) return rc;
+    c->m.pairs = 0;
+    if (n_clusters) *n_clusters = 0;
+    if (n == 0) return GKD_OK;
+    ABI_GUARD_BEGIN
+    Selection sel{};
+    sel.within = false;
+    sel.max_dist = max_dist;
+    sel.cluster = true;
+    std::unique_ptr<HostForest> hf;
+    if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hf.reset(new HostForest(n));
+    sel.host_forest = hf.get();
+    if ((rc = forest_begin(c, n))) return rc;
+    HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
+    if ((rc = run_pairs(c, hp, gkd_outputs{}, &sel))) return rc;
+    return forest_finish(c, n, hf.get(), label, n, nullptr, n_clusters);
+    ABI_GUARD_END(c)
+}
+
+int gkd_query_vs_ref_clusters(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, double max_dist,
+                              uint32_t *q_label, uint32_t *r_label) {
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: max_dist is NaN");
+    if (!q_label && !r_label) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: both outputs are NULL");
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: null id array");
+    if ((uint64_t)nq + nr >= 0xFFFFFFFFull) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: %u + %u nodes", nq, nr);
+    const void *ps[2] = {q_label, r_label};
+    int rc = hits_host_ok(c, ps, 2);
+    if (rc) return rc;
+    c->m.pairs = 0;
+    const uint32_t nodes = nq + nr;
+    if (nodes == 0) return GKD_OK;
+    ABI_GUARD_BEGIN
+    Selection sel{};
+    sel.within = false;
+    sel.max_dist = max_dist;
+    sel.cluster = true;
+    sel.b_base = nq;
+    std::unique_ptr<HostForest> hf;
+    if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hf.reset(new HostForest(nodes));
+    sel.host_forest = hf.get();
+    if ((rc = forest_begin(c, nodes))) return rc;
+    if (nq && nr && (rc = rect_selection(c, q, nq, r, nr, sel))) return rc;
+    return forest_finish(c, nodes, hf.get(), q_label, nq, r_label, nullptr);
     ABI_GUARD_END(c)
 }
 

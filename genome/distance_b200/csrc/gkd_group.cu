@@ -6,7 +6,8 @@
 // FASTA file.  The pair matrix shards with no reduction (SURVEY section 8e): member x owns its diagonal
 // block and the blocks (x, (x+s) mod R), s = 1..R/2 (the half-way block of an even ring is split between
 // its two members), exactly the schedule of genome/distance_b200/sharding.py (the one-process-per-GPU
-// torch.distributed layer); here the transport is a peer copy instead of NCCL send/recv.
+// torch.distributed layer); here the transport is a peer copy instead of NCCL send/recv.  The cluster form also
+// uses the host union-find of gkd_internal.cuh.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -19,6 +20,7 @@
 #include <vector>
 
 #include "gkd.h"
+#include "gkd_internal.cuh"  // HostForest
 
 // host FASTA scanner (fasta.cpp)
 struct FastaPiece {
@@ -176,21 +178,32 @@ struct NearestSink {
     }
 };
 
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest);
+// gkd_group_all_vs_all_clusters: a member's links (global p, global label[p]) for every node p of its calls with
+// label[p] != p.  A call's labels carry all the connectivity of its links, and the ring computes every pair once, so
+// the union of these links over all members has the components of the whole triangle.
+struct ClusterSink {
+    double max_dist;
+    std::vector<std::pair<uint32_t, uint32_t>> links;
+};
+
+void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
+                 ClusterSink *clusters);
 
 // the ring of one member (runs on its own host thread; no exception may leave the thread).  With `within` the
 // member selects on its device and collects its hits there instead of scattering dense blocks into inter / dist;
-// with `nearest` it collects partial k-nearest lists.
-void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest) {
+// with `nearest` it collects partial k-nearest lists, with `clusters` the links of its calls' components.
+void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
+                       ClusterSink *clusters) {
     try {
-        member_ring(g, x, inter, dist, within, nearest);
+        member_ring(g, x, inter, dist, within, nearest, clusters);
     } catch (const std::exception &ex) {
         g->members[x].rc = GKD_ENOMEM;
         g->members[x].err = ex.what();
     }
 }
 
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest) {
+void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
+                 ClusterSink *clusters) {
     Member &M = g->members[x];
     const uint32_t R = (uint32_t)g->members.size();
     const uint64_t N = g->n_genomes;
@@ -296,8 +309,14 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
         nf.resize(rows_);
         return gkd_neighbors{pos.data(), in.data(), d.data(), nf.data()};
     };
+    std::vector<uint32_t> ql, rl;  // clusters: the labels of one call
     // diagonal block (runs while the first group is in flight)
-    if (m >= 2 && nearest) {
+    if (m >= 2 && clusters) {
+        ql.resize(m);
+        MGK(gkd_all_vs_all_clusters(M.ctx, m, clusters->max_dist, ql.data(), nullptr));
+        for (uint32_t i = 0; i < m; i++)
+            if (ql[i] != i) clusters->links.push_back({M.global_ids[i], M.global_ids[ql[i]]});
+    } else if (m >= 2 && nearest) {
         const uint32_t k = nearest->k;
         const gkd_neighbors nb = side(m, qpos, qi, qd, qn);
         MGK(gkd_all_vs_all_nearest(M.ctx, m, k, nearest->max_dist, &nb));
@@ -343,6 +362,19 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
                 cols.push_back(first + c);
                 col_gid.push_back(g->members[S.src].global_ids[S.p.first + c]);
             }
+        }
+        if (clusters) {
+            const uint32_t nr = (uint32_t)rows.size(), nc = (uint32_t)cols.size();
+            auto gid = [&](uint32_t node) { return node < nr ? M.global_ids[rows[node]] : col_gid[node - nr]; };
+            ql.resize(nr);
+            rl.resize(nc);
+            MGK(gkd_query_vs_ref_clusters(M.ctx, rows.data(), nr, cols.data(), nc, clusters->max_dist, ql.data(), rl.data()));
+            for (uint32_t p = 0; p < nr; p++)
+                if (ql[p] != p) clusters->links.push_back({gid(p), gid(ql[p])});
+            for (uint32_t c = 0; c < nc; c++)
+                if (rl[c] != nr + c) clusters->links.push_back({col_gid[c], gid(rl[c])});
+            MGK(gkd_truncate(M.ctx, m));
+            continue;
         }
         if (nearest) {
             // The lists break ties by position in the call, and a group of panels may span peers (x+1)%R, (x+2)%R, ...,
@@ -597,7 +629,7 @@ int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist) {
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr, nullptr);
+            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr, nullptr, nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -620,7 +652,7 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x], nullptr);
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x], nullptr, nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -659,7 +691,7 @@ int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, cons
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, &sinks[x]);
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, &sinks[x], nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -686,6 +718,38 @@ int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, cons
         return GKD_OK;
     } catch (const std::exception &ex) {
         return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_nearest: %s", ex.what());
+    }
+}
+
+int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label, uint32_t *n_clusters) {
+    if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_clusters: max_dist is NaN");
+    if (!label) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_clusters: null label");
+    if (!g) return GKD_EINVAL;
+    try {
+        for (auto &M : g->members)
+            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
+        std::vector<ClusterSink> sinks(g->members.size(), ClusterSink{max_dist, {}});
+        std::vector<std::thread> threads;
+        for (uint32_t x = 0; x < g->members.size(); x++) {
+            g->members[x].rc = GKD_OK;
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, nullptr, &sinks[x]);
+        }
+        for (auto &t : threads) t.join();
+        for (size_t i = 0; i < g->members.size(); i++)
+            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        const uint32_t N = g->n_genomes;
+        gkd::HostForest forest(N);
+        for (auto &s : sinks)
+            for (const auto &l : s.links) forest.link(l.first, l.second);
+        uint32_t roots = 0;
+        for (uint32_t i = 0; i < N; i++) {
+            label[i] = forest.find(i);
+            roots += label[i] == i ? 1u : 0u;
+        }
+        if (n_clusters) *n_clusters = roots;
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_clusters: %s", ex.what());
     }
 }
 

@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <vector>
+
 #include "gkd.h"
 
 namespace gkd {
@@ -312,6 +314,34 @@ cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t 
 cudaError_t launch_nearest_absorb(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
                                   int both_strands, double max_dist, uint32_t k, int exclude_self, uint32_t a_base,
                                   const uint32_t *join_err, NearestOut state, cudaStream_t s);
+// Single-linkage clusters: a union-find forest parent[0, n) in device memory (invariant parent[x] <= x) followed by
+// one root counter parent[n].  init: parent[x] = x and the counter 0.  link: every pair within max_dist joins its two
+// nodes (UPPER: the set ids; RECT: a_base + query row and b_base + reference column); nothing when join_err (may be
+// nullptr) reads nonzero on the stream.  flatten: parent[x] = the smallest node of x's cluster (a read-only walk;
+// only thread x writes parent[x]), counter = clusters.
+cudaError_t launch_cluster_init(uint32_t *parent, uint32_t n, cudaStream_t s);
+cudaError_t launch_cluster_link(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
+                                int both_strands, double max_dist, uint32_t a_base, uint32_t b_base, const uint32_t *join_err,
+                                uint32_t *parent, cudaStream_t s);
+cudaError_t launch_cluster_flatten(uint32_t *parent, uint32_t n, cudaStream_t s);
+// The same forest on the host (GKD_AMBIG_LITERAL pairs, and the group's merge of its members' components): a link
+// hooks the larger root under the smaller, so find() is the smallest node of the cluster.
+struct HostForest {
+    std::vector<uint32_t> parent;
+    explicit HostForest(uint32_t n) : parent(n) {
+        for (uint32_t x = 0; x < n; x++) parent[x] = x;
+    }
+    uint32_t find(uint32_t x) {
+        while (parent[x] != x) x = parent[x] = parent[parent[x]];
+        return x;
+    }
+    void link(uint32_t a, uint32_t b) {
+        a = find(a);
+        b = find(b);
+        if (a < b) parent[b] = a;
+        else if (b < a) parent[a] = b;
+    }
+};
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless
 // some representative is within max_dist; clears the counts it consumed
 cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *n_reps, uint32_t cand, uint32_t visit,

@@ -137,6 +137,8 @@ const std::vector<OptSpec> FASTA_OPTS = {
     {{"--maxDist"}, true, "report only the pairs with distance <= this (additive option; selected on the GPU)"},
     {{"--nearest"}, true, "report each record's N (1..256) nearest other records within --maxDist (default 1.0), in "
                           "input order, nearest first; a pair can appear twice, once from each end (additive option)"},
+    {{"--clusters"}, false, "report each record's single-linkage cluster at --maxDist: the label of the cluster's first "
+                            "record (additive option; needs --maxDist)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
@@ -191,6 +193,27 @@ uint64_t writeNeighbors(std::ostream &writer, size_t n, uint32_t k, const uint32
     return lines;
 }
 
+// the lines of `fastaDist --clusters`: every record in input order with the label of its cluster's first record
+template <class LabelFn, class CommentFn>
+uint32_t writeClusters(std::ostream &writer, size_t n, const uint32_t *cluster, LabelFn label, CommentFn comment) {
+    std::string line;
+    uint32_t clusters = 0;
+    writer << "seq\tname\tcluster\n";
+    for (size_t i = 0; i < n; i++) {
+        line.clear();
+        line += label(i);
+        line += '\t';
+        line += comment(i);
+        line += '\t';
+        line += label(cluster[i]);
+        line += '\n';
+        writer << line;
+        clusters += cluster[i] == i ? 1u : 0u;
+    }
+    writer.flush();
+    return clusters;
+}
+
 // pairs per gkd_all_vs_all_range_within call of `fastaDist --maxDist`: host memory stays O(range), not O(n^2)
 constexpr uint64_t WITHIN_RANGE = 64ull << 20;
 
@@ -235,6 +258,10 @@ int fastaDist(const std::vector<std::string> &args) {
     const int nearest = p.values.count("--nearest") ? toInt("--nearest", p.values["--nearest"]) : 0;
     if (p.values.count("--nearest") && (nearest < 1 || nearest > 256))
         throw ParseFailureException("Number of neighbors must be between 1 and 256.");
+    // single linkage at the default 1.0 would put every record in one cluster
+    const bool clusters = p.values.count("--clusters") > 0;
+    if (clusters && !within) throw ParseFailureException("--clusters needs --maxDist.");
+    if (clusters && nearest) throw ParseFailureException("--clusters and --nearest cannot be combined.");
     const char *typeName = seqType == KmerType::DNA ? "DNA" : (seqType == KmerType::RNA ? "RNA" : "PROT");
     if (inFile.empty()) logInfo(std::string("Reading ") + typeName + " sequences from the standard input.");
     else if (!readable(inFile)) throw IOException("Input file " + inFile + " is not found or unreadable.");
@@ -285,10 +312,20 @@ int fastaDist(const std::vector<std::string> &args) {
         uint32_t n = 0;
         gcheck(gkd_group_add_fasta_file(grp, inFile.c_str(), &n));
         logInfo(std::to_string(n) + " sequences read from input.");
-        writer << "seq1\tname1\tseq2\tname2\tdistance\n";
+        if (!clusters) writer << "seq1\tname1\tseq2\tname2\tdistance\n";
         gcheck(gkd_group_build(grp));
         logInfo(std::to_string(n) + " sequences cached on " + std::to_string(gpus) + " GPUs. Computing distances.");
         const uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
+        if (clusters) {
+            std::vector<uint32_t> label(n);
+            gcheck(gkd_group_all_vs_all_clusters(grp, maxDist, label.data(), nullptr));
+            const uint32_t found = writeClusters(writer, n, label.data(), [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
+                                                 [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
+            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(found) + " clusters at distance " +
+                    javaDouble(maxDist) + ".");
+            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
+            return 0;
+        }
         if (nearest) {
             const uint32_t k = (uint32_t)nearest;
             std::vector<uint32_t> pos((size_t)n * k), found(n);
@@ -338,9 +375,21 @@ int fastaDist(const std::vector<std::string> &args) {
     logInfo(std::to_string(seqs.size()) + " sequences read from input.");
     // runReporter (:134-165): the batch cache and the per-row parallel streams are what the engine
     // replaces; every pair i<j is computed in one batched launch and printed in list order
-    writer << "seq1\tname1\tseq2\tname2\tdistance\n";
+    if (!clusters) writer << "seq1\tname1\tseq2\tname2\tdistance\n";
     engine.build();
     logInfo(std::to_string(seqs.size()) + " sequences cached. Computing distances.");
+    if (clusters) {
+        // each pair i < j is intersected once and linked on the GPU; only the n labels leave it
+        const size_t n = seqs.size();
+        std::vector<uint32_t> label(n);
+        engine.check(gkd_all_vs_all_clusters(engine.raw(), (uint32_t)n, maxDist, label.data(), nullptr));
+        const uint32_t found = writeClusters(writer, n, label.data(), [&](size_t i) { return seqs[i].getGenomeId(); },
+                                             [&](size_t i) { return seqs[i].getGenomeName(); });
+        logInfo(std::to_string(n < 2 ? 0 : n * (n - 1) / 2) + " pairs computed in 1 batches, " + std::to_string(found) +
+                " clusters at distance " + javaDouble(maxDist) + ".");
+        writeMetrics(metricsFile, "fastaDist", engine.raw(), n < 2 ? 0 : n * (n - 1) / 2, 1);
+        return 0;
+    }
     if (nearest) {
         // each pair i < j is intersected once and offered to both rows; only the n*k lists leave the GPU
         const uint32_t k = (uint32_t)nearest;

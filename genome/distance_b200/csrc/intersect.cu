@@ -33,6 +33,8 @@
 // ~4.25 per key (low word + table share), see DESIGN.md section 4 for the measured limiter.
 #include <cstdlib>
 
+#include <cuda/atomic>
+
 #include "gkd_internal.cuh"
 
 namespace gkd {
@@ -861,6 +863,118 @@ cudaError_t launch_nearest_absorb(const SetDesc *sets, PairSource src, const uin
     }
     k_nearest_absorb<<<targets, NEAR_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, k, exclude_self,
                                                       i0, i1, a_base, join_err, state);
+    return cudaGetLastError();
+}
+
+// Clusters, accumulating form: single linkage at max_dist as a union-find forest `parent` over the call's nodes in HBM,
+// kept across the chunks and launches of one call like the nearest lists.  Invariant parent[x] <= x, so a root is the
+// smallest node of its tree and the flattened forest is the label the API returns.
+//   link:  find both roots, hook the larger under the smaller with a CAS that succeeds only while it is still a root;
+//          a failed CAS means another thread hooked that root, so the loop resumes from the value it returned.
+//   find:  path halving; its stores only ever write a smaller ancestor of the same tree (a non-root stays a
+//          non-root, a root is only written by the CAS), so racing finds and links keep the forest valid.
+// Loads go through device-scope relaxed atomics: a plain load may be served by a stale L1 line of another SM's write.
+// No thread waits for another, so every loop ends.  Like k_nearest_absorb, a launch whose block join overflowed links
+// nothing (the chunk is redone by the merge kernel): an overflowed attempt could only undercount, but this way every
+// link is decided on final counts.
+constexpr int CLUSTER_THREADS = 256;
+
+__device__ __forceinline__ uint32_t uf_load(uint32_t *p) {
+    return cuda::atomic_ref<uint32_t, cuda::thread_scope_device>(*p).load(cuda::memory_order_relaxed);
+}
+
+__device__ __forceinline__ void uf_store(uint32_t *p, uint32_t v) {
+    cuda::atomic_ref<uint32_t, cuda::thread_scope_device>(*p).store(v, cuda::memory_order_relaxed);
+}
+
+__device__ __forceinline__ uint32_t uf_find(uint32_t *__restrict__ parent, uint32_t x) {
+    uint32_t p = uf_load(parent + x);
+    while (p != x) {
+        const uint32_t gp = uf_load(parent + p);
+        if (gp != p) uf_store(parent + x, gp);
+        x = gp;
+        p = uf_load(parent + x);
+    }
+    return x;
+}
+
+__device__ __forceinline__ void uf_union(uint32_t *__restrict__ parent, uint32_t a, uint32_t b) {
+    a = uf_find(parent, a);
+    b = uf_find(parent, b);
+    while (a != b) {
+        const uint32_t hi = max(a, b), lo = min(a, b);
+        const uint32_t old = atomicCAS(parent + hi, hi, lo);
+        if (old == hi) return;
+        a = uf_find(parent, old);
+        b = uf_find(parent, lo);
+    }
+}
+
+__global__ void __launch_bounds__(CLUSTER_THREADS)
+    k_cluster_link(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
+                   const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t a_base, uint32_t b_base,
+                   const uint32_t *__restrict__ join_err, uint32_t *__restrict__ parent) {
+    if (join_err && *join_err) return;
+    const bool rect = src.mode == PAIRS_RECT;
+    for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < src.count; t += (uint64_t)gridDim.x * blockDim.x) {
+        uint32_t ida, idb;
+        decode_pair(src, t, ida, idb);
+        uint64_t I, sa, sb;
+        double d;
+        pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+        if (!(d <= max_dist)) continue;
+        if (rect) uf_union(parent, a_base + (uint32_t)(t / src.n), b_base + (uint32_t)(t % src.n));
+        else uf_union(parent, ida, idb);
+    }
+}
+
+// the root of x without writing: every value read is an ancestor of x or its root, so the walk ends at the root
+__device__ __forceinline__ uint32_t uf_root(uint32_t *__restrict__ parent, uint32_t x) {
+    for (uint32_t p = uf_load(parent + x); p != x; p = uf_load(parent + x)) x = p;
+    return x;
+}
+
+// every node to its root, *n_roots += roots.  The labels live in `parent`, so only thread x writes parent[x], and it
+// writes its root: a path-halving find here could store a stale ancestor over a node's label after that node's own
+// thread had written the root.
+__global__ void __launch_bounds__(CLUSTER_THREADS) k_cluster_flatten(uint32_t *__restrict__ parent, uint32_t n, uint32_t *__restrict__ n_roots) {
+    const uint32_t x = blockIdx.x * blockDim.x + threadIdx.x;
+    bool root = false;
+    if (x < n) {
+        const uint32_t r = uf_root(parent, x);
+        root = r == x;
+        if (!root) uf_store(parent + x, r);
+    }
+    const uint32_t roots = __popc(__ballot_sync(0xffffffffu, root));
+    if ((threadIdx.x & 31) == 0 && roots) atomicAdd(n_roots, roots);
+}
+
+__global__ void __launch_bounds__(CLUSTER_THREADS) k_cluster_init(uint32_t *__restrict__ parent, uint32_t n) {
+    const uint32_t x = blockIdx.x * blockDim.x + threadIdx.x;
+    if (x < n) parent[x] = x;
+    if (x == n) parent[x] = 0;  // the root counter of k_cluster_flatten
+}
+
+cudaError_t launch_cluster_init(uint32_t *parent, uint32_t n, cudaStream_t s) {
+    k_cluster_init<<<(unsigned)(((uint64_t)n + CLUSTER_THREADS) / CLUSTER_THREADS), CLUSTER_THREADS, 0, s>>>(parent, n);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_cluster_link(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
+                                int both_strands, double max_dist, uint32_t a_base, uint32_t b_base, const uint32_t *join_err,
+                                uint32_t *parent, cudaStream_t s) {
+    if (src.count == 0) return cudaSuccess;
+    const uint64_t need = (src.count + CLUSTER_THREADS - 1) / CLUSTER_THREADS;  // grid-stride beyond 8192 CTAs
+    const uint64_t blocks = need < 8192 ? need : 8192;
+    k_cluster_link<<<(unsigned)blocks, CLUSTER_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, a_base,
+                                                                 b_base, join_err, parent);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_cluster_flatten(uint32_t *parent, uint32_t n, cudaStream_t s) {
+    if (n == 0) return cudaSuccess;
+    k_cluster_flatten<<<(unsigned)(((uint64_t)n + CLUSTER_THREADS - 1) / CLUSTER_THREADS), CLUSTER_THREADS, 0, s>>>(parent, n,
+                                                                                                                  parent + n);
     return cudaGetLastError();
 }
 

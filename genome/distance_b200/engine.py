@@ -333,6 +333,24 @@ class Engine:
         self._ck(self._L.gkd_all_vs_all_nearest(self._h, n, int(k), float(max_dist), C.byref(nb)))
         return out
 
+    def all_vs_all_clusters(self, max_dist: float, n: int = None):
+        """(labels, n_clusters): single-linkage clusters of the first n sets (default: all) at max_dist, i.e. the
+        connected components of the pairs with distance <= max_dist; labels[i] (uint32) is the smallest id of i's
+        cluster.  Every pair is intersected once and only the labels leave the device"""
+        n = len(self) if n is None else int(n)
+        labels, count = np.empty(n, dtype=np.uint32), C.c_uint32()
+        self._ck(self._L.gkd_all_vs_all_clusters(self._h, n, float(max_dist), labels.ctypes.data, C.byref(count)))
+        return labels, count.value
+
+    def query_vs_ref_clusters(self, q: Sequence[int], r: Sequence[int], max_dist: float):
+        """(q_label, r_label): the components of the bipartite graph of the query x reference pairs within max_dist;
+        node i is q[i] and node len(q) + j is r[j], and each label is the smallest node of its component"""
+        qa, ra = np.ascontiguousarray(q, dtype=np.uint32), np.ascontiguousarray(r, dtype=np.uint32)
+        ql, rl = np.empty(qa.size, dtype=np.uint32), np.empty(ra.size, dtype=np.uint32)
+        self._ck(self._L.gkd_query_vs_ref_clusters(self._h, qa.ctypes.data, qa.size, ra.ctypes.data, ra.size,
+                                                   float(max_dist), ql.ctypes.data, rl.ctypes.data))
+        return ql, rl
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -509,3 +527,9 @@ class Group:
         out, nb = _neighbors(len(self), k)
         self._ck(self._L.gkd_group_all_vs_all_nearest(self._h, int(k), float(max_dist), C.byref(nb)))
         return out
+
+    def all_vs_all_clusters(self, max_dist: float):
+        """(labels, n_clusters) over all global ids: the single-context Engine.all_vs_all_clusters result"""
+        labels, count = np.empty(len(self), dtype=np.uint32), C.c_uint32()
+        self._ck(self._L.gkd_group_all_vs_all_clusters(self._h, float(max_dist), labels.ctypes.data, C.byref(count)))
+        return labels, count.value

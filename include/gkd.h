@@ -269,6 +269,18 @@ int gkd_all_vs_all_nearest(gkd_ctx *ctx, uint32_t n, uint32_t k, double max_dist
 int gkd_query_vs_ref_nearest_ex(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
                                 double max_dist, int exclude_self, const gkd_neighbors *q_side, const gkd_neighbors *r_side);
 
+/* Single-linkage clusters of the first n sets at max_dist: i and j are in one cluster when a chain of pairs, each with
+ * distance <= max_dist (the comparison of gkd_*_within), joins them.  label[i] = the smallest id of i's cluster;
+ * *n_clusters (may be NULL; host memory) = number of clusters.  Every pair i < j is intersected once; only the labels
+ * leave the device.  label may be host or device memory (host only for GKD_AMBIG_LITERAL).  A negative max_dist gives
+ * singletons. */
+int gkd_all_vs_all_clusters(gkd_ctx *ctx, uint32_t n, double max_dist, uint32_t *label, uint32_t *n_clusters);
+/* The components of one query x reference pass: node i is q[i], node nq + j is r[j] (positions, also when an id is on
+ * both sides); the links are the pairs (q[i], r[j]) within max_dist.  q_label[i] / r_label[j] = the smallest node of the
+ * component.  Either output may be NULL, not both; host or device memory as for gkd_all_vs_all_clusters. */
+int gkd_query_vs_ref_clusters(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr,
+                              double max_dist, uint32_t *q_label, uint32_t *r_label);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -302,6 +314,10 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out);
  * selects its diagonal block and both directions of its ring blocks on its own device; the host merges the partial
  * lists of every id.  The arrays of out are host memory, N*k (n_found: N). */
 int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, const gkd_neighbors *out);
+/* gkd_all_vs_all_clusters over all global ids; equal to one context's labels.  Every member clusters its diagonal block
+ * and each ring block on its own device; the host joins the components of every call (O(rows + columns) per call).
+ * label is host memory (N entries); *n_clusters may be NULL. */
+int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label, uint32_t *n_clusters);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

@@ -237,3 +237,13 @@ JNIEXPORT jint JNICALL FN(allVsAllNearest)(JNIEnv *env, jclass c, jlong h, jint 
     if (p) (*env)->ReleaseIntArrayElements(env, pos, p, 0);
     return rc;
 }
+
+/* single-linkage clusters of the first n sets at maxDist: label holds n entries, the smallest id of each set's cluster */
+JNIEXPORT jint JNICALL FN(allVsAllClusters)(JNIEnv *env, jclass c, jlong h, jint n, jdouble maxDist, jintArray label) {
+    (void)c;
+    if (!label || n < 0 || (*env)->GetArrayLength(env, label) < n) return GKD_EINVAL;
+    jint *l = (*env)->GetIntArrayElements(env, label, NULL);
+    int rc = l ? gkd_all_vs_all_clusters(CTX(h), (uint32_t)n, maxDist, (uint32_t *)l, NULL) : GKD_ENOMEM;
+    if (l) (*env)->ReleaseIntArrayElements(env, label, l, 0);
+    return rc;
+}

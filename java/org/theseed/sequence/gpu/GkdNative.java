@@ -47,6 +47,9 @@ final class GkdNative {
      *  every pair is intersected once: pos and dist (length n * k, row-major; unused slots -1 and -1.0), nFound
      *  (length n) */
     static native int allVsAllNearest(long ctx, int n, int k, double maxDist, int[] pos, double[] dist, int[] nFound);
+    /** single-linkage clusters of the first n sets at maxDist: label (length n) receives the smallest id of each set's
+     *  cluster */
+    static native int allVsAllClusters(long ctx, int n, double maxDist, int[] label);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

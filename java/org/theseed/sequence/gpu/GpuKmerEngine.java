@@ -185,6 +185,16 @@ public class GpuKmerEngine implements AutoCloseable {
         return found;
     }
 
+    /** single-linkage clusters of every set at maxDist (dereplication): two sets share a cluster when a chain of pairs,
+     *  each with distance &lt;= maxDist, joins them; label[i] is the smallest id of set i's cluster, so label[i] == i
+     *  marks a cluster's first member.  Every pair is intersected once and only the labels leave the GPU. */
+    public synchronized int[] allVsAllClusters(double maxDist) {
+        this.build();
+        int[] label = new int[this.size()];
+        check(GkdNative.allVsAllClusters(this.ctx, label.length, maxDist, label));
+        return label;
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
