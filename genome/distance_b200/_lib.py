@@ -83,6 +83,7 @@ SYMBOLS = {
     "gkd_group_all_vs_all_within": (_i32, [_vp, _dbl, C.POINTER(GkdHits)]),
     "gkd_group_all_vs_all_nearest": (_i32, [_vp, _u32, _dbl, C.POINTER(GkdNeighbors)]),
     "gkd_group_all_vs_all_clusters": (_i32, [_vp, _dbl, _vp, _pu32]),
+    "gkd_group_all_vs_all_linkage": (_i32, [_vp, _dbl, C.POINTER(GkdHits)]),
     "gkd_build_sets": (_i32, [_vp]),
     "gkd_set_size": (_i32, [_vp, _u32, _pu64, _pu64, _pu64]),
     "gkd_export_set": (_i32, [_vp, _u32, _vp, _u64, _pu64]),
@@ -111,6 +112,8 @@ SYMBOLS = {
     "gkd_all_vs_all_nearest": (_i32, [_vp, _u32, _u32, _dbl, C.POINTER(GkdNeighbors)]),
     "gkd_all_vs_all_clusters": (_i32, [_vp, _u32, _dbl, _vp, _pu32]),
     "gkd_query_vs_ref_clusters": (_i32, [_vp, _vp, _u32, _vp, _u32, _dbl, _vp, _vp]),
+    "gkd_all_vs_all_linkage": (_i32, [_vp, _u32, _dbl, C.POINTER(GkdHits)]),
+    "gkd_query_vs_ref_linkage": (_i32, [_vp, _vp, _u32, _vp, _u32, _dbl, _vp, _vp, C.POINTER(GkdHits)]),
     "gkd_hash_set": (_i32, [_vp, _u32, _u32, _i32, _vp, _pu32]),
     "gkd_sketch_distances": (_i32, [_vp, _u32, _i32, _vp, _vp, _u64, _vp]),
     "gkd_format_double": (_i32, [_dbl, C.c_char_p, C.c_size_t]),

@@ -129,6 +129,7 @@ struct gkd_ctx {
     DevBuf hit_a, hit_b, sel_cta;  // selection epilogues: hit ids / positions (nearest: ref_pos, n_found), tile offsets + total
     DevBuf nn_pos, nn_inter, nn_dist, nn_found;  // accumulating nearest selection: per-target lists of one call
     DevBuf uf_parent;  // cluster selection: the union-find forest of one call and its root counter
+    DevBuf lk_forest, lk_state;  // linkage selection: the spanning forest of one call and its Boruvka state
     int isect_algo = 0;  // GKD_ISECT_ALGO: 0 = choose per call, 1 = bucket merge only, 2 = block join whenever it applies
     bool use_msd = true;  // GKD_SORT_ALGO=lsd pins the LSD path
     bool sets_dirty = true;
@@ -989,6 +990,18 @@ struct HostLists {
     }
 };
 
+// One linkage call: the forest of its launches so far.  Node of a reported edge (a, b): a and b + b_off.
+struct LinkCall {
+    uint32_t nodes = 0, b_off = 0;
+    std::vector<uint32_t> key;   // key of every node (empty: the node itself); uploaded to c->lk_state when not empty
+    uint32_t n_dev = 0;          // edges of the device forest c->lk_forest
+    std::vector<LinkEdge> host;  // GKD_AMBIG_LITERAL: the forest of the pairs completed on the host
+    LinkEdge edge(uint32_t a, uint32_t b, uint64_t inter, double dist) const {
+        const uint32_t na = a, nb = b + b_off;
+        return link_edge(a, b, inter, dist, na, nb, key.empty() ? na : key[na], key.empty() ? nb : key[nb]);
+    }
+};
+
 // What a selection call wants instead of the dense outputs (run_pairs with sel == nullptr writes gkd_outputs).
 struct Selection {
     bool within;          // true: pairs with dist <= max_dist (gkd_hits); false: k nearest (rows and / or absorb) or clusters
@@ -1008,6 +1021,7 @@ struct Selection {
     bool cluster;         // link the pairs within max_dist in the forest c->uf_parent (RECT: reference column j is node
     uint32_t b_base;      // b_base + j, query row r is node a_base + r), or in host_forest when the pairs are completed
     HostForest *host_forest;  // on the host (GKD_AMBIG_LITERAL; nullptr otherwise)
+    LinkCall *link;       // linkage: replace the call's forest with MSF(forest u the chunk's pairs within max_dist)
 };
 
 // GKD_AMBIG_LITERAL: the chunk's pairs were completed on the host (inter / dist of pairs done .. done+cnt), so the
@@ -1040,6 +1054,18 @@ void host_select(const HostPairs &hp, const Selection &sel, uint64_t done, uint6
                 sel.host_forest->link(a, b);
             }
         }
+        return;
+    }
+    if (sel.link) {  // Kruskal on the host forest and the chunk's edges, in the order of k_link_edges
+        LinkCall &L = *sel.link;
+        for (uint64_t t = 0; t < cnt; t++) {
+            if (!(dist[t] <= sel.max_dist)) continue;
+            uint32_t a, b;
+            if (hp.mode == PAIRS_RECT) a = sel.a_base + (uint32_t)((done + t) / hp.nb), b = (uint32_t)((done + t) % hp.nb);
+            else host_pair_ids(hp, done + t, a, b);
+            L.host.push_back(L.edge(a, b, inter[t], dist[t]));
+        }
+        host_msf(L.host, L.nodes);
         return;
     }
     if (sel.absorb) {
@@ -1079,6 +1105,44 @@ void host_select(const HostPairs &hp, const Selection &sel, uint64_t done, uint6
 
 constexpr int SELECT_REDO = 1;  // select_chunk: a join table overflowed; nothing of the attempt was kept
 
+// Linkage, one chunk whose n_chunk edges are compacted at the front of hit_a / hit_b / d_inter / d_dist: the forest so
+// far is copied behind them and the Boruvka rounds replace it with MSF(forest u chunk).  Records ev[7] after the
+// rounds and reads the new forest's size (4 bytes).
+static int link_chunk(gkd_ctx *c, LinkCall &L, uint64_t n_chunk) {
+    if (n_chunk == 0) {  // the forest stands
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        return GKD_OK;
+    }
+    const uint32_t N = L.nodes;
+    uint64_t *fi = (uint64_t *)c->lk_forest.p;  // 24 B per node: inter, dist, a, b
+    double *fd = (double *)(fi + N);
+    uint32_t *fa = (uint32_t *)(fd + N), *fb = fa + N;
+    const uint64_t f = L.n_dev;
+    if (f) {
+        CK(cudaMemcpyAsync((uint32_t *)c->hit_a.p + n_chunk, fa, f * 4, cudaMemcpyDeviceToDevice, c->stream));
+        CK(cudaMemcpyAsync((uint32_t *)c->hit_b.p + n_chunk, fb, f * 4, cudaMemcpyDeviceToDevice, c->stream));
+        CK(cudaMemcpyAsync((uint64_t *)c->d_inter.p + n_chunk, fi, f * 8, cudaMemcpyDeviceToDevice, c->stream));
+        CK(cudaMemcpyAsync((double *)c->d_dist.p + n_chunk, fd, f * 8, cudaMemcpyDeviceToDevice, c->stream));
+    }
+    const LinkState st = link_state_at(c->lk_state.p, N);
+    const LinkGraph g{(const uint32_t *)c->hit_a.p, (const uint32_t *)c->hit_b.p, (const uint64_t *)c->d_inter.p,
+                      (const double *)c->d_dist.p, n_chunk + f, L.b_off, L.key.empty() ? nullptr : st.key};
+    if (g.n_edges >= LINK_NONE) return fail(c, GKD_EINVAL, "linkage: %llu edges in one pass", (unsigned long long)g.n_edges);
+    uint32_t rounds = 1;
+    while (rounds < LINK_MAX_ROUNDS && (1ull << rounds) < N) rounds++;
+    nvtxRangePushA("gkd kernel 5: linkage rounds");
+    CK(launch_link_rounds(g, st, LinkForest{fa, fb, fi, fd}, rounds, c->stream));
+    nvtxRangePop();
+    c->m.launches += 1 + 5 * rounds;
+    uint32_t n_forest = 0;
+    CK(cudaEventRecord(c->ev[7], c->stream));
+    CK(cudaMemcpyAsync(&n_forest, st.n_forest, 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    L.n_dev = n_forest;
+    return GKD_OK;
+}
+
 // The selection epilogue of one chunk whose kernel-4 launches are queued: launches the within or nearest selection,
 // then copies back only the hits (within: plus the chunk's 8-byte hit total) or the rows' best lists (nearest).  The
 // absorb form merges the chunk into the device lists instead, which are copied once by the caller (lists_finish), and
@@ -1111,6 +1175,20 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         c->m.launches += wcap ? 3 : 2;
         CK(cudaEventRecord(c->ev[7], c->stream));
         CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
+    } else if (sel.link) {
+        // every edge of the chunk within max_dist, with room behind them for the forest so far (link_chunk)
+        const uint64_t room = cnt + sel.link->nodes;
+        nctas = select_within_ctas(cnt);
+        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
+        if ((rc = ensure(c, c->hit_a, room * 4)) || (rc = ensure(c, c->hit_b, room * 4))) return rc;
+        if ((rc = ensure(c, c->d_inter, room * 8)) || (rc = ensure(c, c->d_dist, room * 8))) return rc;
+        const HitsOut ho{(uint32_t *)c->hit_a.p, (uint32_t *)c->hit_b.p, (uint64_t *)c->d_inter.p, (double *)c->d_dist.p};
+        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
+        nvtxRangePushA("gkd kernel 5: linkage edges");
+        CK(launch_select_within(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.a_base, cnt, ho, cta, cta + nctas, c->stream));
+        nvtxRangePop();
+        c->m.launches += 3;
+        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
     } else if (sel.rows) {
         const uint64_t slots = (uint64_t)hp.na * sel.k;
         if (sel.ref_pos && (rc = ensure(c, c->hit_a, slots * 4))) return rc;
@@ -1141,9 +1219,11 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         nvtxRangePop();
         c->m.launches++;
     }
-    if (!sel.within) CK(cudaEventRecord(c->ev[7], c->stream));
+    if (!sel.within && !sel.link) CK(cudaEventRecord(c->ev[7], c->stream));
     CK(cudaStreamSynchronize(c->stream));
     if (join_err) return SELECT_REDO;
+    // linkage: the forest outlives the chunk, so the rounds start only once the host has seen that the join held
+    if (sel.link && (rc = link_chunk(c, *sel.link, chunk_hits))) return rc;
     struct {
         void *dst;
         const void *src;
@@ -1163,7 +1243,7 @@ int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const S
         copies[2] = {sel.dist, c->d_dist.p, slots * 8};
         copies[3] = {sel.n_found, c->hit_b.p, (uint64_t)hp.na * 4};
     }
-    uint64_t d2h = sel.within ? 8 : 0;
+    uint64_t d2h = sel.within ? 8 : (sel.link ? 12 : 0);
     for (const auto &cp : copies) {
         if (!cp.dst || !cp.bytes) continue;
         CK(cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, cudaMemcpyDefault, c->stream));
@@ -1628,7 +1708,7 @@ int gkd_destroy(gkd_ctx *c) {
                       &c->d_cb, &c->ids_a, &c->ids_b, &c->work_counter, &c->sk_cand, &c->sk_misc, &c->sk_sig,
                       &c->sk_len, &c->sk_out, &c->msd_genomes, &c->msd_bins32, &c->msd_bins64, &c->msd_gstat,
                       &c->gr_reps, &c->gr_flags, &c->join_rows, &c->join_err, &c->hit_a, &c->hit_b, &c->sel_cta, &c->nn_pos, &c->nn_inter,
-                      &c->nn_dist, &c->nn_found, &c->uf_parent};
+                      &c->nn_dist, &c->nn_found, &c->uf_parent, &c->lk_forest, &c->lk_state};
     for (DevBuf *b : bufs)
         if (b->p) cudaFreeAsync(b->p, c->stream);
     cudaStreamSynchronize(c->stream);
@@ -2545,6 +2625,129 @@ int gkd_query_vs_ref_clusters(gkd_ctx *c, const uint32_t *q, uint32_t nq, const 
     if ((rc = forest_begin(c, nodes))) return rc;
     if (nq && nr && (rc = rect_selection(c, q, nq, r, nr, sel))) return rc;
     return forest_finish(c, nodes, hf.get(), q_label, nq, r_label, nullptr);
+    ABI_GUARD_END(c)
+}
+
+// ---- single-linkage hierarchy --------------------------------------------------------------------------------
+// node keys of a rectangle: q_key[i] for node i and r_key[j] for node nq + j, or the node itself where an array is NULL.
+// key stays empty when both are NULL.  Checked before the context is used: the keys must be distinct.
+static int link_keys(gkd_ctx *c, const uint32_t *q_key, uint32_t nq, const uint32_t *r_key, uint32_t nr,
+                     std::vector<uint32_t> &key) {
+    if (!q_key && !r_key) return GKD_OK;
+    ABI_GUARD_BEGIN
+    key.resize((uint64_t)nq + nr);
+    for (uint32_t i = 0; i < nq; i++) key[i] = q_key ? q_key[i] : i;
+    for (uint32_t j = 0; j < nr; j++) key[(uint64_t)nq + j] = r_key ? r_key[j] : nq + j;
+    std::vector<uint32_t> sorted(key);
+    std::sort(sorted.begin(), sorted.end());
+    if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
+        return fail(c, GKD_EINVAL, "gkd_query_vs_ref_linkage: node keys are not distinct");
+    return GKD_OK;
+    ABI_GUARD_END(c)
+}
+
+// an empty forest on the device, and the node keys there when the caller passed any
+static int link_begin(gkd_ctx *c, LinkCall &L) {
+    int rc;
+    if ((rc = ensure(c, c->lk_forest, (uint64_t)L.nodes * 24)) || (rc = ensure(c, c->lk_state, link_state_bytes(L.nodes))))
+        return rc;
+    if (!L.key.empty())
+        CK(cudaMemcpyAsync(link_state_at(c->lk_state.p, L.nodes).key, L.key.data(), (uint64_t)L.nodes * 4, cudaMemcpyHostToDevice,
+                           c->stream));
+    L.n_dev = 0;
+    return GKD_OK;
+}
+
+// The forest to the caller, once, at the end of the call: the device forest is copied to the host and merged with the
+// host forest of GKD_AMBIG_LITERAL launches by one Kruskal pass, which also sorts it (a forest keeps every edge).
+static int link_finish(gkd_ctx *c, LinkCall &L, gkd_hits *out) {
+    std::vector<LinkEdge> edges = std::move(L.host);
+    const uint64_t f = L.n_dev, N = L.nodes;
+    if (f) {
+        std::vector<uint64_t> in(f);
+        std::vector<double> d(f);
+        std::vector<uint32_t> a(f), b(f);
+        const uint64_t *fi = (const uint64_t *)c->lk_forest.p;
+        const double *fd = (const double *)(fi + N);
+        const uint32_t *fa = (const uint32_t *)(fd + N), *fb = fa + N;
+        CK(cudaMemcpyAsync(in.data(), fi, f * 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(d.data(), fd, f * 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(a.data(), fa, f * 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(b.data(), fb, f * 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += f * 24;
+        for (uint64_t t = 0; t < f; t++) edges.push_back(L.edge(a[t], b[t], in[t], d[t]));
+    }
+    host_msf(edges, L.nodes);
+    out->n = edges.size();
+    const uint64_t w = std::min<uint64_t>(out->n, out->cap);
+    if (w == 0) return GKD_OK;
+    std::vector<uint32_t> a(w), b(w);
+    std::vector<uint64_t> in(w);
+    std::vector<double> d(w);
+    for (uint64_t t = 0; t < w; t++) a[t] = edges[t].a, b[t] = edges[t].b, in[t] = edges[t].inter, d[t] = edges[t].dist;
+    if (out->a) CK(cudaMemcpyAsync(out->a, a.data(), w * 4, cudaMemcpyDefault, c->stream));
+    if (out->b) CK(cudaMemcpyAsync(out->b, b.data(), w * 4, cudaMemcpyDefault, c->stream));
+    if (out->inter) CK(cudaMemcpyAsync(out->inter, in.data(), w * 8, cudaMemcpyDefault, c->stream));
+    if (out->dist) CK(cudaMemcpyAsync(out->dist, d.data(), w * 8, cudaMemcpyDefault, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return GKD_OK;
+}
+
+int gkd_all_vs_all_linkage(gkd_ctx *c, uint32_t n, double max_dist, gkd_hits *out) {
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_linkage: max_dist is NaN");
+    if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_linkage: null out");
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "linkage over %u sets but only %zu exist", n, c->genomes.size());
+    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
+    int rc = hits_host_ok(c, ps, 4);
+    if (rc) return rc;
+    c->m.pairs = 0;
+    out->n = 0;
+    if (n < 2) return GKD_OK;
+    ABI_GUARD_BEGIN
+    LinkCall L;
+    L.nodes = n;
+    Selection sel{};
+    sel.within = false;
+    sel.max_dist = max_dist;
+    sel.link = &L;
+    if ((rc = link_begin(c, L))) return rc;
+    HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
+    if ((rc = run_pairs(c, hp, gkd_outputs{}, &sel))) return rc;
+    return link_finish(c, L, out);
+    ABI_GUARD_END(c)
+}
+
+int gkd_query_vs_ref_linkage(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, double max_dist,
+                             const uint32_t *q_key, const uint32_t *r_key, gkd_hits *out) {
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_linkage: max_dist is NaN");
+    if (!out) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_linkage: null out");
+    if ((uint64_t)nq + nr >= 0xFFFFFFFFull) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_linkage: %u + %u nodes", nq, nr);
+    std::vector<uint32_t> key;
+    int rc = link_keys(c, q_key, nq, r_key, nr, key);
+    if (rc) return rc;
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_linkage: null id array");
+    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
+    if ((rc = hits_host_ok(c, ps, 4))) return rc;
+    c->m.pairs = 0;
+    out->n = 0;
+    if (nq == 0 || nr == 0) return GKD_OK;
+    ABI_GUARD_BEGIN
+    LinkCall L;
+    L.nodes = nq + nr;
+    L.b_off = nq;
+    L.key = std::move(key);
+    Selection sel{};
+    sel.within = false;
+    sel.max_dist = max_dist;
+    sel.link = &L;
+    if ((rc = link_begin(c, L))) return rc;
+    if ((rc = rect_selection(c, q, nq, r, nr, sel))) return rc;
+    return link_finish(c, L, out);
     ABI_GUARD_END(c)
 }
 

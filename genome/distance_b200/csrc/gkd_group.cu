@@ -6,8 +6,8 @@
 // FASTA file.  The pair matrix shards with no reduction (SURVEY section 8e): member x owns its diagonal
 // block and the blocks (x, (x+s) mod R), s = 1..R/2 (the half-way block of an even ring is split between
 // its two members), exactly the schedule of genome/distance_b200/sharding.py (the one-process-per-GPU
-// torch.distributed layer); here the transport is a peer copy instead of NCCL send/recv.  The cluster form also
-// uses the host union-find of gkd_internal.cuh.
+// torch.distributed layer); here the transport is a peer copy instead of NCCL send/recv.  The cluster and linkage
+// forms also use the host union-find of gkd_internal.cuh.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -20,7 +20,7 @@
 #include <vector>
 
 #include "gkd.h"
-#include "gkd_internal.cuh"  // HostForest
+#include "gkd_internal.cuh"  // HostForest, host_msf
 
 // host FASTA scanner (fasta.cpp)
 struct FastaPiece {
@@ -186,16 +186,25 @@ struct ClusterSink {
     std::vector<std::pair<uint32_t, uint32_t>> links;
 };
 
+// gkd_group_all_vs_all_linkage: the forest edges of a member's calls in global ids (a < b).  The ring computes every
+// pair once, so MSF(union of the calls' forests) = MSF(triangle) under one strict order: every call breaks ties by global
+// ids (its keys), and an edge a call's forest left out is the maximum of a cycle of the whole graph.
+struct LinkageSink {
+    double max_dist;
+    std::vector<gkd::LinkEdge> edges;
+};
+
 void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
-                 ClusterSink *clusters);
+                 ClusterSink *clusters, LinkageSink *linkage);
 
 // the ring of one member (runs on its own host thread; no exception may leave the thread).  With `within` the
 // member selects on its device and collects its hits there instead of scattering dense blocks into inter / dist;
-// with `nearest` it collects partial k-nearest lists, with `clusters` the links of its calls' components.
+// with `nearest` it collects partial k-nearest lists, with `clusters` the links of its calls' components, with
+// `linkage` their spanning forests.
 void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
-                       ClusterSink *clusters) {
+                       ClusterSink *clusters, LinkageSink *linkage) {
     try {
-        member_ring(g, x, inter, dist, within, nearest, clusters);
+        member_ring(g, x, inter, dist, within, nearest, clusters, linkage);
     } catch (const std::exception &ex) {
         g->members[x].rc = GKD_ENOMEM;
         g->members[x].err = ex.what();
@@ -203,7 +212,7 @@ void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, 
 }
 
 void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
-                 ClusterSink *clusters) {
+                 ClusterSink *clusters, LinkageSink *linkage) {
     Member &M = g->members[x];
     const uint32_t R = (uint32_t)g->members.size();
     const uint64_t N = g->n_genomes;
@@ -310,8 +319,26 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
         return gkd_neighbors{pos.data(), in.data(), d.data(), nf.data()};
     };
     std::vector<uint32_t> ql, rl;  // clusters: the labels of one call
+    // linkage: the forest of one call, at most nodes - 1 edges
+    auto forest = [&](uint64_t nodes, auto call, auto gid_a, auto gid_b) -> int {
+        ha.resize(nodes);
+        hb.resize(nodes);
+        bi.resize(nodes);
+        bd.resize(nodes);
+        gkd_hits h{ha.data(), hb.data(), bi.data(), bd.data(), nodes, 0};
+        const int rc = call(h);
+        if (rc != GKD_OK) return rc;
+        for (uint64_t t = 0; t < h.n; t++) {
+            const uint32_t ga = gid_a(ha[t]), gb = gid_b(hb[t]), lo = std::min(ga, gb), hi = std::max(ga, gb);
+            linkage->edges.push_back(gkd::link_edge(lo, hi, bi[t], bd[t], lo, hi, lo, hi));
+        }
+        return GKD_OK;
+    };
     // diagonal block (runs while the first group is in flight)
-    if (m >= 2 && clusters) {
+    if (m >= 2 && linkage) {
+        auto own = [&](uint32_t i) { return M.global_ids[i]; };  // ascending, so local order is global order
+        MGK(forest(m, [&](gkd_hits &h) { return gkd_all_vs_all_linkage(M.ctx, m, linkage->max_dist, &h); }, own, own));
+    } else if (m >= 2 && clusters) {
         ql.resize(m);
         MGK(gkd_all_vs_all_clusters(M.ctx, m, clusters->max_dist, ql.data(), nullptr));
         for (uint32_t i = 0; i < m; i++)
@@ -362,6 +389,21 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
                 cols.push_back(first + c);
                 col_gid.push_back(g->members[S.src].global_ids[S.p.first + c]);
             }
+        }
+        if (linkage) {
+            // keyed by global id: the columns may span peers on both sides of this member's ids, and ties must be broken
+            // as one context over all ids breaks them
+            const uint32_t nr = (uint32_t)rows.size(), nc = (uint32_t)cols.size();
+            std::vector<uint32_t> row_gid(nr);
+            for (uint32_t p = 0; p < nr; p++) row_gid[p] = M.global_ids[rows[p]];
+            MGK(forest((uint64_t)nr + nc - 1,
+                       [&](gkd_hits &h) {
+                           return gkd_query_vs_ref_linkage(M.ctx, rows.data(), nr, cols.data(), nc, linkage->max_dist,
+                                                           row_gid.data(), col_gid.data(), &h);
+                       },
+                       [&](uint32_t p) { return row_gid[p]; }, [&](uint32_t c) { return col_gid[c]; }));
+            MGK(gkd_truncate(M.ctx, m));
+            continue;
         }
         if (clusters) {
             const uint32_t nr = (uint32_t)rows.size(), nc = (uint32_t)cols.size();
@@ -629,7 +671,7 @@ int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist) {
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr, nullptr, nullptr);
+            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr, nullptr, nullptr, nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -652,7 +694,7 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x], nullptr, nullptr);
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x], nullptr, nullptr, nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -691,7 +733,7 @@ int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, cons
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, &sinks[x], nullptr);
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, &sinks[x], nullptr, nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -732,7 +774,7 @@ int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label
         std::vector<std::thread> threads;
         for (uint32_t x = 0; x < g->members.size(); x++) {
             g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, nullptr, &sinks[x]);
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, nullptr, &sinks[x], nullptr);
         }
         for (auto &t : threads) t.join();
         for (size_t i = 0; i < g->members.size(); i++)
@@ -750,6 +792,42 @@ int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label
         return GKD_OK;
     } catch (const std::exception &ex) {
         return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_clusters: %s", ex.what());
+    }
+}
+
+int gkd_group_all_vs_all_linkage(gkd_group *g, double max_dist, gkd_hits *out) {
+    if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_linkage: max_dist is NaN");
+    if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_linkage: null out");
+    if (!g) return GKD_EINVAL;
+    try {
+        for (auto &M : g->members)
+            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
+        std::vector<LinkageSink> sinks(g->members.size(), LinkageSink{max_dist, {}});
+        std::vector<std::thread> threads;
+        for (uint32_t x = 0; x < g->members.size(); x++) {
+            g->members[x].rc = GKD_OK;
+            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, nullptr, nullptr, &sinks[x]);
+        }
+        for (auto &t : threads) t.join();
+        for (size_t i = 0; i < g->members.size(); i++)
+            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        std::vector<gkd::LinkEdge> edges;
+        for (auto &s : sinks) {
+            edges.insert(edges.end(), s.edges.begin(), s.edges.end());
+            std::vector<gkd::LinkEdge>().swap(s.edges);
+        }
+        gkd::host_msf(edges, g->n_genomes);
+        out->n = edges.size();
+        const uint64_t w = std::min<uint64_t>(out->n, out->cap);
+        for (uint64_t t = 0; t < w; t++) {
+            if (out->a) out->a[t] = edges[t].a;
+            if (out->b) out->b[t] = edges[t].b;
+            if (out->inter) out->inter[t] = edges[t].inter;
+            if (out->dist) out->dist[t] = edges[t].dist;
+        }
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_linkage: %s", ex.what());
     }
 }
 

@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
+#include <cstring>
 #include <vector>
 
 #include "gkd.h"
@@ -342,6 +344,67 @@ struct HostForest {
         else if (b < a) parent[a] = b;
     }
 };
+// Single-linkage hierarchy: the minimum spanning forest (MSF) of the pairs within max_dist under the strict order
+// (distance bits, min key, max key) of the two nodes.  One Boruvka pass (launch_link_rounds) replaces the device forest F
+// with MSF(F u E) for a graph whose edge list is E_chunk followed by F, copied there by the caller.
+struct LinkGraph {
+    const uint32_t *a, *b;  // as launch_select_within writes them; the nodes are a and b + b_off
+    const uint64_t *inter;
+    const double *dist;
+    uint64_t n_edges;       // < LINK_NONE
+    uint32_t b_off;         // RECT: nq (reference column j is node nq + j); UPPER: 0
+    const uint32_t *key;    // key of every node (nullptr: the node itself)
+};
+constexpr uint32_t LINK_NONE = 0xFFFFFFFFu;
+// O(nodes) device state of one call, carved from one buffer of link_state_bytes(nodes)
+struct LinkState {
+    unsigned long long *best_d, *best_k;  // per component root: the minimum crossing edge's distance bits, then key pair
+    uint32_t *best_e;                     // ... and its edge index
+    uint32_t *comp, *hook;                // component root of every node; the root a root hooks under in this round
+    uint32_t *hooked;                     // hooked[r] != 0: round r - 1 hooked something (hooked[0] = 1)
+    uint32_t *n_forest;                   // edges written to the new forest
+    uint32_t *key;                        // node keys, when the caller passed any
+    uint32_t nodes;
+};
+struct LinkForest {  // the new forest: <= nodes - 1 edges
+    uint32_t *a, *b;
+    uint64_t *inter;
+    double *dist;
+};
+constexpr uint32_t LINK_MAX_ROUNDS = 32;
+uint64_t link_state_bytes(uint32_t nodes);
+LinkState link_state_at(void *base, uint32_t nodes);
+// rounds = ceil(log2(nodes)) Boruvka rounds, queued without a host read; a round after one that hooked nothing exits
+// at once.  On return *st.n_forest (device) is the number of edges of the new forest f.
+cudaError_t launch_link_rounds(const LinkGraph &g, const LinkState &st, const LinkForest &f, uint32_t rounds, cudaStream_t s);
+// The same forest on the host: Kruskal in the strict order.  Used for GKD_AMBIG_LITERAL pairs, to sort the device forest
+// at the end of a call (a forest keeps every edge), and for the group's merge of its members' forests.
+struct LinkEdge {
+    uint64_t dbits, keys;  // distance bits, (min key << 32) | max key
+    uint32_t na, nb;       // nodes
+    uint32_t a, b;         // as reported
+    uint64_t inter;
+    double dist;
+};
+inline LinkEdge link_edge(uint32_t a, uint32_t b, uint64_t inter, double dist, uint32_t na, uint32_t nb, uint32_t ka, uint32_t kb) {
+    LinkEdge e{0, (uint64_t)std::min(ka, kb) << 32 | std::max(ka, kb), na, nb, a, b, inter, dist};
+    std::memcpy(&e.dbits, &dist, 8);
+    return e;
+}
+// edges <- MSF(edges) over nodes [0, nodes), ascending
+inline void host_msf(std::vector<LinkEdge> &edges, uint32_t nodes) {
+    std::sort(edges.begin(), edges.end(), [](const LinkEdge &x, const LinkEdge &y) {
+        return x.dbits < y.dbits || (x.dbits == y.dbits && x.keys < y.keys);
+    });
+    HostForest f(nodes);
+    size_t kept = 0;
+    for (const LinkEdge &e : edges) {
+        if (f.find(e.na) == f.find(e.nb)) continue;
+        f.link(e.na, e.nb);
+        edges[kept++] = e;
+    }
+    edges.resize(kept);
+}
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless
 // some representative is within max_dist; clears the counts it consumed
 cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *n_reps, uint32_t cand, uint32_t visit,

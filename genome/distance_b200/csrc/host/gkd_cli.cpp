@@ -139,6 +139,8 @@ const std::vector<OptSpec> FASTA_OPTS = {
                           "input order, nearest first; a pair can appear twice, once from each end (additive option)"},
     {{"--clusters"}, false, "report each record's single-linkage cluster at --maxDist: the label of the cluster's first "
                             "record (additive option; needs --maxDist)"},
+    {{"--linkage"}, false, "report the single-linkage hierarchy up to --maxDist (default 1.0, the whole tree): one line "
+                           "per merge of single-linkage agglomeration, in merge order (additive option)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
@@ -262,6 +264,9 @@ int fastaDist(const std::vector<std::string> &args) {
     const bool clusters = p.values.count("--clusters") > 0;
     if (clusters && !within) throw ParseFailureException("--clusters needs --maxDist.");
     if (clusters && nearest) throw ParseFailureException("--clusters and --nearest cannot be combined.");
+    const bool linkage = p.values.count("--linkage") > 0;
+    if (linkage && nearest) throw ParseFailureException("--linkage and --nearest cannot be combined.");
+    if (linkage && clusters) throw ParseFailureException("--linkage and --clusters cannot be combined.");
     const char *typeName = seqType == KmerType::DNA ? "DNA" : (seqType == KmerType::RNA ? "RNA" : "PROT");
     if (inFile.empty()) logInfo(std::string("Reading ") + typeName + " sequences from the standard input.");
     else if (!readable(inFile)) throw IOException("Input file " + inFile + " is not found or unreadable.");
@@ -322,6 +327,20 @@ int fastaDist(const std::vector<std::string> &args) {
             const uint32_t found = writeClusters(writer, n, label.data(), [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
                                                  [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
             logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(found) + " clusters at distance " +
+                    javaDouble(maxDist) + ".");
+            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
+            return 0;
+        }
+        if (linkage) {
+            const uint64_t cap = n ? n - 1 : 0;
+            std::vector<uint32_t> a(cap), b(cap);
+            std::vector<double> d(cap);
+            gkd_hits h{a.data(), b.data(), nullptr, d.data(), cap, 0};
+            gcheck(gkd_group_all_vs_all_linkage(grp, maxDist, &h));
+            writeHits(writer, a.data(), b.data(), d.data(), h.n, [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
+                      [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
+            writer.flush();
+            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(h.n) + " merges up to distance " +
                     javaDouble(maxDist) + ".");
             writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
             return 0;
@@ -388,6 +407,21 @@ int fastaDist(const std::vector<std::string> &args) {
         logInfo(std::to_string(n < 2 ? 0 : n * (n - 1) / 2) + " pairs computed in 1 batches, " + std::to_string(found) +
                 " clusters at distance " + javaDouble(maxDist) + ".");
         writeMetrics(metricsFile, "fastaDist", engine.raw(), n < 2 ? 0 : n * (n - 1) / 2, 1);
+        return 0;
+    }
+    if (linkage) {
+        // each pair i < j is intersected once; only the spanning forest (<= n - 1 edges) leaves the GPU
+        const uint64_t n = seqs.size(), total = n < 2 ? 0 : n * (n - 1) / 2, cap = n ? n - 1 : 0;
+        std::vector<uint32_t> a(cap), b(cap);
+        std::vector<double> d(cap);
+        gkd_hits h{a.data(), b.data(), nullptr, d.data(), cap, 0};
+        engine.check(gkd_all_vs_all_linkage(engine.raw(), (uint32_t)n, maxDist, &h));
+        writeHits(writer, a.data(), b.data(), d.data(), h.n, [&](size_t i) { return seqs[i].getGenomeId(); },
+                  [&](size_t i) { return seqs[i].getGenomeName(); });
+        writer.flush();
+        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(h.n) + " merges up to distance " +
+                javaDouble(maxDist) + ".");
+        writeMetrics(metricsFile, "fastaDist", engine.raw(), total, 1);
         return 0;
     }
     if (nearest) {

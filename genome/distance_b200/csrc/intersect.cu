@@ -978,6 +978,148 @@ cudaError_t launch_cluster_flatten(uint32_t *parent, uint32_t n, cudaStream_t s)
     return cudaGetLastError();
 }
 
+// Linkage, Boruvka form: the minimum spanning forest of an edge list (a chunk's edges within max_dist, compacted by
+// k_select_within, followed by the forest of the earlier chunks) under the strict order (distance bits, min key, max key).
+// Every round starts from the components of the previous one (comp[x] = root):
+//   edges 0:  every edge between two components offers its distance bits to both roots' best_d (atomicMin);
+//   edges 1:  an edge with the winning distance offers its key pair to best_k;
+//   edges 2:  the one edge with both (the order is strict) writes its index to best_e;
+//   hook:     every root with a best edge hooks under the root at its other end and appends the edge to the new forest;
+//             of a mutual pair (both roots chose the same edge) only the larger root hooks, so each edge enters once and
+//             the hooks form trees;
+//   relabel:  each root jumps its own hook pointer to its tree's root (only thread x writes hook[x]; every value read
+//             is an ancestor, so the walk ends), every node takes its root's final root, and best_* are reset.
+// Every component with a crossing edge merges in a round, so ceil(log2 nodes) rounds finish the forest.  The host
+// queues them all; a round whose predecessor hooked nothing (hooked[r] == 0) exits at once.
+constexpr int LINK_THREADS = 256;
+
+__device__ __forceinline__ unsigned long long link_load64(unsigned long long *p) {
+    return cuda::atomic_ref<unsigned long long, cuda::thread_scope_device>(*p).load(cuda::memory_order_relaxed);
+}
+
+// atomicMin only when it can lower the value: most offers lose, and the relaxed load keeps them off the atomic unit
+__device__ __forceinline__ void link_offer(unsigned long long *p, unsigned long long v) {
+    if (v < link_load64(p)) atomicMin(p, v);
+}
+
+__device__ __forceinline__ unsigned long long link_keys(const LinkGraph &g, uint32_t na, uint32_t nb) {
+    const uint32_t ka = g.key ? g.key[na] : na, kb = g.key ? g.key[nb] : nb;
+    return (unsigned long long)min(ka, kb) << 32 | max(ka, kb);
+}
+
+__global__ void __launch_bounds__(LINK_THREADS) k_link_init(LinkState st, uint32_t rounds) {
+    const uint32_t x = blockIdx.x * blockDim.x + threadIdx.x;
+    if (x < st.nodes) {
+        st.comp[x] = st.hook[x] = x;
+        st.best_d[x] = st.best_k[x] = ~0ull;
+        st.best_e[x] = LINK_NONE;
+    }
+    if (x <= rounds) st.hooked[x] = x == 0 ? 1u : 0u;
+    if (x == 0) *st.n_forest = 0;
+}
+
+template <int PHASE>
+__global__ void __launch_bounds__(LINK_THREADS) k_link_edges(LinkGraph g, LinkState st, uint32_t round) {
+    if (st.hooked[round] == 0) return;
+    for (uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; e < g.n_edges; e += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t na = g.a[e], nb = g.b[e] + g.b_off;
+        const uint32_t ca = st.comp[na], cb = st.comp[nb];
+        if (ca == cb) continue;
+        const unsigned long long d = (unsigned long long)__double_as_longlong(g.dist[e]);
+        if (PHASE == 0) {
+            link_offer(st.best_d + ca, d);
+            link_offer(st.best_d + cb, d);
+            continue;
+        }
+        const bool at_a = st.best_d[ca] == d, at_b = st.best_d[cb] == d;
+        if (!at_a && !at_b) continue;
+        const unsigned long long kp = link_keys(g, na, nb);
+        if (PHASE == 1) {
+            if (at_a) link_offer(st.best_k + ca, kp);
+            if (at_b) link_offer(st.best_k + cb, kp);
+        } else {
+            if (at_a && st.best_k[ca] == kp) st.best_e[ca] = (uint32_t)e;
+            if (at_b && st.best_k[cb] == kp) st.best_e[cb] = (uint32_t)e;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(LINK_THREADS) k_link_hook(LinkGraph g, LinkState st, LinkForest f, uint32_t round) {
+    if (st.hooked[round] == 0) return;
+    const uint32_t x = blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t e = LINK_NONE, y = x;
+    if (x < st.nodes && st.comp[x] == x) e = st.best_e[x];
+    if (e != LINK_NONE) {
+        const uint32_t ca = st.comp[g.a[e]], cb = st.comp[g.b[e] + g.b_off];
+        y = ca == x ? cb : ca;
+        if (st.best_e[y] == e && x < y) e = LINK_NONE;  // mutual: the smaller root stays a root
+    }
+    const bool hooks = e != LINK_NONE;
+    const uint32_t lane = threadIdx.x & 31, mask = __ballot_sync(0xffffffffu, hooks);
+    if (!mask) return;
+    uint32_t at = 0;
+    if (lane == 0) at = atomicAdd(st.n_forest, (uint32_t)__popc(mask));
+    at = __shfl_sync(0xffffffffu, at, 0) + __popc(mask & ((1u << lane) - 1u));
+    if (!hooks) return;
+    st.hook[x] = y;
+    f.a[at] = g.a[e];
+    f.b[at] = g.b[e];
+    f.inter[at] = g.inter[e];
+    f.dist[at] = g.dist[e];
+    if (lane == __ffs(mask) - 1) st.hooked[round + 1] = 1u;
+}
+
+__global__ void __launch_bounds__(LINK_THREADS) k_link_relabel(LinkState st, uint32_t round) {
+    if (st.hooked[round + 1] == 0) return;  // nothing merged: the labels stand and the later rounds exit
+    const uint32_t x = blockIdx.x * blockDim.x + threadIdx.x;
+    if (x >= st.nodes) return;
+    uint32_t r = st.comp[x];
+    if (r == x) {
+        for (uint32_t p = uf_load(st.hook + x), gp = uf_load(st.hook + p); gp != p; gp = uf_load(st.hook + p)) {
+            p = gp;
+            uf_store(st.hook + x, p);
+        }
+        r = uf_load(st.hook + x);
+    } else {
+        for (uint32_t p = uf_load(st.hook + r); p != r; p = uf_load(st.hook + r)) r = p;
+    }
+    st.comp[x] = r;
+    st.best_d[x] = st.best_k[x] = ~0ull;
+    st.best_e[x] = LINK_NONE;
+}
+
+uint64_t link_state_bytes(uint32_t nodes) { return (uint64_t)nodes * (16 + 16) + (LINK_MAX_ROUNDS + 2) * 4 + 16; }
+
+LinkState link_state_at(void *base, uint32_t nodes) {
+    LinkState st{};
+    char *p = (char *)base;
+    st.best_d = (unsigned long long *)p;
+    st.best_k = st.best_d + nodes;
+    st.best_e = (uint32_t *)(st.best_k + nodes);
+    st.comp = st.best_e + nodes;
+    st.hook = st.comp + nodes;
+    st.key = st.hook + nodes;
+    st.hooked = st.key + nodes;
+    st.n_forest = st.hooked + LINK_MAX_ROUNDS + 1;
+    st.nodes = nodes;
+    return st;
+}
+
+cudaError_t launch_link_rounds(const LinkGraph &g, const LinkState &st, const LinkForest &f, uint32_t rounds, cudaStream_t s) {
+    const unsigned node_blocks = (unsigned)(((uint64_t)st.nodes + LINK_THREADS - 1) / LINK_THREADS);
+    const uint64_t need = (g.n_edges + LINK_THREADS - 1) / LINK_THREADS;  // grid-stride beyond 8192 CTAs
+    const unsigned edge_blocks = (unsigned)(need < 8192 ? (need ? need : 1) : 8192);
+    k_link_init<<<(unsigned)((std::max<uint64_t>(st.nodes, rounds + 1) + LINK_THREADS - 1) / LINK_THREADS), LINK_THREADS, 0, s>>>(st, rounds);
+    for (uint32_t r = 0; r < rounds; r++) {
+        k_link_edges<0><<<edge_blocks, LINK_THREADS, 0, s>>>(g, st, r);
+        k_link_edges<1><<<edge_blocks, LINK_THREADS, 0, s>>>(g, st, r);
+        k_link_edges<2><<<edge_blocks, LINK_THREADS, 0, s>>>(g, st, r);
+        k_link_hook<<<node_blocks, LINK_THREADS, 0, s>>>(g, st, f, r);
+        k_link_relabel<<<node_blocks, LINK_THREADS, 0, s>>>(st, r);
+    }
+    return cudaGetLastError();
+}
+
 // Greedy representative pass (DistanceRepsProcessor.java:185-201, FastaDistanceRepsProcessor.java:124-146): the
 // candidate was intersected with every current representative (counts[t] for reps[t]); it joins the list unless
 // one of them is within max_dist.  The list and its length live on the device, so the host queues the launches

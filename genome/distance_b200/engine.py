@@ -22,9 +22,10 @@ assert PACKED_DTYPE.itemsize == C.sizeof(GkdPackedSet)
 FIRST_HITS_CAP = 1 << 20
 
 
-def _select(call, pairs: int):
-    """(a, b, inter, dist) numpy arrays of a gkd_hits call `call(hits)` (count-then-fetch, see FIRST_HITS_CAP)"""
-    cap = min(pairs, FIRST_HITS_CAP)
+def _select(call, pairs: int, cap: int = None):
+    """(a, b, inter, dist) numpy arrays of a gkd_hits call `call(hits)` (count-then-fetch, see FIRST_HITS_CAP; a cap
+    known to suffice, such as nodes - 1 for a spanning forest, makes it one call)"""
+    cap = min(pairs, FIRST_HITS_CAP) if cap is None else cap
     while True:
         a, b = np.empty(cap, dtype=np.uint32), np.empty(cap, dtype=np.uint32)
         inter, dist = np.empty(cap, dtype=np.uint64), np.empty(cap, dtype=np.float64)
@@ -351,6 +352,29 @@ class Engine:
                                                    float(max_dist), ql.ctypes.data, rl.ctypes.data))
         return ql, rl
 
+    def all_vs_all_linkage(self, max_dist: float, n: int = None):
+        """(a, b, inter, dist): the single-linkage hierarchy of the first n sets (default: all) up to max_dist, i.e. the
+        minimum spanning forest of the pairs within max_dist under the order (distance bits, a, b), in ascending order
+        (the merge order of single-linkage agglomeration).  Every pair is intersected once; only the forest leaves the
+        device"""
+        n = len(self) if n is None else int(n)
+        return _select(lambda h: self._ck(self._L.gkd_all_vs_all_linkage(self._h, n, float(max_dist), C.byref(h))),
+                       max(n - 1, 0), max(n - 1, 0))
+
+    def query_vs_ref_linkage(self, q: Sequence[int], r: Sequence[int], max_dist: float, q_key=None, r_key=None):
+        """(a, b, inter, dist): the forest of one query x reference pass; node i is q[i] and node len(q) + j is r[j], an
+        edge reports a = i and b = j.  Ties are broken by the nodes' (min key, max key); keys default to the nodes and
+        must be distinct"""
+        qa, ra = np.ascontiguousarray(q, dtype=np.uint32), np.ascontiguousarray(r, dtype=np.uint32)
+        qk = None if q_key is None else np.ascontiguousarray(q_key, dtype=np.uint32)
+        rk = None if r_key is None else np.ascontiguousarray(r_key, dtype=np.uint32)
+        if (qk is not None and qk.size != qa.size) or (rk is not None and rk.size != ra.size):
+            raise ValueError("q_key / r_key must have one entry per query / reference")
+        nodes = max(qa.size + ra.size - 1, 0)
+        return _select(lambda h: self._ck(self._L.gkd_query_vs_ref_linkage(
+            self._h, qa.ctypes.data, qa.size, ra.ctypes.data, ra.size, float(max_dist),
+            None if qk is None else qk.ctypes.data, None if rk is None else rk.ctypes.data, C.byref(h))), nodes, nodes)
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -533,3 +557,8 @@ class Group:
         labels, count = np.empty(len(self), dtype=np.uint32), C.c_uint32()
         self._ck(self._L.gkd_group_all_vs_all_clusters(self._h, float(max_dist), labels.ctypes.data, C.byref(count)))
         return labels, count.value
+
+    def all_vs_all_linkage(self, max_dist: float):
+        """(a, b, inter, dist) over all global ids: the single-context Engine.all_vs_all_linkage result"""
+        n = max(len(self) - 1, 0)
+        return _select(lambda h: self._ck(self._L.gkd_group_all_vs_all_linkage(self._h, float(max_dist), C.byref(h))), n, n)

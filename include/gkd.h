@@ -281,6 +281,23 @@ int gkd_all_vs_all_clusters(gkd_ctx *ctx, uint32_t n, double max_dist, uint32_t 
 int gkd_query_vs_ref_clusters(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr,
                               double max_dist, uint32_t *q_label, uint32_t *r_label);
 
+/* The single-linkage hierarchy of the first n sets up to max_dist: the minimum spanning forest of the pairs i < j with
+ * distance <= max_dist (the comparison of gkd_*_within), under the strict order (distance bits, a, b).  out receives its
+ * edges in ascending order, which is the merge order of single-linkage agglomeration; a, b (a < b), inter and dist are
+ * bit-identical to the dense call's.  out->n = n - (clusters at max_dist); only the first min(n, cap) are written, so
+ * cap = n - 1 always suffices.  For every t <= max_dist the components of the edges with dist <= t are the clusters of
+ * gkd_all_vs_all_clusters(t).  Any array may be NULL; host or device memory as for gkd_hits.  A negative max_dist gives
+ * no edges, max_dist = 1.0 a spanning tree.  Every pair is intersected once.  Device memory: one chunk of compacted
+ * edges (24 B x 64 Mi pairs = 1.5 GiB at most) and O(n) forest state (56 B per node); only the forest leaves the
+ * device. */
+int gkd_all_vs_all_linkage(gkd_ctx *ctx, uint32_t n, double max_dist, gkd_hits *out);
+/* The same over one query x reference pass, with the nodes of gkd_query_vs_ref_clusters: node i is q[i], node nq + j is
+ * r[j]; an edge (a = i, b = j) joins them when dist(q[i], r[j]) <= max_dist.  Ties are broken by (min key, max key) of
+ * the two nodes; the key of node i is q_key[i] and of node nq + j is r_key[j] (host arrays), or the node itself when the
+ * array is NULL.  Keys must be distinct (GKD_EINVAL otherwise).  out->n <= nq + nr - 1. */
+int gkd_query_vs_ref_linkage(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr,
+                             double max_dist, const uint32_t *q_key, const uint32_t *r_key, gkd_hits *out);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -318,6 +335,10 @@ int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, cons
  * and each ring block on its own device; the host joins the components of every call (O(rows + columns) per call).
  * label is host memory (N entries); *n_clusters may be NULL. */
 int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label, uint32_t *n_clusters);
+/* gkd_all_vs_all_linkage over all global ids; equal to one context's forest, bit for bit.  Every member computes the
+ * forest of its diagonal block and of each ring call (keyed by global id) on its own device; the host merges them by
+ * Kruskal in the order (distance bits, global a, global b).  The arrays of out are host memory. */
+int gkd_group_all_vs_all_linkage(gkd_group *g, double max_dist, gkd_hits *out);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

@@ -247,3 +247,28 @@ JNIEXPORT jint JNICALL FN(allVsAllClusters)(JNIEnv *env, jclass c, jlong h, jint
     if (l) (*env)->ReleaseIntArrayElements(env, label, l, 0);
     return rc;
 }
+
+/* the single-linkage hierarchy of the first n sets up to maxDist: a, b, dist hold n - 1 entries (the forest edges in
+ * merge order); nEdges[0] receives their number */
+JNIEXPORT jint JNICALL FN(allVsAllLinkage)(JNIEnv *env, jclass c, jlong h, jint n, jdouble maxDist, jintArray a,
+                                           jintArray b, jdoubleArray dist, jintArray nEdges) {
+    (void)c;
+    if (!a || !b || !dist || !nEdges || n < 0 || (*env)->GetArrayLength(env, nEdges) < 1) return GKD_EINVAL;
+    const jint cap = n > 0 ? n - 1 : 0;
+    if ((*env)->GetArrayLength(env, a) < cap || (*env)->GetArrayLength(env, b) < cap ||
+        (*env)->GetArrayLength(env, dist) < cap)
+        return GKD_EINVAL;
+    jint *pa = (*env)->GetIntArrayElements(env, a, NULL);
+    jint *pb = (*env)->GetIntArrayElements(env, b, NULL);
+    jdouble *d = (*env)->GetDoubleArrayElements(env, dist, NULL);
+    gkd_hits out = {(uint32_t *)pa, (uint32_t *)pb, NULL, d, (uint64_t)cap, 0};
+    int rc = (pa && pb && d) ? gkd_all_vs_all_linkage(CTX(h), (uint32_t)n, maxDist, &out) : GKD_ENOMEM;
+    if (d) (*env)->ReleaseDoubleArrayElements(env, dist, d, 0);
+    if (pb) (*env)->ReleaseIntArrayElements(env, b, pb, 0);
+    if (pa) (*env)->ReleaseIntArrayElements(env, a, pa, 0);
+    if (rc == GKD_OK) {
+        jint ne = (jint)out.n;
+        (*env)->SetIntArrayRegion(env, nEdges, 0, 1, &ne);
+    }
+    return rc;
+}

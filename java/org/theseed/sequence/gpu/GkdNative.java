@@ -50,6 +50,9 @@ final class GkdNative {
     /** single-linkage clusters of the first n sets at maxDist: label (length n) receives the smallest id of each set's
      *  cluster */
     static native int allVsAllClusters(long ctx, int n, double maxDist, int[] label);
+    /** the single-linkage hierarchy of the first n sets up to maxDist: the minimum spanning forest of the pairs within
+     *  maxDist in merge order; a, b, dist (length n - 1) receive its edges (a &lt; b), nEdges[0] their number */
+    static native int allVsAllLinkage(long ctx, int n, double maxDist, int[] a, int[] b, double[] dist, int[] nEdges);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

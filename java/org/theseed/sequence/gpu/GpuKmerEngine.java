@@ -195,6 +195,18 @@ public class GpuKmerEngine implements AutoCloseable {
         return label;
     }
 
+    /** the single-linkage hierarchy of every set up to maxDist (1.0: the whole tree): the merges of single-linkage
+     *  agglomeration in order, i.e. the minimum spanning forest of the pairs within maxDist under (distance, a, b).
+     *  a, b and dist (at least size() - 1 entries) receive the merged pair (a &lt; b) and its distance; returns the
+     *  number of merges, size() minus the clusters at maxDist.  The clusters at any t &lt;= maxDist are the components
+     *  of the merges with dist &lt;= t.  Every pair is intersected once and only the merges leave the GPU. */
+    public synchronized int allVsAllLinkage(double maxDist, int[] a, int[] b, double[] dist) {
+        this.build();
+        int[] merges = new int[1];
+        check(GkdNative.allVsAllLinkage(this.ctx, this.size(), maxDist, a, b, dist, merges));
+        return merges[0];
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
