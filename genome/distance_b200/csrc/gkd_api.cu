@@ -956,6 +956,391 @@ bool plan_join(gkd_ctx *c, const HostPairs &hp, uint64_t first, uint64_t count, 
     return true;
 }
 
+// The sets of one call: the largest sizes and levels (kernel 4's work split) and whether any has literal k-mers
+struct SetScan {
+    uint64_t max_n = 0, max_pal = 0;
+    uint32_t max_level = 0, max_pal_level = 0;
+    bool any_lit = false;
+    int see(gkd_ctx *c, uint32_t id) {
+        const int rc = check_built(c, id);
+        if (rc) return rc;
+        const GenomeRec &g = c->genomes[id];
+        max_n = std::max<uint64_t>(max_n, g.desc.main.n);
+        max_pal = std::max<uint64_t>(max_pal, g.desc.pal.n);
+        max_level = std::max(max_level, g.desc.main.level);
+        max_pal_level = std::max(max_pal_level, g.desc.pal.level);
+        any_lit = any_lit || !g.lit.empty();
+        return GKD_OK;
+    }
+};
+
+// Kernel 4's work split for `pairs` pairs whose sets have at most nmax keys and level lmax: a pair is walked in
+// 32-bucket groups at the level of its larger set; an item is a run of groups of one pair.  Few pairs -> small items so
+// every warp has work; many pairs -> eight items per pair, so the warps that share a pair read neighbouring parts of its
+// two key streams.  gkd_config.segment_keys, when set, fixes the item size instead.
+IsectPlan make_plan(const gkd_ctx *c, uint64_t pairs, uint64_t nmax, uint32_t lmax, bool one_item) {
+    IsectPlan p{};
+    p.low_bits = c->low_bits;
+    p.tmax = c->isect_tmax;
+    p.level_min = c->lvl_min;
+    uint32_t L = std::max(level_for((uint32_t)nmax, p.tmax), c->lvl_min);
+    L = std::min(L, lmax);
+    const uint64_t max_groups = ((1ull << L) + 31) >> 5;
+    uint64_t gpi;
+    if (one_item || max_groups <= 64) gpi = max_groups;  // tiny sets: a pair is one item (the per-item set-up would dominate)
+    else if (c->cfg.segment_keys) gpi = std::max<uint64_t>(1, c->cfg.segment_keys / (64ull * p.tmax));
+    else {
+        const uint64_t warps = (uint64_t)c->n_sms * intersect_warps_per_sm(c->low_bits);
+        const long double total_groups = (long double)pairs * max_groups;
+        gpi = (uint64_t)std::min<long double>(total_groups / (long double)(warps * 8), (long double)(max_groups / 8));
+    }
+    gpi = std::min<uint64_t>(std::max<uint64_t>(gpi, 1), max_groups);
+    p.groups_per_item = (uint32_t)gpi;
+    p.items_per_pair = (uint32_t)((max_groups + gpi - 1) / gpi);
+    return p;
+}
+
+// One chunk of run_pairs once its kernel-4 launches are queued: pairs done .. done + cnt of hp and their counts
+struct Chunk {
+    const HostPairs &hp;
+    const PairSource &src;
+    uint64_t done, cnt;
+    const SetDesc *sets;
+    const uint32_t *counts, *pal;  // pal: nullptr unless the palindrome counts are needed
+    int both;
+    const uint32_t *join_err;      // the block join's overflow flag on the device; nullptr when the merge kernel ran
+    // pair t of the chunk as reported: RECT (a_base + query row, reference position), otherwise the two set ids
+    void pair(uint32_t a_base, uint64_t t, uint32_t &a, uint32_t &b) const {
+        if (hp.mode == PAIRS_RECT) a = a_base + (uint32_t)((done + t) / hp.nb), b = (uint32_t)((done + t) % hp.nb);
+        else host_pair_ids(hp, done + t, a, b);
+    }
+};
+
+// What a call computes from the counts of kernel 4: one form of kernel 5.  run_pairs owns the chunk loop and the redo of
+// a chunk whose join table overflowed; the form owns its state, its launches, its copies and its rule for pairs that are
+// completed on the host.  The bytes queue() and keep() read back are counted only for a chunk that is kept.
+struct Form {
+    uint32_t a_base = 0;              // RECT: position in the caller's q of this launch's first query row (run_rect)
+    std::vector<uint64_t> lit_inter;  // GKD_AMBIG_LITERAL: the chunk's pairs, completed on the host
+    std::vector<double> lit_dist;
+    virtual ~Form() = default;
+    // the chunk's kernel-5 launches, then the reads the host needs once the stream is synchronised; records ev[7]
+    virtual int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) = 0;
+    // the join held: the chunk is kept
+    virtual int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) { return GKD_OK; }
+    // GKD_AMBIG_LITERAL: host memory for the chunk's dense values (inter is required) ...
+    virtual gkd_outputs literal_outputs(const Chunk &e) {
+        lit_inter.resize(e.cnt);
+        lit_dist.resize(e.cnt);
+        return gkd_outputs{lit_inter.data(), lit_dist.data(), nullptr, nullptr};
+    }
+    // ... and the form's rule on them once they are completed, the same as its device kernels'
+    virtual void host(const Chunk &e, const uint64_t *inter, const double *dist) {}
+};
+
+// a read of `bytes` from the device into dst (host or device memory), skipped when dst is nullptr; counted in d2h
+int read_back(gkd_ctx *c, void *dst, const void *src, uint64_t bytes, uint64_t &d2h) {
+    if (!dst || !bytes) return GKD_OK;
+    CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, c->stream));
+    d2h += bytes;
+    return GKD_OK;
+}
+
+// kernel 5, dense form: the chunk's values to o[0, cnt); a nullptr member of o is not computed
+int dense_epilogue(gkd_ctx *c, const Chunk &e, const gkd_outputs &o, uint64_t &d2h) {
+    int rc;
+    if (o.inter && (rc = ensure(c, c->d_inter, e.cnt * 8))) return rc;
+    if (o.dist && (rc = ensure(c, c->d_dist, e.cnt * 8))) return rc;
+    if (o.contain_a && (rc = ensure(c, c->d_ca, e.cnt * 8))) return rc;
+    if (o.contain_b && (rc = ensure(c, c->d_cb, e.cnt * 8))) return rc;
+    EpilogueOut eo{o.inter ? (uint64_t *)c->d_inter.p : nullptr, o.dist ? (double *)c->d_dist.p : nullptr,
+                   o.contain_a ? (double *)c->d_ca.p : nullptr, o.contain_b ? (double *)c->d_cb.p : nullptr};
+    nvtxRangePushA("gkd kernel 5: distance epilogue");
+    CK(launch_epilogue(e.sets, e.src, e.counts, e.pal, e.both, eo, c->stream));
+    nvtxRangePop();
+    c->m.launches++;
+    CK(cudaEventRecord(c->ev[7], c->stream));
+    // queued before the overflow flag is read: a redo rewrites the same slots
+    if ((rc = read_back(c, o.inter, c->d_inter.p, e.cnt * 8, d2h)) || (rc = read_back(c, o.dist, c->d_dist.p, e.cnt * 8, d2h)) ||
+        (rc = read_back(c, o.contain_a, c->d_ca.p, e.cnt * 8, d2h)) || (rc = read_back(c, o.contain_b, c->d_cb.p, e.cnt * 8, d2h)))
+        return rc;
+    return GKD_OK;
+}
+
+// gkd_all_vs_all*, gkd_query_vs_ref*, gkd_pairs*: every pair's values to the caller's outputs
+struct Dense : Form {
+    gkd_outputs out;
+    explicit Dense(const gkd_outputs &o) : out(o) {}
+    gkd_outputs at(const Chunk &e) const {  // the chunk's part of out (RECT: from row a_base of the caller's block)
+        const uint64_t t = (uint64_t)a_base * e.hp.nb + e.done;
+        return gkd_outputs{out.inter ? out.inter + t : nullptr, out.dist ? out.dist + t : nullptr,
+                           out.contain_a ? out.contain_a + t : nullptr, out.contain_b ? out.contain_b + t : nullptr};
+    }
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override { return dense_epilogue(c, e, at(e), d2h); }
+    gkd_outputs literal_outputs(const Chunk &e) override {
+        gkd_outputs o = at(e);
+        if (!o.inter) {
+            lit_inter.resize(e.cnt);
+            o.inter = lit_inter.data();
+        }
+        return o;
+    }
+};
+
+int run_pairs(gkd_ctx *c, const HostPairs &hp, Form &f) {
+    int rc = upload_sets(c);
+    if (rc) return rc;
+    const bool nuc = c->cfg.alphabet != GKD_PROT;
+    const bool both = nuc && c->cfg.strand_mode == GKD_STRAND_BOTH;
+    const bool need_pal = both && (c->k % 2 == 0);
+    c->m.pairs = hp.count;
+    c->m.intersect_bytes = 0;
+    c->m.intersect_ms = c->m.epilogue_ms = 0;
+
+    // validate ids, gather sizes for the work split and the byte accounting
+    SetScan s;
+    long double sum_bytes = 0;
+    auto size_of = [&](uint32_t id) -> uint64_t { return c->genomes[id].desc.main.n; };
+    if (hp.mode == PAIRS_UPPER) {
+        for (uint32_t i = 0; i < hp.n; i++)
+            if ((rc = s.see(c, i))) return rc;
+        // bytes of the requested range, row by row
+        uint32_t i0 = 0, j0 = 1;
+        if (hp.count) upper_pair(hp.first, hp.n, i0, j0);
+        uint64_t left = hp.count;
+        std::vector<uint64_t> prefix(hp.n + 1, 0);
+        for (uint32_t i = 0; i < hp.n; i++) prefix[i + 1] = prefix[i] + size_of(i);
+        for (uint32_t i = i0, j = j0; left > 0 && i + 1 < hp.n; i++, j = i + 1) {
+            uint64_t in_row = std::min<uint64_t>(left, hp.n - j);
+            sum_bytes += 8.0L * ((long double)in_row * size_of(i) + (long double)(prefix[j + in_row] - prefix[j]));
+            left -= in_row;
+        }
+    } else if (hp.mode == PAIRS_RECT) {
+        uint64_t sq = 0, sr = 0;
+        for (uint32_t i = 0; i < hp.na; i++) {
+            if ((rc = s.see(c, hp.a[i]))) return rc;
+            sq += size_of(hp.a[i]);
+        }
+        for (uint32_t i = 0; i < hp.nb; i++) {
+            if ((rc = s.see(c, hp.b[i]))) return rc;
+            sr += size_of(hp.b[i]);
+        }
+        sum_bytes = 8.0L * ((long double)sq * hp.nb + (long double)sr * hp.na);
+    } else {
+        for (uint64_t t = 0; t < hp.count; t++) {
+            if ((rc = s.see(c, hp.a[t])) || (rc = s.see(c, hp.b[t]))) return rc;
+            sum_bytes += 8.0L * (size_of(hp.a[t]) + size_of(hp.b[t]));
+        }
+    }
+    c->m.intersect_bytes = (uint64_t)sum_bytes;
+    c->m.total_intersect_bytes += (uint64_t)sum_bytes;
+    c->m.total_pairs += hp.count;
+    if (hp.count == 0) return GKD_OK;
+    const IsectPlan plan = make_plan(c, hp.count, s.max_n, s.max_level, false);
+    const IsectPlan pal_plan = make_plan(c, hp.count, s.max_pal, s.max_pal_level, true);
+
+    // device id arrays
+    PairSource src{};
+    src.mode = hp.mode;
+    src.n = hp.n;
+    if (hp.mode != PAIRS_UPPER) {
+        if ((rc = ensure(c, c->ids_a, (uint64_t)hp.na * 4))) return rc;
+        if ((rc = ensure(c, c->ids_b, (uint64_t)hp.nb * 4))) return rc;
+        CK(cudaMemcpyAsync(c->ids_a.p, hp.a, (uint64_t)hp.na * 4, cudaMemcpyHostToDevice, c->stream));
+        CK(cudaMemcpyAsync(c->ids_b.p, hp.b, (uint64_t)hp.nb * 4, cudaMemcpyHostToDevice, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+    }
+    if ((rc = ensure(c, c->work_counter, 8))) return rc;
+
+    bool join_banned = false;  // set when a join table overflowed: the chunk is redone by the merge kernel
+    JoinPlan jplan{};
+    std::vector<uint32_t> jrows;
+    for (uint64_t done = 0; done < hp.count;) {
+        const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, hp.count - done);
+        src.count = cnt;
+        bool jswapped = false;
+        const bool use_join = !join_banned && plan_join(c, hp, hp.mode == PAIRS_UPPER ? hp.first + done : 0, cnt, jplan, jrows, jswapped);
+        if (hp.mode == PAIRS_UPPER) {
+            src.first = hp.first + done;
+            src.a = src.b = nullptr;
+        } else if (hp.mode == PAIRS_RECT) {
+            // run_rect splits by query rows, so a rectangle always fits one launch
+            src.first = 0;
+            src.a = (const uint32_t *)c->ids_a.p;
+            src.b = (const uint32_t *)c->ids_b.p;
+            if (hp.count > PAIR_CHUNK) return fail(c, GKD_EINVAL, "query x reference block larger than %llu pairs", (unsigned long long)PAIR_CHUNK);
+        } else {
+            src.first = 0;
+            src.a = (const uint32_t *)c->ids_a.p + done;
+            src.b = (const uint32_t *)c->ids_b.p + done;
+        }
+        if ((rc = ensure(c, c->counts, cnt * 4))) return rc;
+        CK(cudaMemsetAsync(c->counts.p, 0, cnt * 4, c->stream));
+        if (need_pal) {
+            if ((rc = ensure(c, c->pal_counts, cnt * 4))) return rc;
+            CK(cudaMemsetAsync(c->pal_counts.p, 0, cnt * 4, c->stream));
+        }
+
+        if (use_join) {
+            if ((rc = ensure(c, c->join_rows, jrows.size() * 4))) return rc;
+            if ((rc = ensure(c, c->join_err, 4))) return rc;
+            CK(cudaMemcpyAsync(c->join_rows.p, jrows.data(), jrows.size() * 4, cudaMemcpyHostToDevice, c->stream));
+            CK(cudaMemsetAsync(c->join_err.p, 0, 4, c->stream));
+            jplan.rows = (const uint32_t *)c->join_rows.p;
+            if (hp.mode == PAIRS_RECT) {
+                jplan.row_ids = (const uint32_t *)(jswapped ? c->ids_b.p : c->ids_a.p);
+                jplan.col_ids = (const uint32_t *)(jswapped ? c->ids_a.p : c->ids_b.p);
+            }
+        }
+        CK(cudaEventRecord(c->ev[4], c->stream));
+        if (use_join) {
+            nvtxRangePushA("gkd kernel 4: block join");
+            CK(launch_join((const SetDesc *)c->d_sets.p, jplan, (uint32_t *)c->counts.p,
+                           (unsigned long long *)c->work_counter.p, (uint32_t *)c->join_err.p, c->n_sms, c->stream));
+        } else {
+            nvtxRangePushA("gkd kernel 4: bucket-merge intersect");
+            CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 0, plan, (uint32_t *)c->counts.p,
+                                (unsigned long long *)c->work_counter.p, c->n_sms, c->stream));
+        }
+        nvtxRangePop();
+        CK(cudaEventRecord(c->ev[5], c->stream));
+        c->m.intersect_kernel = use_join ? 5u : (c->low_bits == 32 ? 3u : 4u);
+        uint32_t join_err = 0;
+        if (use_join) {
+            // a table that would overflow flags the launch; the chunk is then redone by the merge kernel
+            CK(cudaMemcpyAsync(&join_err, c->join_err.p, 4, cudaMemcpyDeviceToHost, c->stream));
+        }
+        c->m.launches++;
+        c->m.intersect_launches++;
+        if (need_pal && s.max_pal) {
+            CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 1, pal_plan, (uint32_t *)c->pal_counts.p,
+                                (unsigned long long *)c->work_counter.p, c->n_sms, c->stream));
+            c->m.launches++;
+        }
+        CK(cudaEventRecord(c->ev[6], c->stream));
+        const Chunk e{hp, src, done, cnt, (const SetDesc *)c->d_sets.p, (const uint32_t *)c->counts.p,
+                      need_pal ? (const uint32_t *)c->pal_counts.p : nullptr, both ? 1 : 0,
+                      use_join ? (const uint32_t *)c->join_err.p : nullptr};
+        // with literal side lists the pairs are completed on the host, which needs the counts: the dense epilogue runs
+        // into host memory and the form takes the completed pairs
+        uint64_t d2h = 0;
+        const gkd_outputs lit = s.any_lit ? f.literal_outputs(e) : gkd_outputs{};
+        if ((rc = s.any_lit ? dense_epilogue(c, e, lit, d2h) : f.queue(c, e, d2h))) return rc;
+        CK(cudaStreamSynchronize(c->stream));
+        if (join_err) {  // the attempt keeps nothing
+            join_banned = true;
+            continue;
+        }
+        if (!s.any_lit && (rc = f.keep(c, e, d2h))) return rc;
+        c->m.d2h_bytes += d2h;
+        const double ims = elapsed(c->ev[4], c->ev[5]);
+        c->m.intersect_ms += ims;
+        c->m.total_intersect_ms += ims;
+        c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+        if (s.any_lit) {
+            // GKD_AMBIG_LITERAL: add the literal k-mers both sets share and redo the formula with the
+            // full sizes (outputs must be host memory in this mode)
+            for (uint64_t t = 0; t < cnt; t++) {
+                uint32_t a, b;
+                host_pair_ids(hp, done + t, a, b);
+                const GenomeRec &ga = c->genomes[a], &gb = c->genomes[b];
+                if (ga.lit.empty() && gb.lit.empty()) continue;
+                const uint64_t I = lit.inter[t] + literal_intersection(ga.lit, gb.lit);
+                const uint64_t sa = both_size(c, ga), sb = both_size(c, gb);
+                lit.inter[t] = I;
+                if (lit.dist) lit.dist[t] = host_distance(I, sa, sb);
+                if (lit.contain_a) lit.contain_a[t] = sa ? (double)I / (double)sa : 0.0;
+                if (lit.contain_b) lit.contain_b[t] = sb ? (double)I / (double)sb : 0.0;
+            }
+            f.host(e, lit.inter, lit.dist);
+        }
+        done += PAIR_CHUNK;
+    }
+    return GKD_OK;
+}
+
+// A query x reference call, split by query rows so that each launch stays under PAIR_CHUNK pairs and every row is
+// complete in one launch; f.a_base is the launch's first row.  The call's metrics add up its launches.
+int run_rect(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, Form &f) {
+    const uint32_t rows_per = (uint32_t)std::max<uint64_t>(1, PAIR_CHUNK / nr);
+    uint64_t pairs = 0, bytes = 0;
+    double ims = 0, ems = 0;
+    for (uint32_t q0 = 0; q0 < nq; q0 += rows_per) {
+        const uint32_t rows = std::min(rows_per, nq - q0);
+        HostPairs hp{PAIRS_RECT, nr, 0, (uint64_t)rows * nr, q + q0, r, rows, nr};
+        f.a_base = q0;
+        const int rc = run_pairs(c, hp, f);
+        if (rc) return rc;
+        pairs += c->m.pairs;
+        bytes += c->m.intersect_bytes;
+        ims += c->m.intersect_ms;
+        ems += c->m.epilogue_ms;
+    }
+    c->m.pairs = pairs;
+    c->m.intersect_bytes = bytes;
+    c->m.intersect_ms = ims;
+    c->m.epilogue_ms = ems;
+    return GKD_OK;
+}
+
+// ---- selection forms --------------------------------------------------------------------------------------------
+// gkd_*_within: the pairs with dist <= max_dist, in enumeration order, to the caller's hits.  hits.n counts every hit so
+// far and is the next write position, so a chunk's hits are read back only once the chunk is kept.
+struct Within : Form {
+    double max_dist;
+    gkd_hits &h;
+    uint64_t wcap = 0;  // hits of the chunk the device buffers hold
+    unsigned long long chunk_hits = 0;
+    Within(double d, gkd_hits &hits) : max_dist(d), h(hits) {}
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        const bool any_out = h.a || h.b || h.inter || h.dist;
+        wcap = (any_out && h.n < h.cap) ? std::min<uint64_t>(e.cnt, h.cap - h.n) : 0;
+        const uint64_t nctas = select_within_ctas(e.cnt);
+        int rc;
+        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
+        if (h.a && (rc = ensure(c, c->hit_a, wcap * 4))) return rc;
+        if (h.b && (rc = ensure(c, c->hit_b, wcap * 4))) return rc;
+        if (h.inter && (rc = ensure(c, c->d_inter, wcap * 8))) return rc;
+        if (h.dist && (rc = ensure(c, c->d_dist, wcap * 8))) return rc;
+        const HitsOut ho{h.a ? (uint32_t *)c->hit_a.p : nullptr, h.b ? (uint32_t *)c->hit_b.p : nullptr,
+                         h.inter ? (uint64_t *)c->d_inter.p : nullptr, h.dist ? (double *)c->d_dist.p : nullptr};
+        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
+        nvtxRangePushA("gkd kernel 5: within selection");
+        CK(launch_select_within(e.sets, e.src, e.counts, e.pal, e.both, max_dist, a_base, wcap, ho, cta, cta + nctas, c->stream));
+        nvtxRangePop();
+        c->m.launches += wcap ? 3 : 2;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
+        d2h += 8;
+        return GKD_OK;
+    }
+    int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        const uint64_t w = std::min<uint64_t>(chunk_hits, wcap);
+        int rc;
+        if ((rc = read_back(c, h.a ? h.a + h.n : nullptr, c->hit_a.p, w * 4, d2h)) ||
+            (rc = read_back(c, h.b ? h.b + h.n : nullptr, c->hit_b.p, w * 4, d2h)) ||
+            (rc = read_back(c, h.inter ? h.inter + h.n : nullptr, c->d_inter.p, w * 8, d2h)) ||
+            (rc = read_back(c, h.dist ? h.dist + h.n : nullptr, c->d_dist.p, w * 8, d2h)))
+            return rc;
+        CK(cudaStreamSynchronize(c->stream));
+        h.n += chunk_hits;
+        return GKD_OK;
+    }
+    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {
+        for (uint64_t t = 0; t < e.cnt; t++) {
+            if (!(dist[t] <= max_dist)) continue;
+            const uint64_t at = h.n++;
+            if (at >= h.cap) continue;
+            uint32_t a, b;
+            e.pair(a_base, t, a, b);
+            if (h.a) h.a[at] = a;
+            if (h.b) h.b[at] = b;
+            if (h.inter) h.inter[at] = inter[t];
+            if (h.dist) h.dist[at] = dist[t];
+        }
+    }
+};
+
 // GKD_AMBIG_LITERAL: the per-target lists of an accumulating nearest selection, kept on the host because the pairs
 // are completed there.  Same layout and unused entry as the device lists (c->nn_*); n[t] entries of target t are used.
 struct HostLists {
@@ -990,535 +1375,343 @@ struct HostLists {
     }
 };
 
-// One linkage call: the forest of its launches so far.  Node of a reported edge (a, b): a and b + b_off.
-struct LinkCall {
-    uint32_t nodes = 0, b_off = 0;
-    std::vector<uint32_t> key;   // key of every node (empty: the node itself); uploaded to c->lk_state when not empty
-    uint32_t n_dev = 0;          // edges of the device forest c->lk_forest
-    std::vector<LinkEdge> host;  // GKD_AMBIG_LITERAL: the forest of the pairs completed on the host
+// gkd_*_nearest: the k nearest within max_dist by (distance bits, position).  rows (RECT only): each query row's list,
+// complete in every launch (k_select_nearest) and read back once the chunk is kept.  lists: per-target lists that the
+// launches merge into (k_nearest_absorb; UPPER: both ends of every pair, RECT: each reference's nearest queries), on the
+// device (c->nn_*) or, when the pairs are completed on the host, in host_lists; read once by finish().
+struct Nearest : Form {
+    uint32_t k;
+    double max_dist;
+    int exclude_self;
+    const gkd_neighbors *rows, *lists;  // either may be nullptr
+    uint32_t targets;
+    std::unique_ptr<HostLists> host_lists;
+    Nearest(uint32_t k_, double d, int excl, const gkd_neighbors *rows_, const gkd_neighbors *lists_, uint32_t targets_)
+        : k(k_), max_dist(d), exclude_self(excl), rows(rows_), lists(lists_), targets(targets_) {}
+    int start(gkd_ctx *c) {  // every per-target list unused
+        if (!lists) return GKD_OK;
+        if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) host_lists.reset(new HostLists(targets, k));
+        const uint64_t slots = (uint64_t)targets * k;
+        int rc;
+        if ((rc = ensure(c, c->nn_pos, slots * 4)) || (rc = ensure(c, c->nn_inter, slots * 8)) ||
+            (rc = ensure(c, c->nn_dist, slots * 8)) || (rc = ensure(c, c->nn_found, (uint64_t)targets * 4)))
+            return rc;
+        const double none = -1.0;
+        uint64_t none_bits;
+        std::memcpy(&none_bits, &none, 8);
+        CK(cudaMemsetAsync(c->nn_pos.p, 0xFF, slots * 4, c->stream));
+        CK(cudaMemsetAsync(c->nn_inter.p, 0, slots * 8, c->stream));
+        CK(cudaMemsetAsync(c->nn_found.p, 0, (uint64_t)targets * 4, c->stream));
+        CK(launch_fill_u64((uint64_t *)c->nn_dist.p, slots, none_bits, c->stream));
+        c->m.launches++;
+        return GKD_OK;
+    }
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        int rc;
+        if (rows) {
+            const uint64_t slots = (uint64_t)e.hp.na * k;
+            if (rows->pos && (rc = ensure(c, c->hit_a, slots * 4))) return rc;
+            if (rows->n_found && (rc = ensure(c, c->hit_b, (uint64_t)e.hp.na * 4))) return rc;
+            if (rows->inter && (rc = ensure(c, c->d_inter, slots * 8))) return rc;
+            if (rows->dist && (rc = ensure(c, c->d_dist, slots * 8))) return rc;
+            const NearestOut no{rows->pos ? (uint32_t *)c->hit_a.p : nullptr, rows->inter ? (uint64_t *)c->d_inter.p : nullptr,
+                                rows->dist ? (double *)c->d_dist.p : nullptr, rows->n_found ? (uint32_t *)c->hit_b.p : nullptr};
+            nvtxRangePushA("gkd kernel 5: nearest selection");
+            CK(launch_select_nearest(e.sets, e.src, e.hp.na, e.counts, e.pal, e.both, max_dist, k, exclude_self, no, c->stream));
+            nvtxRangePop();
+            c->m.launches++;
+        }
+        if (lists) {
+            // the lists outlive this chunk: the kernel itself skips a chunk whose join overflowed
+            const NearestOut st{(uint32_t *)c->nn_pos.p, (uint64_t *)c->nn_inter.p, (double *)c->nn_dist.p, (uint32_t *)c->nn_found.p};
+            nvtxRangePushA("gkd kernel 5: nearest absorb");
+            CK(launch_nearest_absorb(e.sets, e.src, e.counts, e.pal, e.both, max_dist, k, exclude_self, a_base, e.join_err, st, c->stream));
+            nvtxRangePop();
+            c->m.launches++;
+        }
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        return GKD_OK;
+    }
+    int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        if (!rows) return GKD_OK;
+        const uint64_t slots = (uint64_t)e.hp.na * k, at = (uint64_t)a_base * k;
+        int rc;
+        if ((rc = read_back(c, rows->pos ? rows->pos + at : nullptr, c->hit_a.p, slots * 4, d2h)) ||
+            (rc = read_back(c, rows->inter ? rows->inter + at : nullptr, c->d_inter.p, slots * 8, d2h)) ||
+            (rc = read_back(c, rows->dist ? rows->dist + at : nullptr, c->d_dist.p, slots * 8, d2h)) ||
+            (rc = read_back(c, rows->n_found ? rows->n_found + a_base : nullptr, c->hit_b.p, (uint64_t)e.hp.na * 4, d2h)))
+            return rc;
+        CK(cudaStreamSynchronize(c->stream));
+        return GKD_OK;
+    }
+    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {
+        const HostPairs &hp = e.hp;
+        for (uint64_t t = 0; lists && t < e.cnt; t++) {
+            if (!(dist[t] <= max_dist)) continue;
+            if (hp.mode == PAIRS_RECT) {
+                const uint32_t row = (uint32_t)((e.done + t) / hp.nb), j = (uint32_t)((e.done + t) % hp.nb);
+                if (!(exclude_self && hp.a[row] == hp.b[j])) host_lists->offer(j, a_base + row, inter[t], dist[t]);
+            } else {
+                uint32_t a, b;
+                host_pair_ids(hp, e.done + t, a, b);
+                host_lists->offer(a, b, inter[t], dist[t]);
+                host_lists->offer(b, a, inter[t], dist[t]);
+            }
+        }
+        if (!rows) return;
+        std::vector<uint32_t> js;
+        for (uint32_t row = 0; row < hp.na; row++) {
+            const uint64_t r0 = (uint64_t)row * hp.nb;
+            js.clear();
+            for (uint32_t j = 0; j < hp.nb; j++)
+                if (dist[r0 + j] <= max_dist && !(exclude_self && hp.a[row] == hp.b[j])) js.push_back(j);
+            const size_t m = std::min<size_t>(js.size(), k);
+            std::partial_sort(js.begin(), js.begin() + m, js.end(), [&](uint32_t x, uint32_t y) {
+                return dist[r0 + x] < dist[r0 + y] || (dist[r0 + x] == dist[r0 + y] && x < y);
+            });
+            for (uint32_t i = 0; i < k; i++) {
+                const uint64_t o = (uint64_t)(a_base + row) * k + i;
+                if (rows->pos) rows->pos[o] = i < m ? js[i] : 0xFFFFFFFFu;
+                if (rows->inter) rows->inter[o] = i < m ? inter[r0 + js[i]] : 0;
+                if (rows->dist) rows->dist[o] = i < m ? dist[r0 + js[i]] : -1.0;
+            }
+            if (rows->n_found) rows->n_found[a_base + row] = (uint32_t)m;
+        }
+    }
+    // the lists to the caller, once, at the end of the call.  With host_lists (GKD_AMBIG_LITERAL, host outputs) the
+    // launches that ran on the device are merged into the host lists first.
+    int finish(gkd_ctx *c) {
+        if (!lists) return GKD_OK;
+        const gkd_neighbors &out = *lists;
+        const uint64_t slots = (uint64_t)targets * k;
+        int rc;
+        if (!host_lists) {
+            uint64_t d2h = 0;
+            if ((rc = read_back(c, out.pos, c->nn_pos.p, slots * 4, d2h)) || (rc = read_back(c, out.inter, c->nn_inter.p, slots * 8, d2h)) ||
+                (rc = read_back(c, out.dist, c->nn_dist.p, slots * 8, d2h)) ||
+                (rc = read_back(c, out.n_found, c->nn_found.p, (uint64_t)targets * 4, d2h)))
+                return rc;
+            CK(cudaStreamSynchronize(c->stream));
+            c->m.d2h_bytes += d2h;
+            return GKD_OK;
+        }
+        HostLists dev(targets, k);
+        CK(cudaMemcpyAsync(dev.pos.data(), c->nn_pos.p, slots * 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(dev.inter.data(), c->nn_inter.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(dev.dist.data(), c->nn_dist.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += slots * 20;
+        HostLists &hl = *host_lists;
+        for (uint32_t t = 0; t < targets; t++)
+            for (uint64_t s = (uint64_t)t * k; s < (uint64_t)(t + 1) * k && dev.pos[s] != 0xFFFFFFFFu; s++)
+                hl.offer(t, dev.pos[s], dev.inter[s], dev.dist[s]);
+        if (out.pos) std::memcpy(out.pos, hl.pos.data(), slots * 4);
+        if (out.inter) std::memcpy(out.inter, hl.inter.data(), slots * 8);
+        if (out.dist) std::memcpy(out.dist, hl.dist.data(), slots * 8);
+        if (out.n_found) std::memcpy(out.n_found, hl.n.data(), (uint64_t)targets * 4);
+        return GKD_OK;
+    }
+};
+
+// gkd_*_clusters: the pairs within max_dist link their nodes in the union-find forest c->uf_parent (k_cluster_link;
+// RECT: query row r is node a_base + r, reference column j is node b_base + j), or in host_forest when the pairs are
+// completed on the host.  Nothing is read back before finish().
+struct Clusters : Form {
+    double max_dist;
+    uint32_t nodes, b_base;
+    std::unique_ptr<HostForest> host_forest;
+    Clusters(double d, uint32_t nodes_, uint32_t b_base_) : max_dist(d), nodes(nodes_), b_base(b_base_) {}
+    int start(gkd_ctx *c) {  // every node its own root
+        if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) host_forest.reset(new HostForest(nodes));
+        const int rc = ensure(c, c->uf_parent, ((uint64_t)nodes + 1) * 4);
+        if (rc) return rc;
+        CK(launch_cluster_init((uint32_t *)c->uf_parent.p, nodes, c->stream));
+        c->m.launches++;
+        return GKD_OK;
+    }
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        // the forest outlives this chunk: the kernel itself skips a chunk whose join overflowed
+        nvtxRangePushA("gkd kernel 5: cluster link");
+        CK(launch_cluster_link(e.sets, e.src, e.counts, e.pal, e.both, max_dist, a_base, b_base, e.join_err,
+                               (uint32_t *)c->uf_parent.p, c->stream));
+        nvtxRangePop();
+        c->m.launches++;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        return GKD_OK;
+    }
+    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {  // the rule of k_cluster_link
+        for (uint64_t t = 0; t < e.cnt; t++) {
+            if (!(dist[t] <= max_dist)) continue;
+            uint32_t a, b;
+            e.pair(a_base, t, a, b);
+            host_forest->link(a, b_base + b);
+        }
+    }
+    // The labels to the caller, once, at the end of the call: nodes [0, na) to a_out and [na, nodes) to b_out (either
+    // may be NULL).  With host_forest the launches that ran on the device are merged into it first: every node is linked
+    // to its device label, which carries all of the device links' connectivity.
+    int finish(gkd_ctx *c, uint32_t *a_out, uint32_t na, uint32_t *b_out, uint32_t *n_clusters) {
+        uint32_t *parent = (uint32_t *)c->uf_parent.p;
+        CK(cudaEventRecord(c->ev[6], c->stream));
+        CK(launch_cluster_flatten(parent, nodes, c->stream));
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        c->m.launches++;
+        uint32_t roots = 0;
+        if (!host_forest) {
+            const uint32_t nb = nodes - na;
+            if (a_out && na) CK(cudaMemcpyAsync(a_out, parent, (uint64_t)na * 4, cudaMemcpyDefault, c->stream));
+            if (b_out && nb) CK(cudaMemcpyAsync(b_out, parent + na, (uint64_t)nb * 4, cudaMemcpyDefault, c->stream));
+            CK(cudaMemcpyAsync(&roots, parent + nodes, 4, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            c->m.d2h_bytes += (a_out ? (uint64_t)na * 4 : 0) + (b_out ? (uint64_t)nb * 4 : 0) + 4;
+        } else {
+            std::vector<uint32_t> dev(nodes);
+            CK(cudaMemcpyAsync(dev.data(), parent, (uint64_t)nodes * 4, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            c->m.d2h_bytes += (uint64_t)nodes * 4;
+            for (uint32_t x = 0; x < nodes; x++)
+                if (dev[x] != x) host_forest->link(x, dev[x]);
+            for (uint32_t x = 0; x < nodes; x++) {
+                const uint32_t r = host_forest->find(x);
+                roots += r == x ? 1u : 0u;
+                if (x < na && a_out) a_out[x] = r;
+                if (x >= na && b_out) b_out[x - na] = r;
+            }
+        }
+        c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+        if (n_clusters) *n_clusters = roots;
+        return GKD_OK;
+    }
+};
+
+// gkd_*_linkage: the call's forest so far is replaced, chunk by chunk, with MSF(forest u the chunk's pairs within
+// max_dist).  Node of a reported edge (a, b): a and b + b_off.
+struct Linkage : Form {
+    double max_dist;
+    uint32_t nodes, b_off;
+    std::vector<uint32_t> key;        // key of every node (empty: the node itself); uploaded to c->lk_state when not empty
+    uint32_t n_dev = 0;               // edges of the device forest c->lk_forest
+    std::vector<LinkEdge> host_edges;  // GKD_AMBIG_LITERAL: the forest of the pairs completed on the host
+    unsigned long long chunk_hits = 0;
+    Linkage(double d, uint32_t nodes_, uint32_t b_off_, std::vector<uint32_t> key_)
+        : max_dist(d), nodes(nodes_), b_off(b_off_), key(std::move(key_)) {}
     LinkEdge edge(uint32_t a, uint32_t b, uint64_t inter, double dist) const {
         const uint32_t na = a, nb = b + b_off;
         return link_edge(a, b, inter, dist, na, nb, key.empty() ? na : key[na], key.empty() ? nb : key[nb]);
     }
-};
-
-// What a selection call wants instead of the dense outputs (run_pairs with sel == nullptr writes gkd_outputs).
-struct Selection {
-    bool within;          // true: pairs with dist <= max_dist (gkd_hits); false: k nearest (rows and / or absorb) or clusters
-    double max_dist;
-    gkd_hits *hits;       // within: the caller's arrays; hits->n counts the hits so far and is the next write position
-    uint32_t a_base;      // RECT: position in the caller's q of the first query row of this call
-    uint32_t k;           // nearest
-    int exclude_self;
-    bool rows;            // nearest, RECT: each query row's list, complete in this call (k_select_nearest) ...
-    uint32_t *ref_pos;    // ... written to these outputs of the call's first row (host or device memory)
-    uint64_t *inter;
-    double *dist;
-    uint32_t *n_found;
-    bool absorb;          // nearest: merge the call into the per-target lists c->nn_* (UPPER: both ends of every pair;
-                          // RECT: each reference's nearest queries), or into host_lists when the pairs are completed
-    HostLists *host_lists;  // on the host (GKD_AMBIG_LITERAL; nullptr otherwise)
-    bool cluster;         // link the pairs within max_dist in the forest c->uf_parent (RECT: reference column j is node
-    uint32_t b_base;      // b_base + j, query row r is node a_base + r), or in host_forest when the pairs are completed
-    HostForest *host_forest;  // on the host (GKD_AMBIG_LITERAL; nullptr otherwise)
-    LinkCall *link;       // linkage: replace the call's forest with MSF(forest u the chunk's pairs within max_dist)
-};
-
-// GKD_AMBIG_LITERAL: the chunk's pairs were completed on the host (inter / dist of pairs done .. done+cnt), so the
-// selection runs here with the device kernels' rules
-void host_select(const HostPairs &hp, const Selection &sel, uint64_t done, uint64_t cnt, const uint64_t *inter, const double *dist) {
-    if (sel.within) {
-        gkd_hits &h = *sel.hits;
-        for (uint64_t t = 0; t < cnt; t++) {
-            if (!(dist[t] <= sel.max_dist)) continue;
-            const uint64_t at = h.n++;
-            if (at >= h.cap) continue;
-            uint32_t a, b;
-            if (hp.mode == PAIRS_RECT) a = sel.a_base + (uint32_t)((done + t) / hp.nb), b = (uint32_t)((done + t) % hp.nb);
-            else host_pair_ids(hp, done + t, a, b);
-            if (h.a) h.a[at] = a;
-            if (h.b) h.b[at] = b;
-            if (h.inter) h.inter[at] = inter[t];
-            if (h.dist) h.dist[at] = dist[t];
-        }
-        return;
-    }
-    if (sel.cluster) {  // the rule of k_cluster_link
-        for (uint64_t t = 0; t < cnt; t++) {
-            if (!(dist[t] <= sel.max_dist)) continue;
-            if (hp.mode == PAIRS_RECT) {
-                sel.host_forest->link(sel.a_base + (uint32_t)((done + t) / hp.nb), sel.b_base + (uint32_t)((done + t) % hp.nb));
-            } else {
-                uint32_t a, b;
-                host_pair_ids(hp, done + t, a, b);
-                sel.host_forest->link(a, b);
-            }
-        }
-        return;
-    }
-    if (sel.link) {  // Kruskal on the host forest and the chunk's edges, in the order of k_link_edges
-        LinkCall &L = *sel.link;
-        for (uint64_t t = 0; t < cnt; t++) {
-            if (!(dist[t] <= sel.max_dist)) continue;
-            uint32_t a, b;
-            if (hp.mode == PAIRS_RECT) a = sel.a_base + (uint32_t)((done + t) / hp.nb), b = (uint32_t)((done + t) % hp.nb);
-            else host_pair_ids(hp, done + t, a, b);
-            L.host.push_back(L.edge(a, b, inter[t], dist[t]));
-        }
-        host_msf(L.host, L.nodes);
-        return;
-    }
-    if (sel.absorb) {
-        for (uint64_t t = 0; t < cnt; t++) {
-            if (!(dist[t] <= sel.max_dist)) continue;
-            if (hp.mode == PAIRS_RECT) {
-                const uint32_t row = (uint32_t)((done + t) / hp.nb), j = (uint32_t)((done + t) % hp.nb);
-                if (!(sel.exclude_self && hp.a[row] == hp.b[j])) sel.host_lists->offer(j, sel.a_base + row, inter[t], dist[t]);
-            } else {
-                uint32_t a, b;
-                host_pair_ids(hp, done + t, a, b);
-                sel.host_lists->offer(a, b, inter[t], dist[t]);
-                sel.host_lists->offer(b, a, inter[t], dist[t]);
-            }
-        }
-    }
-    if (!sel.rows) return;
-    std::vector<uint32_t> js;
-    for (uint32_t row = 0; row < hp.na; row++) {
-        const uint64_t r0 = (uint64_t)row * hp.nb;
-        js.clear();
-        for (uint32_t j = 0; j < hp.nb; j++)
-            if (dist[r0 + j] <= sel.max_dist && !(sel.exclude_self && hp.a[row] == hp.b[j])) js.push_back(j);
-        const size_t m = std::min<size_t>(js.size(), sel.k);
-        std::partial_sort(js.begin(), js.begin() + m, js.end(), [&](uint32_t x, uint32_t y) {
-            return dist[r0 + x] < dist[r0 + y] || (dist[r0 + x] == dist[r0 + y] && x < y);
-        });
-        for (uint32_t i = 0; i < sel.k; i++) {
-            const uint64_t o = (uint64_t)row * sel.k + i;
-            if (sel.ref_pos) sel.ref_pos[o] = i < m ? js[i] : 0xFFFFFFFFu;
-            if (sel.inter) sel.inter[o] = i < m ? inter[r0 + js[i]] : 0;
-            if (sel.dist) sel.dist[o] = i < m ? dist[r0 + js[i]] : -1.0;
-        }
-        if (sel.n_found) sel.n_found[row] = (uint32_t)m;
-    }
-}
-
-constexpr int SELECT_REDO = 1;  // select_chunk: a join table overflowed; nothing of the attempt was kept
-
-// Linkage, one chunk whose n_chunk edges are compacted at the front of hit_a / hit_b / d_inter / d_dist: the forest so
-// far is copied behind them and the Boruvka rounds replace it with MSF(forest u chunk).  Records ev[7] after the
-// rounds and reads the new forest's size (4 bytes).
-static int link_chunk(gkd_ctx *c, LinkCall &L, uint64_t n_chunk) {
-    if (n_chunk == 0) {  // the forest stands
-        CK(cudaEventRecord(c->ev[7], c->stream));
-        CK(cudaStreamSynchronize(c->stream));
+    int start(gkd_ctx *c) {  // an empty forest on the device, and the node keys there when the caller passed any
+        int rc;
+        if ((rc = ensure(c, c->lk_forest, (uint64_t)nodes * 24)) || (rc = ensure(c, c->lk_state, link_state_bytes(nodes))))
+            return rc;
+        if (!key.empty())
+            CK(cudaMemcpyAsync(link_state_at(c->lk_state.p, nodes).key, key.data(), (uint64_t)nodes * 4, cudaMemcpyHostToDevice,
+                               c->stream));
+        n_dev = 0;
         return GKD_OK;
     }
-    const uint32_t N = L.nodes;
-    uint64_t *fi = (uint64_t *)c->lk_forest.p;  // 24 B per node: inter, dist, a, b
-    double *fd = (double *)(fi + N);
-    uint32_t *fa = (uint32_t *)(fd + N), *fb = fa + N;
-    const uint64_t f = L.n_dev;
-    if (f) {
-        CK(cudaMemcpyAsync((uint32_t *)c->hit_a.p + n_chunk, fa, f * 4, cudaMemcpyDeviceToDevice, c->stream));
-        CK(cudaMemcpyAsync((uint32_t *)c->hit_b.p + n_chunk, fb, f * 4, cudaMemcpyDeviceToDevice, c->stream));
-        CK(cudaMemcpyAsync((uint64_t *)c->d_inter.p + n_chunk, fi, f * 8, cudaMemcpyDeviceToDevice, c->stream));
-        CK(cudaMemcpyAsync((double *)c->d_dist.p + n_chunk, fd, f * 8, cudaMemcpyDeviceToDevice, c->stream));
-    }
-    const LinkState st = link_state_at(c->lk_state.p, N);
-    const LinkGraph g{(const uint32_t *)c->hit_a.p, (const uint32_t *)c->hit_b.p, (const uint64_t *)c->d_inter.p,
-                      (const double *)c->d_dist.p, n_chunk + f, L.b_off, L.key.empty() ? nullptr : st.key};
-    if (g.n_edges >= LINK_NONE) return fail(c, GKD_EINVAL, "linkage: %llu edges in one pass", (unsigned long long)g.n_edges);
-    uint32_t rounds = 1;
-    while (rounds < LINK_MAX_ROUNDS && (1ull << rounds) < N) rounds++;
-    nvtxRangePushA("gkd kernel 5: linkage rounds");
-    CK(launch_link_rounds(g, st, LinkForest{fa, fb, fi, fd}, rounds, c->stream));
-    nvtxRangePop();
-    c->m.launches += 1 + 5 * rounds;
-    uint32_t n_forest = 0;
-    CK(cudaEventRecord(c->ev[7], c->stream));
-    CK(cudaMemcpyAsync(&n_forest, st.n_forest, 4, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    L.n_dev = n_forest;
-    return GKD_OK;
-}
-
-// The selection epilogue of one chunk whose kernel-4 launches are queued: launches the within or nearest selection,
-// then copies back only the hits (within: plus the chunk's 8-byte hit total) or the rows' best lists (nearest).  The
-// absorb form merges the chunk into the device lists instead, which are copied once by the caller (lists_finish), and
-// the cluster form links it into the device forest, copied once by forest_finish.
-// The hit total and the join overflow flag are read before anything is copied, so a chunk that has to be redone by
-// the merge kernel appends nothing.
-int select_chunk(gkd_ctx *c, const HostPairs &hp, const PairSource &src, const Selection &sel, uint64_t cnt, bool need_pal,
-                 bool both, const uint32_t &join_err, bool use_join) {
-    const SetDesc *sets = (const SetDesc *)c->d_sets.p;
-    const uint32_t *counts = (const uint32_t *)c->counts.p, *pal = need_pal ? (const uint32_t *)c->pal_counts.p : nullptr;
-    int rc;
-    unsigned long long chunk_hits = 0;
-    uint64_t wcap = 0, nctas = 0;
-    if (sel.within) {
-        const gkd_hits &h = *sel.hits;
-        const bool any_out = h.a || h.b || h.inter || h.dist;
-        wcap = (any_out && h.n < h.cap) ? std::min<uint64_t>(cnt, h.cap - h.n) : 0;  // the device buffers hold at most this
-        nctas = select_within_ctas(cnt);
-        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
-        if (h.a && (rc = ensure(c, c->hit_a, wcap * 4))) return rc;
-        if (h.b && (rc = ensure(c, c->hit_b, wcap * 4))) return rc;
-        if (h.inter && (rc = ensure(c, c->d_inter, wcap * 8))) return rc;
-        if (h.dist && (rc = ensure(c, c->d_dist, wcap * 8))) return rc;
-        const HitsOut ho{h.a ? (uint32_t *)c->hit_a.p : nullptr, h.b ? (uint32_t *)c->hit_b.p : nullptr,
-                         h.inter ? (uint64_t *)c->d_inter.p : nullptr, h.dist ? (double *)c->d_dist.p : nullptr};
-        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
-        nvtxRangePushA("gkd kernel 5: within selection");
-        CK(launch_select_within(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.a_base, wcap, ho, cta, cta + nctas, c->stream));
-        nvtxRangePop();
-        c->m.launches += wcap ? 3 : 2;
-        CK(cudaEventRecord(c->ev[7], c->stream));
-        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
-    } else if (sel.link) {
-        // every edge of the chunk within max_dist, with room behind them for the forest so far (link_chunk)
-        const uint64_t room = cnt + sel.link->nodes;
-        nctas = select_within_ctas(cnt);
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        // every edge of the chunk within max_dist, with room behind them for the forest so far (keep)
+        const uint64_t room = e.cnt + nodes;
+        const uint64_t nctas = select_within_ctas(e.cnt);
+        int rc;
         if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
         if ((rc = ensure(c, c->hit_a, room * 4)) || (rc = ensure(c, c->hit_b, room * 4))) return rc;
         if ((rc = ensure(c, c->d_inter, room * 8)) || (rc = ensure(c, c->d_dist, room * 8))) return rc;
         const HitsOut ho{(uint32_t *)c->hit_a.p, (uint32_t *)c->hit_b.p, (uint64_t *)c->d_inter.p, (double *)c->d_dist.p};
         unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
         nvtxRangePushA("gkd kernel 5: linkage edges");
-        CK(launch_select_within(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.a_base, cnt, ho, cta, cta + nctas, c->stream));
+        CK(launch_select_within(e.sets, e.src, e.counts, e.pal, e.both, max_dist, a_base, e.cnt, ho, cta, cta + nctas, c->stream));
         nvtxRangePop();
         c->m.launches += 3;
         CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
-    } else if (sel.rows) {
-        const uint64_t slots = (uint64_t)hp.na * sel.k;
-        if (sel.ref_pos && (rc = ensure(c, c->hit_a, slots * 4))) return rc;
-        if (sel.n_found && (rc = ensure(c, c->hit_b, (uint64_t)hp.na * 4))) return rc;
-        if (sel.inter && (rc = ensure(c, c->d_inter, slots * 8))) return rc;
-        if (sel.dist && (rc = ensure(c, c->d_dist, slots * 8))) return rc;
-        const NearestOut no{sel.ref_pos ? (uint32_t *)c->hit_a.p : nullptr, sel.inter ? (uint64_t *)c->d_inter.p : nullptr,
-                            sel.dist ? (double *)c->d_dist.p : nullptr, sel.n_found ? (uint32_t *)c->hit_b.p : nullptr};
-        nvtxRangePushA("gkd kernel 5: nearest selection");
-        CK(launch_select_nearest(sets, src, hp.na, counts, pal, both ? 1 : 0, sel.max_dist, sel.k, sel.exclude_self, no, c->stream));
+        d2h += 8;
+        return GKD_OK;
+    }
+    // The chunk's chunk_hits edges are compacted at the front of hit_a / hit_b / d_inter / d_dist: the forest so far is
+    // copied behind them and the Boruvka rounds replace it with MSF(forest u chunk).  The forest outlives the chunk, so
+    // the rounds start only once the host has seen that the join held.  Records ev[7] after the rounds and reads the new
+    // forest's size (4 bytes).
+    int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        d2h += 4;
+        if (chunk_hits == 0) {  // the forest stands
+            CK(cudaEventRecord(c->ev[7], c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            return GKD_OK;
+        }
+        const uint32_t N = nodes;
+        uint64_t *fi = (uint64_t *)c->lk_forest.p;  // 24 B per node: inter, dist, a, b
+        double *fd = (double *)(fi + N);
+        uint32_t *fa = (uint32_t *)(fd + N), *fb = fa + N;
+        const uint64_t f = n_dev;
+        if (f) {
+            CK(cudaMemcpyAsync((uint32_t *)c->hit_a.p + chunk_hits, fa, f * 4, cudaMemcpyDeviceToDevice, c->stream));
+            CK(cudaMemcpyAsync((uint32_t *)c->hit_b.p + chunk_hits, fb, f * 4, cudaMemcpyDeviceToDevice, c->stream));
+            CK(cudaMemcpyAsync((uint64_t *)c->d_inter.p + chunk_hits, fi, f * 8, cudaMemcpyDeviceToDevice, c->stream));
+            CK(cudaMemcpyAsync((double *)c->d_dist.p + chunk_hits, fd, f * 8, cudaMemcpyDeviceToDevice, c->stream));
+        }
+        const LinkState st = link_state_at(c->lk_state.p, N);
+        const LinkGraph g{(const uint32_t *)c->hit_a.p, (const uint32_t *)c->hit_b.p, (const uint64_t *)c->d_inter.p,
+                          (const double *)c->d_dist.p, chunk_hits + f, b_off, key.empty() ? nullptr : st.key};
+        if (g.n_edges >= LINK_NONE) return fail(c, GKD_EINVAL, "linkage: %llu edges in one pass", (unsigned long long)g.n_edges);
+        uint32_t rounds = 1;
+        while (rounds < LINK_MAX_ROUNDS && (1ull << rounds) < N) rounds++;
+        nvtxRangePushA("gkd kernel 5: linkage rounds");
+        CK(launch_link_rounds(g, st, LinkForest{fa, fb, fi, fd}, rounds, c->stream));
         nvtxRangePop();
-        c->m.launches++;
-    }
-    if (sel.absorb) {
-        // the lists outlive this chunk: the kernel itself skips a chunk whose join overflowed
-        const NearestOut st{(uint32_t *)c->nn_pos.p, (uint64_t *)c->nn_inter.p, (double *)c->nn_dist.p, (uint32_t *)c->nn_found.p};
-        nvtxRangePushA("gkd kernel 5: nearest absorb");
-        CK(launch_nearest_absorb(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.k, sel.exclude_self, sel.a_base,
-                                 use_join ? (const uint32_t *)c->join_err.p : nullptr, st, c->stream));
-        nvtxRangePop();
-        c->m.launches++;
-    }
-    if (sel.cluster) {
-        // like absorb: the forest outlives this chunk, so the kernel itself skips a chunk whose join overflowed
-        nvtxRangePushA("gkd kernel 5: cluster link");
-        CK(launch_cluster_link(sets, src, counts, pal, both ? 1 : 0, sel.max_dist, sel.a_base, sel.b_base,
-                               use_join ? (const uint32_t *)c->join_err.p : nullptr, (uint32_t *)c->uf_parent.p, c->stream));
-        nvtxRangePop();
-        c->m.launches++;
-    }
-    if (!sel.within && !sel.link) CK(cudaEventRecord(c->ev[7], c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    if (join_err) return SELECT_REDO;
-    // linkage: the forest outlives the chunk, so the rounds start only once the host has seen that the join held
-    if (sel.link && (rc = link_chunk(c, *sel.link, chunk_hits))) return rc;
-    struct {
-        void *dst;
-        const void *src;
-        uint64_t bytes;
-    } copies[4] = {};  // absorb and cluster: nothing leaves the device before the end of the call
-    if (sel.within) {
-        const gkd_hits &h = *sel.hits;
-        const uint64_t w = std::min<uint64_t>(chunk_hits, wcap);
-        copies[0] = {h.a ? h.a + h.n : nullptr, c->hit_a.p, w * 4};
-        copies[1] = {h.b ? h.b + h.n : nullptr, c->hit_b.p, w * 4};
-        copies[2] = {h.inter ? h.inter + h.n : nullptr, c->d_inter.p, w * 8};
-        copies[3] = {h.dist ? h.dist + h.n : nullptr, c->d_dist.p, w * 8};
-    } else if (sel.rows) {
-        const uint64_t slots = (uint64_t)hp.na * sel.k;
-        copies[0] = {sel.ref_pos, c->hit_a.p, slots * 4};
-        copies[1] = {sel.inter, c->d_inter.p, slots * 8};
-        copies[2] = {sel.dist, c->d_dist.p, slots * 8};
-        copies[3] = {sel.n_found, c->hit_b.p, (uint64_t)hp.na * 4};
-    }
-    uint64_t d2h = sel.within ? 8 : (sel.link ? 12 : 0);
-    for (const auto &cp : copies) {
-        if (!cp.dst || !cp.bytes) continue;
-        CK(cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, cudaMemcpyDefault, c->stream));
-        d2h += cp.bytes;
-    }
-    CK(cudaStreamSynchronize(c->stream));
-    if (sel.within) sel.hits->n += chunk_hits;
-    c->m.d2h_bytes += d2h;
-    const double ims = elapsed(c->ev[4], c->ev[5]);
-    c->m.intersect_ms += ims;
-    c->m.total_intersect_ms += ims;
-    c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
-    return GKD_OK;
-}
-
-int run_pairs(gkd_ctx *c, const HostPairs &hp, const gkd_outputs &out, const Selection *sel = nullptr) {
-    int rc = upload_sets(c);
-    if (rc) return rc;
-    const bool nuc = c->cfg.alphabet != GKD_PROT;
-    const bool both = nuc && c->cfg.strand_mode == GKD_STRAND_BOTH;
-    const bool need_pal = both && (c->k % 2 == 0);
-    c->m.pairs = hp.count;
-    c->m.intersect_bytes = 0;
-    c->m.intersect_ms = c->m.epilogue_ms = 0;
-
-    // validate ids, gather sizes for the work split and the byte accounting
-    uint64_t max_n = 0, max_pal = 0;
-    uint32_t max_level = 0, max_pal_level = 0;
-    bool any_lit = false;
-    long double sum_bytes = 0;
-    auto size_of = [&](uint32_t id) -> uint64_t { return c->genomes[id].desc.main.n; };
-    auto see = [&](uint32_t id) {
-        const GenomeRec &g = c->genomes[id];
-        max_n = std::max<uint64_t>(max_n, g.desc.main.n);
-        max_pal = std::max<uint64_t>(max_pal, g.desc.pal.n);
-        max_level = std::max(max_level, g.desc.main.level);
-        max_pal_level = std::max(max_pal_level, g.desc.pal.level);
-        any_lit = any_lit || !g.lit.empty();
-    };
-    if (hp.mode == PAIRS_UPPER) {
-        for (uint32_t i = 0; i < hp.n; i++) {
-            if ((rc = check_built(c, i))) return rc;
-            see(i);
-        }
-        // bytes of the requested range, row by row
-        uint32_t i0 = 0, j0 = 1;
-        if (hp.count) upper_pair(hp.first, hp.n, i0, j0);
-        uint64_t left = hp.count;
-        std::vector<uint64_t> prefix(hp.n + 1, 0);
-        for (uint32_t i = 0; i < hp.n; i++) prefix[i + 1] = prefix[i] + size_of(i);
-        for (uint32_t i = i0, j = j0; left > 0 && i + 1 < hp.n; i++, j = i + 1) {
-            uint64_t in_row = std::min<uint64_t>(left, hp.n - j);
-            sum_bytes += 8.0L * ((long double)in_row * size_of(i) + (long double)(prefix[j + in_row] - prefix[j]));
-            left -= in_row;
-        }
-    } else if (hp.mode == PAIRS_RECT) {
-        uint64_t sq = 0, sr = 0;
-        for (uint32_t i = 0; i < hp.na; i++) {
-            if ((rc = check_built(c, hp.a[i]))) return rc;
-            sq += size_of(hp.a[i]);
-            see(hp.a[i]);
-        }
-        for (uint32_t i = 0; i < hp.nb; i++) {
-            if ((rc = check_built(c, hp.b[i]))) return rc;
-            sr += size_of(hp.b[i]);
-            see(hp.b[i]);
-        }
-        sum_bytes = 8.0L * ((long double)sq * hp.nb + (long double)sr * hp.na);
-    } else {
-        for (uint64_t t = 0; t < hp.count; t++) {
-            if ((rc = check_built(c, hp.a[t]))) return rc;
-            if ((rc = check_built(c, hp.b[t]))) return rc;
-            sum_bytes += 8.0L * (size_of(hp.a[t]) + size_of(hp.b[t]));
-            see(hp.a[t]);
-            see(hp.b[t]);
-        }
-    }
-    c->m.intersect_bytes = (uint64_t)sum_bytes;
-    c->m.total_intersect_bytes += (uint64_t)sum_bytes;
-    c->m.total_pairs += hp.count;
-    if (hp.count == 0) return GKD_OK;
-
-    // work split: a pair is walked in 32-bucket groups at the level of its larger set; an item is a run
-    // of groups of one pair.  Few pairs -> small items so every warp has work; many pairs -> eight items
-    // per pair, so the warps that share a pair read neighbouring parts of its two key streams.
-    auto make_plan = [&](uint64_t nmax, uint32_t lmax, bool one_item) {
-        IsectPlan p{};
-        p.low_bits = c->low_bits;
-        p.tmax = c->isect_tmax;
-        p.level_min = c->lvl_min;
-        uint32_t L = std::max(level_for((uint32_t)nmax, p.tmax), c->lvl_min);
-        L = std::min(L, lmax);
-        const uint64_t max_groups = ((1ull << L) + 31) >> 5;
-        uint64_t gpi;
-        if (one_item || max_groups <= 64) gpi = max_groups;  // tiny sets: a pair is one item (the per-item set-up would dominate)
-        else if (c->cfg.segment_keys) gpi = std::max<uint64_t>(1, c->cfg.segment_keys / (64ull * p.tmax));
-        else {
-            const uint64_t warps = (uint64_t)c->n_sms * intersect_warps_per_sm(c->low_bits);
-            const long double total_groups = (long double)hp.count * max_groups;
-            gpi = (uint64_t)std::min<long double>(total_groups / (long double)(warps * 8), (long double)(max_groups / 8));
-        }
-        gpi = std::min<uint64_t>(std::max<uint64_t>(gpi, 1), max_groups);
-        p.groups_per_item = (uint32_t)gpi;
-        p.items_per_pair = (uint32_t)((max_groups + gpi - 1) / gpi);
-        return p;
-    };
-    const IsectPlan plan = make_plan(max_n, max_level, false);
-    const IsectPlan pal_plan = make_plan(max_pal, max_pal_level, true);
-
-    // device id arrays
-    PairSource src{};
-    src.mode = hp.mode;
-    src.n = hp.n;
-    if (hp.mode != PAIRS_UPPER) {
-        if ((rc = ensure(c, c->ids_a, (uint64_t)hp.na * 4))) return rc;
-        if ((rc = ensure(c, c->ids_b, (uint64_t)hp.nb * 4))) return rc;
-        CK(cudaMemcpyAsync(c->ids_a.p, hp.a, (uint64_t)hp.na * 4, cudaMemcpyHostToDevice, c->stream));
-        CK(cudaMemcpyAsync(c->ids_b.p, hp.b, (uint64_t)hp.nb * 4, cudaMemcpyHostToDevice, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-    }
-    if ((rc = ensure(c, c->work_counter, 8))) return rc;
-
-    bool join_banned = false;  // set when a join table overflowed: the chunk is redone by the merge kernel
-    std::vector<uint64_t> lit_inter;  // selection on a GKD_AMBIG_LITERAL context: the chunk's completed pairs
-    std::vector<double> lit_dist;
-    JoinPlan jplan{};
-    std::vector<uint32_t> jrows;
-    for (uint64_t done = 0; done < hp.count;) {
-        const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, hp.count - done);
-        src.count = cnt;
-        bool jswapped = false;
-        const bool use_join = !join_banned && plan_join(c, hp, hp.mode == PAIRS_UPPER ? hp.first + done : 0, cnt, jplan, jrows, jswapped);
-        if (hp.mode == PAIRS_UPPER) {
-            src.first = hp.first + done;
-            src.a = src.b = nullptr;
-        } else if (hp.mode == PAIRS_RECT) {
-            // gkd_query_vs_ref splits by query rows, so a rectangle always fits one launch
-            src.first = 0;
-            src.a = (const uint32_t *)c->ids_a.p;
-            src.b = (const uint32_t *)c->ids_b.p;
-            if (hp.count > PAIR_CHUNK) return fail(c, GKD_EINVAL, "query x reference block larger than %llu pairs", (unsigned long long)PAIR_CHUNK);
-        } else {
-            src.first = 0;
-            src.a = (const uint32_t *)c->ids_a.p + done;
-            src.b = (const uint32_t *)c->ids_b.p + done;
-        }
-        if ((rc = ensure(c, c->counts, cnt * 4))) return rc;
-        CK(cudaMemsetAsync(c->counts.p, 0, cnt * 4, c->stream));
-        if (need_pal) {
-            if ((rc = ensure(c, c->pal_counts, cnt * 4))) return rc;
-            CK(cudaMemsetAsync(c->pal_counts.p, 0, cnt * 4, c->stream));
-        }
-        // with literal side lists the pairs are completed on the host, which needs the counts; a selection on such a
-        // context runs the dense epilogue into host scratch and selects after the completion (host_select)
-        const bool dev_sel = sel && !any_lit;
-        gkd_outputs o = out;
-        uint64_t at = done;  // where this chunk's dense outputs go in o
-        if (sel && any_lit) {
-            lit_inter.resize(cnt);
-            lit_dist.resize(cnt);
-            o = gkd_outputs{lit_inter.data(), lit_dist.data(), nullptr, nullptr};
-            at = 0;
-        }
-        const bool want_inter = o.inter || any_lit;
-        if (!dev_sel) {
-            if (want_inter && (rc = ensure(c, c->d_inter, cnt * 8))) return rc;
-            if (o.dist && (rc = ensure(c, c->d_dist, cnt * 8))) return rc;
-            if (o.contain_a && (rc = ensure(c, c->d_ca, cnt * 8))) return rc;
-            if (o.contain_b && (rc = ensure(c, c->d_cb, cnt * 8))) return rc;
-        }
-
-        if (use_join) {
-            if ((rc = ensure(c, c->join_rows, jrows.size() * 4))) return rc;
-            if ((rc = ensure(c, c->join_err, 4))) return rc;
-            CK(cudaMemcpyAsync(c->join_rows.p, jrows.data(), jrows.size() * 4, cudaMemcpyHostToDevice, c->stream));
-            CK(cudaMemsetAsync(c->join_err.p, 0, 4, c->stream));
-            jplan.rows = (const uint32_t *)c->join_rows.p;
-            if (hp.mode == PAIRS_RECT) {
-                jplan.row_ids = (const uint32_t *)(jswapped ? c->ids_b.p : c->ids_a.p);
-                jplan.col_ids = (const uint32_t *)(jswapped ? c->ids_a.p : c->ids_b.p);
-            }
-        }
-        CK(cudaEventRecord(c->ev[4], c->stream));
-        if (use_join) {
-            nvtxRangePushA("gkd kernel 4: block join");
-            CK(launch_join((const SetDesc *)c->d_sets.p, jplan, (uint32_t *)c->counts.p,
-                           (unsigned long long *)c->work_counter.p, (uint32_t *)c->join_err.p, c->n_sms, c->stream));
-        } else {
-            nvtxRangePushA("gkd kernel 4: bucket-merge intersect");
-            CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 0, plan, (uint32_t *)c->counts.p,
-                                (unsigned long long *)c->work_counter.p, c->n_sms, c->stream));
-        }
-        nvtxRangePop();
-        CK(cudaEventRecord(c->ev[5], c->stream));
-        c->m.intersect_kernel = use_join ? 5u : (c->low_bits == 32 ? 3u : 4u);
-        uint32_t join_err = 0;
-        if (use_join) {
-            // a table that would overflow flags the launch; the chunk is then redone by the merge kernel
-            CK(cudaMemcpyAsync(&join_err, c->join_err.p, 4, cudaMemcpyDeviceToHost, c->stream));
-        }
-        c->m.launches++;
-        c->m.intersect_launches++;
-        if (need_pal && max_pal) {
-            CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 1, pal_plan, (uint32_t *)c->pal_counts.p,
-                                (unsigned long long *)c->work_counter.p, c->n_sms, c->stream));
-            c->m.launches++;
-        }
-        CK(cudaEventRecord(c->ev[6], c->stream));
-        if (dev_sel) {
-            rc = select_chunk(c, hp, src, *sel, cnt, need_pal, both, join_err, use_join);
-            if (rc == SELECT_REDO) {
-                join_banned = true;
-                continue;
-            }
-            if (rc) return rc;
-            done += PAIR_CHUNK;
-            continue;
-        }
-        EpilogueOut eo{want_inter ? (uint64_t *)c->d_inter.p : nullptr, o.dist ? (double *)c->d_dist.p : nullptr,
-                       o.contain_a ? (double *)c->d_ca.p : nullptr, o.contain_b ? (double *)c->d_cb.p : nullptr};
-        nvtxRangePushA("gkd kernel 5: distance epilogue");
-        CK(launch_epilogue((const SetDesc *)c->d_sets.p, src, (const uint32_t *)c->counts.p,
-                           need_pal ? (const uint32_t *)c->pal_counts.p : nullptr, both ? 1 : 0, eo, c->stream));
-        nvtxRangePop();
-        c->m.launches++;
+        c->m.launches += 1 + 5 * rounds;
+        uint32_t n_forest = 0;
         CK(cudaEventRecord(c->ev[7], c->stream));
-        std::vector<uint64_t> tmp_inter;
-        uint64_t *h_inter = o.inter ? o.inter + at : nullptr;
-        if (any_lit && !h_inter) {
-            tmp_inter.resize(cnt);
-            h_inter = tmp_inter.data();
-        }
-        uint64_t d2h = 0;
-        const struct {
-            void *dst;
-            const void *src;
-        } copies[4] = {{h_inter, c->d_inter.p}, {o.dist ? o.dist + at : nullptr, c->d_dist.p},
-                       {o.contain_a ? o.contain_a + at : nullptr, c->d_ca.p},
-                       {o.contain_b ? o.contain_b + at : nullptr, c->d_cb.p}};
-        for (const auto &cp : copies) {
-            if (!cp.dst) continue;
-            CK(cudaMemcpyAsync(cp.dst, cp.src, cnt * 8, cudaMemcpyDefault, c->stream));
-            d2h += cnt * 8;
-        }
+        CK(cudaMemcpyAsync(&n_forest, st.n_forest, 4, cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
-        if (join_err) {
-            join_banned = true;
-            continue;
-        }
-        c->m.d2h_bytes += d2h;
-        const double ims = elapsed(c->ev[4], c->ev[5]);
-        c->m.intersect_ms += ims;
-        c->m.total_intersect_ms += ims;
-        c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
-        if (any_lit) {
-            // GKD_AMBIG_LITERAL: add the literal k-mers both sets share and redo the formula with the
-            // full sizes (outputs must be host memory in this mode)
-            for (uint64_t t = 0; t < cnt; t++) {
-                uint32_t a, b;
-                host_pair_ids(hp, done + t, a, b);
-                const GenomeRec &ga = c->genomes[a], &gb = c->genomes[b];
-                if (ga.lit.empty() && gb.lit.empty()) continue;
-                const uint64_t I = h_inter[t] + literal_intersection(ga.lit, gb.lit);
-                const uint64_t sa = both_size(c, ga), sb = both_size(c, gb);
-                if (o.inter) o.inter[at + t] = I;
-                if (o.dist) o.dist[at + t] = host_distance(I, sa, sb);
-                if (o.contain_a) o.contain_a[at + t] = sa ? (double)I / (double)sa : 0.0;
-                if (o.contain_b) o.contain_b[at + t] = sb ? (double)I / (double)sb : 0.0;
-            }
-            if (sel) host_select(hp, *sel, done, cnt, lit_inter.data(), lit_dist.data());
-        }
-        done += PAIR_CHUNK;
+        n_dev = n_forest;
+        return GKD_OK;
     }
-    return GKD_OK;
-}
+    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {
+        // Kruskal on the host forest and the chunk's edges, in the order of k_link_edges
+        for (uint64_t t = 0; t < e.cnt; t++) {
+            if (!(dist[t] <= max_dist)) continue;
+            uint32_t a, b;
+            e.pair(a_base, t, a, b);
+            host_edges.push_back(edge(a, b, inter[t], dist[t]));
+        }
+        host_msf(host_edges, nodes);
+    }
+    // The forest to the caller, once, at the end of the call: the device forest is copied to the host and merged with the
+    // host forest by one Kruskal pass, which also sorts it (a forest keeps every edge).
+    int finish(gkd_ctx *c, gkd_hits *out) {
+        std::vector<LinkEdge> edges = std::move(host_edges);
+        const uint64_t f = n_dev, N = nodes;
+        if (f) {
+            std::vector<uint64_t> in(f);
+            std::vector<double> d(f);
+            std::vector<uint32_t> a(f), b(f);
+            const uint64_t *fi = (const uint64_t *)c->lk_forest.p;
+            const double *fd = (const double *)(fi + N);
+            const uint32_t *fa = (const uint32_t *)(fd + N), *fb = fa + N;
+            CK(cudaMemcpyAsync(in.data(), fi, f * 8, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaMemcpyAsync(d.data(), fd, f * 8, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaMemcpyAsync(a.data(), fa, f * 4, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaMemcpyAsync(b.data(), fb, f * 4, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            c->m.d2h_bytes += f * 24;
+            for (uint64_t t = 0; t < f; t++) edges.push_back(edge(a[t], b[t], in[t], d[t]));
+        }
+        host_msf(edges, nodes);
+        out->n = edges.size();
+        const uint64_t w = std::min<uint64_t>(out->n, out->cap);
+        if (w == 0) return GKD_OK;
+        std::vector<uint32_t> a(w), b(w);
+        std::vector<uint64_t> in(w);
+        std::vector<double> d(w);
+        for (uint64_t t = 0; t < w; t++) a[t] = edges[t].a, b[t] = edges[t].b, in[t] = edges[t].inter, d[t] = edges[t].dist;
+        if (out->a) CK(cudaMemcpyAsync(out->a, a.data(), w * 4, cudaMemcpyDefault, c->stream));
+        if (out->b) CK(cudaMemcpyAsync(out->b, b.data(), w * 4, cudaMemcpyDefault, c->stream));
+        if (out->inter) CK(cudaMemcpyAsync(out->inter, in.data(), w * 8, cudaMemcpyDefault, c->stream));
+        if (out->dist) CK(cudaMemcpyAsync(out->dist, d.data(), w * 8, cudaMemcpyDefault, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        return GKD_OK;
+    }
+};
 
 int default_k(int alphabet) { return alphabet == GKD_PROT ? 8 : 21; }
 
@@ -2074,10 +2267,11 @@ int gkd_load_sets(gkd_ctx *c, const char *path, uint32_t *first_id, uint32_t *n_
 }
 
 // ---- distances --------------------------------------------------------------------------------------------
-static int lit_outputs_ok(gkd_ctx *c, const gkd_outputs &o) {
-    // literal side lists are completed on the host, so the outputs must be host memory in that mode
+// Literal side lists are completed (and selected) on the host, so the outputs must be host memory in that mode.  The
+// selections check this before the context is touched, so a bad k or a NaN threshold is GKD_EINVAL even without a
+// usable device.
+static int host_outputs_ok(gkd_ctx *c, std::initializer_list<const void *> ps) {
     if (c->cfg.ambig_policy != GKD_AMBIG_LITERAL) return GKD_OK;
-    const void *ps[4] = {o.inter, o.dist, o.contain_a, o.contain_b};
     for (const void *p : ps)
         if (p && classify(p) == MEM_DEVICE) return fail(c, GKD_EINVAL, "GKD_AMBIG_LITERAL needs host output buffers");
     return GKD_OK;
@@ -2090,11 +2284,12 @@ int gkd_all_vs_all_range_ex(gkd_ctx *c, uint32_t n, uint64_t first, uint64_t cou
     if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "range over %u sets but only %zu exist", n, c->genomes.size());
     uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
     if (first > total || count > total - first) return fail(c, GKD_EINVAL, "pair range [%llu, +%llu) outside 0..%llu", (unsigned long long)first, (unsigned long long)count, (unsigned long long)total);
-    int rc = lit_outputs_ok(c, *out);
+    int rc = host_outputs_ok(c, {out->inter, out->dist, out->contain_a, out->contain_b});
     if (rc) return rc;
     ABI_GUARD_BEGIN
     HostPairs hp{PAIRS_UPPER, n, first, count, nullptr, nullptr, 0, 0};
-    return run_pairs(c, hp, *out);
+    Dense f(*out);
+    return run_pairs(c, hp, f);
     ABI_GUARD_END(c)
 }
 
@@ -2114,35 +2309,15 @@ int gkd_query_vs_ref_ex(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32
     if (!out) return fail(c, GKD_EINVAL, "null outputs");
     CK(cudaSetDevice(c->cfg.device));
     if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref: null id array");
-    int rc = lit_outputs_ok(c, *out);
+    int rc = host_outputs_ok(c, {out->inter, out->dist, out->contain_a, out->contain_b});
     if (rc) return rc;
-    // large blocks are split by query rows so each launch stays under PAIR_CHUNK pairs
     if (nq == 0 || nr == 0) {
         c->m.pairs = 0;
         return GKD_OK;
     }
     ABI_GUARD_BEGIN
-    uint32_t rows_per = (uint32_t)std::max<uint64_t>(1, PAIR_CHUNK / nr);
-    uint64_t pairs = 0, bytes = 0;
-    double ims = 0, ems = 0;
-    for (uint32_t q0 = 0; q0 < nq; q0 += rows_per) {
-        uint32_t rows = std::min(rows_per, nq - q0);
-        HostPairs hp{PAIRS_RECT, nr, 0, (uint64_t)rows * nr, q + q0, r, rows, nr};
-        const uint64_t at = (uint64_t)q0 * nr;
-        gkd_outputs o{out->inter ? out->inter + at : nullptr, out->dist ? out->dist + at : nullptr,
-                      out->contain_a ? out->contain_a + at : nullptr, out->contain_b ? out->contain_b + at : nullptr};
-        rc = run_pairs(c, hp, o);
-        if (rc) return rc;
-        pairs += c->m.pairs;
-        bytes += c->m.intersect_bytes;
-        ims += c->m.intersect_ms;
-        ems += c->m.epilogue_ms;
-    }
-    c->m.pairs = pairs;
-    c->m.intersect_bytes = bytes;
-    c->m.intersect_ms = ims;
-    c->m.epilogue_ms = ems;
-    return GKD_OK;
+    Dense f(*out);
+    return run_rect(c, q, nq, r, nr, f);
     ABI_GUARD_END(c)
 }
 
@@ -2157,11 +2332,12 @@ int gkd_pairs_ex(gkd_ctx *c, const uint32_t *a, const uint32_t *b, uint64_t n_pa
     CK(cudaSetDevice(c->cfg.device));
     if (n_pairs && (!a || !b)) return fail(c, GKD_EINVAL, "gkd_pairs: null id array");
     if (n_pairs > 0xFFFFFFFFull) return fail(c, GKD_EINVAL, "gkd_pairs: more than 2^32 pairs in one call");
-    int rc = lit_outputs_ok(c, *out);
+    int rc = host_outputs_ok(c, {out->inter, out->dist, out->contain_a, out->contain_b});
     if (rc) return rc;
     ABI_GUARD_BEGIN
     HostPairs hp{PAIRS_LIST, 0, 0, n_pairs, a, b, (uint32_t)n_pairs, (uint32_t)n_pairs};
-    return run_pairs(c, hp, *out);
+    Dense f(*out);
+    return run_pairs(c, hp, f);
     ABI_GUARD_END(c)
 }
 
@@ -2181,19 +2357,10 @@ int gkd_greedy_reps(gkd_ctx *c, const uint32_t *order, uint32_t n, double max_di
     const bool nuc = c->cfg.alphabet != GKD_PROT;
     const bool both = nuc && c->cfg.strand_mode == GKD_STRAND_BOTH;
     const bool need_pal = both && (c->k % 2 == 0);
-    uint64_t max_n = 0, max_pal = 0;
-    uint32_t max_level = 0, max_pal_level = 0;
-    bool any_lit = false;
-    for (uint32_t i = 0; i < n; i++) {
-        if ((rc = check_built(c, order[i]))) return rc;
-        const GenomeRec &g = c->genomes[order[i]];
-        max_n = std::max<uint64_t>(max_n, g.desc.main.n);
-        max_pal = std::max<uint64_t>(max_pal, g.desc.pal.n);
-        max_level = std::max(max_level, g.desc.main.level);
-        max_pal_level = std::max(max_pal_level, g.desc.pal.level);
-        any_lit = any_lit || !g.lit.empty();
-    }
-    if (any_lit) {
+    SetScan s;
+    for (uint32_t i = 0; i < n; i++)
+        if ((rc = s.see(c, order[i]))) return rc;
+    if (s.any_lit) {
         // literal ambiguous k-mers are completed on the host: one batched call per candidate
         std::vector<uint32_t> reps, cand;
         std::vector<double> dist;
@@ -2202,9 +2369,9 @@ int gkd_greedy_reps(gkd_ctx *c, const uint32_t *order, uint32_t n, double max_di
             if (!reps.empty()) {
                 cand.assign(reps.size(), order[i]);
                 dist.assign(reps.size(), 1.0);
-                gkd_outputs o{nullptr, dist.data(), nullptr, nullptr};
+                Dense f(gkd_outputs{nullptr, dist.data(), nullptr, nullptr});
                 HostPairs hp{PAIRS_LIST, 0, 0, reps.size(), reps.data(), cand.data(), (uint32_t)reps.size(), (uint32_t)reps.size()};
-                if ((rc = run_pairs(c, hp, o))) return rc;
+                if ((rc = run_pairs(c, hp, f))) return rc;
                 for (double d : dist) found = found || d <= max_dist;
             }
             is_rep[i] = found ? 0 : 1;
@@ -2223,22 +2390,6 @@ int gkd_greedy_reps(gkd_ctx *c, const uint32_t *order, uint32_t n, double max_di
     CK(cudaMemsetAsync(d_nreps, 0, 16, c->stream));
     CK(cudaMemsetAsync(c->counts.p, 0, (uint64_t)n * 4, c->stream));
     if (need_pal) CK(cudaMemsetAsync(c->pal_counts.p, 0, (uint64_t)n * 4, c->stream));
-    const uint64_t warps = (uint64_t)c->n_sms * intersect_warps_per_sm(c->low_bits);
-    auto plan_for = [&](uint64_t nmax, uint32_t lmax, uint64_t pairs, bool one_item) {
-        IsectPlan p{};
-        p.low_bits = c->low_bits;
-        p.tmax = c->isect_tmax;
-        p.level_min = c->lvl_min;
-        uint32_t L = std::min(std::max(level_for((uint32_t)nmax, p.tmax), c->lvl_min), lmax);
-        const uint64_t max_groups = ((1ull << L) + 31) >> 5;
-        uint64_t gpi = max_groups;
-        if (!one_item && max_groups > 64)
-            gpi = (uint64_t)std::min<long double>((long double)pairs * max_groups / (long double)(warps * 8), (long double)(max_groups / 8));
-        gpi = std::min<uint64_t>(std::max<uint64_t>(gpi, 1), max_groups);
-        p.groups_per_item = (uint32_t)gpi;
-        p.items_per_pair = (uint32_t)((max_groups + gpi - 1) / gpi);
-        return p;
-    };
     CK(cudaEventRecord(c->ev[4], c->stream));
     NvtxRange nvtx("gkd greedy representatives (kernels 4+5 per candidate, device-resident list)");
     for (uint32_t i = 0; i < n; i++) {
@@ -2249,12 +2400,12 @@ int gkd_greedy_reps(gkd_ctx *c, const uint32_t *order, uint32_t n, double max_di
             src.count = i;
             src.a = d_reps;
             src.count_ptr = d_nreps;
-            CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 0, plan_for(max_n, max_level, i, false), (uint32_t *)c->counts.p,
+            CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 0, make_plan(c, i, s.max_n, s.max_level, false), (uint32_t *)c->counts.p,
                                 (unsigned long long *)c->work_counter.p, c->n_sms, c->stream));
             c->m.launches++;
             c->m.intersect_launches++;
-            if (need_pal && max_pal) {
-                CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 1, plan_for(max_pal, max_pal_level, i, true),
+            if (need_pal && s.max_pal) {
+                CK(launch_intersect((const SetDesc *)c->d_sets.p, src, 1, make_plan(c, i, s.max_pal, s.max_pal_level, true),
                                     (uint32_t *)c->pal_counts.p, (unsigned long long *)c->work_counter.p, c->n_sms, c->stream));
                 c->m.launches++;
             }
@@ -2291,45 +2442,6 @@ int gkd_pair(gkd_ctx *c, uint32_t a, uint32_t b, uint64_t *inter, uint64_t *uni,
 }
 
 // ---- selections ---------------------------------------------------------------------------------------------
-// The arguments are checked before the context is touched, so a bad k or a NaN threshold is GKD_EINVAL even
-// without a usable device.
-static int hits_host_ok(gkd_ctx *c, const void *const *ps, int n) {
-    // literal side lists are completed and selected on the host, so the outputs must be host memory in that mode
-    if (c->cfg.ambig_policy != GKD_AMBIG_LITERAL) return GKD_OK;
-    for (int i = 0; i < n; i++)
-        if (ps[i] && classify(ps[i]) == MEM_DEVICE) return fail(c, GKD_EINVAL, "GKD_AMBIG_LITERAL needs host output buffers");
-    return GKD_OK;
-}
-
-// a query x reference selection, split by query rows like gkd_query_vs_ref_ex (every row is complete in one launch)
-static int rect_selection(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, const Selection &sel) {
-    const uint32_t rows_per = (uint32_t)std::max<uint64_t>(1, PAIR_CHUNK / nr);
-    uint64_t pairs = 0, bytes = 0;
-    double ims = 0, ems = 0;
-    for (uint32_t q0 = 0; q0 < nq; q0 += rows_per) {
-        const uint32_t rows = std::min(rows_per, nq - q0);
-        HostPairs hp{PAIRS_RECT, nr, 0, (uint64_t)rows * nr, q + q0, r, rows, nr};
-        Selection s = sel;
-        s.a_base = q0;
-        const uint64_t at = (uint64_t)q0 * sel.k;
-        if (s.ref_pos) s.ref_pos += at;
-        if (s.inter) s.inter += at;
-        if (s.dist) s.dist += at;
-        if (s.n_found) s.n_found += q0;
-        const int rc = run_pairs(c, hp, gkd_outputs{}, &s);
-        if (rc) return rc;
-        pairs += c->m.pairs;
-        bytes += c->m.intersect_bytes;
-        ims += c->m.intersect_ms;
-        ems += c->m.epilogue_ms;
-    }
-    c->m.pairs = pairs;
-    c->m.intersect_bytes = bytes;
-    c->m.intersect_ms = ims;
-    c->m.epilogue_ms = ems;
-    return GKD_OK;
-}
-
 int gkd_all_vs_all_range_within(gkd_ctx *c, uint32_t n, uint64_t first, uint64_t count, double max_dist, gkd_hits *out) {
     if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_range_within: null hits");
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_range_within: max_dist is NaN");
@@ -2338,17 +2450,13 @@ int gkd_all_vs_all_range_within(gkd_ctx *c, uint32_t n, uint64_t first, uint64_t
     if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "range over %u sets but only %zu exist", n, c->genomes.size());
     uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
     if (first > total || count > total - first) return fail(c, GKD_EINVAL, "pair range [%llu, +%llu) outside 0..%llu", (unsigned long long)first, (unsigned long long)count, (unsigned long long)total);
-    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
-    int rc = hits_host_ok(c, ps, 4);
+    int rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist});
     if (rc) return rc;
     out->n = 0;
     ABI_GUARD_BEGIN
     HostPairs hp{PAIRS_UPPER, n, first, count, nullptr, nullptr, 0, 0};
-    Selection sel{};
-    sel.within = true;
-    sel.max_dist = max_dist;
-    sel.hits = out;
-    return run_pairs(c, hp, gkd_outputs{}, &sel);
+    Within f(max_dist, *out);
+    return run_pairs(c, hp, f);
     ABI_GUARD_END(c)
 }
 
@@ -2359,8 +2467,7 @@ int gkd_query_vs_ref_within(gkd_ctx *c, const uint32_t *q, uint32_t nq, const ui
     CHECK_CTX(c);
     CK(cudaSetDevice(c->cfg.device));
     if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_within: null id array");
-    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
-    int rc = hits_host_ok(c, ps, 4);
+    int rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist});
     if (rc) return rc;
     out->n = 0;
     if (nq == 0 || nr == 0) {
@@ -2368,11 +2475,8 @@ int gkd_query_vs_ref_within(gkd_ctx *c, const uint32_t *q, uint32_t nq, const ui
         return GKD_OK;
     }
     ABI_GUARD_BEGIN
-    Selection sel{};
-    sel.within = true;
-    sel.max_dist = max_dist;
-    sel.hits = out;
-    return rect_selection(c, q, nq, r, nr, sel);
+    Within f(max_dist, *out);
+    return run_rect(c, q, nq, r, nr, f);
     ABI_GUARD_END(c)
 }
 
@@ -2387,67 +2491,14 @@ static int fill_none(gkd_ctx *c, uint32_t rows, uint32_t k, const gkd_neighbors 
     return GKD_OK;
 }
 
-// the per-target lists of an accumulating nearest call (k_nearest_absorb), all unused
-static int lists_begin(gkd_ctx *c, uint32_t targets, uint32_t k) {
-    const uint64_t slots = (uint64_t)targets * k;
-    int rc;
-    if ((rc = ensure(c, c->nn_pos, slots * 4)) || (rc = ensure(c, c->nn_inter, slots * 8)) ||
-        (rc = ensure(c, c->nn_dist, slots * 8)) || (rc = ensure(c, c->nn_found, (uint64_t)targets * 4)))
-        return rc;
-    const double none = -1.0;
-    uint64_t none_bits;
-    std::memcpy(&none_bits, &none, 8);
-    CK(cudaMemsetAsync(c->nn_pos.p, 0xFF, slots * 4, c->stream));
-    CK(cudaMemsetAsync(c->nn_inter.p, 0, slots * 8, c->stream));
-    CK(cudaMemsetAsync(c->nn_found.p, 0, (uint64_t)targets * 4, c->stream));
-    CK(launch_fill_u64((uint64_t *)c->nn_dist.p, slots, none_bits, c->stream));
-    c->m.launches++;
-    return GKD_OK;
-}
-
-// the lists to the caller, once, at the end of the call.  With host_lists (GKD_AMBIG_LITERAL, host outputs) the
-// launches that ran on the device are merged into the host lists first.
-static int lists_finish(gkd_ctx *c, uint32_t targets, uint32_t k, HostLists *hl, const gkd_neighbors &out) {
-    const uint64_t slots = (uint64_t)targets * k;
-    const struct {
-        void *dst;
-        const void *src;
-        uint64_t bytes;
-    } copies[4] = {{out.pos, c->nn_pos.p, slots * 4}, {out.inter, c->nn_inter.p, slots * 8}, {out.dist, c->nn_dist.p, slots * 8},
-                   {out.n_found, c->nn_found.p, (uint64_t)targets * 4}};
-    if (!hl) {
-        for (const auto &cp : copies) {
-            if (!cp.dst) continue;
-            CK(cudaMemcpyAsync(cp.dst, cp.src, cp.bytes, cudaMemcpyDefault, c->stream));
-            c->m.d2h_bytes += cp.bytes;
-        }
-        CK(cudaStreamSynchronize(c->stream));
-        return GKD_OK;
-    }
-    HostLists dev(targets, k);
-    CK(cudaMemcpyAsync(dev.pos.data(), c->nn_pos.p, slots * 4, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaMemcpyAsync(dev.inter.data(), c->nn_inter.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaMemcpyAsync(dev.dist.data(), c->nn_dist.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    c->m.d2h_bytes += slots * 20;
-    for (uint32_t t = 0; t < targets; t++)
-        for (uint64_t s = (uint64_t)t * k; s < (uint64_t)(t + 1) * k && dev.pos[s] != 0xFFFFFFFFu; s++)
-            hl->offer(t, dev.pos[s], dev.inter[s], dev.dist[s]);
-    if (out.pos) std::memcpy(out.pos, hl->pos.data(), slots * 4);
-    if (out.inter) std::memcpy(out.inter, hl->inter.data(), slots * 8);
-    if (out.dist) std::memcpy(out.dist, hl->dist.data(), slots * 8);
-    if (out.n_found) std::memcpy(out.n_found, hl->n.data(), (uint64_t)targets * 4);
-    return GKD_OK;
-}
-
 static int nearest_args_ok(gkd_ctx *c, const char *fn, uint32_t k, double max_dist) {
     if (k < 1 || k > NEAREST_MAX_K) return fail(c, GKD_EINVAL, "%s: k = %u is outside 1..%u", fn, k, NEAREST_MAX_K);
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "%s: max_dist is NaN", fn);
     return GKD_OK;
 }
 
-// gkd_query_vs_ref_nearest(_ex): the q side by k_select_nearest (rows complete in every launch), the r side through
-// the per-target lists across the launches of rect_selection
+// gkd_query_vs_ref_nearest(_ex): the q side as row lists (complete in every launch), the r side through the per-target
+// lists across the launches of run_rect
 static int nearest_rect(gkd_ctx *c, const char *fn, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
                         double max_dist, int exclude_self, const gkd_neighbors *qs, const gkd_neighbors *rs) {
     int rc = nearest_args_ok(c, fn, k, max_dist);
@@ -2458,31 +2509,16 @@ static int nearest_rect(gkd_ctx *c, const char *fn, const uint32_t *q, uint32_t 
     if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "%s: null id array", fn);
     const gkd_neighbors none{};
     const gkd_neighbors &a = qs ? *qs : none, &b = rs ? *rs : none;
-    const void *ps[8] = {a.pos, a.inter, a.dist, a.n_found, b.pos, b.inter, b.dist, b.n_found};
-    if ((rc = hits_host_ok(c, ps, 8))) return rc;
+    if ((rc = host_outputs_ok(c, {a.pos, a.inter, a.dist, a.n_found, b.pos, b.inter, b.dist, b.n_found}))) return rc;
     c->m.pairs = 0;
     ABI_GUARD_BEGIN
     if (nq == 0 || nr == 0) {  // no pair: every list is empty
         if ((rc = fill_none(c, nq, k, qs))) return rc;
         return fill_none(c, nr, k, rs);
     }
-    Selection sel{};
-    sel.within = false;
-    sel.max_dist = max_dist;
-    sel.k = k;
-    sel.exclude_self = exclude_self ? 1 : 0;
-    sel.rows = qs != nullptr;
-    sel.ref_pos = a.pos;
-    sel.inter = a.inter;
-    sel.dist = a.dist;
-    sel.n_found = a.n_found;
-    sel.absorb = rs != nullptr;
-    std::unique_ptr<HostLists> hl;
-    if (rs && c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hl.reset(new HostLists(nr, k));
-    sel.host_lists = hl.get();
-    if (rs && (rc = lists_begin(c, nr, k))) return rc;
-    if ((rc = rect_selection(c, q, nq, r, nr, sel))) return rc;
-    return rs ? lists_finish(c, nr, k, hl.get(), *rs) : GKD_OK;
+    Nearest f(k, max_dist, exclude_self ? 1 : 0, qs, rs, nr);
+    if ((rc = f.start(c)) || (rc = run_rect(c, q, nq, r, nr, f))) return rc;
+    return f.finish(c);
     ABI_GUARD_END(c)
 }
 
@@ -2505,97 +2541,34 @@ int gkd_all_vs_all_nearest(gkd_ctx *c, uint32_t n, uint32_t k, double max_dist, 
     CHECK_CTX(c);
     CK(cudaSetDevice(c->cfg.device));
     if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "nearest over %u sets but only %zu exist", n, c->genomes.size());
-    const void *ps[4] = {out->pos, out->inter, out->dist, out->n_found};
-    if ((rc = hits_host_ok(c, ps, 4))) return rc;
+    if ((rc = host_outputs_ok(c, {out->pos, out->inter, out->dist, out->n_found}))) return rc;
     c->m.pairs = 0;
     if (n == 0) return GKD_OK;
     ABI_GUARD_BEGIN
-    Selection sel{};
-    sel.within = false;
-    sel.max_dist = max_dist;
-    sel.k = k;
-    sel.absorb = true;
-    std::unique_ptr<HostLists> hl;
-    if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hl.reset(new HostLists(n, k));
-    sel.host_lists = hl.get();
-    if ((rc = lists_begin(c, n, k))) return rc;
+    Nearest f(k, max_dist, 0, nullptr, out, n);
     HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
-    if ((rc = run_pairs(c, hp, gkd_outputs{}, &sel))) return rc;
-    return lists_finish(c, n, k, hl.get(), *out);
+    if ((rc = f.start(c)) || (rc = run_pairs(c, hp, f))) return rc;
+    return f.finish(c);
     ABI_GUARD_END(c)
 }
 
 // ---- single-linkage clusters ----------------------------------------------------------------------------------
-// the forest of one cluster call (k_cluster_link): every node its own root
-static int forest_begin(gkd_ctx *c, uint32_t nodes) {
-    const int rc = ensure(c, c->uf_parent, ((uint64_t)nodes + 1) * 4);
-    if (rc) return rc;
-    CK(launch_cluster_init((uint32_t *)c->uf_parent.p, nodes, c->stream));
-    c->m.launches++;
-    return GKD_OK;
-}
-
-// The labels to the caller, once, at the end of the call: nodes [0, na) to a_out and [na, nodes) to b_out (either may
-// be NULL).  With hf (GKD_AMBIG_LITERAL, host outputs) the launches that ran on the device are merged into the host
-// forest first: every node is linked to its device label, which carries all of the device links' connectivity.
-static int forest_finish(gkd_ctx *c, uint32_t nodes, HostForest *hf, uint32_t *a_out, uint32_t na, uint32_t *b_out,
-                         uint32_t *n_clusters) {
-    uint32_t *parent = (uint32_t *)c->uf_parent.p;
-    CK(cudaEventRecord(c->ev[6], c->stream));
-    CK(launch_cluster_flatten(parent, nodes, c->stream));
-    CK(cudaEventRecord(c->ev[7], c->stream));
-    c->m.launches++;
-    uint32_t roots = 0;
-    if (!hf) {
-        const uint32_t nb = nodes - na;
-        if (a_out && na) CK(cudaMemcpyAsync(a_out, parent, (uint64_t)na * 4, cudaMemcpyDefault, c->stream));
-        if (b_out && nb) CK(cudaMemcpyAsync(b_out, parent + na, (uint64_t)nb * 4, cudaMemcpyDefault, c->stream));
-        CK(cudaMemcpyAsync(&roots, parent + nodes, 4, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        c->m.d2h_bytes += (a_out ? (uint64_t)na * 4 : 0) + (b_out ? (uint64_t)nb * 4 : 0) + 4;
-    } else {
-        std::vector<uint32_t> dev(nodes);
-        CK(cudaMemcpyAsync(dev.data(), parent, (uint64_t)nodes * 4, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        c->m.d2h_bytes += (uint64_t)nodes * 4;
-        for (uint32_t x = 0; x < nodes; x++)
-            if (dev[x] != x) hf->link(x, dev[x]);
-        for (uint32_t x = 0; x < nodes; x++) {
-            const uint32_t r = hf->find(x);
-            roots += r == x ? 1u : 0u;
-            if (x < na && a_out) a_out[x] = r;
-            if (x >= na && b_out) b_out[x - na] = r;
-        }
-    }
-    c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
-    if (n_clusters) *n_clusters = roots;
-    return GKD_OK;
-}
-
 int gkd_all_vs_all_clusters(gkd_ctx *c, uint32_t n, double max_dist, uint32_t *label, uint32_t *n_clusters) {
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_clusters: max_dist is NaN");
     if (!label) return fail(c, GKD_EINVAL, "gkd_all_vs_all_clusters: null label");
     CHECK_CTX(c);
     CK(cudaSetDevice(c->cfg.device));
     if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "clusters over %u sets but only %zu exist", n, c->genomes.size());
-    const void *ps[1] = {label};
-    int rc = hits_host_ok(c, ps, 1);
+    int rc = host_outputs_ok(c, {label});
     if (rc) return rc;
     c->m.pairs = 0;
     if (n_clusters) *n_clusters = 0;
     if (n == 0) return GKD_OK;
     ABI_GUARD_BEGIN
-    Selection sel{};
-    sel.within = false;
-    sel.max_dist = max_dist;
-    sel.cluster = true;
-    std::unique_ptr<HostForest> hf;
-    if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hf.reset(new HostForest(n));
-    sel.host_forest = hf.get();
-    if ((rc = forest_begin(c, n))) return rc;
+    Clusters f(max_dist, n, 0);
     HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
-    if ((rc = run_pairs(c, hp, gkd_outputs{}, &sel))) return rc;
-    return forest_finish(c, n, hf.get(), label, n, nullptr, n_clusters);
+    if ((rc = f.start(c)) || (rc = run_pairs(c, hp, f))) return rc;
+    return f.finish(c, label, n, nullptr, n_clusters);
     ABI_GUARD_END(c)
 }
 
@@ -2607,24 +2580,16 @@ int gkd_query_vs_ref_clusters(gkd_ctx *c, const uint32_t *q, uint32_t nq, const 
     CK(cudaSetDevice(c->cfg.device));
     if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: null id array");
     if ((uint64_t)nq + nr >= 0xFFFFFFFFull) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: %u + %u nodes", nq, nr);
-    const void *ps[2] = {q_label, r_label};
-    int rc = hits_host_ok(c, ps, 2);
+    int rc = host_outputs_ok(c, {q_label, r_label});
     if (rc) return rc;
     c->m.pairs = 0;
     const uint32_t nodes = nq + nr;
     if (nodes == 0) return GKD_OK;
     ABI_GUARD_BEGIN
-    Selection sel{};
-    sel.within = false;
-    sel.max_dist = max_dist;
-    sel.cluster = true;
-    sel.b_base = nq;
-    std::unique_ptr<HostForest> hf;
-    if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) hf.reset(new HostForest(nodes));
-    sel.host_forest = hf.get();
-    if ((rc = forest_begin(c, nodes))) return rc;
-    if (nq && nr && (rc = rect_selection(c, q, nq, r, nr, sel))) return rc;
-    return forest_finish(c, nodes, hf.get(), q_label, nq, r_label, nullptr);
+    Clusters f(max_dist, nodes, nq);
+    if ((rc = f.start(c))) return rc;
+    if (nq && nr && (rc = run_rect(c, q, nq, r, nr, f))) return rc;
+    return f.finish(c, q_label, nq, r_label, nullptr);
     ABI_GUARD_END(c)
 }
 
@@ -2646,77 +2611,22 @@ static int link_keys(gkd_ctx *c, const uint32_t *q_key, uint32_t nq, const uint3
     ABI_GUARD_END(c)
 }
 
-// an empty forest on the device, and the node keys there when the caller passed any
-static int link_begin(gkd_ctx *c, LinkCall &L) {
-    int rc;
-    if ((rc = ensure(c, c->lk_forest, (uint64_t)L.nodes * 24)) || (rc = ensure(c, c->lk_state, link_state_bytes(L.nodes))))
-        return rc;
-    if (!L.key.empty())
-        CK(cudaMemcpyAsync(link_state_at(c->lk_state.p, L.nodes).key, L.key.data(), (uint64_t)L.nodes * 4, cudaMemcpyHostToDevice,
-                           c->stream));
-    L.n_dev = 0;
-    return GKD_OK;
-}
-
-// The forest to the caller, once, at the end of the call: the device forest is copied to the host and merged with the
-// host forest of GKD_AMBIG_LITERAL launches by one Kruskal pass, which also sorts it (a forest keeps every edge).
-static int link_finish(gkd_ctx *c, LinkCall &L, gkd_hits *out) {
-    std::vector<LinkEdge> edges = std::move(L.host);
-    const uint64_t f = L.n_dev, N = L.nodes;
-    if (f) {
-        std::vector<uint64_t> in(f);
-        std::vector<double> d(f);
-        std::vector<uint32_t> a(f), b(f);
-        const uint64_t *fi = (const uint64_t *)c->lk_forest.p;
-        const double *fd = (const double *)(fi + N);
-        const uint32_t *fa = (const uint32_t *)(fd + N), *fb = fa + N;
-        CK(cudaMemcpyAsync(in.data(), fi, f * 8, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaMemcpyAsync(d.data(), fd, f * 8, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaMemcpyAsync(a.data(), fa, f * 4, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaMemcpyAsync(b.data(), fb, f * 4, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        c->m.d2h_bytes += f * 24;
-        for (uint64_t t = 0; t < f; t++) edges.push_back(L.edge(a[t], b[t], in[t], d[t]));
-    }
-    host_msf(edges, L.nodes);
-    out->n = edges.size();
-    const uint64_t w = std::min<uint64_t>(out->n, out->cap);
-    if (w == 0) return GKD_OK;
-    std::vector<uint32_t> a(w), b(w);
-    std::vector<uint64_t> in(w);
-    std::vector<double> d(w);
-    for (uint64_t t = 0; t < w; t++) a[t] = edges[t].a, b[t] = edges[t].b, in[t] = edges[t].inter, d[t] = edges[t].dist;
-    if (out->a) CK(cudaMemcpyAsync(out->a, a.data(), w * 4, cudaMemcpyDefault, c->stream));
-    if (out->b) CK(cudaMemcpyAsync(out->b, b.data(), w * 4, cudaMemcpyDefault, c->stream));
-    if (out->inter) CK(cudaMemcpyAsync(out->inter, in.data(), w * 8, cudaMemcpyDefault, c->stream));
-    if (out->dist) CK(cudaMemcpyAsync(out->dist, d.data(), w * 8, cudaMemcpyDefault, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    return GKD_OK;
-}
-
 int gkd_all_vs_all_linkage(gkd_ctx *c, uint32_t n, double max_dist, gkd_hits *out) {
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_linkage: max_dist is NaN");
     if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_linkage: null out");
     CHECK_CTX(c);
     CK(cudaSetDevice(c->cfg.device));
     if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "linkage over %u sets but only %zu exist", n, c->genomes.size());
-    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
-    int rc = hits_host_ok(c, ps, 4);
+    int rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist});
     if (rc) return rc;
     c->m.pairs = 0;
     out->n = 0;
     if (n < 2) return GKD_OK;
     ABI_GUARD_BEGIN
-    LinkCall L;
-    L.nodes = n;
-    Selection sel{};
-    sel.within = false;
-    sel.max_dist = max_dist;
-    sel.link = &L;
-    if ((rc = link_begin(c, L))) return rc;
+    Linkage f(max_dist, n, 0, {});
     HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
-    if ((rc = run_pairs(c, hp, gkd_outputs{}, &sel))) return rc;
-    return link_finish(c, L, out);
+    if ((rc = f.start(c)) || (rc = run_pairs(c, hp, f))) return rc;
+    return f.finish(c, out);
     ABI_GUARD_END(c)
 }
 
@@ -2731,23 +2641,14 @@ int gkd_query_vs_ref_linkage(gkd_ctx *c, const uint32_t *q, uint32_t nq, const u
     CHECK_CTX(c);
     CK(cudaSetDevice(c->cfg.device));
     if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_linkage: null id array");
-    const void *ps[4] = {out->a, out->b, out->inter, out->dist};
-    if ((rc = hits_host_ok(c, ps, 4))) return rc;
+    if ((rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist}))) return rc;
     c->m.pairs = 0;
     out->n = 0;
     if (nq == 0 || nr == 0) return GKD_OK;
     ABI_GUARD_BEGIN
-    LinkCall L;
-    L.nodes = nq + nr;
-    L.b_off = nq;
-    L.key = std::move(key);
-    Selection sel{};
-    sel.within = false;
-    sel.max_dist = max_dist;
-    sel.link = &L;
-    if ((rc = link_begin(c, L))) return rc;
-    if ((rc = rect_selection(c, q, nq, r, nr, sel))) return rc;
-    return link_finish(c, L, out);
+    Linkage f(max_dist, nq + nr, nq, std::move(key));
+    if ((rc = f.start(c)) || (rc = run_rect(c, q, nq, r, nr, f))) return rc;
+    return f.finish(c, out);
     ABI_GUARD_END(c)
 }
 

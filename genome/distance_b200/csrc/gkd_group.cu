@@ -20,7 +20,7 @@
 #include <vector>
 
 #include "gkd.h"
-#include "gkd_internal.cuh"  // HostForest, host_msf
+#include "gkd_internal.cuh"  // HostForest, host_msf, NEAREST_MAX_K
 
 // host FASTA scanner (fasta.cpp)
 struct FastaPiece {
@@ -139,90 +139,71 @@ inline uint64_t row_start(uint64_t i, uint64_t n) { return i * (2 * n - i - 1) /
         }                                                     \
     } while (0)
 
+// What a group call computes: every member runs its own form over its diagonal block and over each of its ring calls
+// (member_ring), in global ids, and the entry point merges the members' forms.
+struct RingForm {
+    virtual ~RingForm() = default;
+    // the member's own sets, local ids 0 .. m-1 (m >= 2)
+    virtual int diagonal(Member &M, uint32_t m) = 0;
+    // the member's rows (local ids) x the adopted columns cols; col_gid: the global id of every column
+    virtual int block(Member &M, const std::vector<uint32_t> &rows, const std::vector<uint32_t> &cols,
+                      const std::vector<uint32_t> &col_gid) = 0;
+};
+
+// gkd_group_all_vs_all: every block scattered into the caller's triangle
+struct RingDense : RingForm {
+    uint64_t N;
+    uint64_t *inter;
+    double *dist;
+    std::vector<uint64_t> bi;
+    std::vector<double> bd;
+    RingDense(uint64_t n, uint64_t *inter_, double *dist_) : N(n), inter(inter_), dist(dist_) {}
+    void put(uint32_t ga, uint32_t gb, uint64_t t) {  // entry t of the call to pair (ga, gb)
+        if (ga > gb) std::swap(ga, gb);
+        const uint64_t o = row_start(ga, N) + (gb - ga - 1);
+        if (inter) inter[o] = bi[t];
+        if (dist) dist[o] = bd[t];
+    }
+    int diagonal(Member &M, uint32_t m) override {
+        const uint64_t cnt = (uint64_t)m * (m - 1) / 2;
+        bi.resize(cnt);
+        bd.resize(cnt);
+        const int rc = gkd_all_vs_all_range(M.ctx, m, 0, cnt, bi.data(), bd.data());
+        if (rc != GKD_OK) return rc;
+        uint64_t t = 0;
+        for (uint32_t i = 0; i < m; i++)
+            for (uint32_t j = i + 1; j < m; j++, t++) put(M.global_ids[i], M.global_ids[j], t);
+        return GKD_OK;
+    }
+    int block(Member &M, const std::vector<uint32_t> &rows, const std::vector<uint32_t> &cols,
+              const std::vector<uint32_t> &col_gid) override {
+        bi.resize(rows.size() * cols.size());
+        bd.resize(bi.size());
+        const int rc = gkd_query_vs_ref(M.ctx, rows.data(), (uint32_t)rows.size(), cols.data(), (uint32_t)cols.size(), bi.data(), bd.data());
+        if (rc != GKD_OK) return rc;
+        for (size_t r = 0; r < rows.size(); r++)
+            for (size_t c = 0; c < cols.size(); c++) put(M.global_ids[rows[r]], col_gid[c], r * cols.size() + c);
+        return GKD_OK;
+    }
+};
+
 // gkd_group_all_vs_all_within: a member's hits in global ids (a < b); no dense result exists on this path
 struct GroupHit {
     uint32_t a, b;
     uint64_t inter;
     double dist;
 };
-struct WithinSink {
-    double max_dist;
-    std::vector<GroupHit> hits;
-};
 // first capacity a member offers a within call; a call with more hits is repeated with the exact total
 constexpr uint64_t WITHIN_FIRST_CAP = 4ull << 20;
-
-// gkd_group_all_vs_all_nearest: a member's partial lists by global id.  A pair is computed once in the whole ring, so
-// the global top k of an id, by (distance bits, global id), is the top k of the union of its partial top-k lists.
-constexpr uint32_t NEAREST_MAX_K = 256;
-struct Neighbor {
-    uint64_t key;  // distance bits (distances are non-negative: the bits order like the values)
-    uint32_t id;
-    uint64_t inter;
-    bool operator<(const Neighbor &o) const { return key < o.key || (key == o.key && id < o.id); }
-};
-struct NearestSink {
-    uint32_t k;
+struct RingWithin : RingForm {
     double max_dist;
-    std::vector<std::vector<Neighbor>> lists;  // global id -> <= k entries after every call
-    void add(uint32_t target, uint32_t id, uint64_t inter, double d) {
-        uint64_t key;
-        memcpy(&key, &d, 8);
-        lists[target].push_back(Neighbor{key, id, inter});
-    }
-    void keep_best(uint32_t target) {
-        std::vector<Neighbor> &l = lists[target];
-        if (l.size() <= k) return;
-        std::partial_sort(l.begin(), l.begin() + k, l.end());
-        l.resize(k);
-    }
-};
-
-// gkd_group_all_vs_all_clusters: a member's links (global p, global label[p]) for every node p of its calls with
-// label[p] != p.  A call's labels carry all the connectivity of its links, and the ring computes every pair once, so
-// the union of these links over all members has the components of the whole triangle.
-struct ClusterSink {
-    double max_dist;
-    std::vector<std::pair<uint32_t, uint32_t>> links;
-};
-
-// gkd_group_all_vs_all_linkage: the forest edges of a member's calls in global ids (a < b).  The ring computes every
-// pair once, so MSF(union of the calls' forests) = MSF(triangle) under one strict order: every call breaks ties by global
-// ids (its keys), and an edge a call's forest left out is the maximum of a cycle of the whole graph.
-struct LinkageSink {
-    double max_dist;
-    std::vector<gkd::LinkEdge> edges;
-};
-
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
-                 ClusterSink *clusters, LinkageSink *linkage);
-
-// the ring of one member (runs on its own host thread; no exception may leave the thread).  With `within` the
-// member selects on its device and collects its hits there instead of scattering dense blocks into inter / dist;
-// with `nearest` it collects partial k-nearest lists, with `clusters` the links of its calls' components, with
-// `linkage` their spanning forests.
-void member_all_vs_all(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
-                       ClusterSink *clusters, LinkageSink *linkage) {
-    try {
-        member_ring(g, x, inter, dist, within, nearest, clusters, linkage);
-    } catch (const std::exception &ex) {
-        g->members[x].rc = GKD_ENOMEM;
-        g->members[x].err = ex.what();
-    }
-}
-
-void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, WithinSink *within, NearestSink *nearest,
-                 ClusterSink *clusters, LinkageSink *linkage) {
-    Member &M = g->members[x];
-    const uint32_t R = (uint32_t)g->members.size();
-    const uint64_t N = g->n_genomes;
-    const uint32_t m = (uint32_t)M.global_ids.size();
-    MCK(cudaSetDevice(M.device));
+    std::vector<GroupHit> hits;
+    std::vector<uint32_t> ha, hb;  // hit positions of one call
     std::vector<uint64_t> bi;
     std::vector<double> bd;
-    std::vector<uint32_t> ha, hb;  // within: hit positions of one call
-    uint64_t nh = 0;
-    auto fetch = [&](uint64_t pairs, auto call) -> int {  // one within call, repeated once with cap = n if it was short
+    explicit RingWithin(double d) : max_dist(d) {}
+    template <class Call>
+    int fetch(uint64_t pairs, Call call, uint64_t &nh) {  // one within call, repeated once with cap = n if it was short
         uint64_t cap = std::min(pairs, WITHIN_FIRST_CAP);
         for (;;) {
             ha.resize(cap);
@@ -236,13 +217,194 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
             if (h.n <= cap) return GKD_OK;
             cap = h.n;
         }
-    };
-    auto put = [&](uint32_t ga, uint32_t gb, uint64_t I, double d) {
-        if (ga > gb) std::swap(ga, gb);
-        const uint64_t t = row_start(ga, N) + (gb - ga - 1);
-        if (inter) inter[t] = I;
-        if (dist) dist[t] = d;
-    };
+    }
+    int diagonal(Member &M, uint32_t m) override {
+        const uint64_t cnt = (uint64_t)m * (m - 1) / 2;
+        uint64_t nh = 0;
+        const int rc = fetch(cnt, [&](gkd_hits &h) { return gkd_all_vs_all_range_within(M.ctx, m, 0, cnt, max_dist, &h); }, nh);
+        if (rc != GKD_OK) return rc;
+        for (uint64_t t = 0; t < nh; t++) hits.push_back({M.global_ids[ha[t]], M.global_ids[hb[t]], bi[t], bd[t]});
+        return GKD_OK;
+    }
+    int block(Member &M, const std::vector<uint32_t> &rows, const std::vector<uint32_t> &cols,
+              const std::vector<uint32_t> &col_gid) override {
+        uint64_t nh = 0;
+        const int rc = fetch((uint64_t)rows.size() * cols.size(), [&](gkd_hits &h) {
+            return gkd_query_vs_ref_within(M.ctx, rows.data(), (uint32_t)rows.size(), cols.data(), (uint32_t)cols.size(), max_dist, &h);
+        }, nh);
+        if (rc != GKD_OK) return rc;
+        for (uint64_t t = 0; t < nh; t++) {
+            const uint32_t ga = M.global_ids[rows[ha[t]]], gb = col_gid[hb[t]];
+            hits.push_back({std::min(ga, gb), std::max(ga, gb), bi[t], bd[t]});
+        }
+        return GKD_OK;
+    }
+};
+
+// gkd_group_all_vs_all_nearest: a member's partial lists by global id.  A pair is computed once in the whole ring, so
+// the global top k of an id, by (distance bits, global id), is the top k of the union of its partial top-k lists.
+struct Neighbor {
+    uint64_t key;  // distance bits (distances are non-negative: the bits order like the values)
+    uint32_t id;
+    uint64_t inter;
+    bool operator<(const Neighbor &o) const { return key < o.key || (key == o.key && id < o.id); }
+};
+struct RingNearest : RingForm {
+    uint32_t k;
+    double max_dist;
+    std::vector<std::vector<Neighbor>> lists;  // global id -> <= k entries after every call
+    std::vector<uint32_t> qpos, qn, rpos, rn;  // the lists of one call, per side
+    std::vector<uint64_t> qi, ri;
+    std::vector<double> qd, rd;
+    RingNearest(uint32_t k_, double d, uint32_t n) : k(k_), max_dist(d), lists(n) {}
+    void add(uint32_t target, uint32_t id, uint64_t inter, double d) {
+        uint64_t key;
+        memcpy(&key, &d, 8);
+        lists[target].push_back(Neighbor{key, id, inter});
+    }
+    void keep_best(uint32_t target) {
+        std::vector<Neighbor> &l = lists[target];
+        if (l.size() <= k) return;
+        std::partial_sort(l.begin(), l.begin() + k, l.end());
+        l.resize(k);
+    }
+    gkd_neighbors side(size_t rows, std::vector<uint32_t> &pos, std::vector<uint64_t> &in, std::vector<double> &d,
+                       std::vector<uint32_t> &nf) {
+        pos.resize(rows * k);
+        in.resize(rows * k);
+        d.resize(rows * k);
+        nf.resize(rows);
+        return gkd_neighbors{pos.data(), in.data(), d.data(), nf.data()};
+    }
+    int diagonal(Member &M, uint32_t m) override {
+        const gkd_neighbors nb = side(m, qpos, qi, qd, qn);
+        const int rc = gkd_all_vs_all_nearest(M.ctx, m, k, max_dist, &nb);
+        if (rc != GKD_OK) return rc;
+        for (uint32_t i = 0; i < m; i++)
+            for (uint32_t s = 0; s < qn[i]; s++) {
+                const uint64_t o = (uint64_t)i * k + s;
+                add(M.global_ids[i], M.global_ids[qpos[o]], qi[o], qd[o]);
+            }
+        return GKD_OK;
+    }
+    int block(Member &M, const std::vector<uint32_t> &rows, const std::vector<uint32_t> &cols,
+              const std::vector<uint32_t> &col_gid) override {
+        // The lists break ties by position in the call, and a group of panels may span peers (x+1)%R, (x+2)%R, ...,
+        // whose global ids are not ascending: order the columns by global id so that position order is id order.
+        // The rows are this member's own ids, ascending.
+        std::vector<uint32_t> order(cols.size());
+        for (uint32_t c = 0; c < order.size(); c++) order[c] = c;
+        std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return col_gid[a] < col_gid[b]; });
+        std::vector<uint32_t> scols(cols.size()), sgid(cols.size());
+        for (size_t c = 0; c < order.size(); c++) scols[c] = cols[order[c]], sgid[c] = col_gid[order[c]];
+        const gkd_neighbors qs = side(rows.size(), qpos, qi, qd, qn), rs = side(cols.size(), rpos, ri, rd, rn);
+        const int rc = gkd_query_vs_ref_nearest_ex(M.ctx, rows.data(), (uint32_t)rows.size(), scols.data(), (uint32_t)scols.size(),
+                                                   k, max_dist, 0, &qs, &rs);
+        if (rc != GKD_OK) return rc;
+        for (size_t r = 0; r < rows.size(); r++) {
+            const uint32_t target = M.global_ids[rows[r]];
+            for (uint32_t s = 0; s < qn[r]; s++) {
+                const uint64_t o = (uint64_t)r * k + s;
+                add(target, sgid[qpos[o]], qi[o], qd[o]);
+            }
+            keep_best(target);
+        }
+        for (size_t c = 0; c < scols.size(); c++) {
+            for (uint32_t s = 0; s < rn[c]; s++) {
+                const uint64_t o = (uint64_t)c * k + s;
+                add(sgid[c], M.global_ids[rows[rpos[o]]], ri[o], rd[o]);
+            }
+            keep_best(sgid[c]);
+        }
+        return GKD_OK;
+    }
+};
+
+// gkd_group_all_vs_all_clusters: a member's links (global p, global label[p]) for every node p of its calls with
+// label[p] != p.  A call's labels carry all the connectivity of its links, and the ring computes every pair once, so
+// the union of these links over all members has the components of the whole triangle.
+struct RingClusters : RingForm {
+    double max_dist;
+    std::vector<std::pair<uint32_t, uint32_t>> links;
+    std::vector<uint32_t> ql, rl;  // the labels of one call
+    explicit RingClusters(double d) : max_dist(d) {}
+    int diagonal(Member &M, uint32_t m) override {
+        ql.resize(m);
+        const int rc = gkd_all_vs_all_clusters(M.ctx, m, max_dist, ql.data(), nullptr);
+        if (rc != GKD_OK) return rc;
+        for (uint32_t i = 0; i < m; i++)
+            if (ql[i] != i) links.push_back({M.global_ids[i], M.global_ids[ql[i]]});
+        return GKD_OK;
+    }
+    int block(Member &M, const std::vector<uint32_t> &rows, const std::vector<uint32_t> &cols,
+              const std::vector<uint32_t> &col_gid) override {
+        const uint32_t nr = (uint32_t)rows.size(), nc = (uint32_t)cols.size();
+        auto gid = [&](uint32_t node) { return node < nr ? M.global_ids[rows[node]] : col_gid[node - nr]; };
+        ql.resize(nr);
+        rl.resize(nc);
+        const int rc = gkd_query_vs_ref_clusters(M.ctx, rows.data(), nr, cols.data(), nc, max_dist, ql.data(), rl.data());
+        if (rc != GKD_OK) return rc;
+        for (uint32_t p = 0; p < nr; p++)
+            if (ql[p] != p) links.push_back({gid(p), gid(ql[p])});
+        for (uint32_t c = 0; c < nc; c++)
+            if (rl[c] != nr + c) links.push_back({col_gid[c], gid(rl[c])});
+        return GKD_OK;
+    }
+};
+
+// gkd_group_all_vs_all_linkage: the forest edges of a member's calls in global ids (a < b).  The ring computes every
+// pair once, so MSF(union of the calls' forests) = MSF(triangle) under one strict order: every call breaks ties by global
+// ids (its keys), and an edge a call's forest left out is the maximum of a cycle of the whole graph.
+struct RingLinkage : RingForm {
+    double max_dist;
+    std::vector<gkd::LinkEdge> edges;
+    std::vector<uint32_t> ha, hb;
+    std::vector<uint64_t> bi;
+    std::vector<double> bd;
+    explicit RingLinkage(double d) : max_dist(d) {}
+    // the forest of one call, at most nodes - 1 edges
+    template <class Call, class GidA, class GidB>
+    int forest(uint64_t nodes, Call call, GidA gid_a, GidB gid_b) {
+        ha.resize(nodes);
+        hb.resize(nodes);
+        bi.resize(nodes);
+        bd.resize(nodes);
+        gkd_hits h{ha.data(), hb.data(), bi.data(), bd.data(), nodes, 0};
+        const int rc = call(h);
+        if (rc != GKD_OK) return rc;
+        for (uint64_t t = 0; t < h.n; t++) {
+            const uint32_t ga = gid_a(ha[t]), gb = gid_b(hb[t]), lo = std::min(ga, gb), hi = std::max(ga, gb);
+            edges.push_back(gkd::link_edge(lo, hi, bi[t], bd[t], lo, hi, lo, hi));
+        }
+        return GKD_OK;
+    }
+    int diagonal(Member &M, uint32_t m) override {
+        auto own = [&](uint32_t i) { return M.global_ids[i]; };  // ascending, so local order is global order
+        return forest(m, [&](gkd_hits &h) { return gkd_all_vs_all_linkage(M.ctx, m, max_dist, &h); }, own, own);
+    }
+    int block(Member &M, const std::vector<uint32_t> &rows, const std::vector<uint32_t> &cols,
+              const std::vector<uint32_t> &col_gid) override {
+        // keyed by global id: the columns may span peers on both sides of this member's ids, and ties must be broken
+        // as one context over all ids breaks them
+        const uint32_t nr = (uint32_t)rows.size(), nc = (uint32_t)cols.size();
+        std::vector<uint32_t> row_gid(nr);
+        for (uint32_t p = 0; p < nr; p++) row_gid[p] = M.global_ids[rows[p]];
+        return forest((uint64_t)nr + nc - 1,
+                      [&](gkd_hits &h) {
+                          return gkd_query_vs_ref_linkage(M.ctx, rows.data(), nr, cols.data(), nc, max_dist, row_gid.data(),
+                                                          col_gid.data(), &h);
+                      },
+                      [&](uint32_t p) { return row_gid[p]; }, [&](uint32_t c) { return col_gid[c]; });
+    }
+};
+
+// The ring of one member (runs on its own host thread; no exception may leave the thread): its diagonal block while the
+// first group of peer panels is in flight, then one call per group, each through the member's form.
+void member_ring(gkd_group *g, uint32_t x, RingForm &f) {
+    Member &M = g->members[x];
+    const uint32_t R = (uint32_t)g->members.size();
+    const uint32_t m = (uint32_t)M.global_ids.size();
+    MCK(cudaSetDevice(M.device));
     // transfer slots: (panel to receive, its owner, my rows)
     struct Slot {
         Panel p;
@@ -304,69 +466,8 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
     };
     if (!groups.empty()) post(0);
     if (M.rc) return;
-
-    // nearest: host lists of one call, per side
-    std::vector<uint32_t> qpos, qn, rpos, rn;
-    std::vector<uint64_t> qi, ri;
-    std::vector<double> qd, rd;
-    auto side = [&](size_t rows_, std::vector<uint32_t> &pos, std::vector<uint64_t> &in, std::vector<double> &d,
-                    std::vector<uint32_t> &nf) {
-        const size_t slots = rows_ * nearest->k;
-        pos.resize(slots);
-        in.resize(slots);
-        d.resize(slots);
-        nf.resize(rows_);
-        return gkd_neighbors{pos.data(), in.data(), d.data(), nf.data()};
-    };
-    std::vector<uint32_t> ql, rl;  // clusters: the labels of one call
-    // linkage: the forest of one call, at most nodes - 1 edges
-    auto forest = [&](uint64_t nodes, auto call, auto gid_a, auto gid_b) -> int {
-        ha.resize(nodes);
-        hb.resize(nodes);
-        bi.resize(nodes);
-        bd.resize(nodes);
-        gkd_hits h{ha.data(), hb.data(), bi.data(), bd.data(), nodes, 0};
-        const int rc = call(h);
-        if (rc != GKD_OK) return rc;
-        for (uint64_t t = 0; t < h.n; t++) {
-            const uint32_t ga = gid_a(ha[t]), gb = gid_b(hb[t]), lo = std::min(ga, gb), hi = std::max(ga, gb);
-            linkage->edges.push_back(gkd::link_edge(lo, hi, bi[t], bd[t], lo, hi, lo, hi));
-        }
-        return GKD_OK;
-    };
-    // diagonal block (runs while the first group is in flight)
-    if (m >= 2 && linkage) {
-        auto own = [&](uint32_t i) { return M.global_ids[i]; };  // ascending, so local order is global order
-        MGK(forest(m, [&](gkd_hits &h) { return gkd_all_vs_all_linkage(M.ctx, m, linkage->max_dist, &h); }, own, own));
-    } else if (m >= 2 && clusters) {
-        ql.resize(m);
-        MGK(gkd_all_vs_all_clusters(M.ctx, m, clusters->max_dist, ql.data(), nullptr));
-        for (uint32_t i = 0; i < m; i++)
-            if (ql[i] != i) clusters->links.push_back({M.global_ids[i], M.global_ids[ql[i]]});
-    } else if (m >= 2 && nearest) {
-        const uint32_t k = nearest->k;
-        const gkd_neighbors nb = side(m, qpos, qi, qd, qn);
-        MGK(gkd_all_vs_all_nearest(M.ctx, m, k, nearest->max_dist, &nb));
-        for (uint32_t i = 0; i < m; i++)
-            for (uint32_t s = 0; s < qn[i]; s++) {
-                const uint64_t o = (uint64_t)i * k + s;
-                nearest->add(M.global_ids[i], M.global_ids[qpos[o]], qi[o], qd[o]);
-            }
-    } else if (m >= 2 && within) {
-        const uint64_t cnt = (uint64_t)m * (m - 1) / 2;
-        MGK(fetch(cnt, [&](gkd_hits &h) { return gkd_all_vs_all_range_within(M.ctx, m, 0, cnt, within->max_dist, &h); }));
-        for (uint64_t t = 0; t < nh; t++) within->hits.push_back({M.global_ids[ha[t]], M.global_ids[hb[t]], bi[t], bd[t]});
-    } else if (m >= 2) {
-        const uint64_t cnt = (uint64_t)m * (m - 1) / 2;
-        bi.resize(cnt);
-        bd.resize(cnt);
-        MGK(gkd_all_vs_all_range(M.ctx, m, 0, cnt, bi.data(), bd.data()));
-        uint64_t t = 0;
-        for (uint32_t i = 0; i < m; i++)
-            for (uint32_t j = i + 1; j < m; j++, t++) put(M.global_ids[i], M.global_ids[j], bi[t], bd[t]);
-    }
+    if (m >= 2) MGK(f.diagonal(M, m));
     std::vector<uint32_t> rows, cols, col_gid;  // col_gid: global id of every column of the call
-    std::vector<uint32_t> order;
     for (size_t gi = 0; gi < groups.size(); gi++) {
         if (gi + 1 < groups.size()) {
             // buffer (gi+1)&1 was last used by group gi-1, whose sets were dropped (and the stream drained) below
@@ -390,93 +491,32 @@ void member_ring(gkd_group *g, uint32_t x, uint64_t *inter, double *dist, Within
                 col_gid.push_back(g->members[S.src].global_ids[S.p.first + c]);
             }
         }
-        if (linkage) {
-            // keyed by global id: the columns may span peers on both sides of this member's ids, and ties must be broken
-            // as one context over all ids breaks them
-            const uint32_t nr = (uint32_t)rows.size(), nc = (uint32_t)cols.size();
-            std::vector<uint32_t> row_gid(nr);
-            for (uint32_t p = 0; p < nr; p++) row_gid[p] = M.global_ids[rows[p]];
-            MGK(forest((uint64_t)nr + nc - 1,
-                       [&](gkd_hits &h) {
-                           return gkd_query_vs_ref_linkage(M.ctx, rows.data(), nr, cols.data(), nc, linkage->max_dist,
-                                                           row_gid.data(), col_gid.data(), &h);
-                       },
-                       [&](uint32_t p) { return row_gid[p]; }, [&](uint32_t c) { return col_gid[c]; }));
-            MGK(gkd_truncate(M.ctx, m));
-            continue;
-        }
-        if (clusters) {
-            const uint32_t nr = (uint32_t)rows.size(), nc = (uint32_t)cols.size();
-            auto gid = [&](uint32_t node) { return node < nr ? M.global_ids[rows[node]] : col_gid[node - nr]; };
-            ql.resize(nr);
-            rl.resize(nc);
-            MGK(gkd_query_vs_ref_clusters(M.ctx, rows.data(), nr, cols.data(), nc, clusters->max_dist, ql.data(), rl.data()));
-            for (uint32_t p = 0; p < nr; p++)
-                if (ql[p] != p) clusters->links.push_back({gid(p), gid(ql[p])});
-            for (uint32_t c = 0; c < nc; c++)
-                if (rl[c] != nr + c) clusters->links.push_back({col_gid[c], gid(rl[c])});
-            MGK(gkd_truncate(M.ctx, m));
-            continue;
-        }
-        if (nearest) {
-            // The lists break ties by position in the call, and a group of panels may span peers (x+1)%R, (x+2)%R, ...,
-            // whose global ids are not ascending: order the columns by global id so that position order is id order.
-            // The rows are this member's own ids, ascending.
-            order.resize(cols.size());
-            for (uint32_t c = 0; c < order.size(); c++) order[c] = c;
-            std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return col_gid[a] < col_gid[b]; });
-            std::vector<uint32_t> scols(cols.size()), sgid(cols.size());
-            for (size_t c = 0; c < order.size(); c++) scols[c] = cols[order[c]], sgid[c] = col_gid[order[c]];
-            const uint32_t k = nearest->k;
-            const gkd_neighbors qs = side(rows.size(), qpos, qi, qd, qn), rs = side(cols.size(), rpos, ri, rd, rn);
-            MGK(gkd_query_vs_ref_nearest_ex(M.ctx, rows.data(), (uint32_t)rows.size(), scols.data(), (uint32_t)scols.size(), k,
-                                            nearest->max_dist, 0, &qs, &rs));
-            for (size_t r = 0; r < rows.size(); r++) {
-                const uint32_t target = M.global_ids[rows[r]];
-                for (uint32_t s = 0; s < qn[r]; s++) {
-                    const uint64_t o = (uint64_t)r * k + s;
-                    nearest->add(target, sgid[qpos[o]], qi[o], qd[o]);
-                }
-                nearest->keep_best(target);
-            }
-            for (size_t c = 0; c < scols.size(); c++) {
-                for (uint32_t s = 0; s < rn[c]; s++) {
-                    const uint64_t o = (uint64_t)c * k + s;
-                    nearest->add(sgid[c], M.global_ids[rows[rpos[o]]], ri[o], rd[o]);
-                }
-                nearest->keep_best(sgid[c]);
-            }
-            MGK(gkd_truncate(M.ctx, m));
-            continue;
-        }
-        if (within) {
-            MGK(fetch((uint64_t)rows.size() * cols.size(), [&](gkd_hits &h) {
-                return gkd_query_vs_ref_within(M.ctx, rows.data(), (uint32_t)rows.size(), cols.data(), (uint32_t)cols.size(),
-                                               within->max_dist, &h);
-            }));
-            for (uint64_t t = 0; t < nh; t++) {
-                const uint32_t ga = M.global_ids[rows[ha[t]]], gb = col_gid[hb[t]];
-                within->hits.push_back({std::min(ga, gb), std::max(ga, gb), bi[t], bd[t]});
-            }
-            MGK(gkd_truncate(M.ctx, m));
-            continue;
-        }
-        bi.resize((size_t)rows.size() * cols.size());
-        bd.resize(bi.size());
-        MGK(gkd_query_vs_ref(M.ctx, rows.data(), (uint32_t)rows.size(), cols.data(), (uint32_t)cols.size(), bi.data(), bd.data()));
-        size_t col0 = 0;
-        for (size_t k = G.s0; k < G.s1; k++) {
-            const Slot &S = slots[k];
-            const std::vector<uint32_t> &their = g->members[S.src].global_ids;
-            for (uint32_t r = S0.row0; r < S0.row1; r++)
-                for (uint32_t c = 0; c < S.p.count; c++) {
-                    const size_t t = (size_t)(r - S0.row0) * cols.size() + col0 + c;
-                    put(M.global_ids[r], their[S.p.first + c], bi[t], bd[t]);
-                }
-            col0 += S.p.count;
-        }
+        MGK(f.block(M, rows, cols, col_gid));
         MGK(gkd_truncate(M.ctx, m));
     }
+}
+
+// Every member's ring with its own form forms[x], one host thread per member; the first member error is the group's
+template <class Form>
+int run_members(gkd_group *g, std::vector<Form> &forms) {
+    for (auto &M : g->members)
+        if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
+    std::vector<std::thread> threads;
+    for (uint32_t x = 0; x < g->members.size(); x++) {
+        g->members[x].rc = GKD_OK;
+        threads.emplace_back([g, x, &f = forms[x]]() {
+            try {
+                member_ring(g, x, f);
+            } catch (const std::exception &ex) {
+                g->members[x].rc = GKD_ENOMEM;
+                g->members[x].err = ex.what();
+            }
+        });
+    }
+    for (auto &t : threads) t.join();
+    for (size_t i = 0; i < g->members.size(); i++)
+        if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+    return GKD_OK;
 }
 
 }  // namespace
@@ -666,17 +706,8 @@ int gkd_group_build(gkd_group *g) {
 int gkd_group_all_vs_all(gkd_group *g, uint64_t *inter, double *dist) {
     if (!g) return GKD_EINVAL;
     try {
-        for (auto &M : g->members)
-            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
-        std::vector<std::thread> threads;
-        for (uint32_t x = 0; x < g->members.size(); x++) {
-            g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, inter, dist, nullptr, nullptr, nullptr, nullptr);
-        }
-        for (auto &t : threads) t.join();
-        for (size_t i = 0; i < g->members.size(); i++)
-            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
-        return GKD_OK;
+        std::vector<RingDense> forms(g->members.size(), RingDense(g->n_genomes, inter, dist));
+        return run_members(g, forms);
     } catch (const std::exception &ex) {
         return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all: %s", ex.what());
     }
@@ -687,23 +718,15 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
     if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_within: max_dist is NaN");
     if (!g) return GKD_EINVAL;
     try {
-        for (auto &M : g->members)
-            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
         out->n = 0;
-        std::vector<WithinSink> sinks(g->members.size(), WithinSink{max_dist, {}});
-        std::vector<std::thread> threads;
-        for (uint32_t x = 0; x < g->members.size(); x++) {
-            g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, &sinks[x], nullptr, nullptr, nullptr);
-        }
-        for (auto &t : threads) t.join();
-        for (size_t i = 0; i < g->members.size(); i++)
-            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        std::vector<RingWithin> forms(g->members.size(), RingWithin(max_dist));
+        const int rc = run_members(g, forms);
+        if (rc != GKD_OK) return rc;
         // the members own disjoint pairs: one sort by (a, b) gives the order of one context's row-major triangle
         std::vector<GroupHit> all;
-        for (auto &s : sinks) {
-            all.insert(all.end(), s.hits.begin(), s.hits.end());
-            std::vector<GroupHit>().swap(s.hits);
+        for (auto &f : forms) {
+            all.insert(all.end(), f.hits.begin(), f.hits.end());
+            std::vector<GroupHit>().swap(f.hits);
         }
         std::sort(all.begin(), all.end(), [](const GroupHit &p, const GroupHit &q) { return p.a < q.a || (p.a == q.a && p.b < q.b); });
         out->n = all.size();
@@ -721,29 +744,22 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
 }
 
 int gkd_group_all_vs_all_nearest(gkd_group *g, uint32_t k, double max_dist, const gkd_neighbors *out) {
-    if (k < 1 || k > NEAREST_MAX_K) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nearest: k = %u is outside 1..%u", k, NEAREST_MAX_K);
+    if (k < 1 || k > gkd::NEAREST_MAX_K)
+        return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nearest: k = %u is outside 1..%u", k, gkd::NEAREST_MAX_K);
     if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nearest: max_dist is NaN");
     if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nearest: null output");
     if (!g) return GKD_EINVAL;
     try {
-        for (auto &M : g->members)
-            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
         const uint32_t N = g->n_genomes;
-        std::vector<NearestSink> sinks(g->members.size(), NearestSink{k, max_dist, std::vector<std::vector<Neighbor>>(N)});
-        std::vector<std::thread> threads;
-        for (uint32_t x = 0; x < g->members.size(); x++) {
-            g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, &sinks[x], nullptr, nullptr);
-        }
-        for (auto &t : threads) t.join();
-        for (size_t i = 0; i < g->members.size(); i++)
-            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        std::vector<RingNearest> forms(g->members.size(), RingNearest(k, max_dist, N));
+        const int rc = run_members(g, forms);
+        if (rc != GKD_OK) return rc;
         std::vector<Neighbor> all;
         for (uint32_t t = 0; t < N; t++) {
             all.clear();
-            for (auto &s : sinks) {
-                all.insert(all.end(), s.lists[t].begin(), s.lists[t].end());
-                std::vector<Neighbor>().swap(s.lists[t]);
+            for (auto &f : forms) {
+                all.insert(all.end(), f.lists[t].begin(), f.lists[t].end());
+                std::vector<Neighbor>().swap(f.lists[t]);
             }
             const size_t m = std::min<size_t>(all.size(), k);
             std::partial_sort(all.begin(), all.begin() + m, all.end());
@@ -768,21 +784,13 @@ int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label
     if (!label) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_clusters: null label");
     if (!g) return GKD_EINVAL;
     try {
-        for (auto &M : g->members)
-            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
-        std::vector<ClusterSink> sinks(g->members.size(), ClusterSink{max_dist, {}});
-        std::vector<std::thread> threads;
-        for (uint32_t x = 0; x < g->members.size(); x++) {
-            g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, nullptr, &sinks[x], nullptr);
-        }
-        for (auto &t : threads) t.join();
-        for (size_t i = 0; i < g->members.size(); i++)
-            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        std::vector<RingClusters> forms(g->members.size(), RingClusters(max_dist));
+        const int rc = run_members(g, forms);
+        if (rc != GKD_OK) return rc;
         const uint32_t N = g->n_genomes;
         gkd::HostForest forest(N);
-        for (auto &s : sinks)
-            for (const auto &l : s.links) forest.link(l.first, l.second);
+        for (auto &f : forms)
+            for (const auto &l : f.links) forest.link(l.first, l.second);
         uint32_t roots = 0;
         for (uint32_t i = 0; i < N; i++) {
             label[i] = forest.find(i);
@@ -800,21 +808,13 @@ int gkd_group_all_vs_all_linkage(gkd_group *g, double max_dist, gkd_hits *out) {
     if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_linkage: null out");
     if (!g) return GKD_EINVAL;
     try {
-        for (auto &M : g->members)
-            if (M.arenas.empty() && !M.global_ids.empty()) return gfail(g, GKD_ESTATE, "call gkd_group_build first");
-        std::vector<LinkageSink> sinks(g->members.size(), LinkageSink{max_dist, {}});
-        std::vector<std::thread> threads;
-        for (uint32_t x = 0; x < g->members.size(); x++) {
-            g->members[x].rc = GKD_OK;
-            threads.emplace_back(member_all_vs_all, g, x, nullptr, nullptr, nullptr, nullptr, nullptr, &sinks[x]);
-        }
-        for (auto &t : threads) t.join();
-        for (size_t i = 0; i < g->members.size(); i++)
-            if (g->members[i].rc != GKD_OK) return gfail(g, g->members[i].rc, "member %zu: %s", i, g->members[i].err.c_str());
+        std::vector<RingLinkage> forms(g->members.size(), RingLinkage(max_dist));
+        const int rc = run_members(g, forms);
+        if (rc != GKD_OK) return rc;
         std::vector<gkd::LinkEdge> edges;
-        for (auto &s : sinks) {
-            edges.insert(edges.end(), s.edges.begin(), s.edges.end());
-            std::vector<gkd::LinkEdge>().swap(s.edges);
+        for (auto &f : forms) {
+            edges.insert(edges.end(), f.edges.begin(), f.edges.end());
+            std::vector<gkd::LinkEdge>().swap(f.edges);
         }
         gkd::host_msf(edges, g->n_genomes);
         out->n = edges.size();

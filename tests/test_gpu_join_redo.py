@@ -1,4 +1,4 @@
-"""The block-join overflow redo (csrc/join.cu k_join, gkd_api.cu run_pairs / select_chunk, intersect.cu
+"""The block-join overflow redo (csrc/join.cu k_join, gkd_api.cu run_pairs and its forms, intersect.cu
 k_nearest_absorb), forced and checked against exact oracles.
 
 Kernel 4's block join flags a task when the rows of one key range would fill more than 62.5 % of its shared-memory

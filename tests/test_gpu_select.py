@@ -10,7 +10,8 @@ Join-overflow redo: a block-join table is flagged (and the chunk redone by the m
 range fill more than 62.5 % of its slots.  With uniform keys that does not happen: GKD_JOIN_FILL is clamped to 45 % and
 every row's range count keeps its expected share under that target (the 45 % fill is covered below).  Coarse set
 tables and skewed imported key sets do overflow; tests/test_gpu_join_redo.py forces the redo that way and checks that
-the within and nearest selections of a redone chunk are copied and counted once (select_chunk in gkd_api.cu).
+the within and nearest selections of a redone chunk are copied and counted once (run_pairs and the Within /
+Nearest forms in gkd_api.cu).
 """
 import ctypes as C
 import os
