@@ -51,7 +51,10 @@ typedef enum gkd_alphabet { GKD_DNA = 0, GKD_PROT = 1, GKD_RNA = 2 } gkd_alphabe
  *   GKD_STRAND_BOTH      - reference semantics: the set holds the k-mers of the sequence and of its
  *                          reverse complement, so |S| = 2|C| - P and I = 2|C_A n C_B| - P_I where C
  *                          are canonical k-mers and P counts reverse-palindromic ones (even K only)
- *   GKD_STRAND_CANONICAL - plain Jaccard over canonical k-mers (identical doubles for odd K)        */
+ *   GKD_STRAND_CANONICAL - plain Jaccard over canonical k-mers.  For odd K (no palindromes) the
+ *                          distances equal GKD_STRAND_BOTH's bit for bit while |C_A| + |C_B| < 2^30:
+ *                          the both-strand Java int sum 2(|C_A| + |C_B|) wraps at 2^31 before the
+ *                          canonical sum does (not tested: it needs about 10^9 keys)               */
 typedef enum gkd_strand_mode { GKD_STRAND_BOTH = 0, GKD_STRAND_CANONICAL = 1 } gkd_strand_mode;
 
 /* What to do with a nucleotide k-mer that contains a character outside acgt (after lower-casing; u reads

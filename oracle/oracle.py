@@ -239,6 +239,13 @@ def py_kmer_set(contigs, k: int, alphabet: int = DNA, ambig: int = AMBIG_SKIP) -
     return out
 
 
+def py_canonical_set(contigs, k: int, alphabet: int = DNA) -> set:
+    """the set GKD_STRAND_CANONICAL counts: min(s, revcomp(s)) of every k-mer of py_kmer_set (lower-case
+    lexicographic order is the 2-bit key order a < c < g < t); protein sets are returned as they are"""
+    kmers = py_kmer_set(contigs, k, alphabet)
+    return kmers if alphabet == PROT else {min(s, py_revcomp(s)) for s in kmers}
+
+
 def py_distance(a: set, b: set) -> Tuple[int, float]:
     inter = sum(1 for x in b if x in a)
     if inter == 0:
