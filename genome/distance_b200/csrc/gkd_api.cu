@@ -10,7 +10,6 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <memory>
 #include <new>
 #include <string>
 #include <unordered_map>
@@ -130,6 +129,7 @@ struct gkd_ctx {
     DevBuf nn_pos, nn_inter, nn_dist, nn_found;  // accumulating nearest selection: per-target lists of one call
     DevBuf uf_parent;  // cluster selection: the union-find forest of one call and its root counter
     DevBuf lk_forest, lk_state;  // linkage selection: the spanning forest of one call and its Boruvka state
+    DevBuf lit_size, lit_inter;  // GKD_AMBIG_LITERAL: literal k-mers per set, and per pair of a chunk those both sets share
     int isect_algo = 0;  // GKD_ISECT_ALGO: 0 = choose per call, 1 = bucket merge only, 2 = block join whenever it applies
     bool use_msd = true;  // GKD_SORT_ALGO=lsd pins the LSD path
     bool sets_dirty = true;
@@ -781,10 +781,20 @@ int upload_sets(gkd_ctx *c) {
     if (!c->sets_dirty) return GKD_OK;
     const size_t n = c->genomes.size();
     std::vector<SetDesc> h(n);
-    for (size_t i = 0; i < n; i++) h[i] = c->genomes[i].desc;
+    std::vector<uint32_t> lit(n);
+    bool any_lit = false;
+    for (size_t i = 0; i < n; i++) {
+        h[i] = c->genomes[i].desc;
+        lit[i] = (uint32_t)c->genomes[i].lit.size();
+        any_lit = any_lit || lit[i];
+    }
     int rc = ensure(c, c->d_sets, std::max<size_t>(n, 1) * sizeof(SetDesc));
     if (rc) return rc;
     if (n) CK(cudaMemcpyAsync(c->d_sets.p, h.data(), n * sizeof(SetDesc), cudaMemcpyHostToDevice, c->stream));
+    if (any_lit) {
+        if ((rc = ensure(c, c->lit_size, n * 4))) return rc;
+        CK(cudaMemcpyAsync(c->lit_size.p, lit.data(), n * 4, cudaMemcpyHostToDevice, c->stream));
+    }
     CK(cudaStreamSynchronize(c->stream));
     c->sets_dirty = false;
     return GKD_OK;
@@ -844,17 +854,6 @@ int check_built(gkd_ctx *c, uint32_t id) {
     if (id >= c->genomes.size()) return fail(c, GKD_EINVAL, "set id %u out of range (have %zu)", id, c->genomes.size());
     if (!c->genomes[id].built) return fail(c, GKD_ESTATE, "set %u has not been built; call gkd_build_sets first", id);
     return GKD_OK;
-}
-
-// SequenceKmers.distance on the host, for the pairs the literal side lists complete (same double formula
-// as kernel 5)
-double host_distance(uint64_t I, uint64_t sa, uint64_t sb) {
-    double ret = 1.0, similarity = (double)I;
-    if (similarity > 0) {
-        int32_t sum = (int32_t)((uint32_t)sa + (uint32_t)sb);
-        ret = 1.0 - similarity / ((double)sum - similarity);
-    }
-    return ret;
 }
 
 uint64_t both_size(const gkd_ctx *c, const GenomeRec &g) {
@@ -1005,37 +1004,20 @@ struct Chunk {
     const HostPairs &hp;
     const PairSource &src;
     uint64_t done, cnt;
-    const SetDesc *sets;
-    const uint32_t *counts, *pal;  // pal: nullptr unless the palindrome counts are needed
-    int both;
-    const uint32_t *join_err;      // the block join's overflow flag on the device; nullptr when the merge kernel ran
-    // pair t of the chunk as reported: RECT (a_base + query row, reference position), otherwise the two set ids
-    void pair(uint32_t a_base, uint64_t t, uint32_t &a, uint32_t &b) const {
-        if (hp.mode == PAIRS_RECT) a = a_base + (uint32_t)((done + t) / hp.nb), b = (uint32_t)((done + t) % hp.nb);
-        else host_pair_ids(hp, done + t, a, b);
-    }
+    PairCounts pc;
+    const uint32_t *join_err;  // the block join's overflow flag on the device; nullptr when the merge kernel ran
 };
 
 // What a call computes from the counts of kernel 4: one form of kernel 5.  run_pairs owns the chunk loop and the redo of
-// a chunk whose join table overflowed; the form owns its state, its launches, its copies and its rule for pairs that are
-// completed on the host.  The bytes queue() and keep() read back are counted only for a chunk that is kept.
+// a chunk whose join table overflowed; the form owns its state, its launches and its copies.  The bytes queue() and
+// keep() read back are counted only for a chunk that is kept.
 struct Form {
-    uint32_t a_base = 0;              // RECT: position in the caller's q of this launch's first query row (run_rect)
-    std::vector<uint64_t> lit_inter;  // GKD_AMBIG_LITERAL: the chunk's pairs, completed on the host
-    std::vector<double> lit_dist;
+    uint32_t a_base = 0;  // RECT: position in the caller's q of this launch's first query row (run_rect)
     virtual ~Form() = default;
     // the chunk's kernel-5 launches, then the reads the host needs once the stream is synchronised; records ev[7]
     virtual int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) = 0;
     // the join held: the chunk is kept
     virtual int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) { return GKD_OK; }
-    // GKD_AMBIG_LITERAL: host memory for the chunk's dense values (inter is required) ...
-    virtual gkd_outputs literal_outputs(const Chunk &e) {
-        lit_inter.resize(e.cnt);
-        lit_dist.resize(e.cnt);
-        return gkd_outputs{lit_inter.data(), lit_dist.data(), nullptr, nullptr};
-    }
-    // ... and the form's rule on them once they are completed, the same as its device kernels'
-    virtual void host(const Chunk &e, const uint64_t *inter, const double *dist) {}
 };
 
 // a read of `bytes` from the device into dst (host or device memory), skipped when dst is nullptr; counted in d2h
@@ -1046,44 +1028,33 @@ int read_back(gkd_ctx *c, void *dst, const void *src, uint64_t bytes, uint64_t &
     return GKD_OK;
 }
 
-// kernel 5, dense form: the chunk's values to o[0, cnt); a nullptr member of o is not computed
-int dense_epilogue(gkd_ctx *c, const Chunk &e, const gkd_outputs &o, uint64_t &d2h) {
-    int rc;
-    if (o.inter && (rc = ensure(c, c->d_inter, e.cnt * 8))) return rc;
-    if (o.dist && (rc = ensure(c, c->d_dist, e.cnt * 8))) return rc;
-    if (o.contain_a && (rc = ensure(c, c->d_ca, e.cnt * 8))) return rc;
-    if (o.contain_b && (rc = ensure(c, c->d_cb, e.cnt * 8))) return rc;
-    EpilogueOut eo{o.inter ? (uint64_t *)c->d_inter.p : nullptr, o.dist ? (double *)c->d_dist.p : nullptr,
-                   o.contain_a ? (double *)c->d_ca.p : nullptr, o.contain_b ? (double *)c->d_cb.p : nullptr};
-    nvtxRangePushA("gkd kernel 5: distance epilogue");
-    CK(launch_epilogue(e.sets, e.src, e.counts, e.pal, e.both, eo, c->stream));
-    nvtxRangePop();
-    c->m.launches++;
-    CK(cudaEventRecord(c->ev[7], c->stream));
-    // queued before the overflow flag is read: a redo rewrites the same slots
-    if ((rc = read_back(c, o.inter, c->d_inter.p, e.cnt * 8, d2h)) || (rc = read_back(c, o.dist, c->d_dist.p, e.cnt * 8, d2h)) ||
-        (rc = read_back(c, o.contain_a, c->d_ca.p, e.cnt * 8, d2h)) || (rc = read_back(c, o.contain_b, c->d_cb.p, e.cnt * 8, d2h)))
-        return rc;
-    return GKD_OK;
-}
-
-// gkd_all_vs_all*, gkd_query_vs_ref*, gkd_pairs*: every pair's values to the caller's outputs
+// gkd_all_vs_all*, gkd_query_vs_ref*, gkd_pairs*: every pair's values to the caller's outputs; a nullptr member of the
+// outputs is not computed
 struct Dense : Form {
     gkd_outputs out;
     explicit Dense(const gkd_outputs &o) : out(o) {}
-    gkd_outputs at(const Chunk &e) const {  // the chunk's part of out (RECT: from row a_base of the caller's block)
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        // the chunk's part of out (RECT: from row a_base of the caller's block)
         const uint64_t t = (uint64_t)a_base * e.hp.nb + e.done;
-        return gkd_outputs{out.inter ? out.inter + t : nullptr, out.dist ? out.dist + t : nullptr,
-                           out.contain_a ? out.contain_a + t : nullptr, out.contain_b ? out.contain_b + t : nullptr};
-    }
-    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override { return dense_epilogue(c, e, at(e), d2h); }
-    gkd_outputs literal_outputs(const Chunk &e) override {
-        gkd_outputs o = at(e);
-        if (!o.inter) {
-            lit_inter.resize(e.cnt);
-            o.inter = lit_inter.data();
-        }
-        return o;
+        const gkd_outputs o{out.inter ? out.inter + t : nullptr, out.dist ? out.dist + t : nullptr,
+                            out.contain_a ? out.contain_a + t : nullptr, out.contain_b ? out.contain_b + t : nullptr};
+        int rc;
+        if (o.inter && (rc = ensure(c, c->d_inter, e.cnt * 8))) return rc;
+        if (o.dist && (rc = ensure(c, c->d_dist, e.cnt * 8))) return rc;
+        if (o.contain_a && (rc = ensure(c, c->d_ca, e.cnt * 8))) return rc;
+        if (o.contain_b && (rc = ensure(c, c->d_cb, e.cnt * 8))) return rc;
+        EpilogueOut eo{o.inter ? (uint64_t *)c->d_inter.p : nullptr, o.dist ? (double *)c->d_dist.p : nullptr,
+                       o.contain_a ? (double *)c->d_ca.p : nullptr, o.contain_b ? (double *)c->d_cb.p : nullptr};
+        nvtxRangePushA("gkd kernel 5: distance epilogue");
+        CK(launch_epilogue(e.src, e.pc, eo, c->stream));
+        nvtxRangePop();
+        c->m.launches++;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        // queued before the overflow flag is read: a redo rewrites the same slots
+        if ((rc = read_back(c, o.inter, c->d_inter.p, e.cnt * 8, d2h)) || (rc = read_back(c, o.dist, c->d_dist.p, e.cnt * 8, d2h)) ||
+            (rc = read_back(c, o.contain_a, c->d_ca.p, e.cnt * 8, d2h)) || (rc = read_back(c, o.contain_b, c->d_cb.p, e.cnt * 8, d2h)))
+            return rc;
+        return GKD_OK;
     }
 };
 
@@ -1154,7 +1125,7 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, Form &f) {
 
     bool join_banned = false;  // set when a join table overflowed: the chunk is redone by the merge kernel
     JoinPlan jplan{};
-    std::vector<uint32_t> jrows;
+    std::vector<uint32_t> jrows, lit_inter;
     for (uint64_t done = 0; done < hp.count;) {
         const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, hp.count - done);
         src.count = cnt;
@@ -1218,42 +1189,41 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, Form &f) {
             c->m.launches++;
         }
         CK(cudaEventRecord(c->ev[6], c->stream));
-        const Chunk e{hp, src, done, cnt, (const SetDesc *)c->d_sets.p, (const uint32_t *)c->counts.p,
-                      need_pal ? (const uint32_t *)c->pal_counts.p : nullptr, both ? 1 : 0,
-                      use_join ? (const uint32_t *)c->join_err.p : nullptr};
-        // with literal side lists the pairs are completed on the host, which needs the counts: the dense epilogue runs
-        // into host memory and the form takes the completed pairs
+        PairCounts pc{(const SetDesc *)c->d_sets.p, (const uint32_t *)c->counts.p,
+                      need_pal ? (const uint32_t *)c->pal_counts.p : nullptr, s.any_lit ? (const uint32_t *)c->lit_size.p : nullptr,
+                      nullptr, both ? 1 : 0};
+        if (s.any_lit) {
+            // GKD_AMBIG_LITERAL: the literal k-mers live on the host, so the part of I they share is counted here while
+            // kernel 4 runs; kernel 5 adds it, and the sizes, to the counts
+            lit_inter.resize(cnt);
+            bool shared = false;
+            for (uint64_t t = 0; t < cnt; t++) {
+                uint32_t a, b;
+                host_pair_ids(hp, done + t, a, b);
+                lit_inter[t] = (uint32_t)literal_intersection(c->genomes[a].lit, c->genomes[b].lit);
+                shared = shared || lit_inter[t];
+            }
+            if (shared) {
+                if ((rc = ensure(c, c->lit_inter, cnt * 4))) return rc;
+                CK(cudaMemcpyAsync(c->lit_inter.p, lit_inter.data(), cnt * 4, cudaMemcpyHostToDevice, c->stream));
+                c->m.h2d_bytes += cnt * 4;
+                pc.lit_inter = (const uint32_t *)c->lit_inter.p;
+            }
+        }
+        const Chunk e{hp, src, done, cnt, pc, use_join ? (const uint32_t *)c->join_err.p : nullptr};
         uint64_t d2h = 0;
-        const gkd_outputs lit = s.any_lit ? f.literal_outputs(e) : gkd_outputs{};
-        if ((rc = s.any_lit ? dense_epilogue(c, e, lit, d2h) : f.queue(c, e, d2h))) return rc;
+        if ((rc = f.queue(c, e, d2h))) return rc;
         CK(cudaStreamSynchronize(c->stream));
         if (join_err) {  // the attempt keeps nothing
             join_banned = true;
             continue;
         }
-        if (!s.any_lit && (rc = f.keep(c, e, d2h))) return rc;
+        if ((rc = f.keep(c, e, d2h))) return rc;
         c->m.d2h_bytes += d2h;
         const double ims = elapsed(c->ev[4], c->ev[5]);
         c->m.intersect_ms += ims;
         c->m.total_intersect_ms += ims;
         c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
-        if (s.any_lit) {
-            // GKD_AMBIG_LITERAL: add the literal k-mers both sets share and redo the formula with the
-            // full sizes (outputs must be host memory in this mode)
-            for (uint64_t t = 0; t < cnt; t++) {
-                uint32_t a, b;
-                host_pair_ids(hp, done + t, a, b);
-                const GenomeRec &ga = c->genomes[a], &gb = c->genomes[b];
-                if (ga.lit.empty() && gb.lit.empty()) continue;
-                const uint64_t I = lit.inter[t] + literal_intersection(ga.lit, gb.lit);
-                const uint64_t sa = both_size(c, ga), sb = both_size(c, gb);
-                lit.inter[t] = I;
-                if (lit.dist) lit.dist[t] = host_distance(I, sa, sb);
-                if (lit.contain_a) lit.contain_a[t] = sa ? (double)I / (double)sa : 0.0;
-                if (lit.contain_b) lit.contain_b[t] = sb ? (double)I / (double)sb : 0.0;
-            }
-            f.host(e, lit.inter, lit.dist);
-        }
         done += PAIR_CHUNK;
     }
     return GKD_OK;
@@ -1306,7 +1276,7 @@ struct Within : Form {
                          h.inter ? (uint64_t *)c->d_inter.p : nullptr, h.dist ? (double *)c->d_dist.p : nullptr};
         unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
         nvtxRangePushA("gkd kernel 5: within selection");
-        CK(launch_select_within(e.sets, e.src, e.counts, e.pal, e.both, max_dist, a_base, wcap, ho, cta, cta + nctas, c->stream));
+        CK(launch_select_within(e.src, e.pc, max_dist, a_base, wcap, ho, cta, cta + nctas, c->stream));
         nvtxRangePop();
         c->m.launches += wcap ? 3 : 2;
         CK(cudaEventRecord(c->ev[7], c->stream));
@@ -1326,71 +1296,22 @@ struct Within : Form {
         h.n += chunk_hits;
         return GKD_OK;
     }
-    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {
-        for (uint64_t t = 0; t < e.cnt; t++) {
-            if (!(dist[t] <= max_dist)) continue;
-            const uint64_t at = h.n++;
-            if (at >= h.cap) continue;
-            uint32_t a, b;
-            e.pair(a_base, t, a, b);
-            if (h.a) h.a[at] = a;
-            if (h.b) h.b[at] = b;
-            if (h.inter) h.inter[at] = inter[t];
-            if (h.dist) h.dist[at] = dist[t];
-        }
-    }
-};
-
-// GKD_AMBIG_LITERAL: the per-target lists of an accumulating nearest selection, kept on the host because the pairs
-// are completed there.  Same layout and unused entry as the device lists (c->nn_*); n[t] entries of target t are used.
-struct HostLists {
-    uint32_t k = 0;
-    std::vector<uint32_t> pos, n;
-    std::vector<uint64_t> inter;
-    std::vector<double> dist;
-    HostLists(uint32_t targets, uint32_t k_) : k(k_), pos((uint64_t)targets * k_, 0xFFFFFFFFu), n(targets, 0),
-                                               inter((uint64_t)targets * k_, 0), dist((uint64_t)targets * k_, -1.0) {}
-    // the admission rule of k_nearest_absorb: below the k-th entry in (distance bits, position)
-    void offer(uint32_t tg, uint32_t nb, uint64_t I, double d) {
-        const uint64_t base = (uint64_t)tg * k;
-        uint64_t key;
-        std::memcpy(&key, &d, 8);
-        auto below = [&](uint64_t s) {
-            uint64_t ks;
-            std::memcpy(&ks, &dist[s], 8);
-            return key < ks || (key == ks && nb < pos[s]);
-        };
-        uint32_t &m = n[tg];
-        if (m == k && !below(base + k - 1)) return;
-        uint32_t at = m == k ? k - 1 : m;
-        for (; at > 0 && below(base + at - 1); at--) {
-            pos[base + at] = pos[base + at - 1];
-            inter[base + at] = inter[base + at - 1];
-            dist[base + at] = dist[base + at - 1];
-        }
-        pos[base + at] = nb;
-        inter[base + at] = I;
-        dist[base + at] = d;
-        if (m < k) m++;
-    }
 };
 
 // gkd_*_nearest: the k nearest within max_dist by (distance bits, position).  rows (RECT only): each query row's list,
-// complete in every launch (k_select_nearest) and read back once the chunk is kept.  lists: per-target lists that the
-// launches merge into (k_nearest_absorb; UPPER: both ends of every pair, RECT: each reference's nearest queries), on the
-// device (c->nn_*) or, when the pairs are completed on the host, in host_lists; read once by finish().
+// complete in every launch (k_select_nearest) and read back once the chunk is kept.  lists: per-target lists on the
+// device (c->nn_*) that the launches merge into (k_nearest_absorb; UPPER: both ends of every pair, RECT: each
+// reference's nearest queries), read once by finish().
 struct Nearest : Form {
     uint32_t k;
     double max_dist;
     int exclude_self;
     const gkd_neighbors *rows, *lists;  // either may be nullptr
     uint32_t targets;
-    std::unique_ptr<HostLists> host_lists;
     Nearest(uint32_t k_, double d, int excl, const gkd_neighbors *rows_, const gkd_neighbors *lists_, uint32_t targets_)
         : k(k_), max_dist(d), exclude_self(excl), rows(rows_), lists(lists_), targets(targets_) {}
     int start(gkd_ctx *c) {  // every per-target list unused
         if (!lists) return GKD_OK;
-        if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) host_lists.reset(new HostLists(targets, k));
         const uint64_t slots = (uint64_t)targets * k;
         int rc;
         if ((rc = ensure(c, c->nn_pos, slots * 4)) || (rc = ensure(c, c->nn_inter, slots * 8)) ||
@@ -1417,7 +1338,7 @@ struct Nearest : Form {
             const NearestOut no{rows->pos ? (uint32_t *)c->hit_a.p : nullptr, rows->inter ? (uint64_t *)c->d_inter.p : nullptr,
                                 rows->dist ? (double *)c->d_dist.p : nullptr, rows->n_found ? (uint32_t *)c->hit_b.p : nullptr};
             nvtxRangePushA("gkd kernel 5: nearest selection");
-            CK(launch_select_nearest(e.sets, e.src, e.hp.na, e.counts, e.pal, e.both, max_dist, k, exclude_self, no, c->stream));
+            CK(launch_select_nearest(e.src, e.hp.na, e.pc, max_dist, k, exclude_self, no, c->stream));
             nvtxRangePop();
             c->m.launches++;
         }
@@ -1425,7 +1346,7 @@ struct Nearest : Form {
             // the lists outlive this chunk: the kernel itself skips a chunk whose join overflowed
             const NearestOut st{(uint32_t *)c->nn_pos.p, (uint64_t *)c->nn_inter.p, (double *)c->nn_dist.p, (uint32_t *)c->nn_found.p};
             nvtxRangePushA("gkd kernel 5: nearest absorb");
-            CK(launch_nearest_absorb(e.sets, e.src, e.counts, e.pal, e.both, max_dist, k, exclude_self, a_base, e.join_err, st, c->stream));
+            CK(launch_nearest_absorb(e.src, e.pc, max_dist, k, exclude_self, a_base, e.join_err, st, c->stream));
             nvtxRangePop();
             c->m.launches++;
         }
@@ -1444,85 +1365,30 @@ struct Nearest : Form {
         CK(cudaStreamSynchronize(c->stream));
         return GKD_OK;
     }
-    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {
-        const HostPairs &hp = e.hp;
-        for (uint64_t t = 0; lists && t < e.cnt; t++) {
-            if (!(dist[t] <= max_dist)) continue;
-            if (hp.mode == PAIRS_RECT) {
-                const uint32_t row = (uint32_t)((e.done + t) / hp.nb), j = (uint32_t)((e.done + t) % hp.nb);
-                if (!(exclude_self && hp.a[row] == hp.b[j])) host_lists->offer(j, a_base + row, inter[t], dist[t]);
-            } else {
-                uint32_t a, b;
-                host_pair_ids(hp, e.done + t, a, b);
-                host_lists->offer(a, b, inter[t], dist[t]);
-                host_lists->offer(b, a, inter[t], dist[t]);
-            }
-        }
-        if (!rows) return;
-        std::vector<uint32_t> js;
-        for (uint32_t row = 0; row < hp.na; row++) {
-            const uint64_t r0 = (uint64_t)row * hp.nb;
-            js.clear();
-            for (uint32_t j = 0; j < hp.nb; j++)
-                if (dist[r0 + j] <= max_dist && !(exclude_self && hp.a[row] == hp.b[j])) js.push_back(j);
-            const size_t m = std::min<size_t>(js.size(), k);
-            std::partial_sort(js.begin(), js.begin() + m, js.end(), [&](uint32_t x, uint32_t y) {
-                return dist[r0 + x] < dist[r0 + y] || (dist[r0 + x] == dist[r0 + y] && x < y);
-            });
-            for (uint32_t i = 0; i < k; i++) {
-                const uint64_t o = (uint64_t)(a_base + row) * k + i;
-                if (rows->pos) rows->pos[o] = i < m ? js[i] : 0xFFFFFFFFu;
-                if (rows->inter) rows->inter[o] = i < m ? inter[r0 + js[i]] : 0;
-                if (rows->dist) rows->dist[o] = i < m ? dist[r0 + js[i]] : -1.0;
-            }
-            if (rows->n_found) rows->n_found[a_base + row] = (uint32_t)m;
-        }
-    }
-    // the lists to the caller, once, at the end of the call.  With host_lists (GKD_AMBIG_LITERAL, host outputs) the
-    // launches that ran on the device are merged into the host lists first.
+    // the lists to the caller, once, at the end of the call
     int finish(gkd_ctx *c) {
         if (!lists) return GKD_OK;
         const gkd_neighbors &out = *lists;
         const uint64_t slots = (uint64_t)targets * k;
         int rc;
-        if (!host_lists) {
-            uint64_t d2h = 0;
-            if ((rc = read_back(c, out.pos, c->nn_pos.p, slots * 4, d2h)) || (rc = read_back(c, out.inter, c->nn_inter.p, slots * 8, d2h)) ||
-                (rc = read_back(c, out.dist, c->nn_dist.p, slots * 8, d2h)) ||
-                (rc = read_back(c, out.n_found, c->nn_found.p, (uint64_t)targets * 4, d2h)))
-                return rc;
-            CK(cudaStreamSynchronize(c->stream));
-            c->m.d2h_bytes += d2h;
-            return GKD_OK;
-        }
-        HostLists dev(targets, k);
-        CK(cudaMemcpyAsync(dev.pos.data(), c->nn_pos.p, slots * 4, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaMemcpyAsync(dev.inter.data(), c->nn_inter.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaMemcpyAsync(dev.dist.data(), c->nn_dist.p, slots * 8, cudaMemcpyDeviceToHost, c->stream));
+        uint64_t d2h = 0;
+        if ((rc = read_back(c, out.pos, c->nn_pos.p, slots * 4, d2h)) || (rc = read_back(c, out.inter, c->nn_inter.p, slots * 8, d2h)) ||
+            (rc = read_back(c, out.dist, c->nn_dist.p, slots * 8, d2h)) ||
+            (rc = read_back(c, out.n_found, c->nn_found.p, (uint64_t)targets * 4, d2h)))
+            return rc;
         CK(cudaStreamSynchronize(c->stream));
-        c->m.d2h_bytes += slots * 20;
-        HostLists &hl = *host_lists;
-        for (uint32_t t = 0; t < targets; t++)
-            for (uint64_t s = (uint64_t)t * k; s < (uint64_t)(t + 1) * k && dev.pos[s] != 0xFFFFFFFFu; s++)
-                hl.offer(t, dev.pos[s], dev.inter[s], dev.dist[s]);
-        if (out.pos) std::memcpy(out.pos, hl.pos.data(), slots * 4);
-        if (out.inter) std::memcpy(out.inter, hl.inter.data(), slots * 8);
-        if (out.dist) std::memcpy(out.dist, hl.dist.data(), slots * 8);
-        if (out.n_found) std::memcpy(out.n_found, hl.n.data(), (uint64_t)targets * 4);
+        c->m.d2h_bytes += d2h;
         return GKD_OK;
     }
 };
 
 // gkd_*_clusters: the pairs within max_dist link their nodes in the union-find forest c->uf_parent (k_cluster_link;
-// RECT: query row r is node a_base + r, reference column j is node b_base + j), or in host_forest when the pairs are
-// completed on the host.  Nothing is read back before finish().
+// RECT: query row r is node a_base + r, reference column j is node b_base + j).  Nothing is read back before finish().
 struct Clusters : Form {
     double max_dist;
     uint32_t nodes, b_base;
-    std::unique_ptr<HostForest> host_forest;
     Clusters(double d, uint32_t nodes_, uint32_t b_base_) : max_dist(d), nodes(nodes_), b_base(b_base_) {}
     int start(gkd_ctx *c) {  // every node its own root
-        if (c->cfg.ambig_policy == GKD_AMBIG_LITERAL) host_forest.reset(new HostForest(nodes));
         const int rc = ensure(c, c->uf_parent, ((uint64_t)nodes + 1) * 4);
         if (rc) return rc;
         CK(launch_cluster_init((uint32_t *)c->uf_parent.p, nodes, c->stream));
@@ -1532,24 +1398,14 @@ struct Clusters : Form {
     int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         // the forest outlives this chunk: the kernel itself skips a chunk whose join overflowed
         nvtxRangePushA("gkd kernel 5: cluster link");
-        CK(launch_cluster_link(e.sets, e.src, e.counts, e.pal, e.both, max_dist, a_base, b_base, e.join_err,
-                               (uint32_t *)c->uf_parent.p, c->stream));
+        CK(launch_cluster_link(e.src, e.pc, max_dist, a_base, b_base, e.join_err, (uint32_t *)c->uf_parent.p, c->stream));
         nvtxRangePop();
         c->m.launches++;
         CK(cudaEventRecord(c->ev[7], c->stream));
         return GKD_OK;
     }
-    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {  // the rule of k_cluster_link
-        for (uint64_t t = 0; t < e.cnt; t++) {
-            if (!(dist[t] <= max_dist)) continue;
-            uint32_t a, b;
-            e.pair(a_base, t, a, b);
-            host_forest->link(a, b_base + b);
-        }
-    }
     // The labels to the caller, once, at the end of the call: nodes [0, na) to a_out and [na, nodes) to b_out (either
-    // may be NULL).  With host_forest the launches that ran on the device are merged into it first: every node is linked
-    // to its device label, which carries all of the device links' connectivity.
+    // may be NULL).
     int finish(gkd_ctx *c, uint32_t *a_out, uint32_t na, uint32_t *b_out, uint32_t *n_clusters) {
         uint32_t *parent = (uint32_t *)c->uf_parent.p;
         CK(cudaEventRecord(c->ev[6], c->stream));
@@ -1557,27 +1413,12 @@ struct Clusters : Form {
         CK(cudaEventRecord(c->ev[7], c->stream));
         c->m.launches++;
         uint32_t roots = 0;
-        if (!host_forest) {
-            const uint32_t nb = nodes - na;
-            if (a_out && na) CK(cudaMemcpyAsync(a_out, parent, (uint64_t)na * 4, cudaMemcpyDefault, c->stream));
-            if (b_out && nb) CK(cudaMemcpyAsync(b_out, parent + na, (uint64_t)nb * 4, cudaMemcpyDefault, c->stream));
-            CK(cudaMemcpyAsync(&roots, parent + nodes, 4, cudaMemcpyDeviceToHost, c->stream));
-            CK(cudaStreamSynchronize(c->stream));
-            c->m.d2h_bytes += (a_out ? (uint64_t)na * 4 : 0) + (b_out ? (uint64_t)nb * 4 : 0) + 4;
-        } else {
-            std::vector<uint32_t> dev(nodes);
-            CK(cudaMemcpyAsync(dev.data(), parent, (uint64_t)nodes * 4, cudaMemcpyDeviceToHost, c->stream));
-            CK(cudaStreamSynchronize(c->stream));
-            c->m.d2h_bytes += (uint64_t)nodes * 4;
-            for (uint32_t x = 0; x < nodes; x++)
-                if (dev[x] != x) host_forest->link(x, dev[x]);
-            for (uint32_t x = 0; x < nodes; x++) {
-                const uint32_t r = host_forest->find(x);
-                roots += r == x ? 1u : 0u;
-                if (x < na && a_out) a_out[x] = r;
-                if (x >= na && b_out) b_out[x - na] = r;
-            }
-        }
+        const uint32_t nb = nodes - na;
+        if (a_out && na) CK(cudaMemcpyAsync(a_out, parent, (uint64_t)na * 4, cudaMemcpyDefault, c->stream));
+        if (b_out && nb) CK(cudaMemcpyAsync(b_out, parent + na, (uint64_t)nb * 4, cudaMemcpyDefault, c->stream));
+        CK(cudaMemcpyAsync(&roots, parent + nodes, 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += (a_out ? (uint64_t)na * 4 : 0) + (b_out ? (uint64_t)nb * 4 : 0) + 4;
         c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
         if (n_clusters) *n_clusters = roots;
         return GKD_OK;
@@ -1591,7 +1432,6 @@ struct Linkage : Form {
     uint32_t nodes, b_off;
     std::vector<uint32_t> key;        // key of every node (empty: the node itself); uploaded to c->lk_state when not empty
     uint32_t n_dev = 0;               // edges of the device forest c->lk_forest
-    std::vector<LinkEdge> host_edges;  // GKD_AMBIG_LITERAL: the forest of the pairs completed on the host
     unsigned long long chunk_hits = 0;
     Linkage(double d, uint32_t nodes_, uint32_t b_off_, std::vector<uint32_t> key_)
         : max_dist(d), nodes(nodes_), b_off(b_off_), key(std::move(key_)) {}
@@ -1620,7 +1460,7 @@ struct Linkage : Form {
         const HitsOut ho{(uint32_t *)c->hit_a.p, (uint32_t *)c->hit_b.p, (uint64_t *)c->d_inter.p, (double *)c->d_dist.p};
         unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
         nvtxRangePushA("gkd kernel 5: linkage edges");
-        CK(launch_select_within(e.sets, e.src, e.counts, e.pal, e.both, max_dist, a_base, e.cnt, ho, cta, cta + nctas, c->stream));
+        CK(launch_select_within(e.src, e.pc, max_dist, a_base, e.cnt, ho, cta, cta + nctas, c->stream));
         nvtxRangePop();
         c->m.launches += 3;
         CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
@@ -1666,20 +1506,10 @@ struct Linkage : Form {
         n_dev = n_forest;
         return GKD_OK;
     }
-    void host(const Chunk &e, const uint64_t *inter, const double *dist) override {
-        // Kruskal on the host forest and the chunk's edges, in the order of k_link_edges
-        for (uint64_t t = 0; t < e.cnt; t++) {
-            if (!(dist[t] <= max_dist)) continue;
-            uint32_t a, b;
-            e.pair(a_base, t, a, b);
-            host_edges.push_back(edge(a, b, inter[t], dist[t]));
-        }
-        host_msf(host_edges, nodes);
-    }
-    // The forest to the caller, once, at the end of the call: the device forest is copied to the host and merged with the
-    // host forest by one Kruskal pass, which also sorts it (a forest keeps every edge).
+    // The forest to the caller, once, at the end of the call: the device forest is copied to the host and sorted there by
+    // one Kruskal pass (a forest keeps every edge).
     int finish(gkd_ctx *c, gkd_hits *out) {
-        std::vector<LinkEdge> edges = std::move(host_edges);
+        std::vector<LinkEdge> edges;
         const uint64_t f = n_dev, N = nodes;
         if (f) {
             std::vector<uint64_t> in(f);
@@ -1901,7 +1731,7 @@ int gkd_destroy(gkd_ctx *c) {
                       &c->d_cb, &c->ids_a, &c->ids_b, &c->work_counter, &c->sk_cand, &c->sk_misc, &c->sk_sig,
                       &c->sk_len, &c->sk_out, &c->msd_genomes, &c->msd_bins32, &c->msd_bins64, &c->msd_gstat,
                       &c->gr_reps, &c->gr_flags, &c->join_rows, &c->join_err, &c->hit_a, &c->hit_b, &c->sel_cta, &c->nn_pos, &c->nn_inter,
-                      &c->nn_dist, &c->nn_found, &c->uf_parent, &c->lk_forest, &c->lk_state};
+                      &c->nn_dist, &c->nn_found, &c->uf_parent, &c->lk_forest, &c->lk_state, &c->lit_size, &c->lit_inter};
     for (DevBuf *b : bufs)
         if (b->p) cudaFreeAsync(b->p, c->stream);
     cudaStreamSynchronize(c->stream);
@@ -2267,9 +2097,9 @@ int gkd_load_sets(gkd_ctx *c, const char *path, uint32_t *first_id, uint32_t *n_
 }
 
 // ---- distances --------------------------------------------------------------------------------------------
-// Literal side lists are completed (and selected) on the host, so the outputs must be host memory in that mode.  The
-// selections check this before the context is touched, so a bad k or a NaN threshold is GKD_EINVAL even without a
-// usable device.
+// gkd.h publishes host memory as the only output memory of a GKD_AMBIG_LITERAL context, so device buffers are refused
+// in that mode.  The selections check this before the context is touched, so a bad k or a NaN threshold is GKD_EINVAL
+// even without a usable device.
 static int host_outputs_ok(gkd_ctx *c, std::initializer_list<const void *> ps) {
     if (c->cfg.ambig_policy != GKD_AMBIG_LITERAL) return GKD_OK;
     for (const void *p : ps)
@@ -2361,7 +2191,8 @@ int gkd_greedy_reps(gkd_ctx *c, const uint32_t *order, uint32_t n, double max_di
     for (uint32_t i = 0; i < n; i++)
         if ((rc = s.see(c, order[i]))) return rc;
     if (s.any_lit) {
-        // literal ambiguous k-mers are completed on the host: one batched call per candidate
+        // the shared literal k-mers of a pair are counted on the host per chunk, which the device-resident list below
+        // cannot wait for: one batched call per candidate
         std::vector<uint32_t> reps, cand;
         std::vector<double> dist;
         for (uint32_t i = 0; i < n; i++) {

@@ -279,14 +279,28 @@ uint32_t join_cfg_slots(int cfg);  // slots of the shared-memory table
 uint32_t join_cfg_rows(int cfg);   // rows per block (32 or 64)
 cudaError_t launch_join(const SetDesc *sets, const JoinPlan &plan, uint32_t *counts, unsigned long long *work_counter,
                         uint32_t *err, int n_sms, cudaStream_t s);
+// What kernel 5 values the pairs of a chunk from: kernel 4's counts, indexed by chunk position t like the pair source,
+// and the sets.  GKD_AMBIG_LITERAL sets also hold literal k-mers (collected and intersected on the host), which add to
+// I and to both sizes.
+struct PairCounts {
+    const SetDesc *sets;
+    const uint32_t *counts;      // |C_A n C_B|
+    const uint32_t *pal_counts;  // its palindromic part, or nullptr (not needed)
+    const uint32_t *lit_size;    // per set id: literal k-mers of the set, or nullptr (no set of the call has any)
+    const uint32_t *lit_inter;   // per chunk position: literal k-mers both sets share, or nullptr (none in the chunk)
+    int both;                    // GKD_STRAND_BOTH on nucleotides
+#ifdef __CUDACC__
+    // I, |A|, |B| and SequenceKmers.distance of pair t, sets ida and idb (intersect.cu)
+    __device__ void value(uint64_t t, uint32_t ida, uint32_t idb, uint64_t &I, uint64_t &sa, uint64_t &sb, double &dist) const;
+#endif
+};
 struct EpilogueOut {
     uint64_t *inter;     // similarity() of the reference: |A n B| (both strands under GKD_STRAND_BOTH)
     double *dist;        // SequenceKmers.distance
     double *contain_a;   // I / |A|  (0 when |A| == 0)
     double *contain_b;   // I / |B|
 };
-cudaError_t launch_epilogue(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                            int both_strands, EpilogueOut out, cudaStream_t s);
+cudaError_t launch_epilogue(PairSource src, const PairCounts &pc, EpilogueOut out, cudaStream_t s);
 // kernel 5, selection forms (replace launch_epilogue for the within / nearest calls)
 struct HitsOut {         // any member may be nullptr
     uint32_t *a, *b;     // UPPER / LIST: set ids; RECT: a_base + query row, reference position
@@ -302,32 +316,28 @@ struct NearestOut {      // rows * k row-major, n_found per row; any member may 
 };
 uint64_t select_within_ctas(uint64_t count);  // entries of the `cta` scratch array of launch_select_within
 // pairs with dist <= max_dist compacted in enumeration order into out[0 .. min(hits, cap)); *total = hits of the launch
-cudaError_t launch_select_within(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                                 int both_strands, double max_dist, uint32_t a_base, uint64_t cap, HitsOut out,
-                                 unsigned long long *cta, unsigned long long *total, cudaStream_t s);
+cudaError_t launch_select_within(PairSource src, const PairCounts &pc, double max_dist, uint32_t a_base, uint64_t cap,
+                                 HitsOut out, unsigned long long *cta, unsigned long long *total, cudaStream_t s);
 // PAIRS_RECT only: per query row the <= k (<= NEAREST_MAX_K) nearest references within max_dist, ties by position
-cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t rows, const uint32_t *counts,
-                                  const uint32_t *pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
-                                  NearestOut out, cudaStream_t s);
+cudaError_t launch_select_nearest(PairSource src, uint32_t rows, const PairCounts &pc, double max_dist, uint32_t k,
+                                  int exclude_self, NearestOut out, cudaStream_t s);
 // PAIRS_UPPER or PAIRS_RECT: merge the launch into per-target lists that persist across launches (`state`, every member
 // set; targets * k slots, filled with the unused entry before the first launch).  UPPER: every pair (i, j) is offered
 // to target i (neighbour j) and target j (neighbour i); RECT: to reference column j, neighbour a_base + query row.
 // Writes nothing when join_err (may be nullptr) reads nonzero on the stream.
-cudaError_t launch_nearest_absorb(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                                  int both_strands, double max_dist, uint32_t k, int exclude_self, uint32_t a_base,
-                                  const uint32_t *join_err, NearestOut state, cudaStream_t s);
+cudaError_t launch_nearest_absorb(PairSource src, const PairCounts &pc, double max_dist, uint32_t k, int exclude_self,
+                                  uint32_t a_base, const uint32_t *join_err, NearestOut state, cudaStream_t s);
 // Single-linkage clusters: a union-find forest parent[0, n) in device memory (invariant parent[x] <= x) followed by
 // one root counter parent[n].  init: parent[x] = x and the counter 0.  link: every pair within max_dist joins its two
 // nodes (UPPER: the set ids; RECT: a_base + query row and b_base + reference column); nothing when join_err (may be
 // nullptr) reads nonzero on the stream.  flatten: parent[x] = the smallest node of x's cluster (a read-only walk;
 // only thread x writes parent[x]), counter = clusters.
 cudaError_t launch_cluster_init(uint32_t *parent, uint32_t n, cudaStream_t s);
-cudaError_t launch_cluster_link(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                                int both_strands, double max_dist, uint32_t a_base, uint32_t b_base, const uint32_t *join_err,
-                                uint32_t *parent, cudaStream_t s);
+cudaError_t launch_cluster_link(PairSource src, const PairCounts &pc, double max_dist, uint32_t a_base, uint32_t b_base,
+                                const uint32_t *join_err, uint32_t *parent, cudaStream_t s);
 cudaError_t launch_cluster_flatten(uint32_t *parent, uint32_t n, cudaStream_t s);
-// The same forest on the host (GKD_AMBIG_LITERAL pairs, and the group's merge of its members' components): a link
-// hooks the larger root under the smaller, so find() is the smallest node of the cluster.
+// The same forest on the host (the group's merge of its members' components): a link hooks the larger root under the
+// smaller, so find() is the smallest node of the cluster.
 struct HostForest {
     std::vector<uint32_t> parent;
     explicit HostForest(uint32_t n) : parent(n) {
@@ -377,8 +387,8 @@ LinkState link_state_at(void *base, uint32_t nodes);
 // rounds = ceil(log2(nodes)) Boruvka rounds, queued without a host read; a round after one that hooked nothing exits
 // at once.  On return *st.n_forest (device) is the number of edges of the new forest f.
 cudaError_t launch_link_rounds(const LinkGraph &g, const LinkState &st, const LinkForest &f, uint32_t rounds, cudaStream_t s);
-// The same forest on the host: Kruskal in the strict order.  Used for GKD_AMBIG_LITERAL pairs, to sort the device forest
-// at the end of a call (a forest keeps every edge), and for the group's merge of its members' forests.
+// The same forest on the host: Kruskal in the strict order.  Used to sort the device forest at the end of a call (a
+// forest keeps every edge), and for the group's merge of its members' forests.
 struct LinkEdge {
     uint64_t dbits, keys;  // distance bits, (min key << 32) | max key
     uint32_t na, nb;       // nodes

@@ -479,11 +479,13 @@ cudaError_t launch_intersect(const SetDesc *sets, PairSource src, int use_pal, c
 }
 
 // ---- kernel 5: distance epilogue ----------------------------------------------------------------------
-// SequenceKmers.similarity / distance of one pair from the canonical counts (c = |C_A n C_B|, cp = palindromic part)
+// SequenceKmers.similarity / distance of one pair from the canonical counts (c = |C_A n C_B|, cp = palindromic part) and
+// the literal k-mers (li shared, la and lb of each set; 0 outside GKD_AMBIG_LITERAL)
 __device__ __forceinline__ void pair_result(const SetDesc *__restrict__ sets, uint32_t ida, uint32_t idb, uint64_t c, uint64_t cp,
-                                            int both_strands, uint64_t &I, uint64_t &sa, uint64_t &sb, double &dist) {
-    const uint32_t nA = sets[ida].main.n, nB = sets[idb].main.n;
-    const uint32_t pA = sets[ida].pal.n, pB = sets[idb].pal.n;
+                                            uint32_t li, uint32_t la, uint32_t lb, int both_strands, uint64_t &I, uint64_t &sa,
+                                            uint64_t &sb, double &dist) {
+    const uint32_t nA = __ldg(&sets[ida].main.n), nB = __ldg(&sets[idb].main.n);
+    const uint32_t pA = __ldg(&sets[ida].pal.n), pB = __ldg(&sets[idb].pal.n);
     if (both_strands) {
         // the reference's sets hold both strands: |S| = 2|C| - P, I = 2|C_A n C_B| - P(C_A n C_B)
         I = 2 * c - cp;
@@ -494,6 +496,9 @@ __device__ __forceinline__ void pair_result(const SetDesc *__restrict__ sets, ui
         sa = nA;
         sb = nB;
     }
+    I += li;
+    sa += la;
+    sb += lb;
     dist = 1.0;
     const double similarity = (double)I;
     if (similarity > 0) {
@@ -504,16 +509,21 @@ __device__ __forceinline__ void pair_result(const SetDesc *__restrict__ sets, ui
     }
 }
 
-__global__ void __launch_bounds__(256)
-    k_epilogue(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
-               const uint32_t *__restrict__ pal_counts, int both_strands, EpilogueOut out) {
+// everything it reads is constant while kernel 5 runs: read-only cache loads
+__device__ __forceinline__ void PairCounts::value(uint64_t t, uint32_t ida, uint32_t idb, uint64_t &I, uint64_t &sa,
+                                                  uint64_t &sb, double &dist) const {
+    pair_result(sets, ida, idb, __ldg(counts + t), pal_counts ? __ldg(pal_counts + t) : 0, lit_inter ? __ldg(lit_inter + t) : 0,
+                lit_size ? __ldg(lit_size + ida) : 0, lit_size ? __ldg(lit_size + idb) : 0, both, I, sa, sb, dist);
+}
+
+__global__ void __launch_bounds__(256) k_epilogue(PairSource src, PairCounts pc, EpilogueOut out) {
     uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= src.count) return;
     uint32_t ida, idb;
     decode_pair(src, t, ida, idb);
     uint64_t I, sa, sb;
     double d;
-    pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+    pc.value(t, ida, idb, I, sa, sb, d);
     if (out.inter) out.inter[t] = I;
     if (out.dist) out.dist[t] = d;
     if (out.contain_a) out.contain_a[t] = sa ? (double)I / (double)sa : 0.0;
@@ -521,7 +531,7 @@ __global__ void __launch_bounds__(256)
 }
 
 // ---- kernel 5, selection forms: only the chosen pairs leave the device ------------------------------------------
-// Both compute every pair with decode_pair + pair_result, so a selected pair's inter and dist are the dense call's.
+// Both compute every pair with decode_pair + PairCounts::value, so a selected pair's inter and dist are the dense call's.
 //
 // Within: pairs with dist <= max_dist, compacted in enumeration order.  A CTA owns a tile of SEL_TILE consecutive
 // pairs; pass 1 counts its hits, one CTA scans the tile totals (exclusive offsets + the launch total), and pass 2
@@ -534,9 +544,8 @@ uint64_t select_within_ctas(uint64_t count) { return (count + SEL_TILE - 1) / SE
 
 template <bool WRITE>
 __global__ void __launch_bounds__(SEL_THREADS)
-    k_select_within(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
-                    const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t a_base, uint64_t cap,
-                    HitsOut out, unsigned long long *__restrict__ cta) {
+    k_select_within(PairSource src, PairCounts pc, double max_dist, uint32_t a_base, uint64_t cap, HitsOut out,
+                    unsigned long long *__restrict__ cta) {
     __shared__ uint32_t s_warp[SEL_THREADS / 32];
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint64_t tile0 = (uint64_t)blockIdx.x * SEL_TILE;
@@ -551,7 +560,7 @@ __global__ void __launch_bounds__(SEL_THREADS)
         if (t < src.count) {
             decode_pair(src, t, ida, idb);
             uint64_t sa, sb;
-            pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+            pc.value(t, ida, idb, I, sa, sb, d);
             hit = d <= max_dist;
         }
         if (!WRITE) {
@@ -628,17 +637,13 @@ __global__ void __launch_bounds__(1024) k_select_scan(unsigned long long *__rest
     if (threadIdx.x == 1023) *total = run;
 }
 
-cudaError_t launch_select_within(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                                 int both_strands, double max_dist, uint32_t a_base, uint64_t cap, HitsOut out,
-                                 unsigned long long *cta, unsigned long long *total, cudaStream_t s) {
+cudaError_t launch_select_within(PairSource src, const PairCounts &pc, double max_dist, uint32_t a_base, uint64_t cap,
+                                 HitsOut out, unsigned long long *cta, unsigned long long *total, cudaStream_t s) {
     if (src.count == 0) return cudaMemsetAsync(total, 0, sizeof(unsigned long long), s);
     const uint64_t blocks = select_within_ctas(src.count);
-    k_select_within<false><<<(unsigned)blocks, SEL_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, a_base,
-                                                                   cap, out, cta);
+    k_select_within<false><<<(unsigned)blocks, SEL_THREADS, 0, s>>>(src, pc, max_dist, a_base, cap, out, cta);
     k_select_scan<<<1, 1024, 0, s>>>(cta, blocks, total);
-    if (cap)
-        k_select_within<true><<<(unsigned)blocks, SEL_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist,
-                                                                      a_base, cap, out, cta);
+    if (cap) k_select_within<true><<<(unsigned)blocks, SEL_THREADS, 0, s>>>(src, pc, max_dist, a_base, cap, out, cta);
     return cudaGetLastError();
 }
 
@@ -692,9 +697,7 @@ __device__ __forceinline__ void near_write(const unsigned long long *s_key, cons
 }
 
 __global__ void __launch_bounds__(NEAR_THREADS)
-    k_select_nearest(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
-                     const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
-                     NearestOut out) {
+    k_select_nearest(PairSource src, PairCounts pc, double max_dist, uint32_t k, int exclude_self, NearestOut out) {
     __shared__ unsigned long long s_key[NEAR_SLOTS];
     __shared__ unsigned long long s_inter[NEAR_SLOTS];
     __shared__ uint32_t s_pos[NEAR_SLOTS];
@@ -717,7 +720,7 @@ __global__ void __launch_bounds__(NEAR_THREADS)
             if (!(exclude_self && ida == idb)) {
                 uint64_t I, sa, sb;
                 double d;
-                pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+                pc.value(t, ida, idb, I, sa, sb, d);
                 const unsigned long long key = (unsigned long long)__double_as_longlong(d);
                 // a later reference with the k-th best distance loses the tie: strictly smaller only
                 if (d <= max_dist && key < thr) {
@@ -740,11 +743,10 @@ __global__ void __launch_bounds__(NEAR_THREADS)
     near_write(s_key, s_inter, s_pos, k, tid, row, out);
 }
 
-cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t rows, const uint32_t *counts,
-                                  const uint32_t *pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
-                                  NearestOut out, cudaStream_t s) {
+cudaError_t launch_select_nearest(PairSource src, uint32_t rows, const PairCounts &pc, double max_dist, uint32_t k,
+                                  int exclude_self, NearestOut out, cudaStream_t s) {
     if (rows == 0) return cudaSuccess;
-    k_select_nearest<<<rows, NEAR_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, k, exclude_self, out);
+    k_select_nearest<<<rows, NEAR_THREADS, 0, s>>>(src, pc, max_dist, k, exclude_self, out);
     return cudaGetLastError();
 }
 
@@ -761,9 +763,8 @@ cudaError_t launch_select_nearest(const SetDesc *sets, PairSource src, uint32_t 
 __device__ __forceinline__ uint64_t upper_row_start(uint64_t i, uint64_t n) { return i * (2 * n - i - 1) / 2; }
 
 __global__ void __launch_bounds__(NEAR_THREADS)
-    k_nearest_absorb(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
-                     const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t k, int exclude_self,
-                     uint32_t i0, uint32_t i1, uint32_t a_base, const uint32_t *__restrict__ join_err, NearestOut state) {
+    k_nearest_absorb(PairSource src, PairCounts pc, double max_dist, uint32_t k, int exclude_self, uint32_t i0, uint32_t i1,
+                     uint32_t a_base, const uint32_t *__restrict__ join_err, NearestOut state) {
     if (join_err && *join_err) return;
     __shared__ unsigned long long s_key[NEAR_SLOTS];
     __shared__ unsigned long long s_inter[NEAR_SLOTS];
@@ -828,7 +829,7 @@ __global__ void __launch_bounds__(NEAR_THREADS)
         if (have) {
             uint64_t I, sa, sb;
             double d;
-            pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+            pc.value(t, ida, idb, I, sa, sb, d);
             const unsigned long long key = (unsigned long long)__double_as_longlong(d);
             if (d <= max_dist && (key < thr || (key == thr && nb < thr_pos))) {
                 const uint32_t slot = NEAR_THREADS + atomicAdd(&s_n, 1u);
@@ -851,9 +852,8 @@ __global__ void __launch_bounds__(NEAR_THREADS)
     if (changed) near_write(s_key, s_inter, s_pos, k, tid, tg, state);
 }
 
-cudaError_t launch_nearest_absorb(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                                  int both_strands, double max_dist, uint32_t k, int exclude_self, uint32_t a_base,
-                                  const uint32_t *join_err, NearestOut state, cudaStream_t s) {
+cudaError_t launch_nearest_absorb(PairSource src, const PairCounts &pc, double max_dist, uint32_t k, int exclude_self,
+                                  uint32_t a_base, const uint32_t *join_err, NearestOut state, cudaStream_t s) {
     if (src.count == 0) return cudaSuccess;
     uint32_t i0 = 0, i1 = 0, j = 0, targets = src.n;
     if (src.mode == PAIRS_UPPER) {
@@ -861,8 +861,7 @@ cudaError_t launch_nearest_absorb(const SetDesc *sets, PairSource src, const uin
         upper_pair(src.first + src.count - 1, src.n, i1, j);
         targets = src.n - i0;
     }
-    k_nearest_absorb<<<targets, NEAR_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, k, exclude_self,
-                                                      i0, i1, a_base, join_err, state);
+    k_nearest_absorb<<<targets, NEAR_THREADS, 0, s>>>(src, pc, max_dist, k, exclude_self, i0, i1, a_base, join_err, state);
     return cudaGetLastError();
 }
 
@@ -911,8 +910,7 @@ __device__ __forceinline__ void uf_union(uint32_t *__restrict__ parent, uint32_t
 }
 
 __global__ void __launch_bounds__(CLUSTER_THREADS)
-    k_cluster_link(const SetDesc *__restrict__ sets, PairSource src, const uint32_t *__restrict__ counts,
-                   const uint32_t *__restrict__ pal_counts, int both_strands, double max_dist, uint32_t a_base, uint32_t b_base,
+    k_cluster_link(PairSource src, PairCounts pc, double max_dist, uint32_t a_base, uint32_t b_base,
                    const uint32_t *__restrict__ join_err, uint32_t *__restrict__ parent) {
     if (join_err && *join_err) return;
     const bool rect = src.mode == PAIRS_RECT;
@@ -921,7 +919,7 @@ __global__ void __launch_bounds__(CLUSTER_THREADS)
         decode_pair(src, t, ida, idb);
         uint64_t I, sa, sb;
         double d;
-        pair_result(sets, ida, idb, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+        pc.value(t, ida, idb, I, sa, sb, d);
         if (!(d <= max_dist)) continue;
         if (rect) uf_union(parent, a_base + (uint32_t)(t / src.n), b_base + (uint32_t)(t % src.n));
         else uf_union(parent, ida, idb);
@@ -960,14 +958,12 @@ cudaError_t launch_cluster_init(uint32_t *parent, uint32_t n, cudaStream_t s) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_cluster_link(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                                int both_strands, double max_dist, uint32_t a_base, uint32_t b_base, const uint32_t *join_err,
-                                uint32_t *parent, cudaStream_t s) {
+cudaError_t launch_cluster_link(PairSource src, const PairCounts &pc, double max_dist, uint32_t a_base, uint32_t b_base,
+                                const uint32_t *join_err, uint32_t *parent, cudaStream_t s) {
     if (src.count == 0) return cudaSuccess;
     const uint64_t need = (src.count + CLUSTER_THREADS - 1) / CLUSTER_THREADS;  // grid-stride beyond 8192 CTAs
     const uint64_t blocks = need < 8192 ? need : 8192;
-    k_cluster_link<<<(unsigned)blocks, CLUSTER_THREADS, 0, s>>>(sets, src, counts, pal_counts, both_strands, max_dist, a_base,
-                                                                 b_base, join_err, parent);
+    k_cluster_link<<<(unsigned)blocks, CLUSTER_THREADS, 0, s>>>(src, pc, max_dist, a_base, b_base, join_err, parent);
     return cudaGetLastError();
 }
 
@@ -1123,7 +1119,8 @@ cudaError_t launch_link_rounds(const LinkGraph &g, const LinkState &st, const Li
 // Greedy representative pass (DistanceRepsProcessor.java:185-201, FastaDistanceRepsProcessor.java:124-146): the
 // candidate was intersected with every current representative (counts[t] for reps[t]); it joins the list unless
 // one of them is within max_dist.  The list and its length live on the device, so the host queues the launches
-// of every candidate back to back without reading anything.
+// of every candidate back to back without reading anything.  The sets have no literal k-mers: gkd_greedy_reps runs the
+// dense calls for those.
 __global__ void __launch_bounds__(256)
     k_greedy_decide(const SetDesc *__restrict__ sets, uint32_t *__restrict__ reps, uint32_t *__restrict__ n_reps, uint32_t cand,
                     uint32_t visit, uint32_t *__restrict__ counts, uint32_t *__restrict__ pal_counts, int both_strands,
@@ -1136,7 +1133,7 @@ __global__ void __launch_bounds__(256)
     for (uint32_t t = threadIdx.x; t < n; t += blockDim.x) {
         uint64_t I, sa, sb;
         double d;
-        pair_result(sets, reps[t], cand, counts[t], pal_counts ? pal_counts[t] : 0, both_strands, I, sa, sb, d);
+        pair_result(sets, reps[t], cand, counts[t], pal_counts ? pal_counts[t] : 0, 0, 0, 0, both_strands, I, sa, sb, d);
         found |= d <= max_dist ? 1 : 0;
         counts[t] = 0;  // ready for the next candidate
         if (pal_counts) pal_counts[t] = 0;
@@ -1159,11 +1156,10 @@ cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *
     return cudaGetLastError();
 }
 
-cudaError_t launch_epilogue(const SetDesc *sets, PairSource src, const uint32_t *counts, const uint32_t *pal_counts,
-                            int both_strands, EpilogueOut out, cudaStream_t s) {
+cudaError_t launch_epilogue(PairSource src, const PairCounts &pc, EpilogueOut out, cudaStream_t s) {
     if (src.count == 0) return cudaSuccess;
     uint64_t blocks = (src.count + 255) / 256;
-    k_epilogue<<<(unsigned)blocks, 256, 0, s>>>(sets, src, counts, pal_counts, both_strands, out);
+    k_epilogue<<<(unsigned)blocks, 256, 0, s>>>(src, pc, out);
     return cudaGetLastError();
 }
 

@@ -225,7 +225,7 @@ int gkd_pair(gkd_ctx *ctx, uint32_t a, uint32_t b, uint64_t *inter, uint64_t *un
 /* ---- selections: only the chosen pairs leave the device (kernel 5 replaced by a selection epilogue) ----------
  * Pairs whose distance is <= max_dist (the comparison gkd_greedy_reps uses), in the enumeration order of the call.
  * Any array may be NULL; pointers may be host or device memory, like gkd_outputs (host memory only for a
- * GKD_AMBIG_LITERAL context, whose pairs are completed and selected on the host). */
+ * GKD_AMBIG_LITERAL context, whose shared literal k-mers are counted on the host). */
 typedef struct gkd_hits {
     uint32_t *a;      /* all-vs-all: id i (i < j);  query_vs_ref: position of the query in q */
     uint32_t *b;      /* all-vs-all: id j;          query_vs_ref: position of the reference in r */

@@ -304,8 +304,8 @@ def test_redo_only_in_the_second_chunk(monkeypatch):
 
 
 def test_literal_ambiguous_context():
-    """GKD_AMBIG_LITERAL with runs of N: pairs with a literal side are completed and linked on the host; a rectangle of
-    sets without literals runs on the device and is merged into the host forest at the end"""
+    """GKD_AMBIG_LITERAL with runs of N: kernel 5 adds the shared literal k-mers, counted on the host, and links on the
+    device; a rectangle of sets without literals runs as in a skip context"""
     rng = np.random.default_rng(9)
     seqs = []
     for i, s in enumerate(_seqs(40, [60_000] * 12)):

@@ -288,8 +288,8 @@ def test_redo_only_in_the_second_chunk(monkeypatch):
 
 
 def test_literal_ambiguous_context():
-    """GKD_AMBIG_LITERAL with runs of N: pairs with a literal side feed a host forest by Kruskal; a rectangle of sets
-    without literals runs on the device and is merged into the host forest at the end"""
+    """GKD_AMBIG_LITERAL with runs of N: kernel 5 adds the shared literal k-mers, counted on the host, and the forest is
+    built on the device; a rectangle of sets without literals runs as in a skip context"""
     rng = np.random.default_rng(9)
     seqs = []
     for i, s in enumerate(tc._seqs(40, [60_000] * 12)):

@@ -199,7 +199,8 @@ def test_ex_reference_side_accumulates_over_launches():
 
 
 def test_literal_ambiguous_context():
-    """GKD_AMBIG_LITERAL with runs of N: the pairs are completed on the host and the lists are kept there"""
+    """GKD_AMBIG_LITERAL with runs of N: kernel 5 adds the shared literal k-mers, counted on the host, and the lists
+    are kept on the device"""
     rng = np.random.default_rng(9)
     seqs = []
     for s in _seqs(40, [60_000] * 12):

@@ -217,8 +217,9 @@ def test_nearest_over_several_launches():
                 _check_nearest([g[x0:x0 + 40] for g in got], want)
 
 
-def test_literal_ambiguous_context_selects_after_host_completion():
-    """GKD_AMBIG_LITERAL with runs of N: the pairs are completed on the host and selected there"""
+def test_literal_ambiguous_context():
+    """GKD_AMBIG_LITERAL with runs of N: kernel 5 adds the shared literal k-mers, counted on the host, and selects on
+    the device"""
     rng = np.random.default_rng(9)
     seqs = []
     for s in _seqs(40, [60_000] * 12):
