@@ -5,6 +5,7 @@
 #include <nvtx3/nvToolsExt.h>
 
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -1008,16 +1009,23 @@ struct Chunk {
     const uint32_t *join_err;  // the block join's overflow flag on the device; nullptr when the merge kernel ran
 };
 
-// What a call computes from the counts of kernel 4: one form of kernel 5.  run_pairs owns the chunk loop and the redo of
-// a chunk whose join table overflowed; the form owns its state, its launches and its copies.  The bytes queue() and
-// keep() read back are counted only for a chunk that is kept.
+// What a call computes from the counts of kernel 4: one form of kernel 5.  run_call owns the call (checks, start, chunk
+// loop, finish), run_pairs the chunk loop and the redo of a chunk whose join table overflowed; the form owns its outputs,
+// its state, its launches and its copies, and its answer to a call without pairs.  The bytes queue() and keep() read
+// back are counted only for a chunk that is kept.
 struct Form {
     uint32_t a_base = 0;  // RECT: position in the caller's q of this launch's first query row (run_rect)
     virtual ~Form() = default;
+    // the caller's output buffers (unused entries nullptr)
+    virtual std::array<const void *, 8> outputs() const = 0;
+    // before the first chunk, also when the call has no pairs
+    virtual int start(gkd_ctx *c) { return GKD_OK; }
     // the chunk's kernel-5 launches, then the reads the host needs once the stream is synchronised; records ev[7]
     virtual int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) = 0;
     // the join held: the chunk is kept
     virtual int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) { return GKD_OK; }
+    // after the last chunk, also when the call has no pairs
+    virtual int finish(gkd_ctx *c) { return GKD_OK; }
 };
 
 // a read of `bytes` from the device into dst (host or device memory), skipped when dst is nullptr; counted in d2h
@@ -1033,6 +1041,7 @@ int read_back(gkd_ctx *c, void *dst, const void *src, uint64_t bytes, uint64_t &
 struct Dense : Form {
     gkd_outputs out;
     explicit Dense(const gkd_outputs &o) : out(o) {}
+    std::array<const void *, 8> outputs() const override { return {out.inter, out.dist, out.contain_a, out.contain_b}; }
     int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         // the chunk's part of out (RECT: from row a_base of the caller's block)
         const uint64_t t = (uint64_t)a_base * e.hp.nb + e.done;
@@ -1229,17 +1238,19 @@ int run_pairs(gkd_ctx *c, const HostPairs &hp, Form &f) {
     return GKD_OK;
 }
 
-// A query x reference call, split by query rows so that each launch stays under PAIR_CHUNK pairs and every row is
-// complete in one launch; f.a_base is the launch's first row.  The call's metrics add up its launches.
-int run_rect(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, Form &f) {
+// A query x reference block with at least one pair (hp: q = a, nq = na, r = b, nr = nb), split by query rows so that
+// each launch stays under PAIR_CHUNK pairs and every row is complete in one launch; f.a_base is the launch's first row.
+// The call's metrics add up its launches.
+int run_rect(gkd_ctx *c, const HostPairs &hp, Form &f) {
+    const uint32_t nq = hp.na, nr = hp.nb;
     const uint32_t rows_per = (uint32_t)std::max<uint64_t>(1, PAIR_CHUNK / nr);
     uint64_t pairs = 0, bytes = 0;
     double ims = 0, ems = 0;
     for (uint32_t q0 = 0; q0 < nq; q0 += rows_per) {
         const uint32_t rows = std::min(rows_per, nq - q0);
-        HostPairs hp{PAIRS_RECT, nr, 0, (uint64_t)rows * nr, q + q0, r, rows, nr};
+        const HostPairs part{PAIRS_RECT, nr, 0, (uint64_t)rows * nr, hp.a + q0, hp.b, rows, nr};
         f.a_base = q0;
-        const int rc = run_pairs(c, hp, f);
+        const int rc = run_pairs(c, part, f);
         if (rc) return rc;
         pairs += c->m.pairs;
         bytes += c->m.intersect_bytes;
@@ -1262,6 +1273,11 @@ struct Within : Form {
     uint64_t wcap = 0;  // hits of the chunk the device buffers hold
     unsigned long long chunk_hits = 0;
     Within(double d, gkd_hits &hits) : max_dist(d), h(hits) {}
+    std::array<const void *, 8> outputs() const override { return {h.a, h.b, h.inter, h.dist}; }
+    int start(gkd_ctx *c) override {
+        h.n = 0;
+        return GKD_OK;
+    }
     int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         const bool any_out = h.a || h.b || h.inter || h.dist;
         wcap = (any_out && h.n < h.cap) ? std::min<uint64_t>(e.cnt, h.cap - h.n) : 0;
@@ -1298,35 +1314,63 @@ struct Within : Form {
     }
 };
 
-// gkd_*_nearest: the k nearest within max_dist by (distance bits, position).  rows (RECT only): each query row's list,
-// complete in every launch (k_select_nearest) and read back once the chunk is kept.  lists: per-target lists on the
-// device (c->nn_*) that the launches merge into (k_nearest_absorb; UPPER: both ends of every pair, RECT: each
-// reference's nearest queries), read once by finish().
+// gkd_*_nearest: the k nearest within max_dist by (distance bits, position).  rows (RECT only): each of the n_rows query
+// rows' list, complete in every launch (k_select_nearest) and read back once the chunk is kept.  lists: per-target lists
+// on the device (c->nn_*) that the launches merge into (k_nearest_absorb; UPPER: both ends of every pair, RECT: each
+// reference's nearest queries), read once by finish().  A list nothing was offered to is unused: every slot pos
+// 0xFFFFFFFF, inter 0, dist -1.0, and n_found 0.
 struct Nearest : Form {
     uint32_t k;
     double max_dist;
     int exclude_self;
     const gkd_neighbors *rows, *lists;  // either may be nullptr
-    uint32_t targets;
-    Nearest(uint32_t k_, double d, int excl, const gkd_neighbors *rows_, const gkd_neighbors *lists_, uint32_t targets_)
-        : k(k_), max_dist(d), exclude_self(excl), rows(rows_), lists(lists_), targets(targets_) {}
-    int start(gkd_ctx *c) {  // every per-target list unused
-        if (!lists) return GKD_OK;
-        const uint64_t slots = (uint64_t)targets * k;
+    uint32_t n_rows, targets;
+    bool rows_kept = false;
+    Nearest(uint32_t k_, double d, int excl, const gkd_neighbors *rows_, uint32_t n_rows_, const gkd_neighbors *lists_,
+            uint32_t targets_)
+        : k(k_), max_dist(d), exclude_self(excl), rows(rows_), lists(lists_), n_rows(n_rows_), targets(targets_) {}
+    std::array<const void *, 8> outputs() const override {
+        const gkd_neighbors none{};
+        const gkd_neighbors &a = rows ? *rows : none, &b = lists ? *lists : none;
+        return {a.pos, a.inter, a.dist, a.n_found, b.pos, b.inter, b.dist, b.n_found};
+    }
+    // the device buffers of one side's lists
+    struct Bufs {
+        DevBuf &pos, &inter, &dist, &found;
+    };
+    static Bufs row_bufs(gkd_ctx *c) { return {c->hit_a, c->d_inter, c->d_dist, c->hit_b}; }
+    static Bufs list_bufs(gkd_ctx *c) { return {c->nn_pos, c->nn_inter, c->nn_dist, c->nn_found}; }
+    // n unused lists in d
+    int fill_unused(gkd_ctx *c, const Bufs &d, uint64_t n) {
+        if (n == 0) return GKD_OK;
+        const uint64_t slots = n * k;
         int rc;
-        if ((rc = ensure(c, c->nn_pos, slots * 4)) || (rc = ensure(c, c->nn_inter, slots * 8)) ||
-            (rc = ensure(c, c->nn_dist, slots * 8)) || (rc = ensure(c, c->nn_found, (uint64_t)targets * 4)))
+        if ((rc = ensure(c, d.pos, slots * 4)) || (rc = ensure(c, d.inter, slots * 8)) || (rc = ensure(c, d.dist, slots * 8)) ||
+            (rc = ensure(c, d.found, n * 4)))
             return rc;
         const double none = -1.0;
         uint64_t none_bits;
         std::memcpy(&none_bits, &none, 8);
-        CK(cudaMemsetAsync(c->nn_pos.p, 0xFF, slots * 4, c->stream));
-        CK(cudaMemsetAsync(c->nn_inter.p, 0, slots * 8, c->stream));
-        CK(cudaMemsetAsync(c->nn_found.p, 0, (uint64_t)targets * 4, c->stream));
-        CK(launch_fill_u64((uint64_t *)c->nn_dist.p, slots, none_bits, c->stream));
+        CK(cudaMemsetAsync(d.pos.p, 0xFF, slots * 4, c->stream));
+        CK(cudaMemsetAsync(d.inter.p, 0, slots * 8, c->stream));
+        CK(cudaMemsetAsync(d.found.p, 0, n * 4, c->stream));
+        CK(launch_fill_u64((uint64_t *)d.dist.p, slots, none_bits, c->stream));
         c->m.launches++;
         return GKD_OK;
     }
+    // lists [0, n) of d to lists [at, at + n) of out, then the stream is synchronised
+    int read_lists(gkd_ctx *c, const Bufs &d, uint64_t n, const gkd_neighbors &out, uint64_t at, uint64_t &d2h) {
+        const uint64_t slots = n * k, o = at * k;
+        int rc;
+        if ((rc = read_back(c, out.pos ? out.pos + o : nullptr, d.pos.p, slots * 4, d2h)) ||
+            (rc = read_back(c, out.inter ? out.inter + o : nullptr, d.inter.p, slots * 8, d2h)) ||
+            (rc = read_back(c, out.dist ? out.dist + o : nullptr, d.dist.p, slots * 8, d2h)) ||
+            (rc = read_back(c, out.n_found ? out.n_found + at : nullptr, d.found.p, n * 4, d2h)))
+            return rc;
+        CK(cudaStreamSynchronize(c->stream));
+        return GKD_OK;
+    }
+    int start(gkd_ctx *c) override { return lists ? fill_unused(c, list_bufs(c), targets) : GKD_OK; }
     int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         int rc;
         if (rows) {
@@ -1355,40 +1399,34 @@ struct Nearest : Form {
     }
     int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         if (!rows) return GKD_OK;
-        const uint64_t slots = (uint64_t)e.hp.na * k, at = (uint64_t)a_base * k;
-        int rc;
-        if ((rc = read_back(c, rows->pos ? rows->pos + at : nullptr, c->hit_a.p, slots * 4, d2h)) ||
-            (rc = read_back(c, rows->inter ? rows->inter + at : nullptr, c->d_inter.p, slots * 8, d2h)) ||
-            (rc = read_back(c, rows->dist ? rows->dist + at : nullptr, c->d_dist.p, slots * 8, d2h)) ||
-            (rc = read_back(c, rows->n_found ? rows->n_found + a_base : nullptr, c->hit_b.p, (uint64_t)e.hp.na * 4, d2h)))
-            return rc;
-        CK(cudaStreamSynchronize(c->stream));
-        return GKD_OK;
+        rows_kept = true;
+        return read_lists(c, row_bufs(c), e.hp.na, *rows, a_base, d2h);
     }
-    // the lists to the caller, once, at the end of the call
-    int finish(gkd_ctx *c) {
-        if (!lists) return GKD_OK;
-        const gkd_neighbors &out = *lists;
-        const uint64_t slots = (uint64_t)targets * k;
+    // the lists to the caller, once, at the end of the call; rows no launch reached (no reference) are unused
+    int finish(gkd_ctx *c) override {
         int rc;
         uint64_t d2h = 0;
-        if ((rc = read_back(c, out.pos, c->nn_pos.p, slots * 4, d2h)) || (rc = read_back(c, out.inter, c->nn_inter.p, slots * 8, d2h)) ||
-            (rc = read_back(c, out.dist, c->nn_dist.p, slots * 8, d2h)) ||
-            (rc = read_back(c, out.n_found, c->nn_found.p, (uint64_t)targets * 4, d2h)))
+        if (rows && !rows_kept &&
+            ((rc = fill_unused(c, row_bufs(c), n_rows)) || (rc = read_lists(c, row_bufs(c), n_rows, *rows, 0, d2h))))
             return rc;
-        CK(cudaStreamSynchronize(c->stream));
+        if (lists && (rc = read_lists(c, list_bufs(c), targets, *lists, 0, d2h))) return rc;
         c->m.d2h_bytes += d2h;
         return GKD_OK;
     }
 };
 
 // gkd_*_clusters: the pairs within max_dist link their nodes in the union-find forest c->uf_parent (k_cluster_link;
-// RECT: query row r is node a_base + r, reference column j is node b_base + j).  Nothing is read back before finish().
+// RECT: query row r is node a_base + r, reference column j is node b_base + j).  Nothing is read back before finish(),
+// which writes the labels of nodes [0, na) to a_out and of [na, nodes) to b_out (either may be NULL).
 struct Clusters : Form {
     double max_dist;
-    uint32_t nodes, b_base;
-    Clusters(double d, uint32_t nodes_, uint32_t b_base_) : max_dist(d), nodes(nodes_), b_base(b_base_) {}
-    int start(gkd_ctx *c) {  // every node its own root
+    uint32_t nodes, b_base, na;
+    uint32_t *a_out, *b_out, *n_clusters;
+    Clusters(double d, uint32_t nodes_, uint32_t b_base_, uint32_t *a_out_, uint32_t na_, uint32_t *b_out_,
+             uint32_t *n_clusters_)
+        : max_dist(d), nodes(nodes_), b_base(b_base_), na(na_), a_out(a_out_), b_out(b_out_), n_clusters(n_clusters_) {}
+    std::array<const void *, 8> outputs() const override { return {a_out, b_out}; }
+    int start(gkd_ctx *c) override {  // every node its own root
         const int rc = ensure(c, c->uf_parent, ((uint64_t)nodes + 1) * 4);
         if (rc) return rc;
         CK(launch_cluster_init((uint32_t *)c->uf_parent.p, nodes, c->stream));
@@ -1404,9 +1442,8 @@ struct Clusters : Form {
         CK(cudaEventRecord(c->ev[7], c->stream));
         return GKD_OK;
     }
-    // The labels to the caller, once, at the end of the call: nodes [0, na) to a_out and [na, nodes) to b_out (either
-    // may be NULL).
-    int finish(gkd_ctx *c, uint32_t *a_out, uint32_t na, uint32_t *b_out, uint32_t *n_clusters) {
+    // the labels to the caller, once, at the end of the call
+    int finish(gkd_ctx *c) override {
         uint32_t *parent = (uint32_t *)c->uf_parent.p;
         CK(cudaEventRecord(c->ev[6], c->stream));
         CK(launch_cluster_flatten(parent, nodes, c->stream));
@@ -1433,13 +1470,16 @@ struct Linkage : Form {
     std::vector<uint32_t> key;        // key of every node (empty: the node itself); uploaded to c->lk_state when not empty
     uint32_t n_dev = 0;               // edges of the device forest c->lk_forest
     unsigned long long chunk_hits = 0;
-    Linkage(double d, uint32_t nodes_, uint32_t b_off_, std::vector<uint32_t> key_)
-        : max_dist(d), nodes(nodes_), b_off(b_off_), key(std::move(key_)) {}
+    gkd_hits *out;
+    Linkage(double d, uint32_t nodes_, uint32_t b_off_, std::vector<uint32_t> key_, gkd_hits *out_)
+        : max_dist(d), nodes(nodes_), b_off(b_off_), key(std::move(key_)), out(out_) {}
+    std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->inter, out->dist}; }
     LinkEdge edge(uint32_t a, uint32_t b, uint64_t inter, double dist) const {
         const uint32_t na = a, nb = b + b_off;
         return link_edge(a, b, inter, dist, na, nb, key.empty() ? na : key[na], key.empty() ? nb : key[nb]);
     }
-    int start(gkd_ctx *c) {  // an empty forest on the device, and the node keys there when the caller passed any
+    int start(gkd_ctx *c) override {  // an empty forest on the device, and the node keys there when the caller passed any
+        out->n = 0;
         int rc;
         if ((rc = ensure(c, c->lk_forest, (uint64_t)nodes * 24)) || (rc = ensure(c, c->lk_state, link_state_bytes(nodes))))
             return rc;
@@ -1508,7 +1548,7 @@ struct Linkage : Form {
     }
     // The forest to the caller, once, at the end of the call: the device forest is copied to the host and sorted there by
     // one Kruskal pass (a forest keeps every edge).
-    int finish(gkd_ctx *c, gkd_hits *out) {
+    int finish(gkd_ctx *c) override {
         std::vector<LinkEdge> edges;
         const uint64_t f = n_dev, N = nodes;
         if (f) {
@@ -1542,6 +1582,62 @@ struct Linkage : Form {
         return GKD_OK;
     }
 };
+
+// the triangle over the first n sets, and the block of queries q x references r
+HostPairs triangle(uint32_t n) { return {PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0}; }
+HostPairs block(const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr) {
+    return {PAIRS_RECT, nr, 0, (uint64_t)nq * nr, q, r, nq, nr};
+}
+
+// gkd.h publishes host memory as the only output memory of a GKD_AMBIG_LITERAL context, so device buffers are refused in
+// that mode
+int host_outputs_ok(gkd_ctx *c, const char *fn, const std::array<const void *, 8> &ps) {
+    if (c->cfg.ambig_policy != GKD_AMBIG_LITERAL) return GKD_OK;
+    for (const void *p : ps)
+        if (p && classify(p) == MEM_DEVICE) return fail(c, GKD_EINVAL, "%s: GKD_AMBIG_LITERAL needs host output buffers", fn);
+    return GKD_OK;
+}
+
+// One pair call on one device, for every form: the context, the shape of the pairs (messages start with fn), the
+// caller's outputs, every id the call names (also when it has no pairs), then the form's start, the chunks and the
+// form's finish.  RECT: hp is the caller's whole block.
+int run_call(gkd_ctx *c, const char *fn, const HostPairs &hp, Form &f) {
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    if (hp.mode == PAIRS_UPPER) {
+        if (hp.n > c->genomes.size()) return fail(c, GKD_EINVAL, "%s: %u sets but only %zu exist", fn, hp.n, c->genomes.size());
+        const uint64_t total = (uint64_t)hp.n * (hp.n - 1) / 2;
+        if (hp.first > total || hp.count > total - hp.first)
+            return fail(c, GKD_EINVAL, "%s: pair range [%llu, +%llu) outside 0..%llu", fn, (unsigned long long)hp.first,
+                        (unsigned long long)hp.count, (unsigned long long)total);
+    } else {
+        if ((hp.na && !hp.a) || (hp.nb && !hp.b)) return fail(c, GKD_EINVAL, "%s: null id array", fn);
+        if (hp.mode == PAIRS_LIST && hp.count > 0xFFFFFFFFull)
+            return fail(c, GKD_EINVAL, "%s: more than 2^32 pairs in one call", fn);
+    }
+    int rc = host_outputs_ok(c, fn, f.outputs());
+    if (rc) return rc;
+    // the metrics of this call alone (run_pairs sets them again for each launch)
+    c->m.pairs = c->m.intersect_bytes = 0;
+    c->m.intersect_ms = c->m.epilogue_ms = 0;
+    ABI_GUARD_BEGIN
+    if (hp.mode == PAIRS_UPPER) {
+        for (uint32_t i = 0; i < hp.n; i++)
+            if ((rc = check_built(c, i))) return rc;
+    } else if (hp.mode == PAIRS_RECT) {
+        for (uint32_t i = 0; i < hp.na; i++)
+            if ((rc = check_built(c, hp.a[i]))) return rc;
+        for (uint32_t j = 0; j < hp.nb; j++)
+            if ((rc = check_built(c, hp.b[j]))) return rc;
+    } else {
+        for (uint64_t t = 0; t < hp.count; t++)
+            if ((rc = check_built(c, hp.a[t])) || (rc = check_built(c, hp.b[t]))) return rc;
+    }
+    if ((rc = f.start(c))) return rc;
+    if (hp.count && (rc = hp.mode == PAIRS_RECT ? run_rect(c, hp, f) : run_pairs(c, hp, f))) return rc;
+    return f.finish(c);
+    ABI_GUARD_END(c)
+}
 
 int default_k(int alphabet) { return alphabet == GKD_PROT ? 8 : 21; }
 
@@ -2097,30 +2193,10 @@ int gkd_load_sets(gkd_ctx *c, const char *path, uint32_t *first_id, uint32_t *n_
 }
 
 // ---- distances --------------------------------------------------------------------------------------------
-// gkd.h publishes host memory as the only output memory of a GKD_AMBIG_LITERAL context, so device buffers are refused
-// in that mode.  The selections check this before the context is touched, so a bad k or a NaN threshold is GKD_EINVAL
-// even without a usable device.
-static int host_outputs_ok(gkd_ctx *c, std::initializer_list<const void *> ps) {
-    if (c->cfg.ambig_policy != GKD_AMBIG_LITERAL) return GKD_OK;
-    for (const void *p : ps)
-        if (p && classify(p) == MEM_DEVICE) return fail(c, GKD_EINVAL, "GKD_AMBIG_LITERAL needs host output buffers");
-    return GKD_OK;
-}
-
 int gkd_all_vs_all_range_ex(gkd_ctx *c, uint32_t n, uint64_t first, uint64_t count, const gkd_outputs *out) {
-    CHECK_CTX(c);
-    if (!out) return fail(c, GKD_EINVAL, "null outputs");
-    CK(cudaSetDevice(c->cfg.device));
-    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "range over %u sets but only %zu exist", n, c->genomes.size());
-    uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
-    if (first > total || count > total - first) return fail(c, GKD_EINVAL, "pair range [%llu, +%llu) outside 0..%llu", (unsigned long long)first, (unsigned long long)count, (unsigned long long)total);
-    int rc = host_outputs_ok(c, {out->inter, out->dist, out->contain_a, out->contain_b});
-    if (rc) return rc;
-    ABI_GUARD_BEGIN
-    HostPairs hp{PAIRS_UPPER, n, first, count, nullptr, nullptr, 0, 0};
+    if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_range_ex: null outputs");
     Dense f(*out);
-    return run_pairs(c, hp, f);
-    ABI_GUARD_END(c)
+    return run_call(c, "gkd_all_vs_all_range_ex", HostPairs{PAIRS_UPPER, n, first, count, nullptr, nullptr, 0, 0}, f);
 }
 
 int gkd_all_vs_all_range(gkd_ctx *c, uint32_t n, uint64_t first, uint64_t count, uint64_t *inter, double *dist) {
@@ -2135,20 +2211,9 @@ int gkd_all_vs_all(gkd_ctx *c, uint64_t *inter, double *dist) {
 }
 
 int gkd_query_vs_ref_ex(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, const gkd_outputs *out) {
-    CHECK_CTX(c);
-    if (!out) return fail(c, GKD_EINVAL, "null outputs");
-    CK(cudaSetDevice(c->cfg.device));
-    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref: null id array");
-    int rc = host_outputs_ok(c, {out->inter, out->dist, out->contain_a, out->contain_b});
-    if (rc) return rc;
-    if (nq == 0 || nr == 0) {
-        c->m.pairs = 0;
-        return GKD_OK;
-    }
-    ABI_GUARD_BEGIN
+    if (!out) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_ex: null outputs");
     Dense f(*out);
-    return run_rect(c, q, nq, r, nr, f);
-    ABI_GUARD_END(c)
+    return run_call(c, "gkd_query_vs_ref_ex", block(q, nq, r, nr), f);
 }
 
 int gkd_query_vs_ref(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint64_t *inter, double *dist) {
@@ -2157,18 +2222,9 @@ int gkd_query_vs_ref(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t 
 }
 
 int gkd_pairs_ex(gkd_ctx *c, const uint32_t *a, const uint32_t *b, uint64_t n_pairs, const gkd_outputs *out) {
-    CHECK_CTX(c);
-    if (!out) return fail(c, GKD_EINVAL, "null outputs");
-    CK(cudaSetDevice(c->cfg.device));
-    if (n_pairs && (!a || !b)) return fail(c, GKD_EINVAL, "gkd_pairs: null id array");
-    if (n_pairs > 0xFFFFFFFFull) return fail(c, GKD_EINVAL, "gkd_pairs: more than 2^32 pairs in one call");
-    int rc = host_outputs_ok(c, {out->inter, out->dist, out->contain_a, out->contain_b});
-    if (rc) return rc;
-    ABI_GUARD_BEGIN
-    HostPairs hp{PAIRS_LIST, 0, 0, n_pairs, a, b, (uint32_t)n_pairs, (uint32_t)n_pairs};
+    if (!out) return fail(c, GKD_EINVAL, "gkd_pairs_ex: null outputs");
     Dense f(*out);
-    return run_pairs(c, hp, f);
-    ABI_GUARD_END(c)
+    return run_call(c, "gkd_pairs_ex", HostPairs{PAIRS_LIST, 0, 0, n_pairs, a, b, (uint32_t)n_pairs, (uint32_t)n_pairs}, f);
 }
 
 int gkd_pairs(gkd_ctx *c, const uint32_t *a, const uint32_t *b, uint64_t n_pairs, uint64_t *inter, double *dist) {
@@ -2276,50 +2332,16 @@ int gkd_pair(gkd_ctx *c, uint32_t a, uint32_t b, uint64_t *inter, uint64_t *uni,
 int gkd_all_vs_all_range_within(gkd_ctx *c, uint32_t n, uint64_t first, uint64_t count, double max_dist, gkd_hits *out) {
     if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_range_within: null hits");
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_range_within: max_dist is NaN");
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "range over %u sets but only %zu exist", n, c->genomes.size());
-    uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
-    if (first > total || count > total - first) return fail(c, GKD_EINVAL, "pair range [%llu, +%llu) outside 0..%llu", (unsigned long long)first, (unsigned long long)count, (unsigned long long)total);
-    int rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist});
-    if (rc) return rc;
-    out->n = 0;
-    ABI_GUARD_BEGIN
-    HostPairs hp{PAIRS_UPPER, n, first, count, nullptr, nullptr, 0, 0};
     Within f(max_dist, *out);
-    return run_pairs(c, hp, f);
-    ABI_GUARD_END(c)
+    return run_call(c, "gkd_all_vs_all_range_within", HostPairs{PAIRS_UPPER, n, first, count, nullptr, nullptr, 0, 0}, f);
 }
 
 int gkd_query_vs_ref_within(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, double max_dist,
                             gkd_hits *out) {
     if (!out) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_within: null hits");
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_within: max_dist is NaN");
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_within: null id array");
-    int rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist});
-    if (rc) return rc;
-    out->n = 0;
-    if (nq == 0 || nr == 0) {
-        c->m.pairs = 0;
-        return GKD_OK;
-    }
-    ABI_GUARD_BEGIN
     Within f(max_dist, *out);
-    return run_rect(c, q, nq, r, nr, f);
-    ABI_GUARD_END(c)
-}
-
-// rows * k unused entries (and n_found 0) in every member of out
-static int fill_none(gkd_ctx *c, uint32_t rows, uint32_t k, const gkd_neighbors *out) {
-    if (!out || rows == 0) return GKD_OK;
-    const uint64_t slots = (uint64_t)rows * k;
-    if (out->pos) CK(cudaMemcpy(out->pos, std::vector<uint32_t>(slots, 0xFFFFFFFFu).data(), slots * 4, cudaMemcpyDefault));
-    if (out->inter) CK(cudaMemcpy(out->inter, std::vector<uint64_t>(slots, 0).data(), slots * 8, cudaMemcpyDefault));
-    if (out->dist) CK(cudaMemcpy(out->dist, std::vector<double>(slots, -1.0).data(), slots * 8, cudaMemcpyDefault));
-    if (out->n_found) CK(cudaMemcpy(out->n_found, std::vector<uint32_t>(rows, 0).data(), (uint64_t)rows * 4, cudaMemcpyDefault));
-    return GKD_OK;
+    return run_call(c, "gkd_query_vs_ref_within", block(q, nq, r, nr), f);
 }
 
 static int nearest_args_ok(gkd_ctx *c, const char *fn, uint32_t k, double max_dist) {
@@ -2328,100 +2350,47 @@ static int nearest_args_ok(gkd_ctx *c, const char *fn, uint32_t k, double max_di
     return GKD_OK;
 }
 
-// gkd_query_vs_ref_nearest(_ex): the q side as row lists (complete in every launch), the r side through the per-target
-// lists across the launches of run_rect
-static int nearest_rect(gkd_ctx *c, const char *fn, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
-                        double max_dist, int exclude_self, const gkd_neighbors *qs, const gkd_neighbors *rs) {
-    int rc = nearest_args_ok(c, fn, k, max_dist);
-    if (rc) return rc;
-    if (!qs && !rs) return fail(c, GKD_EINVAL, "%s: both sides are NULL", fn);
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "%s: null id array", fn);
-    const gkd_neighbors none{};
-    const gkd_neighbors &a = qs ? *qs : none, &b = rs ? *rs : none;
-    if ((rc = host_outputs_ok(c, {a.pos, a.inter, a.dist, a.n_found, b.pos, b.inter, b.dist, b.n_found}))) return rc;
-    c->m.pairs = 0;
-    ABI_GUARD_BEGIN
-    if (nq == 0 || nr == 0) {  // no pair: every list is empty
-        if ((rc = fill_none(c, nq, k, qs))) return rc;
-        return fill_none(c, nr, k, rs);
-    }
-    Nearest f(k, max_dist, exclude_self ? 1 : 0, qs, rs, nr);
-    if ((rc = f.start(c)) || (rc = run_rect(c, q, nq, r, nr, f))) return rc;
-    return f.finish(c);
-    ABI_GUARD_END(c)
-}
-
 int gkd_query_vs_ref_nearest(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
                              double max_dist, int exclude_self, uint32_t *ref_pos, uint64_t *inter, double *dist,
                              uint32_t *n_found) {
     const gkd_neighbors qs{ref_pos, inter, dist, n_found};
-    return nearest_rect(c, "gkd_query_vs_ref_nearest", q, nq, r, nr, k, max_dist, exclude_self, &qs, nullptr);
+    return gkd_query_vs_ref_nearest_ex(c, q, nq, r, nr, k, max_dist, exclude_self, &qs, nullptr);
 }
 
+// the q side as row lists (complete in every launch), the r side through the per-target lists across the launches
 int gkd_query_vs_ref_nearest_ex(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, uint32_t k,
                                 double max_dist, int exclude_self, const gkd_neighbors *q_side, const gkd_neighbors *r_side) {
-    return nearest_rect(c, "gkd_query_vs_ref_nearest_ex", q, nq, r, nr, k, max_dist, exclude_self, q_side, r_side);
+    const char *fn = "gkd_query_vs_ref_nearest_ex";
+    int rc = nearest_args_ok(c, fn, k, max_dist);
+    if (rc) return rc;
+    if (!q_side && !r_side) return fail(c, GKD_EINVAL, "%s: both sides are NULL", fn);
+    Nearest f(k, max_dist, exclude_self ? 1 : 0, q_side, nq, r_side, nr);
+    return run_call(c, fn, block(q, nq, r, nr), f);
 }
 
 int gkd_all_vs_all_nearest(gkd_ctx *c, uint32_t n, uint32_t k, double max_dist, const gkd_neighbors *out) {
     int rc = nearest_args_ok(c, "gkd_all_vs_all_nearest", k, max_dist);
     if (rc) return rc;
     if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_nearest: null output");
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "nearest over %u sets but only %zu exist", n, c->genomes.size());
-    if ((rc = host_outputs_ok(c, {out->pos, out->inter, out->dist, out->n_found}))) return rc;
-    c->m.pairs = 0;
-    if (n == 0) return GKD_OK;
-    ABI_GUARD_BEGIN
-    Nearest f(k, max_dist, 0, nullptr, out, n);
-    HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
-    if ((rc = f.start(c)) || (rc = run_pairs(c, hp, f))) return rc;
-    return f.finish(c);
-    ABI_GUARD_END(c)
+    Nearest f(k, max_dist, 0, nullptr, 0, out, n);
+    return run_call(c, "gkd_all_vs_all_nearest", triangle(n), f);
 }
 
 // ---- single-linkage clusters ----------------------------------------------------------------------------------
 int gkd_all_vs_all_clusters(gkd_ctx *c, uint32_t n, double max_dist, uint32_t *label, uint32_t *n_clusters) {
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_clusters: max_dist is NaN");
     if (!label) return fail(c, GKD_EINVAL, "gkd_all_vs_all_clusters: null label");
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "clusters over %u sets but only %zu exist", n, c->genomes.size());
-    int rc = host_outputs_ok(c, {label});
-    if (rc) return rc;
-    c->m.pairs = 0;
-    if (n_clusters) *n_clusters = 0;
-    if (n == 0) return GKD_OK;
-    ABI_GUARD_BEGIN
-    Clusters f(max_dist, n, 0);
-    HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
-    if ((rc = f.start(c)) || (rc = run_pairs(c, hp, f))) return rc;
-    return f.finish(c, label, n, nullptr, n_clusters);
-    ABI_GUARD_END(c)
+    Clusters f(max_dist, n, 0, label, n, nullptr, n_clusters);
+    return run_call(c, "gkd_all_vs_all_clusters", triangle(n), f);
 }
 
 int gkd_query_vs_ref_clusters(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, double max_dist,
                               uint32_t *q_label, uint32_t *r_label) {
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: max_dist is NaN");
     if (!q_label && !r_label) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: both outputs are NULL");
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: null id array");
     if ((uint64_t)nq + nr >= 0xFFFFFFFFull) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_clusters: %u + %u nodes", nq, nr);
-    int rc = host_outputs_ok(c, {q_label, r_label});
-    if (rc) return rc;
-    c->m.pairs = 0;
-    const uint32_t nodes = nq + nr;
-    if (nodes == 0) return GKD_OK;
-    ABI_GUARD_BEGIN
-    Clusters f(max_dist, nodes, nq);
-    if ((rc = f.start(c))) return rc;
-    if (nq && nr && (rc = run_rect(c, q, nq, r, nr, f))) return rc;
-    return f.finish(c, q_label, nq, r_label, nullptr);
-    ABI_GUARD_END(c)
+    Clusters f(max_dist, nq + nr, nq, q_label, nq, r_label, nullptr);
+    return run_call(c, "gkd_query_vs_ref_clusters", block(q, nq, r, nr), f);
 }
 
 // ---- single-linkage hierarchy --------------------------------------------------------------------------------
@@ -2445,20 +2414,8 @@ static int link_keys(gkd_ctx *c, const uint32_t *q_key, uint32_t nq, const uint3
 int gkd_all_vs_all_linkage(gkd_ctx *c, uint32_t n, double max_dist, gkd_hits *out) {
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "gkd_all_vs_all_linkage: max_dist is NaN");
     if (!out) return fail(c, GKD_EINVAL, "gkd_all_vs_all_linkage: null out");
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if (n > c->genomes.size()) return fail(c, GKD_EINVAL, "linkage over %u sets but only %zu exist", n, c->genomes.size());
-    int rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist});
-    if (rc) return rc;
-    c->m.pairs = 0;
-    out->n = 0;
-    if (n < 2) return GKD_OK;
-    ABI_GUARD_BEGIN
-    Linkage f(max_dist, n, 0, {});
-    HostPairs hp{PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0};
-    if ((rc = f.start(c)) || (rc = run_pairs(c, hp, f))) return rc;
-    return f.finish(c, out);
-    ABI_GUARD_END(c)
+    Linkage f(max_dist, n, 0, {}, out);
+    return run_call(c, "gkd_all_vs_all_linkage", triangle(n), f);
 }
 
 int gkd_query_vs_ref_linkage(gkd_ctx *c, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr, double max_dist,
@@ -2469,18 +2426,8 @@ int gkd_query_vs_ref_linkage(gkd_ctx *c, const uint32_t *q, uint32_t nq, const u
     std::vector<uint32_t> key;
     int rc = link_keys(c, q_key, nq, r_key, nr, key);
     if (rc) return rc;
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    if ((nq && !q) || (nr && !r)) return fail(c, GKD_EINVAL, "gkd_query_vs_ref_linkage: null id array");
-    if ((rc = host_outputs_ok(c, {out->a, out->b, out->inter, out->dist}))) return rc;
-    c->m.pairs = 0;
-    out->n = 0;
-    if (nq == 0 || nr == 0) return GKD_OK;
-    ABI_GUARD_BEGIN
-    Linkage f(max_dist, nq + nr, nq, std::move(key));
-    if ((rc = f.start(c)) || (rc = run_rect(c, q, nq, r, nr, f))) return rc;
-    return f.finish(c, out);
-    ABI_GUARD_END(c)
+    Linkage f(max_dist, nq + nr, nq, std::move(key), out);
+    return run_call(c, "gkd_query_vs_ref_linkage", block(q, nq, r, nr), f);
 }
 
 // ---- MinHash sketches ---------------------------------------------------------------------------------------

@@ -145,17 +145,74 @@ const std::vector<OptSpec> FASTA_OPTS = {
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
 
+// The sets fastaDist reports on: one context, or a group of contexts, one per device, with the pair matrix sharded over
+// them (gkd_group_*).  Every report is written once, from these calls.
+struct DistSource {
+    std::unique_ptr<KmerEngine> engine;  // exactly one of engine and grp is set
+    gkd_group *grp = nullptr;
+    int gpus = 1;
+    uint32_t n = 0;  // sets
+    DistSource(KmerType type, int k, int device, const std::vector<int32_t> &devices)
+        : gpus(devices.empty() ? 1 : (int)devices.size()) {
+        if (devices.empty()) {
+            engine.reset(new KmerEngine(type, k, device));
+            return;
+        }
+        gkd_config cfg{};
+        cfg.k = k;
+        cfg.alphabet = (int)type;
+        if (gkd_group_create(&grp, &cfg, devices.data(), (uint32_t)devices.size()) != GKD_OK)
+            throw std::runtime_error(gkd_group_last_error(nullptr));
+    }
+    ~DistSource() {
+        if (grp) gkd_group_destroy(grp);
+    }
+    void check(int rc) const {
+        if (engine) return engine->check(rc);
+        if (rc == GKD_EIO) throw IOException(gkd_group_last_error(grp));
+        if (rc == GKD_EINVAL) throw ParseFailureException(gkd_group_last_error(grp));
+        if (rc != GKD_OK) throw std::runtime_error(gkd_group_last_error(grp));
+    }
+    // every record of a FASTA file as its own set
+    void addFasta(const std::string &path) {
+        if (engine) n = (uint32_t)engine->addFasta(path).size();
+        else check(gkd_group_add_fasta_file(grp, path.c_str(), &n));
+    }
+    void build() { check(engine ? gkd_build_sets(engine->raw()) : gkd_group_build(grp)); }
+    const char *label(size_t i) const {
+        return engine ? gkd_label(engine->raw(), (uint32_t)i) : gkd_group_label(grp, (uint32_t)i);
+    }
+    const char *comment(size_t i) const {
+        return engine ? gkd_comment(engine->raw(), (uint32_t)i) : gkd_group_comment(grp, (uint32_t)i);
+    }
+    // the context whose metrics --metrics writes
+    gkd_ctx *metricsCtx() const { return engine ? engine->raw() : gkd_group_member(grp, 0); }
+    void allVsAll(double *dist) const {
+        check(engine ? gkd_all_vs_all(engine->raw(), nullptr, dist) : gkd_group_all_vs_all(grp, nullptr, dist));
+    }
+    void nearest(uint32_t k, double maxDist, const gkd_neighbors &nb) const {
+        check(engine ? gkd_all_vs_all_nearest(engine->raw(), n, k, maxDist, &nb)
+                     : gkd_group_all_vs_all_nearest(grp, k, maxDist, &nb));
+    }
+    void clusters(double maxDist, uint32_t *label) const {
+        check(engine ? gkd_all_vs_all_clusters(engine->raw(), n, maxDist, label, nullptr)
+                     : gkd_group_all_vs_all_clusters(grp, maxDist, label, nullptr));
+    }
+    void linkage(double maxDist, gkd_hits &h) const {
+        check(engine ? gkd_all_vs_all_linkage(engine->raw(), n, maxDist, &h) : gkd_group_all_vs_all_linkage(grp, maxDist, &h));
+    }
+};
+
 // one report line of fastaDist (:188-192)
-template <class LabelFn, class CommentFn>
-void writePairLine(std::ostream &writer, std::string &line, size_t i, size_t j, double dist, LabelFn label, CommentFn comment) {
+void writePairLine(std::ostream &writer, std::string &line, size_t i, size_t j, double dist, const DistSource &src) {
     line.clear();
-    line += label(i);
+    line += src.label(i);
     line += '\t';
-    line += comment(i);
+    line += src.comment(i);
     line += '\t';
-    line += label(j);
+    line += src.label(j);
     line += '\t';
-    line += comment(j);
+    line += src.comment(j);
     line += '\t';
     line += javaDouble(dist);
     line += '\n';
@@ -163,51 +220,46 @@ void writePairLine(std::ostream &writer, std::string &line, size_t i, size_t j, 
 }
 
 // the report lines of fastaDist (:188-192), in list order
-template <class LabelFn, class CommentFn>
-size_t writePairs(std::ostream &writer, size_t n, const std::vector<double> &dist, LabelFn label, CommentFn comment) {
+size_t writePairs(std::ostream &writer, const std::vector<double> &dist, const DistSource &src) {
     size_t t = 0;
     std::string line;
-    for (size_t i = 0; i < n; i++)
-        for (size_t j = i + 1; j < n; j++, t++) writePairLine(writer, line, i, j, dist[t], label, comment);
+    for (size_t i = 0; i < src.n; i++)
+        for (size_t j = i + 1; j < src.n; j++, t++) writePairLine(writer, line, i, j, dist[t], src);
     writer.flush();
     return t;
 }
 
 // the lines of the full report whose distance is <= maxDist, in the same order: hits of gkd_*_within (a < b)
-template <class LabelFn, class CommentFn>
-void writeHits(std::ostream &writer, const uint32_t *a, const uint32_t *b, const double *dist, uint64_t n, LabelFn label,
-               CommentFn comment) {
+void writeHits(std::ostream &writer, const uint32_t *a, const uint32_t *b, const double *dist, uint64_t n,
+               const DistSource &src) {
     std::string line;
-    for (uint64_t t = 0; t < n; t++) writePairLine(writer, line, a[t], b[t], dist[t], label, comment);
+    for (uint64_t t = 0; t < n; t++) writePairLine(writer, line, a[t], b[t], dist[t], src);
 }
 
 // the lines of `fastaDist --nearest`: for each record in input order its neighbours (n*k lists of gkd_*_nearest), record
 // first, in ascending distance and then input order
-template <class LabelFn, class CommentFn>
-uint64_t writeNeighbors(std::ostream &writer, size_t n, uint32_t k, const uint32_t *pos, const double *dist,
-                        const uint32_t *found, LabelFn label, CommentFn comment) {
+uint64_t writeNeighbors(std::ostream &writer, uint32_t k, const uint32_t *pos, const double *dist, const uint32_t *found,
+                        const DistSource &src) {
     std::string line;
     uint64_t lines = 0;
-    for (size_t i = 0; i < n; i++)
-        for (uint32_t s = 0; s < found[i]; s++, lines++)
-            writePairLine(writer, line, i, pos[i * k + s], dist[i * k + s], label, comment);
+    for (size_t i = 0; i < src.n; i++)
+        for (uint32_t s = 0; s < found[i]; s++, lines++) writePairLine(writer, line, i, pos[i * k + s], dist[i * k + s], src);
     writer.flush();
     return lines;
 }
 
 // the lines of `fastaDist --clusters`: every record in input order with the label of its cluster's first record
-template <class LabelFn, class CommentFn>
-uint32_t writeClusters(std::ostream &writer, size_t n, const uint32_t *cluster, LabelFn label, CommentFn comment) {
+uint32_t writeClusters(std::ostream &writer, const uint32_t *cluster, const DistSource &src) {
     std::string line;
     uint32_t clusters = 0;
     writer << "seq\tname\tcluster\n";
-    for (size_t i = 0; i < n; i++) {
+    for (size_t i = 0; i < src.n; i++) {
         line.clear();
-        line += label(i);
+        line += src.label(i);
         line += '\t';
-        line += comment(i);
+        line += src.comment(i);
         line += '\t';
-        line += label(cluster[i]);
+        line += src.label(cluster[i]);
         line += '\n';
         writer << line;
         clusters += cluster[i] == i ? 1u : 0u;
@@ -293,72 +345,73 @@ int fastaDist(const std::vector<std::string> &args) {
     }
     const std::string metricsFile = p.values.count("--metrics") ? p.values["--metrics"] : "";
     if (gpus < 1) throw ParseFailureException("Number of GPUs must be at least 1.");
-    if (gpus > 1 || !deviceList.empty()) {
-        // the pair matrix sharded over a group of contexts, one per device (gkd_group_*); same report
-        if (inFile.empty()) throw ParseFailureException("--gpus needs an input file (--input).");
-        gkd_config cfg{};
-        cfg.k = kmerSize;
-        cfg.alphabet = (int)seqType;
-        std::vector<int32_t> devices = deviceList;
-        if (devices.empty())
-            for (int d = 0; d < gpus; d++) devices.push_back(device + d);
-        gkd_group *grp = nullptr;
-        if (gkd_group_create(&grp, &cfg, devices.data(), (uint32_t)devices.size()) != GKD_OK)
-            throw std::runtime_error(gkd_group_last_error(nullptr));
-        struct Closer {
-            gkd_group *g;
-            ~Closer() { gkd_group_destroy(g); }
-        } closer{grp};
-        auto gcheck = [&](int rc) {
-            if (rc == GKD_EIO) throw IOException(gkd_group_last_error(grp));
-            if (rc == GKD_EINVAL) throw ParseFailureException(gkd_group_last_error(grp));
-            if (rc != GKD_OK) throw std::runtime_error(gkd_group_last_error(grp));
-        };
-        uint32_t n = 0;
-        gcheck(gkd_group_add_fasta_file(grp, inFile.c_str(), &n));
-        logInfo(std::to_string(n) + " sequences read from input.");
-        if (!clusters) writer << "seq1\tname1\tseq2\tname2\tdistance\n";
-        gcheck(gkd_group_build(grp));
-        logInfo(std::to_string(n) + " sequences cached on " + std::to_string(gpus) + " GPUs. Computing distances.");
-        const uint64_t total = n < 2 ? 0 : (uint64_t)n * (n - 1) / 2;
-        if (clusters) {
-            std::vector<uint32_t> label(n);
-            gcheck(gkd_group_all_vs_all_clusters(grp, maxDist, label.data(), nullptr));
-            const uint32_t found = writeClusters(writer, n, label.data(), [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
-                                                 [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
-            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(found) + " clusters at distance " +
-                    javaDouble(maxDist) + ".");
-            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
-            return 0;
-        }
-        if (linkage) {
-            const uint64_t cap = n ? n - 1 : 0;
-            std::vector<uint32_t> a(cap), b(cap);
-            std::vector<double> d(cap);
-            gkd_hits h{a.data(), b.data(), nullptr, d.data(), cap, 0};
-            gcheck(gkd_group_all_vs_all_linkage(grp, maxDist, &h));
-            writeHits(writer, a.data(), b.data(), d.data(), h.n, [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
-                      [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
-            writer.flush();
-            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(h.n) + " merges up to distance " +
-                    javaDouble(maxDist) + ".");
-            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
-            return 0;
-        }
-        if (nearest) {
-            const uint32_t k = (uint32_t)nearest;
-            std::vector<uint32_t> pos((size_t)n * k), found(n);
-            std::vector<double> d((size_t)n * k);
-            const gkd_neighbors nb{pos.data(), nullptr, d.data(), found.data()};
-            gcheck(gkd_group_all_vs_all_nearest(grp, k, maxDist, &nb));
-            const uint64_t lines = writeNeighbors(writer, n, k, pos.data(), d.data(), found.data(),
-                                                  [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
-                                                  [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
-            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(lines) + " neighbor lines.");
-            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
-            return 0;
-        }
-        if (within) {
+    // more than one GPU, or an explicit device list: the pair matrix sharded over a group, one context per device
+    std::vector<int32_t> devices = deviceList;
+    if (devices.empty() && gpus > 1)
+        for (int d = 0; d < gpus; d++) devices.push_back(device + d);
+    if (!devices.empty() && inFile.empty()) throw ParseFailureException("--gpus needs an input file (--input).");
+    DistSource src(seqType, kmerSize, device, devices);
+    src.addFasta(inFile.empty() ? "-" : inFile);
+    logInfo(std::to_string(src.n) + " sequences read from input.");
+    // runReporter (:134-165): the batch cache and the per-row parallel streams are what the engine
+    // replaces; every pair i<j is computed in one batched launch and printed in list order
+    if (!clusters) writer << "seq1\tname1\tseq2\tname2\tdistance\n";
+    src.build();
+    logInfo(std::to_string(src.n) + " sequences cached" + (src.grp ? " on " + std::to_string(src.gpus) + " GPUs" : "") +
+            ". Computing distances.");
+    const uint64_t n = src.n, total = n < 2 ? 0 : n * (n - 1) / 2;
+    if (clusters) {
+        // each pair i < j is intersected once and linked on the GPU; only the n labels leave it
+        std::vector<uint32_t> label(n);
+        src.clusters(maxDist, label.data());
+        const uint32_t found = writeClusters(writer, label.data(), src);
+        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(found) + " clusters at distance " +
+                javaDouble(maxDist) + ".");
+        writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);
+        return 0;
+    }
+    if (linkage) {
+        // each pair i < j is intersected once; only the spanning forest (<= n - 1 edges) leaves the GPU
+        const uint64_t cap = n ? n - 1 : 0;
+        std::vector<uint32_t> a(cap), b(cap);
+        std::vector<double> d(cap);
+        gkd_hits h{a.data(), b.data(), nullptr, d.data(), cap, 0};
+        src.linkage(maxDist, h);
+        writeHits(writer, a.data(), b.data(), d.data(), h.n, src);
+        writer.flush();
+        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(h.n) + " merges up to distance " +
+                javaDouble(maxDist) + ".");
+        writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);
+        return 0;
+    }
+    if (nearest) {
+        // each pair i < j is intersected once and offered to both rows; only the n*k lists leave the GPU
+        const uint32_t k = (uint32_t)nearest;
+        std::vector<uint32_t> pos(n * k), found(n);
+        std::vector<double> d(n * k);
+        const gkd_neighbors nb{pos.data(), nullptr, d.data(), found.data()};
+        src.nearest(k, maxDist, nb);
+        const uint64_t lines = writeNeighbors(writer, k, pos.data(), d.data(), found.data(), src);
+        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(lines) + " neighbor lines.");
+        writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);
+        return 0;
+    }
+    if (within) {
+        // only the pairs within maxDist leave the GPUs
+        uint64_t hits = 0;
+        if (src.engine) {
+            // the triangle in ranges of <= WITHIN_RANGE pairs
+            const uint64_t room = std::min(total, WITHIN_RANGE);
+            std::unique_ptr<uint32_t[]> a(new uint32_t[room + 1]), b(new uint32_t[room + 1]);
+            std::unique_ptr<double[]> d(new double[room + 1]);
+            for (uint64_t first = 0; first < total; first += WITHIN_RANGE) {
+                const uint64_t cnt = std::min(WITHIN_RANGE, total - first);
+                gkd_hits h{a.get(), b.get(), nullptr, d.get(), cnt, 0};
+                src.check(gkd_all_vs_all_range_within(src.engine->raw(), src.n, first, cnt, maxDist, &h));
+                writeHits(writer, a.get(), b.get(), d.get(), h.n, src);
+                hits += h.n;
+            }
+        } else {
             // every member selects on its device; one call, repeated with the exact capacity if the first was short
             uint64_t cap = std::min<uint64_t>(total, WITHIN_RANGE);
             std::vector<uint32_t> a, b;
@@ -369,103 +422,24 @@ int fastaDist(const std::vector<std::string> &args) {
                 b.resize(cap);
                 d.resize(cap);
                 h = gkd_hits{a.data(), b.data(), nullptr, d.data(), cap, 0};
-                gcheck(gkd_group_all_vs_all_within(grp, maxDist, &h));
+                src.check(gkd_group_all_vs_all_within(src.grp, maxDist, &h));
                 if (h.n <= cap) break;
                 cap = h.n;
             }
-            writeHits(writer, a.data(), b.data(), d.data(), h.n, [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
-                      [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
-            writer.flush();
-            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(h.n) + " within distance " +
-                    javaDouble(maxDist) + ".");
-            writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), total, gpus);
-            return 0;
-        }
-        std::vector<double> dist((size_t)n * (n > 0 ? n - 1 : 0) / 2);
-        gcheck(gkd_group_all_vs_all(grp, nullptr, dist.data()));
-        size_t t = writePairs(writer, n, dist, [&](size_t i) { return gkd_group_label(grp, (uint32_t)i); },
-                              [&](size_t i) { return gkd_group_comment(grp, (uint32_t)i); });
-        logInfo(std::to_string(t) + " pairs computed in 1 batches.");
-        writeMetrics(metricsFile, "fastaDist", gkd_group_member(grp, 0), t, gpus);
-        return 0;
-    }
-    KmerEngine engine(seqType, kmerSize, device);
-    std::vector<SequenceKmers> seqs = engine.addFasta(inFile.empty() ? "-" : inFile);
-    logInfo(std::to_string(seqs.size()) + " sequences read from input.");
-    // runReporter (:134-165): the batch cache and the per-row parallel streams are what the engine
-    // replaces; every pair i<j is computed in one batched launch and printed in list order
-    if (!clusters) writer << "seq1\tname1\tseq2\tname2\tdistance\n";
-    engine.build();
-    logInfo(std::to_string(seqs.size()) + " sequences cached. Computing distances.");
-    if (clusters) {
-        // each pair i < j is intersected once and linked on the GPU; only the n labels leave it
-        const size_t n = seqs.size();
-        std::vector<uint32_t> label(n);
-        engine.check(gkd_all_vs_all_clusters(engine.raw(), (uint32_t)n, maxDist, label.data(), nullptr));
-        const uint32_t found = writeClusters(writer, n, label.data(), [&](size_t i) { return seqs[i].getGenomeId(); },
-                                             [&](size_t i) { return seqs[i].getGenomeName(); });
-        logInfo(std::to_string(n < 2 ? 0 : n * (n - 1) / 2) + " pairs computed in 1 batches, " + std::to_string(found) +
-                " clusters at distance " + javaDouble(maxDist) + ".");
-        writeMetrics(metricsFile, "fastaDist", engine.raw(), n < 2 ? 0 : n * (n - 1) / 2, 1);
-        return 0;
-    }
-    if (linkage) {
-        // each pair i < j is intersected once; only the spanning forest (<= n - 1 edges) leaves the GPU
-        const uint64_t n = seqs.size(), total = n < 2 ? 0 : n * (n - 1) / 2, cap = n ? n - 1 : 0;
-        std::vector<uint32_t> a(cap), b(cap);
-        std::vector<double> d(cap);
-        gkd_hits h{a.data(), b.data(), nullptr, d.data(), cap, 0};
-        engine.check(gkd_all_vs_all_linkage(engine.raw(), (uint32_t)n, maxDist, &h));
-        writeHits(writer, a.data(), b.data(), d.data(), h.n, [&](size_t i) { return seqs[i].getGenomeId(); },
-                  [&](size_t i) { return seqs[i].getGenomeName(); });
-        writer.flush();
-        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(h.n) + " merges up to distance " +
-                javaDouble(maxDist) + ".");
-        writeMetrics(metricsFile, "fastaDist", engine.raw(), total, 1);
-        return 0;
-    }
-    if (nearest) {
-        // each pair i < j is intersected once and offered to both rows; only the n*k lists leave the GPU
-        const uint32_t k = (uint32_t)nearest;
-        const size_t n = seqs.size();
-        std::vector<uint32_t> pos(n * k), found(n);
-        std::vector<double> d(n * k);
-        const gkd_neighbors nb{pos.data(), nullptr, d.data(), found.data()};
-        engine.check(gkd_all_vs_all_nearest(engine.raw(), (uint32_t)n, k, maxDist, &nb));
-        const uint64_t lines = writeNeighbors(writer, n, k, pos.data(), d.data(), found.data(),
-                                              [&](size_t i) { return seqs[i].getGenomeId(); },
-                                              [&](size_t i) { return seqs[i].getGenomeName(); });
-        logInfo(std::to_string(n < 2 ? 0 : n * (n - 1) / 2) + " pairs computed in 1 batches, " + std::to_string(lines) +
-                " neighbor lines.");
-        writeMetrics(metricsFile, "fastaDist", engine.raw(), n < 2 ? 0 : n * (n - 1) / 2, 1);
-        return 0;
-    }
-    if (within) {
-        // the triangle in ranges of <= WITHIN_RANGE pairs; only the pairs within maxDist leave the GPU
-        const uint64_t n = seqs.size(), total = n < 2 ? 0 : n * (n - 1) / 2, room = std::min(total, WITHIN_RANGE);
-        std::unique_ptr<uint32_t[]> a(new uint32_t[room + 1]), b(new uint32_t[room + 1]);
-        std::unique_ptr<double[]> d(new double[room + 1]);
-        uint64_t hits = 0;
-        for (uint64_t first = 0; first < total; first += WITHIN_RANGE) {
-            const uint64_t cnt = std::min(WITHIN_RANGE, total - first);
-            gkd_hits h{a.get(), b.get(), nullptr, d.get(), cnt, 0};
-            engine.check(gkd_all_vs_all_range_within(engine.raw(), (uint32_t)n, first, cnt, maxDist, &h));
-            writeHits(writer, a.get(), b.get(), d.get(), h.n, [&](size_t i) { return seqs[i].getGenomeId(); },
-                      [&](size_t i) { return seqs[i].getGenomeName(); });
-            hits += h.n;
+            writeHits(writer, a.data(), b.data(), d.data(), h.n, src);
+            hits = h.n;
         }
         writer.flush();
         logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(hits) + " within distance " +
                 javaDouble(maxDist) + ".");
-        writeMetrics(metricsFile, "fastaDist", engine.raw(), total, 1);
+        writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);
         return 0;
     }
-    std::vector<double> dist;
-    engine.allVsAll(nullptr, dist);
-    size_t t = writePairs(writer, seqs.size(), dist, [&](size_t i) { return seqs[i].getGenomeId(); },
-                          [&](size_t i) { return seqs[i].getGenomeName(); });
+    std::vector<double> dist(total);
+    src.allVsAll(dist.data());
+    const size_t t = writePairs(writer, dist, src);
     logInfo(std::to_string(t) + " pairs computed in 1 batches.");
-    writeMetrics(metricsFile, "fastaDist", engine.raw(), t, 1);
+    writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), t, src.gpus);
     return 0;
 }
 
