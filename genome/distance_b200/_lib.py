@@ -13,6 +13,7 @@ DNA, PROT, RNA = 0, 1, 2
 STRAND_BOTH, STRAND_CANONICAL = 0, 1
 AMBIG_SKIP, AMBIG_LITERAL = 0, 1
 HASH_JAVA_STRING, HASH_MURMUR3 = 0, 1
+LINK_COMPLETE, LINK_AVERAGE = 1, 2
 ABI_VERSION = 2
 
 
@@ -37,6 +38,11 @@ class GkdHits(C.Structure):
                 ("n", C.c_uint64)]
 
 
+class GkdMerges(C.Structure):
+    _fields_ = [("a", C.c_void_p), ("b", C.c_void_p), ("height", C.c_void_p), ("size", C.c_void_p), ("cap", C.c_uint64),
+                ("n", C.c_uint64)]
+
+
 class GkdNeighbors(C.Structure):
     _fields_ = [("pos", C.c_void_p), ("inter", C.c_void_p), ("dist", C.c_void_p), ("n_found", C.c_void_p)]
 
@@ -48,7 +54,8 @@ class GkdMetrics(C.Structure):
                 ("sort_passes", C.c_uint32), ("intersect_kernel", C.c_uint32), ("keys_unique", C.c_uint64), ("pairs", C.c_uint64),
                 ("intersect_bytes", C.c_uint64), ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64),
                 ("launches", C.c_uint64), ("intersect_launches", C.c_uint64), ("total_pairs", C.c_uint64),
-                ("total_intersect_bytes", C.c_uint64), ("total_intersect_ms", C.c_double), ("reserved", C.c_uint64 * 3)]
+                ("total_intersect_bytes", C.c_uint64), ("total_intersect_ms", C.c_double), ("agglomerate_rounds", C.c_uint64),
+                ("reserved", C.c_uint64 * 2)]
 
 
 # every symbol include/gkd.h declares: name -> (restype, argtypes)
@@ -84,6 +91,7 @@ SYMBOLS = {
     "gkd_group_all_vs_all_nearest": (_i32, [_vp, _u32, _dbl, C.POINTER(GkdNeighbors)]),
     "gkd_group_all_vs_all_clusters": (_i32, [_vp, _dbl, _vp, _pu32]),
     "gkd_group_all_vs_all_linkage": (_i32, [_vp, _dbl, C.POINTER(GkdHits)]),
+    "gkd_group_all_vs_all_agglomerate": (_i32, [_vp, _i32, _dbl, C.POINTER(GkdMerges)]),
     "gkd_build_sets": (_i32, [_vp]),
     "gkd_set_size": (_i32, [_vp, _u32, _pu64, _pu64, _pu64]),
     "gkd_export_set": (_i32, [_vp, _u32, _vp, _u64, _pu64]),
@@ -114,6 +122,8 @@ SYMBOLS = {
     "gkd_query_vs_ref_clusters": (_i32, [_vp, _vp, _u32, _vp, _u32, _dbl, _vp, _vp]),
     "gkd_all_vs_all_linkage": (_i32, [_vp, _u32, _dbl, C.POINTER(GkdHits)]),
     "gkd_query_vs_ref_linkage": (_i32, [_vp, _vp, _u32, _vp, _u32, _dbl, _vp, _vp, C.POINTER(GkdHits)]),
+    "gkd_all_vs_all_agglomerate": (_i32, [_vp, _u32, _i32, _dbl, C.POINTER(GkdMerges)]),
+    "gkd_agglomerate": (_i32, [_vp, _u32, _vp, _i32, _dbl, C.POINTER(GkdMerges)]),
     "gkd_hash_set": (_i32, [_vp, _u32, _u32, _i32, _vp, _pu32]),
     "gkd_sketch_distances": (_i32, [_vp, _u32, _i32, _vp, _vp, _u64, _vp]),
     "gkd_format_double": (_i32, [_dbl, C.c_char_p, C.c_size_t]),

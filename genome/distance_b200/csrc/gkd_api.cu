@@ -1583,6 +1583,161 @@ struct Linkage : Form {
     }
 };
 
+// ---- complete / average linkage ------------------------------------------------------------------------------------
+// S / (N 2^53) rounded to the nearest double, ties to even (S = lo + hi 2^64, N >= 1)
+double agg_round(uint64_t lo, uint64_t hi, uint64_t N) {
+    const unsigned __int128 S = (unsigned __int128)hi << 64 | lo;
+    unsigned __int128 q = S / N, r = S % N;
+    if (q == 0 && r == 0) return 0.0;
+    int e = -53;  // value = (q + r / N) 2^e
+    while (q < ((unsigned __int128)1 << 55)) {  // at least 56 quotient bits: 53 kept, a round bit and two more
+        r <<= 1;
+        q = q << 1 | (r >= N ? 1 : 0);
+        if (r >= N) r -= N;
+        e--;
+    }
+    int bits = 0;
+    for (unsigned __int128 t = q; t; t >>= 1) bits++;
+    const int drop = bits - 53;
+    uint64_t keep = (uint64_t)(q >> drop);
+    const unsigned __int128 rest = q & (((unsigned __int128)1 << drop) - 1), half = (unsigned __int128)1 << (drop - 1);
+    if (rest > half || (rest == half && (r != 0 || (keep & 1)))) keep++;
+    return std::ldexp((double)keep, e + drop);
+}
+
+// One complete- or average-linkage agglomeration on the context's device (gkd_all_vs_all_agglomerate, gkd_agglomerate):
+// start() checks the free memory and sets up the matrix and state of agglomerate.cu in one buffer of the call; the
+// distances are scattered into it (scatter); finish() runs the rounds, reads the merges back and writes them to out in
+// the sequential order.
+struct Agglomeration {
+    const char *fn;
+    uint32_t n;
+    int average;
+    double max_dist;
+    gkd_merges *out;
+    void *buf = nullptr;
+    cudaStream_t stream = nullptr;
+    AggState st{};
+    Agglomeration(const char *fn_, uint32_t n_, int method, double d, gkd_merges *out_)
+        : fn(fn_), n(n_), average(method == GKD_LINK_AVERAGE), max_dist(d), out(out_) {}
+    ~Agglomeration() {
+        if (buf) cudaFreeAsync(buf, stream);
+    }
+    std::array<const void *, 8> outputs() const { return {out->a, out->b, out->height, out->size}; }
+    int start(gkd_ctx *c) {
+        out->n = 0;
+        c->m.agglomerate_rounds = 0;
+        if (n < 2) return GKD_OK;
+        const uint64_t need = agg_state_bytes(n, average);
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        if (need > free_b)
+            return fail(c, GKD_ENOMEM, "%s: %s linkage of %u sets needs %llu bytes of device memory; %llu are free", fn,
+                        average ? "average" : "complete", n, (unsigned long long)need, (unsigned long long)free_b);
+        stream = c->stream;
+        CK(cudaMallocAsync(&buf, need, c->stream));
+        st = agg_state_at(buf, n, average);
+        CK(launch_agg_init(st, c->stream));
+        c->m.launches++;
+        return GKD_OK;
+    }
+    // entries [first, first + count) of the triangle, as doubles in device memory
+    int scatter(gkd_ctx *c, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err) {
+        CK(launch_agg_scatter(st, src, first, count, join_err, c->stream));
+        c->m.launches++;
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) {
+        if (n < 2) return GKD_OK;
+        unsigned long long ctr[AGG_COUNTERS];
+        CK(cudaMemcpyAsync(ctr, st.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += sizeof(ctr);
+        if (ctr[AGG_BAD] != ~0ull) {
+            uint32_t i, j;
+            upper_pair(ctr[AGG_BAD], n, i, j);
+            return fail(c, GKD_EINVAL, "%s: the distance of pair (%u, %u) is not a multiple of 2^-53 in [0, 2]", fn, i, j);
+        }
+        if (max_dist < 0) return GKD_OK;
+        AggThreshold thr{0, 0, max_dist >= 2.0 ? 1 : 0};
+        if (!thr.all) {
+            int e = 0;
+            const double fr = std::frexp(max_dist, &e);  // max_dist = m 2^(e - 53)
+            thr.m = (uint64_t)std::ldexp(fr, 53);
+            thr.shift = e;
+        }
+        // batches of rounds without a host read in between; a batch that ends with AGG_DONE set is the last
+        CK(cudaEventRecord(c->ev[6], c->stream));
+        uint64_t queued = 0;
+        for (uint32_t batch = 8;; batch = std::min<uint32_t>(batch * 2, 512)) {
+            CK(launch_agg_rounds(st, thr, batch, c->n_sms, c->stream));
+            c->m.launches += 4ull * batch;
+            queued += batch;
+            CK(cudaMemcpyAsync(ctr, st.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            c->m.d2h_bytes += sizeof(ctr);
+            if (ctr[AGG_DONE]) break;
+            // every round but the last merges at least one pair
+            if (queued > (uint64_t)n + 1024) return fail(c, GKD_EINVAL, "internal error: %s did not finish in %llu rounds", fn,
+                                                          (unsigned long long)queued);
+        }
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        const uint64_t m = ctr[AGG_N_MERGES];
+        std::vector<AggMerge> ms(m);
+        if (m) CK(cudaMemcpyAsync(ms.data(), st.merges, m * sizeof(AggMerge), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += m * sizeof(AggMerge);
+        c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+        c->m.agglomerate_rounds = ctr[AGG_ROUNDS];
+        // the merge keys strictly increase in the sequential order
+        auto N = [&](const AggMerge &x) -> uint64_t { return average ? (uint64_t)x.sa * x.sb : 1; };
+        std::sort(ms.begin(), ms.end(), [&](const AggMerge &x, const AggMerge &y) {
+            const int k = agg_cmp(x.lo, x.hi, N(x), y.lo, y.hi, N(y));
+            return k < 0 || (k == 0 && (x.a < y.a || (x.a == y.a && x.b < y.b)));
+        });
+        out->n = m;
+        const uint64_t w = std::min<uint64_t>(m, out->cap);
+        if (w == 0) return GKD_OK;
+        std::vector<uint32_t> a(w), b(w), size(w);
+        std::vector<double> h(w);
+        for (uint64_t t = 0; t < w; t++) {
+            const AggMerge &x = ms[t];
+            a[t] = x.a;
+            b[t] = x.b;
+            size[t] = x.sa + x.sb;
+            h[t] = average ? agg_round(x.lo, x.hi, N(x)) : std::ldexp((double)x.lo, -53);
+        }
+        if (out->a) CK(cudaMemcpyAsync(out->a, a.data(), w * 4, cudaMemcpyDefault, c->stream));
+        if (out->b) CK(cudaMemcpyAsync(out->b, b.data(), w * 4, cudaMemcpyDefault, c->stream));
+        if (out->height) CK(cudaMemcpyAsync(out->height, h.data(), w * 8, cudaMemcpyDefault, c->stream));
+        if (out->size) CK(cudaMemcpyAsync(out->size, size.data(), w * 4, cudaMemcpyDefault, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        return GKD_OK;
+    }
+};
+
+// gkd_all_vs_all_agglomerate: each chunk's distances (the dense epilogue's doubles) go straight into the matrix; a chunk
+// whose join overflowed writes nothing and its redo writes the same entries, so the rounds in finish() see final values.
+struct Agglomerate : Form {
+    Agglomeration g;
+    Agglomerate(uint32_t n, int method, double d, gkd_merges *out) : g("gkd_all_vs_all_agglomerate", n, method, d, out) {}
+    std::array<const void *, 8> outputs() const override { return g.outputs(); }
+    int start(gkd_ctx *c) override { return g.start(c); }
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        int rc = ensure(c, c->d_dist, e.cnt * 8);
+        if (rc) return rc;
+        nvtxRangePushA("gkd kernel 5: agglomerate matrix");
+        CK(launch_epilogue(e.src, e.pc, EpilogueOut{nullptr, (double *)c->d_dist.p, nullptr, nullptr}, c->stream));
+        c->m.launches++;
+        rc = g.scatter(c, (const double *)c->d_dist.p, e.src.first, e.cnt, e.join_err);
+        nvtxRangePop();
+        if (rc) return rc;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) override { return g.finish(c); }
+};
+
 // the triangle over the first n sets, and the block of queries q x references r
 HostPairs triangle(uint32_t n) { return {PAIRS_UPPER, n, 0, (uint64_t)n * (n - 1) / 2, nullptr, nullptr, 0, 0}; }
 HostPairs block(const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr) {
@@ -2428,6 +2583,51 @@ int gkd_query_vs_ref_linkage(gkd_ctx *c, const uint32_t *q, uint32_t nq, const u
     if (rc) return rc;
     Linkage f(max_dist, nq + nr, nq, std::move(key), out);
     return run_call(c, "gkd_query_vs_ref_linkage", block(q, nq, r, nr), f);
+}
+
+// ---- complete / average linkage -------------------------------------------------------------------------------
+static int agglomerate_args_ok(gkd_ctx *c, const char *fn, int method, double max_dist, const gkd_merges *out) {
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "%s: max_dist is NaN", fn);
+    if (method != GKD_LINK_COMPLETE && method != GKD_LINK_AVERAGE) return fail(c, GKD_EINVAL, "%s: unknown method %d", fn, method);
+    if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
+    return GKD_OK;
+}
+
+int gkd_all_vs_all_agglomerate(gkd_ctx *c, uint32_t n, int method, double max_dist, gkd_merges *out) {
+    const int rc = agglomerate_args_ok(c, "gkd_all_vs_all_agglomerate", method, max_dist, out);
+    if (rc) return rc;
+    Agglomerate f(n, method, max_dist, out);
+    return run_call(c, "gkd_all_vs_all_agglomerate", triangle(n), f);
+}
+
+int gkd_agglomerate(gkd_ctx *c, uint32_t n, const double *dist, int method, double max_dist, gkd_merges *out) {
+    const char *fn = "gkd_agglomerate";
+    int rc = agglomerate_args_ok(c, fn, method, max_dist, out);
+    if (rc) return rc;
+    if (!dist && n >= 2) return fail(c, GKD_EINVAL, "%s: null dist", fn);
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    Agglomeration g(fn, n, method, max_dist, out);
+    if ((rc = host_outputs_ok(c, fn, g.outputs()))) return rc;
+    c->m.pairs = c->m.intersect_bytes = 0;
+    c->m.intersect_ms = c->m.epilogue_ms = 0;
+    ABI_GUARD_BEGIN
+    if ((rc = g.start(c))) return rc;
+    const uint64_t total = (uint64_t)n * (n - (n > 0)) / 2;
+    const bool on_device = total && classify(dist) == MEM_DEVICE;
+    for (uint64_t first = 0; first < total; first += PAIR_CHUNK) {
+        const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, total - first);
+        const double *src = dist + first;
+        if (!on_device) {  // staged through the scatter's source buffer, in stream order
+            if ((rc = ensure(c, c->d_dist, cnt * 8))) return rc;
+            CK(cudaMemcpyAsync(c->d_dist.p, src, cnt * 8, cudaMemcpyHostToDevice, c->stream));
+            c->m.h2d_bytes += cnt * 8;
+            src = (const double *)c->d_dist.p;
+        }
+        if ((rc = g.scatter(c, src, first, cnt, nullptr))) return rc;
+    }
+    return g.finish(c);
+    ABI_GUARD_END(c)
 }
 
 // ---- MinHash sketches ---------------------------------------------------------------------------------------

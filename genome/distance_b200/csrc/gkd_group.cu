@@ -831,4 +831,25 @@ int gkd_group_all_vs_all_linkage(gkd_group *g, double max_dist, gkd_hits *out) {
     }
 }
 
+int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, gkd_merges *out) {
+    if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_agglomerate: max_dist is NaN");
+    if (method != GKD_LINK_COMPLETE && method != GKD_LINK_AVERAGE)
+        return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_agglomerate: unknown method %d", method);
+    if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_agglomerate: null out");
+    if (!g) return GKD_EINVAL;
+    try {
+        out->n = 0;
+        const uint64_t N = g->n_genomes;
+        std::vector<double> dist(N * (N - (N > 0)) / 2);
+        int rc = gkd_group_all_vs_all(g, nullptr, dist.data());
+        if (rc != GKD_OK) return rc;
+        gkd_ctx *c0 = g->members[0].ctx;
+        if ((rc = gkd_agglomerate(c0, g->n_genomes, dist.data(), method, max_dist, out)) != GKD_OK)
+            return gfail(g, rc, "member 0: %s", gkd_last_error(c0));
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_agglomerate: %s", ex.what());
+    }
+}
+
 }  // extern "C"

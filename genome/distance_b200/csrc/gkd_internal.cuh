@@ -415,6 +415,59 @@ inline void host_msf(std::vector<LinkEdge> &edges, uint32_t nodes) {
     }
     edges.resize(kept);
 }
+// Complete / average linkage (agglomerate.cu): reciprocal-nearest-neighbour rounds over an n x n matrix in HBM.  Slot
+// x holds the cluster labelled x while it is active (size[x] != 0).  Entry (x, y) is one word lo (complete: the max of
+// d 2^53) or two words lo, hi (average: S = sum of d 2^53 as a 128-bit integer), stored at [x n + y] and [y n + x].  A
+// cluster distance is the exact rational S / (N 2^53) with N = 1 (complete) or |A| |B| (average); pairs are ordered by
+// the strict key (S / N, smaller slot, larger slot).
+struct AggMerge {  // one merge as the device appends it (unordered): slots a < b, their sizes, S of the pair
+    uint32_t a, b, sa, sb;
+    uint64_t lo, hi;
+};
+enum AggCounter : uint32_t { AGG_N_STALE = 0, AGG_N_SURV, AGG_N_MERGES, AGG_ROUND_MERGES, AGG_DONE, AGG_ROUNDS, AGG_BAD, AGG_COUNTERS };
+constexpr uint32_t AGG_NONE = 0xFFFFFFFFu;
+struct AggState {
+    uint32_t n;
+    int average;
+    uint64_t *lo, *hi;              // the matrix (hi: average only)
+    uint32_t *size, *nn, *mate;     // per slot: cluster size (0 = inactive), nearest active slot, merge partner this round
+    uint64_t *nn_lo, *nn_hi;        // per slot: S of the nearest pair (N follows from the sizes)
+    uint32_t *stale, *surv;         // rows to rescan; survivors (smaller slot of a merge) of this round
+    unsigned long long *ctr;        // AggCounter; AGG_BAD: the smallest pair index of an invalid input value (~0: none)
+    AggMerge *merges;               // <= n - 1
+};
+struct AggThreshold {  // v <= max_dist  <=>  S <= (m N) << shift (shift < 0: >> -shift); all: every value passes
+    uint64_t m;
+    int shift;
+    int all;
+};
+uint64_t agg_state_bytes(uint32_t n, int average);  // the matrix and the O(n) state, in one buffer
+AggState agg_state_at(void *base, uint32_t n, int average);
+cudaError_t launch_agg_init(const AggState &st, cudaStream_t s);
+// entries [first, first + count) of the row-major strict upper triangle of n, as doubles in src (device), into the
+// matrix; an entry that is not a multiple of 2^-53 in [0, 2] is recorded in AGG_BAD.  Nothing when join_err (may be
+// nullptr) reads nonzero on the stream: the chunk is redone.
+cudaError_t launch_agg_scatter(const AggState &st, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err,
+                               cudaStream_t s);
+// `rounds` rounds queued without a host read; a round after one that merged nothing exits at once (AGG_DONE)
+cudaError_t launch_agg_rounds(const AggState &st, AggThreshold thr, uint32_t rounds, int n_sms, cudaStream_t s);
+// S1 / N1 < S2 / N2 exactly (S 128-bit as lo, hi; 192-bit cross products)
+__host__ __device__ inline int agg_cmp(uint64_t lo1, uint64_t hi1, uint64_t n1, uint64_t lo2, uint64_t hi2, uint64_t n2) {
+    // (lo + hi 2^64) * n as three words w0 + w1 2^64 + w2 2^128
+    auto mul = [](uint64_t lo, uint64_t hi, uint64_t n, uint64_t &w0, uint64_t &w1, uint64_t &w2) {
+        const unsigned __int128 p0 = (unsigned __int128)lo * n, p1 = (unsigned __int128)hi * n + (uint64_t)(p0 >> 64);
+        w0 = (uint64_t)p0;
+        w1 = (uint64_t)p1;
+        w2 = (uint64_t)(p1 >> 64);
+    };
+    uint64_t a0, a1, a2, b0, b1, b2;
+    mul(lo1, hi1, n2, a0, a1, a2);
+    mul(lo2, hi2, n1, b0, b1, b2);
+    if (a2 != b2) return a2 < b2 ? -1 : 1;
+    if (a1 != b1) return a1 < b1 ? -1 : 1;
+    if (a0 != b0) return a0 < b0 ? -1 : 1;
+    return 0;
+}
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless
 // some representative is within max_dist; clears the counts it consumed
 cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *n_reps, uint32_t cand, uint32_t visit,

@@ -141,6 +141,9 @@ const std::vector<OptSpec> FASTA_OPTS = {
                             "record (additive option; needs --maxDist)"},
     {{"--linkage"}, false, "report the single-linkage hierarchy up to --maxDist (default 1.0, the whole tree): one line "
                            "per merge of single-linkage agglomeration, in merge order (additive option)"},
+    {{"--method"}, true, "linkage method of --linkage and --clusters: single (default), complete or average (UPGMA); a "
+                         "complete or average merge line holds the two clusters' first records and the merge height "
+                         "(additive option)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
@@ -200,6 +203,10 @@ struct DistSource {
     }
     void linkage(double maxDist, gkd_hits &h) const {
         check(engine ? gkd_all_vs_all_linkage(engine->raw(), n, maxDist, &h) : gkd_group_all_vs_all_linkage(grp, maxDist, &h));
+    }
+    void agglomerate(int method, double maxDist, gkd_merges &m) const {
+        check(engine ? gkd_all_vs_all_agglomerate(engine->raw(), n, method, maxDist, &m)
+                     : gkd_group_all_vs_all_agglomerate(grp, method, maxDist, &m));
     }
 };
 
@@ -319,6 +326,15 @@ int fastaDist(const std::vector<std::string> &args) {
     const bool linkage = p.values.count("--linkage") > 0;
     if (linkage && nearest) throw ParseFailureException("--linkage and --nearest cannot be combined.");
     if (linkage && clusters) throw ParseFailureException("--linkage and --clusters cannot be combined.");
+    // 0 = single linkage (gkd_*_linkage / gkd_*_clusters), else a gkd_link_method
+    int method = 0;
+    if (p.values.count("--method")) {
+        const std::string &m = p.values["--method"];
+        if (m == "complete") method = GKD_LINK_COMPLETE;
+        else if (m == "average") method = GKD_LINK_AVERAGE;
+        else if (m != "single") throw ParseFailureException("Linkage method must be single, complete or average.");
+        if (!linkage && !clusters) throw ParseFailureException("--method needs --linkage or --clusters.");
+    }
     const char *typeName = seqType == KmerType::DNA ? "DNA" : (seqType == KmerType::RNA ? "RNA" : "PROT");
     if (inFile.empty()) logInfo(std::string("Reading ") + typeName + " sequences from the standard input.");
     else if (!readable(inFile)) throw IOException("Input file " + inFile + " is not found or unreadable.");
@@ -360,6 +376,35 @@ int fastaDist(const std::vector<std::string> &args) {
     logInfo(std::to_string(src.n) + " sequences cached" + (src.grp ? " on " + std::to_string(src.gpus) + " GPUs" : "") +
             ". Computing distances.");
     const uint64_t n = src.n, total = n < 2 ? 0 : n * (n - 1) / 2;
+    if (method && (clusters || linkage)) {
+        // each pair i < j is intersected once; the agglomeration runs on the GPU and only its merges (<= n - 1) leave it
+        const uint64_t cap = n ? n - 1 : 0;
+        std::vector<uint32_t> a(cap), b(cap), size(cap);
+        std::vector<double> d(cap);
+        gkd_merges m{a.data(), b.data(), d.data(), size.data(), cap, 0};
+        src.agglomerate(method, maxDist, m);
+        if (linkage) {
+            writeHits(writer, a.data(), b.data(), d.data(), m.n, src);
+            writer.flush();
+            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(m.n) + " merges up to distance " +
+                    javaDouble(maxDist) + ".");
+        } else {
+            // the clusters at maxDist are the components of the merges; each is labelled by its first record
+            std::vector<uint32_t> label(n);
+            for (uint32_t i = 0; i < n; i++) label[i] = i;
+            auto find = [&](uint32_t x) {
+                while (label[x] != x) x = label[x];
+                return x;
+            };
+            for (uint64_t t = 0; t < m.n; t++) label[find(b[t])] = find(a[t]);  // a < b are both roots' labels
+            for (uint32_t i = 0; i < n; i++) label[i] = find(i);
+            const uint32_t found = writeClusters(writer, label.data(), src);
+            logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(found) + " clusters at distance " +
+                    javaDouble(maxDist) + ".");
+        }
+        writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);
+        return 0;
+    }
     if (clusters) {
         // each pair i < j is intersected once and linked on the GPU; only the n labels leave it
         std::vector<uint32_t> label(n);

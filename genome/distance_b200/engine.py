@@ -9,7 +9,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (AMBIG_LITERAL, AMBIG_SKIP, DNA, PROT, RNA, STRAND_BOTH, STRAND_CANONICAL, GkdConfig, GkdHits,
-                   GkdMetrics, GkdNeighbors, GkdOutputs, GkdPackedSet)
+                   GkdMerges, GkdMetrics, GkdNeighbors, GkdOutputs, GkdPackedSet)
 
 PACKED_DTYPE = np.dtype([("offs_off", "<u8"), ("lows_off", "<u8"), ("pal_offs_off", "<u8"), ("pal_lows_off", "<u8"),
                          ("n", "<u4"), ("n_pal", "<u4"), ("level", "<u4"), ("pal_level", "<u4")])
@@ -43,6 +43,16 @@ def _neighbors(rows: int, k: int):
     pos, inter = np.empty((rows, k), dtype=np.uint32), np.empty((rows, k), dtype=np.uint64)
     dist, found = np.empty((rows, k), dtype=np.float64), np.empty(rows, dtype=np.uint32)
     return (pos, inter, dist, found), GkdNeighbors(pos.ctypes.data, inter.ctypes.data, dist.ctypes.data, found.ctypes.data)
+
+
+def _merges(call, n: int):
+    """(a, b, height, size) numpy arrays of a gkd_merges call `call(merges)`; n - 1 entries always suffice"""
+    cap = max(int(n) - 1, 0)
+    a, b = np.empty(cap, dtype=np.uint32), np.empty(cap, dtype=np.uint32)
+    height, size = np.empty(cap, dtype=np.float64), np.empty(cap, dtype=np.uint32)
+    m = GkdMerges(a.ctypes.data, b.ctypes.data, height.ctypes.data, size.ctypes.data, cap, 0)
+    call(m)
+    return a[:m.n], b[:m.n], height[:m.n], size[:m.n]
 
 
 class GkdError(RuntimeError):
@@ -375,6 +385,36 @@ class Engine:
             self._h, qa.ctypes.data, qa.size, ra.ctypes.data, ra.size, float(max_dist),
             None if qk is None else qk.ctypes.data, None if rk is None else rk.ctypes.data, C.byref(h))), nodes, nodes)
 
+    def all_vs_all_agglomerate(self, method: int, max_dist: float, n: int = None):
+        """(a, b, height, size): the complete- (LINK_COMPLETE) or average-linkage (LINK_AVERAGE) hierarchy of the first
+        n sets (default: all) up to max_dist, one entry per merge in the order of the sequential agglomeration; a < b
+        are the smallest ids of the two clusters and size the size of the merged cluster.  Every pair is intersected
+        once and its distance stays on the device"""
+        n = len(self) if n is None else int(n)
+        return _merges(lambda m: self._ck(self._L.gkd_all_vs_all_agglomerate(self._h, n, int(method), float(max_dist),
+                                                                             C.byref(m))), n)
+
+    def agglomerate(self, dist, method: int, max_dist: float):
+        """all_vs_all_agglomerate over a caller's row-major strict upper triangle of distances (a float64 numpy array
+        or CUDA tensor of n(n-1)/2 entries, read and not modified), on this context's device"""
+        m = int(dist.numel() if _is_torch(dist) else np.asarray(dist).size)
+        n = int(round((1 + (1 + 8 * m) ** 0.5) / 2)) if m else 0
+        if n * (n - 1) // 2 != m:
+            raise ValueError(f"{m} distances are not a strict upper triangle")
+        if _is_torch(dist):
+            import torch
+
+            if dist.dtype != torch.float64 or not dist.is_contiguous():
+                raise ValueError("dist must be a contiguous float64 tensor")
+            ptr, keep = dist.data_ptr(), dist
+        else:
+            keep = np.ascontiguousarray(dist, dtype=np.float64)
+            ptr = keep.ctypes.data
+        out = _merges(lambda mg: self._ck(self._L.gkd_agglomerate(self._h, n, ptr, int(method), float(max_dist),
+                                                                 C.byref(mg))), n)
+        del keep
+        return out
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -562,3 +602,8 @@ class Group:
         """(a, b, inter, dist) over all global ids: the single-context Engine.all_vs_all_linkage result"""
         n = max(len(self) - 1, 0)
         return _select(lambda h: self._ck(self._L.gkd_group_all_vs_all_linkage(self._h, float(max_dist), C.byref(h))), n, n)
+
+    def all_vs_all_agglomerate(self, method: int, max_dist: float):
+        """(a, b, height, size) over all global ids: the single-context Engine.all_vs_all_agglomerate result"""
+        return _merges(lambda m: self._ck(self._L.gkd_group_all_vs_all_agglomerate(self._h, int(method), float(max_dist),
+                                                                                   C.byref(m))), len(self))

@@ -100,7 +100,8 @@ typedef struct gkd_metrics {
     uint64_t total_pairs;            /* the three "last distance call" figures summed since gkd_create / gkd_reset */
     uint64_t total_intersect_bytes;
     double total_intersect_ms;
-    uint64_t reserved[3];
+    uint64_t agglomerate_rounds;  /* rounds that merged something in the last gkd_*_agglomerate call */
+    uint64_t reserved[2];
 } gkd_metrics;
 
 /* ---- lifecycle --------------------------------------------------------------------------- */
@@ -301,6 +302,34 @@ int gkd_all_vs_all_linkage(gkd_ctx *ctx, uint32_t n, double max_dist, gkd_hits *
 int gkd_query_vs_ref_linkage(gkd_ctx *ctx, const uint32_t *q, uint32_t nq, const uint32_t *r, uint32_t nr,
                              double max_dist, const uint32_t *q_key, const uint32_t *r_key, gkd_hits *out);
 
+/* Complete- and average-linkage (UPGMA) hierarchies of the first n sets up to max_dist.  d(x, y) is the dense call's
+ * double; a cluster's label is its smallest id.  Cluster distance v(A, B): complete = max d(a, b); average =
+ * S(A, B) / (|A| |B|) with S = the sum of d(a, b) 2^53 as an exact integer (every distance of kernel 5 is a multiple of
+ * 2^-53 in [0, 2]; a value that is not fails the call with GKD_EINVAL).  The result is the sequential agglomeration that
+ * repeatedly merges the pair of current clusters with the smallest strict key (v, min label, max label) while
+ * v <= max_dist: one entry per merge, in that order, with a < b the two labels, height = v (average: v rounded to the
+ * nearest double, ties to even) and size = |A| + |B|.  out->n = n - (clusters at max_dist); only the first min(n, cap)
+ * entries are written, so cap = n - 1 always suffices.  For every t <= max_dist the clusters at t are the components of
+ * the merges with v <= t.  Any array may be NULL; host or device memory as for gkd_hits.  A negative max_dist gives no
+ * merges.  Single linkage is gkd_all_vs_all_linkage.
+ * Device memory: an n x n matrix of 8 B (complete) or 16 B (average) entries, and O(n) state; the call fails with
+ * GKD_ENOMEM, naming the bytes, when that exceeds the free device memory.  Only the merges (32 B each) leave the
+ * device. */
+typedef enum gkd_link_method { GKD_LINK_COMPLETE = 1, GKD_LINK_AVERAGE = 2 } gkd_link_method;
+typedef struct gkd_merges {
+    uint32_t *a, *b;  /* labels of the two clusters, a < b */
+    double *height;
+    uint32_t *size;   /* |A| + |B| */
+    uint64_t cap;     /* entries each non-NULL array can hold */
+    uint64_t n;       /* out: number of merges; only the first min(n, cap) are written */
+} gkd_merges;
+/* Every pair i < j is intersected once and its distance written straight into the matrix on the device. */
+int gkd_all_vs_all_agglomerate(gkd_ctx *ctx, uint32_t n, int method, double max_dist, gkd_merges *out);
+/* The same agglomeration over a caller's row-major strict upper triangle of n(n-1)/2 distances (host or device memory;
+ * read, not modified), on the context's device.  n is not tied to the context's sets.  One gkd_all_vs_all serves
+ * several methods or thresholds this way. */
+int gkd_agglomerate(gkd_ctx *ctx, uint32_t n, const double *dist, int method, double max_dist, gkd_merges *out);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -342,6 +371,10 @@ int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label
  * forest of its diagonal block and of each ring call (keyed by global id) on its own device; the host merges them by
  * Kruskal in the order (distance bits, global a, global b).  The arrays of out are host memory. */
 int gkd_group_all_vs_all_linkage(gkd_group *g, double max_dist, gkd_hits *out);
+/* gkd_all_vs_all_agglomerate over all global ids; equal to one context's merges, bit for bit.  The members fill a host
+ * triangle of all N(N-1)/2 distances as gkd_group_all_vs_all does (8 B per pair of host memory), then member 0 runs
+ * gkd_agglomerate on it (its device needs the matrix of gkd_agglomerate).  The arrays of out are host memory. */
+int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, gkd_merges *out);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

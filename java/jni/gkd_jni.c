@@ -272,3 +272,31 @@ JNIEXPORT jint JNICALL FN(allVsAllLinkage)(JNIEnv *env, jclass c, jlong h, jint 
     }
     return rc;
 }
+
+/* the complete- (method 1) or average-linkage (method 2) hierarchy of the first n sets up to maxDist: a, b, height, size
+ * hold n - 1 entries (the merges in order); nMerges[0] receives their number */
+JNIEXPORT jint JNICALL FN(allVsAllAgglomerate)(JNIEnv *env, jclass c, jlong h, jint n, jint method, jdouble maxDist,
+                                               jintArray a, jintArray b, jdoubleArray height, jintArray size,
+                                               jintArray nMerges) {
+    (void)c;
+    if (!a || !b || !height || !size || !nMerges || n < 0 || (*env)->GetArrayLength(env, nMerges) < 1) return GKD_EINVAL;
+    const jint cap = n > 0 ? n - 1 : 0;
+    if ((*env)->GetArrayLength(env, a) < cap || (*env)->GetArrayLength(env, b) < cap ||
+        (*env)->GetArrayLength(env, height) < cap || (*env)->GetArrayLength(env, size) < cap)
+        return GKD_EINVAL;
+    jint *pa = (*env)->GetIntArrayElements(env, a, NULL);
+    jint *pb = (*env)->GetIntArrayElements(env, b, NULL);
+    jdouble *ph = (*env)->GetDoubleArrayElements(env, height, NULL);
+    jint *ps = (*env)->GetIntArrayElements(env, size, NULL);
+    gkd_merges out = {(uint32_t *)pa, (uint32_t *)pb, ph, (uint32_t *)ps, (uint64_t)cap, 0};
+    int rc = (pa && pb && ph && ps) ? gkd_all_vs_all_agglomerate(CTX(h), (uint32_t)n, method, maxDist, &out) : GKD_ENOMEM;
+    if (ps) (*env)->ReleaseIntArrayElements(env, size, ps, 0);
+    if (ph) (*env)->ReleaseDoubleArrayElements(env, height, ph, 0);
+    if (pb) (*env)->ReleaseIntArrayElements(env, b, pb, 0);
+    if (pa) (*env)->ReleaseIntArrayElements(env, a, pa, 0);
+    if (rc == GKD_OK) {
+        jint nm = (jint)out.n;
+        (*env)->SetIntArrayRegion(env, nMerges, 0, 1, &nm);
+    }
+    return rc;
+}

@@ -53,6 +53,11 @@ final class GkdNative {
     /** the single-linkage hierarchy of the first n sets up to maxDist: the minimum spanning forest of the pairs within
      *  maxDist in merge order; a, b, dist (length n - 1) receive its edges (a &lt; b), nEdges[0] their number */
     static native int allVsAllLinkage(long ctx, int n, double maxDist, int[] a, int[] b, double[] dist, int[] nEdges);
+    /** the complete- (method 1) or average-linkage (method 2, UPGMA) hierarchy of the first n sets up to maxDist: a, b,
+     *  height, size (length n - 1) receive the merges in order (a &lt; b the clusters' smallest ids, size the merged
+     *  cluster's), nMerges[0] their number */
+    static native int allVsAllAgglomerate(long ctx, int n, int method, double maxDist, int[] a, int[] b, double[] height,
+                                          int[] size, int[] nMerges);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

@@ -207,6 +207,21 @@ public class GpuKmerEngine implements AutoCloseable {
         return merges[0];
     }
 
+    /** linkage methods of allVsAllAgglomerate (gkd_link_method) */
+    public static final int LINK_COMPLETE = 1, LINK_AVERAGE = 2;
+
+    /** the complete- (LINK_COMPLETE) or average-linkage (LINK_AVERAGE, UPGMA) hierarchy of every set up to maxDist
+     *  (1.0: the whole tree): the merges of the sequential agglomeration in order.  a, b, height and size (at least
+     *  size() - 1 entries) receive the two clusters' smallest ids (a &lt; b), the cluster distance (average: rounded to
+     *  the nearest double) and the merged cluster's size; returns the number of merges, size() minus the clusters at
+     *  maxDist.  Every pair is intersected once; the distances stay on the GPU and only the merges leave it. */
+    public synchronized int allVsAllAgglomerate(int method, double maxDist, int[] a, int[] b, double[] height, int[] size) {
+        this.build();
+        int[] merges = new int[1];
+        check(GkdNative.allVsAllAgglomerate(this.ctx, this.size(), method, maxDist, a, b, height, size, merges));
+        return merges[0];
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
