@@ -16,6 +16,10 @@
 // The host queues rounds in batches without reading anything between them.
 #include <cuda_runtime.h>
 
+#include <cstdlib>
+
+#include <cub/device/device_radix_sort.cuh>
+
 #include "gkd_internal.cuh"
 
 namespace gkd {
@@ -49,6 +53,30 @@ __device__ __forceinline__ bool agg_before(const Best &x, const Best &y) {
 __device__ __forceinline__ Best shfl_best(const Best &b, int off) {
     return Best{__shfl_down_sync(0xffffffffu, b.lo, off), __shfl_down_sync(0xffffffffu, b.hi, off),
                 __shfl_down_sync(0xffffffffu, b.N, off), __shfl_down_sync(0xffffffffu, b.k, off)};
+}
+
+// the CTA's best candidate of row i (b: this thread's) to nn[i], nn_lo[i], nn_hi[i]; part: AGG_THREADS / 32 entries of
+// shared memory, free again on return
+__device__ __forceinline__ void row_best(const AggState &st, uint32_t i, Best b, Best *part, uint32_t lane, uint32_t warp) {
+    for (int off = 16; off; off >>= 1) {
+        const Best o = shfl_best(b, off);
+        if (agg_before(o, b)) b = o;
+    }
+    if (lane == 0) part[warp] = b;
+    __syncthreads();
+    if (warp == 0) {
+        b = lane < AGG_THREADS / 32 ? part[lane] : Best{0, 0, 1, AGG_NONE};
+        for (int off = 16; off; off >>= 1) {
+            const Best o = shfl_best(b, off);
+            if (agg_before(o, b)) b = o;
+        }
+        if (lane == 0) {
+            st.nn[i] = b.k;
+            st.nn_lo[i] = b.lo;
+            st.nn_hi[i] = b.hi;
+        }
+    }
+    __syncthreads();  // part[] is reused by the next row
 }
 
 __global__ void __launch_bounds__(AGG_THREADS) k_agg_init(AggState st) {
@@ -100,25 +128,7 @@ __global__ void __launch_bounds__(AGG_THREADS) k_agg_scan(AggState st) {
             const Best c{st.lo[row + k], st.average ? st.hi[row + k] : 0, st.average ? si * sk : 1, k};
             if (agg_before(c, b)) b = c;
         }
-        for (int off = 16; off; off >>= 1) {
-            const Best o = shfl_best(b, off);
-            if (agg_before(o, b)) b = o;
-        }
-        if (lane == 0) part[warp] = b;
-        __syncthreads();
-        if (warp == 0) {
-            b = lane < AGG_THREADS / 32 ? part[lane] : Best{0, 0, 1, AGG_NONE};
-            for (int off = 16; off; off >>= 1) {
-                const Best o = shfl_best(b, off);
-                if (agg_before(o, b)) b = o;
-            }
-            if (lane == 0) {
-                st.nn[i] = b.k;
-                st.nn_lo[i] = b.lo;
-                st.nn_hi[i] = b.hi;
-            }
-        }
-        __syncthreads();  // part[] is reused by the next row
+        row_best(st, i, b, part, lane, warp);
     }
 }
 
@@ -200,21 +210,173 @@ __global__ void __launch_bounds__(AGG_THREADS) k_agg_finalize(AggState st) {
         st.stale[atomicAdd(st.ctr + AGG_N_STALE, 1ull)] = x;
 }
 
-}  // namespace
+// ---- complete linkage from the pairs within max_dist (CsRows) ----------------------------------------------------
+// The rounds above with the matrix replaced by one sorted row per slot.  A pair beyond max_dist is +inf, and so is a
+// tombstone; complete linkage is a max, so the merges up to max_dist are the same.  The update keeps the dense rule
+// that a CTA reads only its own row, its partner's row and the neighbour words of other rows (never written), and that
+// no two CTAs write one word.
 
-uint64_t agg_state_bytes(uint32_t n, int average) {
-    const uint64_t N = n;
-    return N * N * 8 * (average ? 2 : 1) + N * (5 * 4 + 2 * 8) + N * sizeof(AggMerge) + AGG_COUNTERS * 8 + 256;
+__global__ void __launch_bounds__(AGG_THREADS) k_cs_append(const uint32_t *__restrict__ a, const uint32_t *__restrict__ b,
+                                                           const double *__restrict__ dist, uint64_t count, uint32_t n,
+                                                           CsList dst, uint64_t at, unsigned long long *bad) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count) return;
+    const uint32_t x = a[t], y = b[t];
+    const double d = dist[t];
+    const double w = d * 9007199254740992.0;  // d 2^53, exact
+    dst.a[at + t] = min(x, y);
+    dst.b[at + t] = max(x, y);
+    if (x >= n || y >= n || x == y || !(d >= 0.0 && d <= 2.0 && w == floor(w))) {
+        dst.w[at + t] = CS_TOMB;
+        atomicMin(bad, (unsigned long long)(at + t));
+        return;
+    }
+    dst.w[at + t] = (uint64_t)w;
 }
 
+// both directions of every pair: key row << 32 | neighbour, value w
+__global__ void __launch_bounds__(AGG_THREADS) k_cs_directed(CsList l, uint64_t count, uint64_t *__restrict__ keys,
+                                                             uint64_t *__restrict__ vals) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count) return;
+    const uint64_t a = l.a[t], b = l.b[t], w = l.w[t];
+    keys[2 * t] = a << 32 | b;
+    keys[2 * t + 1] = b << 32 | a;
+    vals[2 * t] = vals[2 * t + 1] = w;
+}
+
+// off[r] = the first sorted key of row r (r <= n); nbr = the low words; the smallest repeated key to *dup
+__global__ void __launch_bounds__(AGG_THREADS) k_cs_rows(const uint64_t *__restrict__ keys, uint64_t items, uint32_t n,
+                                                         uint64_t *off, uint32_t *nbr, unsigned long long *dup) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t <= n) {
+        const uint64_t want = t << 32;
+        uint64_t lo = 0, hi = items;
+        while (lo < hi) {
+            const uint64_t mid = (lo + hi) >> 1;
+            if (keys[mid] < want) lo = mid + 1;
+            else hi = mid;
+        }
+        off[t] = lo;
+    }
+    if (t < items) {
+        nbr[t] = (uint32_t)keys[t];
+        if (t && keys[t] == keys[t - 1]) atomicMin(dup, (unsigned long long)keys[t]);
+    }
+}
+
+constexpr uint64_t CS_NOWHERE = ~0ull;
+
+// position of neighbour k in row x, or CS_NOWHERE
+__device__ __forceinline__ uint64_t cs_find(const CsRows &r, uint32_t x, uint32_t k) {
+    uint64_t lo = r.off[x], hi = r.off[x + 1];
+    while (lo < hi) {
+        const uint64_t mid = (lo + hi) >> 1;
+        if (r.nbr[mid] < k) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo < r.off[x + 1] && r.nbr[lo] == k ? lo : CS_NOWHERE;
+}
+
+// e(x, k), CS_TOMB when the pair is absent
+__device__ __forceinline__ uint64_t cs_word(const CsRows &r, uint32_t x, uint32_t k) {
+    const uint64_t p = cs_find(r, x, k);
+    return p == CS_NOWHERE ? CS_TOMB : r.w[p];
+}
+
+__global__ void __launch_bounds__(AGG_THREADS) k_cs_scan(AggState st, CsRows r) {
+    if (st.ctr[AGG_DONE]) return;
+    __shared__ Best part[AGG_THREADS / 32];
+    const uint32_t n_stale = (uint32_t)st.ctr[AGG_N_STALE];
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (uint32_t s = blockIdx.x; s < n_stale; s += gridDim.x) {
+        const uint32_t i = st.stale[s];
+        Best b{0, 0, 1, AGG_NONE};
+        for (uint64_t e = r.off[i] + threadIdx.x; e < r.off[i + 1]; e += AGG_THREADS) {
+            const uint64_t w = r.w[e];
+            if (w == CS_TOMB) continue;
+            const uint32_t k = r.nbr[e];
+            if (!st.size[k]) continue;  // a partner of an earlier round whose entry in this row was left as it was
+            const Best c{w, 0, 1, k};
+            if (agg_before(c, b)) b = c;
+        }
+        row_best(st, i, b, part, lane, warp);
+    }
+}
+
+// One CTA per survivor i with partner j.  Row i's entries: j and the other partners go; another survivor k (partner
+// k') gets the max of e(i, k), e(j, k), e(i, k'), e(j, k'), or a tombstone when one is absent (its own CTA writes the
+// same into row k); a slot k that does not merge gets max(e(i, k), e(j, k)) in row i and in row k, where e(k, j)
+// becomes a tombstone.  A slot that does not merge and is a neighbour of j only loses e(k, j).  The partners' own rows
+// are never read again.
+__global__ void __launch_bounds__(AGG_THREADS) k_cs_update(AggState st, CsRows r) {
+    if (st.ctr[AGG_DONE]) return;
+    const uint32_t n_surv = (uint32_t)st.ctr[AGG_N_SURV];
+    for (uint32_t s = blockIdx.x; s < n_surv; s += gridDim.x) {
+        const uint32_t i = st.surv[s], j = st.mate[i];
+        for (uint64_t e = r.off[j] + threadIdx.x; e < r.off[j + 1]; e += AGG_THREADS) {
+            if (r.w[e] == CS_TOMB) continue;
+            const uint32_t k = r.nbr[e];
+            if (k == i || st.mate[k] != AGG_NONE || !st.size[k]) continue;
+            if (cs_word(r, i, k) == CS_TOMB) r.w[cs_find(r, k, j)] = CS_TOMB;
+        }
+        __syncthreads();  // row i is read above and written below
+        for (uint64_t e = r.off[i] + threadIdx.x; e < r.off[i + 1]; e += AGG_THREADS) {
+            uint64_t v = r.w[e];
+            if (v == CS_TOMB) continue;
+            const uint32_t k = r.nbr[e];
+            if (k == j) {
+                r.w[e] = CS_TOMB;
+                continue;
+            }
+            const uint32_t mk = st.mate[k];
+            if (mk != AGG_NONE) {
+                if (mk < k) continue;  // a partner: the scan skips it by its size from now on, and no thread writes it
+                // CS_TOMB is the largest word, so an absent entry makes the max a tombstone
+                v = max(max(v, cs_word(r, j, k)), max(cs_word(r, i, mk), cs_word(r, j, mk)));
+                r.w[e] = v;
+                continue;
+            }
+            if (!st.size[k]) continue;
+            v = max(v, cs_word(r, j, k));
+            r.w[e] = v;
+            r.w[cs_find(r, k, i)] = v;
+            const uint64_t p = cs_find(r, k, j);
+            if (p != CS_NOWHERE) r.w[p] = CS_TOMB;
+        }
+        // other CTAs test the sizes of merging slots only after their mate, and the outcome is the same before and after
+        if (threadIdx.x == 0) {
+            st.size[i] += st.size[j];
+            st.size[j] = 0;
+        }
+        __syncthreads();
+    }
+}
+
+}  // namespace
+
+uint64_t agg_nodes_bytes(uint32_t n) {
+    const uint64_t N = n;
+    return N * (5 * 4 + 2 * 8) + N * sizeof(AggMerge) + AGG_COUNTERS * 8 + 256;
+}
+
+uint64_t agg_state_bytes(uint32_t n, int average) { return (uint64_t)n * n * 8 * (average ? 2 : 1) + agg_nodes_bytes(n); }
+
 AggState agg_state_at(void *base, uint32_t n, int average) {
+    const uint64_t N = n;
+    uint64_t *lo = (uint64_t *)base;
+    AggState st = agg_nodes_at(lo + N * N * (average ? 2 : 1), n);
+    st.average = average;
+    st.lo = lo;
+    st.hi = average ? lo + N * N : nullptr;
+    return st;
+}
+
+AggState agg_nodes_at(void *base, uint32_t n) {
     AggState st{};
     const uint64_t N = n;
     st.n = n;
-    st.average = average;
-    st.lo = (uint64_t *)base;
-    st.hi = average ? st.lo + N * N : nullptr;
-    uint64_t *w = st.lo + N * N * (average ? 2 : 1);
+    uint64_t *w = (uint64_t *)base;
     st.nn_lo = w;
     st.nn_hi = w + N;
     st.ctr = (unsigned long long *)(w + 2 * N);
@@ -247,6 +409,63 @@ cudaError_t launch_agg_rounds(const AggState &st, AggThreshold thr, uint32_t rou
         k_agg_scan<<<row_blocks, AGG_THREADS, 0, s>>>(st);
         k_agg_pair<<<node_blocks, AGG_THREADS, 0, s>>>(st, thr);
         k_agg_update<<<row_blocks, AGG_THREADS, 0, s>>>(st);
+        k_agg_finalize<<<node_blocks, AGG_THREADS, 0, s>>>(st);
+    }
+    return cudaGetLastError();
+}
+
+uint64_t agg_dense_room() {
+    size_t free_b = 0, total_b = 0;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
+    uint64_t room = free_b;
+    if (const char *e = getenv("GKD_AGG_MAX_BYTES")) room = std::min<uint64_t>(room, strtoull(e, nullptr, 10));
+    return room;
+}
+
+cudaError_t launch_cs_append(const uint32_t *a, const uint32_t *b, const double *dist, uint64_t count, uint32_t n, CsList dst,
+                             uint64_t at, unsigned long long *bad, cudaStream_t s) {
+    if (count == 0) return cudaSuccess;
+    k_cs_append<<<(unsigned)((count + AGG_THREADS - 1) / AGG_THREADS), AGG_THREADS, 0, s>>>(a, b, dist, count, n, dst, at, bad);
+    return cudaGetLastError();
+}
+
+static int cs_end_bit(uint32_t n) {  // keys are below n << 32
+    int bits = 1;
+    while (bits < 32 && ((uint64_t)1 << bits) < n) bits++;
+    return 32 + bits;
+}
+
+cudaError_t cs_sort_temp_bytes(uint64_t pairs, uint32_t n, size_t &bytes) {
+    cub::DoubleBuffer<uint64_t> k(nullptr, nullptr), v(nullptr, nullptr);
+    bytes = 0;
+    return cub::DeviceRadixSort::SortPairs(nullptr, bytes, k, v, (int64_t)(2 * pairs), 0, cs_end_bit(n));
+}
+
+cudaError_t launch_cs_rows(CsList l, uint64_t pairs, uint32_t n, uint64_t *keys[2], uint64_t *vals[2], void *temp,
+                           size_t temp_bytes, uint64_t *off, uint32_t *nbr, unsigned long long *dup, int &current,
+                           cudaStream_t s) {
+    if (pairs) k_cs_directed<<<(unsigned)((pairs + AGG_THREADS - 1) / AGG_THREADS), AGG_THREADS, 0, s>>>(l, pairs, keys[0], vals[0]);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    cub::DoubleBuffer<uint64_t> k(keys[0], keys[1]), v(vals[0], vals[1]);
+    if (pairs && (e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, k, v, (int64_t)(2 * pairs), 0, cs_end_bit(n), s)) != cudaSuccess)
+        return e;
+    current = k.selector;  // the values follow the keys
+    const uint64_t m = std::max<uint64_t>(2 * pairs, (uint64_t)n + 1);
+    k_cs_rows<<<(unsigned)((m + AGG_THREADS - 1) / AGG_THREADS), AGG_THREADS, 0, s>>>(k.Current(), 2 * pairs, n, off, nbr, dup);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_cs_rounds(const AggState &st, CsRows r, AggThreshold thr, uint32_t rounds, int n_sms, cudaStream_t s) {
+    const unsigned node_blocks = (unsigned)(((uint64_t)st.n + AGG_THREADS - 1) / AGG_THREADS);
+    const unsigned row_blocks = (unsigned)std::min<uint64_t>(st.n, (uint64_t)n_sms * 4);
+    for (uint32_t k = 0; k < rounds; k++) {
+        k_cs_scan<<<row_blocks, AGG_THREADS, 0, s>>>(st, r);
+        k_agg_pair<<<node_blocks, AGG_THREADS, 0, s>>>(st, thr);
+        k_cs_update<<<row_blocks, AGG_THREADS, 0, s>>>(st, r);
         k_agg_finalize<<<node_blocks, AGG_THREADS, 0, s>>>(st);
     }
     return cudaGetLastError();

@@ -11,6 +11,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <new>
 #include <string>
 #include <unordered_map>
@@ -1605,6 +1606,71 @@ double agg_round(uint64_t lo, uint64_t hi, uint64_t N) {
     return std::ldexp((double)keep, e + drop);
 }
 
+// v <= max_dist as agg_within tests it (max_dist >= 0)
+AggThreshold agg_threshold(double max_dist) {
+    AggThreshold thr{0, 0, max_dist >= 2.0 ? 1 : 0};
+    if (!thr.all) {
+        int e = 0;
+        const double fr = std::frexp(max_dist, &e);  // max_dist = m 2^(e - 53)
+        thr.m = (uint64_t)std::ldexp(fr, 53);
+        thr.shift = e;
+    }
+    return thr;
+}
+
+// The rounds of an initialised state (rounds(batch) queues `batch` of them) until AGG_DONE, then the merges to out in
+// the sequential order.  The caller has recorded ev[6]; epilogue_ms gains ev[6] .. the end of the rounds.
+int agg_merges(gkd_ctx *c, const char *fn, const AggState &st, gkd_merges *out, const std::function<cudaError_t(uint32_t)> &rounds) {
+    const int average = st.average;
+    unsigned long long ctr[AGG_COUNTERS];
+    // batches of rounds without a host read in between; a batch that ends with AGG_DONE set is the last
+    uint64_t queued = 0;
+    for (uint32_t batch = 8;; batch = std::min<uint32_t>(batch * 2, 512)) {
+        CK(rounds(batch));
+        c->m.launches += 4ull * batch;
+        queued += batch;
+        CK(cudaMemcpyAsync(ctr, st.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += sizeof(ctr);
+        if (ctr[AGG_DONE]) break;
+        // every round but the last merges at least one pair
+        if (queued > (uint64_t)st.n + 1024) return fail(c, GKD_EINVAL, "internal error: %s did not finish in %llu rounds", fn,
+                                                         (unsigned long long)queued);
+    }
+    CK(cudaEventRecord(c->ev[7], c->stream));
+    const uint64_t m = ctr[AGG_N_MERGES];
+    std::vector<AggMerge> ms(m);
+    if (m) CK(cudaMemcpyAsync(ms.data(), st.merges, m * sizeof(AggMerge), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    c->m.d2h_bytes += m * sizeof(AggMerge);
+    c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+    c->m.agglomerate_rounds = ctr[AGG_ROUNDS];
+    // the merge keys strictly increase in the sequential order
+    auto N = [&](const AggMerge &x) -> uint64_t { return average ? (uint64_t)x.sa * x.sb : 1; };
+    std::sort(ms.begin(), ms.end(), [&](const AggMerge &x, const AggMerge &y) {
+        const int k = agg_cmp(x.lo, x.hi, N(x), y.lo, y.hi, N(y));
+        return k < 0 || (k == 0 && (x.a < y.a || (x.a == y.a && x.b < y.b)));
+    });
+    out->n = m;
+    const uint64_t w = std::min<uint64_t>(m, out->cap);
+    if (w == 0) return GKD_OK;
+    std::vector<uint32_t> a(w), b(w), size(w);
+    std::vector<double> h(w);
+    for (uint64_t t = 0; t < w; t++) {
+        const AggMerge &x = ms[t];
+        a[t] = x.a;
+        b[t] = x.b;
+        size[t] = x.sa + x.sb;
+        h[t] = average ? agg_round(x.lo, x.hi, N(x)) : std::ldexp((double)x.lo, -53);
+    }
+    if (out->a) CK(cudaMemcpyAsync(out->a, a.data(), w * 4, cudaMemcpyDefault, c->stream));
+    if (out->b) CK(cudaMemcpyAsync(out->b, b.data(), w * 4, cudaMemcpyDefault, c->stream));
+    if (out->height) CK(cudaMemcpyAsync(out->height, h.data(), w * 8, cudaMemcpyDefault, c->stream));
+    if (out->size) CK(cudaMemcpyAsync(out->size, size.data(), w * 4, cudaMemcpyDefault, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return GKD_OK;
+}
+
 // One complete- or average-linkage agglomeration on the context's device (gkd_all_vs_all_agglomerate, gkd_agglomerate):
 // start() checks the free memory and sets up the matrix and state of agglomerate.cu in one buffer of the call; the
 // distances are scattered into it (scatter); finish() runs the rounds, reads the merges back and writes them to out in
@@ -1628,12 +1694,10 @@ struct Agglomeration {
         out->n = 0;
         c->m.agglomerate_rounds = 0;
         if (n < 2) return GKD_OK;
-        const uint64_t need = agg_state_bytes(n, average);
-        size_t free_b = 0, total_b = 0;
-        CK(cudaMemGetInfo(&free_b, &total_b));
-        if (need > free_b)
+        const uint64_t need = agg_state_bytes(n, average), room = agg_dense_room();
+        if (need > room)
             return fail(c, GKD_ENOMEM, "%s: %s linkage of %u sets needs %llu bytes of device memory; %llu are free", fn,
-                        average ? "average" : "complete", n, (unsigned long long)need, (unsigned long long)free_b);
+                        average ? "average" : "complete", n, (unsigned long long)need, (unsigned long long)room);
         stream = c->stream;
         CK(cudaMallocAsync(&buf, need, c->stream));
         st = agg_state_at(buf, n, average);
@@ -1659,63 +1723,11 @@ struct Agglomeration {
             return fail(c, GKD_EINVAL, "%s: the distance of pair (%u, %u) is not a multiple of 2^-53 in [0, 2]", fn, i, j);
         }
         if (max_dist < 0) return GKD_OK;
-        AggThreshold thr{0, 0, max_dist >= 2.0 ? 1 : 0};
-        if (!thr.all) {
-            int e = 0;
-            const double fr = std::frexp(max_dist, &e);  // max_dist = m 2^(e - 53)
-            thr.m = (uint64_t)std::ldexp(fr, 53);
-            thr.shift = e;
-        }
-        // batches of rounds without a host read in between; a batch that ends with AGG_DONE set is the last
+        const AggThreshold thr = agg_threshold(max_dist);
         CK(cudaEventRecord(c->ev[6], c->stream));
-        uint64_t queued = 0;
-        for (uint32_t batch = 8;; batch = std::min<uint32_t>(batch * 2, 512)) {
-            CK(launch_agg_rounds(st, thr, batch, c->n_sms, c->stream));
-            c->m.launches += 4ull * batch;
-            queued += batch;
-            CK(cudaMemcpyAsync(ctr, st.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, c->stream));
-            CK(cudaStreamSynchronize(c->stream));
-            c->m.d2h_bytes += sizeof(ctr);
-            if (ctr[AGG_DONE]) break;
-            // every round but the last merges at least one pair
-            if (queued > (uint64_t)n + 1024) return fail(c, GKD_EINVAL, "internal error: %s did not finish in %llu rounds", fn,
-                                                          (unsigned long long)queued);
-        }
-        CK(cudaEventRecord(c->ev[7], c->stream));
-        const uint64_t m = ctr[AGG_N_MERGES];
-        std::vector<AggMerge> ms(m);
-        if (m) CK(cudaMemcpyAsync(ms.data(), st.merges, m * sizeof(AggMerge), cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        c->m.d2h_bytes += m * sizeof(AggMerge);
-        c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
-        c->m.agglomerate_rounds = ctr[AGG_ROUNDS];
-        // the merge keys strictly increase in the sequential order
-        auto N = [&](const AggMerge &x) -> uint64_t { return average ? (uint64_t)x.sa * x.sb : 1; };
-        std::sort(ms.begin(), ms.end(), [&](const AggMerge &x, const AggMerge &y) {
-            const int k = agg_cmp(x.lo, x.hi, N(x), y.lo, y.hi, N(y));
-            return k < 0 || (k == 0 && (x.a < y.a || (x.a == y.a && x.b < y.b)));
-        });
-        out->n = m;
-        const uint64_t w = std::min<uint64_t>(m, out->cap);
-        if (w == 0) return GKD_OK;
-        std::vector<uint32_t> a(w), b(w), size(w);
-        std::vector<double> h(w);
-        for (uint64_t t = 0; t < w; t++) {
-            const AggMerge &x = ms[t];
-            a[t] = x.a;
-            b[t] = x.b;
-            size[t] = x.sa + x.sb;
-            h[t] = average ? agg_round(x.lo, x.hi, N(x)) : std::ldexp((double)x.lo, -53);
-        }
-        if (out->a) CK(cudaMemcpyAsync(out->a, a.data(), w * 4, cudaMemcpyDefault, c->stream));
-        if (out->b) CK(cudaMemcpyAsync(out->b, b.data(), w * 4, cudaMemcpyDefault, c->stream));
-        if (out->height) CK(cudaMemcpyAsync(out->height, h.data(), w * 8, cudaMemcpyDefault, c->stream));
-        if (out->size) CK(cudaMemcpyAsync(out->size, size.data(), w * 4, cudaMemcpyDefault, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        return GKD_OK;
+        return agg_merges(c, fn, st, out, [&](uint32_t batch) { return launch_agg_rounds(st, thr, batch, c->n_sms, c->stream); });
     }
 };
-
 // gkd_all_vs_all_agglomerate: each chunk's distances (the dense epilogue's doubles) go straight into the matrix; a chunk
 // whose join overflowed writes nothing and its redo writes the same entries, so the rounds in finish() see final values.
 struct Agglomerate : Form {
@@ -1733,6 +1745,168 @@ struct Agglomerate : Form {
         nvtxRangePop();
         if (rc) return rc;
         CK(cudaEventRecord(c->ev[7], c->stream));
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) override { return g.finish(c); }
+};
+
+// One complete-linkage agglomeration from the pairs within max_dist (gkd_all_vs_all_complete_linkage,
+// gkd_complete_linkage): start() sets up the O(n) state of the rounds; append() adds pairs to one device list that grows
+// with them (16 B per pair); finish() builds the rows of agglomerate.cu from the list and runs the rounds on them (24 B
+// per pair).  While the rows are built the list, the sort's buffers (48 B per pair; the list's buffer is the fourth)
+// and the rows are alive at once: 88 B per pair.  Every allocation is checked against the free device memory first.
+struct SparseComplete {
+    const char *fn;
+    uint32_t n;
+    double max_dist;
+    gkd_merges *out;
+    cudaStream_t stream = nullptr;
+    void *state = nullptr, *list_buf = nullptr, *rows_buf = nullptr;
+    uint64_t cap = 0, hits = 0;  // pairs the list holds room for, and holds
+    CsList list{};
+    AggState st{};
+    SparseComplete(const char *fn_, uint32_t n_, double d, gkd_merges *out_) : fn(fn_), n(n_), max_dist(d), out(out_) {}
+    ~SparseComplete() {
+        for (void *p : {state, list_buf, rows_buf})
+            if (p) cudaFreeAsync(p, stream);
+    }
+    std::array<const void *, 8> outputs() const { return {out->a, out->b, out->height, out->size}; }
+    // bytes more of device memory, or GKD_ENOMEM naming them
+    int room(gkd_ctx *c, uint64_t bytes, const char *what) {
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        if (bytes > free_b)
+            return fail(c, GKD_ENOMEM, "%s: %s for %llu pairs within max_dist needs %llu bytes of device memory; %llu are free", fn,
+                        what, (unsigned long long)hits, (unsigned long long)bytes, (unsigned long long)free_b);
+        return GKD_OK;
+    }
+    int start(gkd_ctx *c) {
+        out->n = 0;
+        c->m.agglomerate_rounds = 0;
+        stream = c->stream;
+        const int rc = room(c, agg_nodes_bytes(n), "the state of the rounds");
+        if (rc) return rc;
+        CK(cudaMallocAsync(&state, agg_nodes_bytes(n), c->stream));
+        st = agg_nodes_at(state, n);
+        CK(launch_agg_init(st, c->stream));
+        c->m.launches++;
+        return GKD_OK;
+    }
+    // count pairs (a, b, dist) in device memory, checked on the device (launch_cs_append)
+    int append(gkd_ctx *c, const uint32_t *a, const uint32_t *b, const double *dist, uint64_t count) {
+        if (hits + count > cap) {
+            const uint64_t want = std::max<uint64_t>(hits + count, std::max<uint64_t>(2 * cap, 1u << 20));
+            int rc = room(c, want * 16, "the pair list");
+            if (rc) return rc;
+            void *p = nullptr;
+            CK(cudaMallocAsync(&p, want * 16, c->stream));
+            const CsList l{(uint32_t *)p, (uint32_t *)p + want, (uint64_t *)((uint32_t *)p + 2 * want)};
+            if (hits) {
+                CK(cudaMemcpyAsync(l.a, list.a, hits * 4, cudaMemcpyDeviceToDevice, c->stream));
+                CK(cudaMemcpyAsync(l.b, list.b, hits * 4, cudaMemcpyDeviceToDevice, c->stream));
+                CK(cudaMemcpyAsync(l.w, list.w, hits * 8, cudaMemcpyDeviceToDevice, c->stream));
+            }
+            if (list_buf) CK(cudaFreeAsync(list_buf, c->stream));
+            list_buf = p;
+            list = l;
+            cap = want;
+        }
+        CK(launch_cs_append(a, b, dist, count, n, list, hits, st.ctr + AGG_BAD, c->stream));
+        c->m.launches += count ? 1 : 0;
+        hits += count;
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) {
+        unsigned long long ctr[AGG_COUNTERS];
+        CK(cudaMemcpyAsync(ctr, st.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += sizeof(ctr);
+        if (ctr[AGG_BAD] != ~0ull) {
+            uint32_t ab[2];
+            CK(cudaMemcpyAsync(ab, list.a + ctr[AGG_BAD], 4, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaMemcpyAsync(ab + 1, list.b + ctr[AGG_BAD], 4, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            const char *why = ab[1] >= n ? "an id that is not below n" : ab[0] == ab[1] ? "two equal ids"
+                                                                      : "a distance that is not a multiple of 2^-53 in [0, 2]";
+            return fail(c, GKD_EINVAL, "%s: pair %llu (%u, %u) has %s", fn, ctr[AGG_BAD], ab[0], ab[1], why);
+        }
+        if (n < 2 || hits == 0) return GKD_OK;
+        // the rows: keys[1] is the list's buffer (at least hits * 16 bytes)
+        CK(cudaEventRecord(c->ev[6], c->stream));
+        size_t temp = 0;
+        CK(cs_sort_temp_bytes(hits, n, temp));
+        const uint64_t items = 2 * hits, off_bytes = ((uint64_t)n + 1) * 8;
+        const uint64_t vals_at = items * 8, alt_at = 2 * vals_at, temp_at = 3 * vals_at;
+        const uint64_t build = temp_at + ((temp + 255) & ~255ull) + 256;
+        int rc = room(c, build, "the row build");
+        if (rc) return rc;
+        void *scratch = nullptr;
+        CK(cudaMallocAsync(&scratch, build, c->stream));
+        char *sc = (char *)scratch;
+        uint64_t *keys[2] = {(uint64_t *)sc, (uint64_t *)list_buf};
+        uint64_t *vals[2] = {(uint64_t *)(sc + vals_at), (uint64_t *)(sc + alt_at)};
+        unsigned long long *dup = (unsigned long long *)(sc + build - 256);
+        // off and nbr go to the front of the rows' buffer; the sorted values are copied behind them below
+        const uint64_t rows_bytes = off_bytes + items * 4 + items * 8 + 64;
+        if ((rc = room(c, rows_bytes, "the rows"))) {
+            cudaFreeAsync(scratch, c->stream);
+            return rc;
+        }
+        CK(cudaMallocAsync(&rows_buf, rows_bytes, c->stream));
+        uint64_t *off = (uint64_t *)rows_buf;
+        uint32_t *nbr = (uint32_t *)(off + n + 1);
+        uint64_t *w = (uint64_t *)(((uintptr_t)(nbr + items) + 7) & ~(uintptr_t)7);
+        CK(cudaMemsetAsync(dup, 0xFF, 8, c->stream));
+        int current = 0;
+        CK(launch_cs_rows(list, hits, n, keys, vals, sc + temp_at, temp, off, nbr, dup, current, c->stream));
+        CK(cudaMemcpyAsync(w, vals[current], items * 8, cudaMemcpyDeviceToDevice, c->stream));
+        c->m.launches += 2;
+        unsigned long long twice = 0;
+        CK(cudaMemcpyAsync(&twice, dup, 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaFreeAsync(scratch, c->stream));
+        CK(cudaFreeAsync(list_buf, c->stream));
+        list_buf = nullptr;
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += 8;
+        if (twice != ~0ull)
+            return fail(c, GKD_EINVAL, "%s: pair (%u, %u) is listed more than once", fn, (uint32_t)(twice >> 32), (uint32_t)twice);
+        if (max_dist < 0) return GKD_OK;
+        const AggThreshold thr = agg_threshold(max_dist);
+        const CsRows r{off, nbr, w};
+        return agg_merges(c, fn, st, out, [&](uint32_t batch) { return launch_cs_rounds(st, r, thr, batch, c->n_sms, c->stream); });
+    }
+};
+
+// gkd_all_vs_all_complete_linkage: each chunk's pairs within max_dist are compacted (as gkd_*_linkage does) and, once the
+// host has seen that the join held, appended to the call's list; the rows are built and the rounds run in finish().
+struct CompleteLinkage : Form {
+    SparseComplete g;
+    unsigned long long chunk_hits = 0;
+    CompleteLinkage(uint32_t n, double d, gkd_merges *out) : g("gkd_all_vs_all_complete_linkage", n, d, out) {}
+    std::array<const void *, 8> outputs() const override { return g.outputs(); }
+    int start(gkd_ctx *c) override { return g.start(c); }
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        const uint64_t nctas = select_within_ctas(e.cnt);
+        int rc;
+        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
+        if ((rc = ensure(c, c->hit_a, e.cnt * 4)) || (rc = ensure(c, c->hit_b, e.cnt * 4)) || (rc = ensure(c, c->d_dist, e.cnt * 8)))
+            return rc;
+        const HitsOut ho{(uint32_t *)c->hit_a.p, (uint32_t *)c->hit_b.p, nullptr, (double *)c->d_dist.p};
+        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
+        nvtxRangePushA("gkd kernel 5: complete linkage pairs");
+        CK(launch_select_within(e.src, e.pc, g.max_dist, a_base, e.cnt, ho, cta, cta + nctas, c->stream));
+        nvtxRangePop();
+        c->m.launches += 3;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
+        d2h += 8;
+        return GKD_OK;
+    }
+    int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        const int rc = g.append(c, (const uint32_t *)c->hit_a.p, (const uint32_t *)c->hit_b.p, (const double *)c->d_dist.p, chunk_hits);
+        if (rc) return rc;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        CK(cudaStreamSynchronize(c->stream));
         return GKD_OK;
     }
     int finish(gkd_ctx *c) override { return g.finish(c); }
@@ -2625,6 +2799,59 @@ int gkd_agglomerate(gkd_ctx *c, uint32_t n, const double *dist, int method, doub
             src = (const double *)c->d_dist.p;
         }
         if ((rc = g.scatter(c, src, first, cnt, nullptr))) return rc;
+    }
+    return g.finish(c);
+    ABI_GUARD_END(c)
+}
+
+// ---- complete linkage from the pairs within max_dist ------------------------------------------------------------
+int gkd_all_vs_all_complete_linkage(gkd_ctx *c, uint32_t n, double max_dist, gkd_merges *out) {
+    const char *fn = "gkd_all_vs_all_complete_linkage";
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "%s: max_dist is NaN", fn);
+    if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
+    CompleteLinkage f(n, max_dist, out);
+    return run_call(c, fn, triangle(n), f);
+}
+
+int gkd_complete_linkage(gkd_ctx *c, uint32_t n, const gkd_hits *pairs, double max_dist, gkd_merges *out) {
+    const char *fn = "gkd_complete_linkage";
+    if (max_dist != max_dist) return fail(c, GKD_EINVAL, "%s: max_dist is NaN", fn);
+    if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
+    if (!pairs) return fail(c, GKD_EINVAL, "%s: null pairs", fn);
+    if (pairs->n && (!pairs->a || !pairs->b || !pairs->dist)) return fail(c, GKD_EINVAL, "%s: null pair array", fn);
+    CHECK_CTX(c);
+    CK(cudaSetDevice(c->cfg.device));
+    SparseComplete g(fn, n, max_dist, out);
+    int rc = host_outputs_ok(c, fn, g.outputs());
+    if (rc) return rc;
+    c->m.pairs = c->m.intersect_bytes = 0;
+    c->m.intersect_ms = c->m.epilogue_ms = 0;
+    ABI_GUARD_BEGIN
+    if ((rc = g.start(c))) return rc;
+    const bool dev_a = pairs->n && classify(pairs->a) == MEM_DEVICE, dev_b = pairs->n && classify(pairs->b) == MEM_DEVICE,
+               dev_d = pairs->n && classify(pairs->dist) == MEM_DEVICE;
+    for (uint64_t first = 0; first < pairs->n; first += PAIR_CHUNK) {
+        const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, pairs->n - first);
+        const uint32_t *a = pairs->a + first, *b = pairs->b + first;
+        const double *d = pairs->dist + first;
+        // host arrays are staged through the selection buffers, in stream order
+        if (!dev_a) {
+            if ((rc = ensure(c, c->hit_a, cnt * 4))) return rc;
+            CK(cudaMemcpyAsync(c->hit_a.p, a, cnt * 4, cudaMemcpyHostToDevice, c->stream));
+            a = (const uint32_t *)c->hit_a.p;
+        }
+        if (!dev_b) {
+            if ((rc = ensure(c, c->hit_b, cnt * 4))) return rc;
+            CK(cudaMemcpyAsync(c->hit_b.p, b, cnt * 4, cudaMemcpyHostToDevice, c->stream));
+            b = (const uint32_t *)c->hit_b.p;
+        }
+        if (!dev_d) {
+            if ((rc = ensure(c, c->d_dist, cnt * 8))) return rc;
+            CK(cudaMemcpyAsync(c->d_dist.p, d, cnt * 8, cudaMemcpyHostToDevice, c->stream));
+            d = (const double *)c->d_dist.p;
+        }
+        c->m.h2d_bytes += (dev_a ? 0 : cnt * 4) + (dev_b ? 0 : cnt * 4) + (dev_d ? 0 : cnt * 8);
+        if ((rc = g.append(c, a, b, d, cnt))) return rc;
     }
     return g.finish(c);
     ABI_GUARD_END(c)

@@ -840,7 +840,22 @@ int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, 
     try {
         out->n = 0;
         const uint64_t N = g->n_genomes;
-        std::vector<double> dist(N * (N - (N > 0)) / 2);
+        // both allocations are checked before any pair is intersected: the host triangle, and the matrix of member 0
+        const uint64_t tri = N * (N - (N > 0)) / 2;
+        std::vector<double> dist;
+        try {
+            dist.resize(tri);
+        } catch (const std::bad_alloc &) {
+            return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_agglomerate: the host triangle of %llu sets needs %llu bytes",
+                         (unsigned long long)N, (unsigned long long)(tri * 8));
+        }
+        if (cudaSetDevice(g->members[0].device) != cudaSuccess)
+            return gfail(g, GKD_ECUDA, "gkd_group_all_vs_all_agglomerate: cannot select the device of member 0");
+        const uint64_t need = gkd::agg_state_bytes(g->n_genomes, method == GKD_LINK_AVERAGE), room = gkd::agg_dense_room();
+        if (N >= 2 && need > room)
+            return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_agglomerate: %s linkage of %llu sets needs %llu bytes of device "
+                         "memory on member 0; %llu are free", method == GKD_LINK_AVERAGE ? "average" : "complete",
+                         (unsigned long long)N, (unsigned long long)need, (unsigned long long)room);
         int rc = gkd_group_all_vs_all(g, nullptr, dist.data());
         if (rc != GKD_OK) return rc;
         gkd_ctx *c0 = g->members[0].ctx;
@@ -849,6 +864,36 @@ int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, 
         return GKD_OK;
     } catch (const std::exception &ex) {
         return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_agglomerate: %s", ex.what());
+    }
+}
+
+int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_merges *out) {
+    if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_complete_linkage: max_dist is NaN");
+    if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_complete_linkage: null out");
+    if (!g) return GKD_EINVAL;
+    try {
+        out->n = 0;
+        // one within pass of the ring, every member keeping all of its hits
+        std::vector<RingWithin> forms(g->members.size(), RingWithin(max_dist));
+        int rc = run_members(g, forms);
+        if (rc != GKD_OK) return rc;
+        std::vector<GroupHit> all;
+        for (auto &f : forms) {
+            all.insert(all.end(), f.hits.begin(), f.hits.end());
+            std::vector<GroupHit>().swap(f.hits);
+        }
+        std::sort(all.begin(), all.end(), [](const GroupHit &p, const GroupHit &q) { return p.a < q.a || (p.a == q.a && p.b < q.b); });
+        std::vector<uint32_t> a(all.size()), b(all.size());
+        std::vector<double> d(all.size());
+        for (size_t t = 0; t < all.size(); t++) a[t] = all[t].a, b[t] = all[t].b, d[t] = all[t].dist;
+        std::vector<GroupHit>().swap(all);
+        const gkd_hits h{a.data(), b.data(), nullptr, d.data(), a.size(), a.size()};
+        gkd_ctx *c0 = g->members[0].ctx;
+        if ((rc = gkd_complete_linkage(c0, g->n_genomes, &h, max_dist, out)) != GKD_OK)
+            return gfail(g, rc, "member 0: %s", gkd_last_error(c0));
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_complete_linkage: %s", ex.what());
     }
 }
 

@@ -451,6 +451,42 @@ cudaError_t launch_agg_scatter(const AggState &st, const double *src, uint64_t f
                                cudaStream_t s);
 // `rounds` rounds queued without a host read; a round after one that merged nothing exits at once (AGG_DONE)
 cudaError_t launch_agg_rounds(const AggState &st, AggThreshold thr, uint32_t rounds, int n_sms, cudaStream_t s);
+// the device bytes a dense agglomeration may take on the current device: the free memory, capped by the environment
+// variable GKD_AGG_MAX_BYTES when it is set (a test pin that reaches the GKD_ENOMEM path at small n)
+uint64_t agg_dense_room();
+// The O(n) state alone (lo and hi nullptr, complete linkage), for the sparse form below
+uint64_t agg_nodes_bytes(uint32_t n);
+AggState agg_nodes_at(void *base, uint32_t n);
+// Complete linkage from the pairs within max_dist (gkd_*_complete_linkage): the same rounds over one CSR row per slot
+// instead of the matrix.  A pair absent from the rows is beyond max_dist, which complete linkage treats as +inf.  Row x
+// holds its neighbours in ascending order, nbr[off[x] .. off[x + 1]), and their words w = d 2^53; a pair that stops
+// being one (a partner merged away, or the merged distance became +inf) is a tombstone: w = CS_TOMB, its neighbour
+// kept so that binary searches stay valid.  24 B per pair (both directions of 4 + 8 B) and 8 B per slot.
+constexpr uint64_t CS_TOMB = ~0ull;
+struct CsRows {
+    const uint64_t *off;
+    const uint32_t *nbr;
+    uint64_t *w;
+};
+struct CsList {  // the pairs of a call as they arrive: a < b and w (16 B per pair)
+    uint32_t *a, *b;
+    uint64_t *w;
+};
+// count pairs (a[t], b[t], dist[t]) (device) to dst[at + t] as (min, max, d 2^53); a pair with an id >= n, two equal
+// ids or a distance that is not a multiple of 2^-53 in [0, 2] stores CS_TOMB and records its index at in *bad
+// (atomicMin)
+cudaError_t launch_cs_append(const uint32_t *a, const uint32_t *b, const double *dist, uint64_t count, uint32_t n, CsList dst,
+                             uint64_t at, unsigned long long *bad, cudaStream_t s);
+// scratch bytes of the radix sort of launch_cs_rows
+cudaError_t cs_sort_temp_bytes(uint64_t pairs, uint32_t n, size_t &bytes);
+// the rows of `pairs` pairs of l: both directions to keys[0] / vals[0] (2 pairs entries each), one radix sort by (row,
+// neighbour) that leaves keys[current] / vals[current] sorted (keys[1] may alias l), then off (n + 1) and nbr.  A key
+// that occurs twice (a pair listed twice) is recorded in *dup (atomicMin; the caller sets it to ~0 first).
+cudaError_t launch_cs_rows(CsList l, uint64_t pairs, uint32_t n, uint64_t *keys[2], uint64_t *vals[2], void *temp,
+                           size_t temp_bytes, uint64_t *off, uint32_t *nbr, unsigned long long *dup, int &current,
+                           cudaStream_t s);
+// launch_agg_rounds over the rows (st from agg_nodes_at)
+cudaError_t launch_cs_rounds(const AggState &st, CsRows r, AggThreshold thr, uint32_t rounds, int n_sms, cudaStream_t s);
 // S1 / N1 < S2 / N2 exactly (S 128-bit as lo, hi; 192-bit cross products)
 __host__ __device__ inline int agg_cmp(uint64_t lo1, uint64_t hi1, uint64_t n1, uint64_t lo2, uint64_t hi2, uint64_t n2) {
     // (lo + hi 2^64) * n as three words w0 + w1 2^64 + w2 2^128

@@ -204,9 +204,21 @@ struct DistSource {
     void linkage(double maxDist, gkd_hits &h) const {
         check(engine ? gkd_all_vs_all_linkage(engine->raw(), n, maxDist, &h) : gkd_group_all_vs_all_linkage(grp, maxDist, &h));
     }
+    // The dense call; when complete linkage fails with GKD_ENOMEM before any pair was intersected (its matrix does not
+    // fit in device memory), the same merges from the pairs within maxDist, whose memory grows with those pairs only
     void agglomerate(int method, double maxDist, gkd_merges &m) const {
-        check(engine ? gkd_all_vs_all_agglomerate(engine->raw(), n, method, maxDist, &m)
-                     : gkd_group_all_vs_all_agglomerate(grp, method, maxDist, &m));
+        gkd_metrics before{}, after{};
+        gkd_get_metrics(metricsCtx(), &before);
+        int rc = engine ? gkd_all_vs_all_agglomerate(engine->raw(), n, method, maxDist, &m)
+                        : gkd_group_all_vs_all_agglomerate(grp, method, maxDist, &m);
+        gkd_get_metrics(metricsCtx(), &after);
+        if (rc == GKD_ENOMEM && method == GKD_LINK_COMPLETE && after.total_pairs == before.total_pairs) {
+            logInfo("The complete-linkage matrix does not fit in device memory: merging from the pairs within distance " +
+                    javaDouble(maxDist) + " instead.");
+            rc = engine ? gkd_all_vs_all_complete_linkage(engine->raw(), n, maxDist, &m)
+                        : gkd_group_all_vs_all_complete_linkage(grp, maxDist, &m);
+        }
+        check(rc);
     }
 };
 

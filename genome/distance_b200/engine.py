@@ -415,6 +415,40 @@ class Engine:
         del keep
         return out
 
+    def all_vs_all_complete_linkage(self, max_dist: float, n: int = None):
+        """(a, b, height, size): all_vs_all_agglomerate(LINK_COMPLETE, max_dist, n), equal bit for bit, from the pairs
+        within max_dist only: device memory grows with those pairs instead of n^2"""
+        n = len(self) if n is None else int(n)
+        return _merges(lambda m: self._ck(self._L.gkd_all_vs_all_complete_linkage(self._h, n, float(max_dist), C.byref(m))), n)
+
+    def complete_linkage(self, n: int, a, b, dist, max_dist: float):
+        """the complete-linkage hierarchy of n records up to max_dist from a caller's pair list: a, b (uint32 ids < n,
+        a != b, each unordered pair at most once) and dist (float64 on the 2^-53 grid in [0, 2]), as numpy arrays or
+        CUDA tensors, in any order; pairs absent from the list are beyond max_dist"""
+        def arr(x, dt, tdt):
+            if _is_torch(x):
+                import torch
+
+                if x.dtype != getattr(torch, tdt) or not x.is_contiguous():
+                    raise ValueError(f"pair arrays must be contiguous {tdt} tensors")
+                return x.data_ptr(), x
+            keep = np.ascontiguousarray(x, dtype=dt)
+            return keep.ctypes.data, keep
+
+        (pa, ka), (pb, kb), (pd, kd) = arr(a, np.uint32, "int32"), arr(b, np.uint32, "int32"), arr(dist, np.float64, "float64")
+        m = int(ka.numel() if _is_torch(ka) else ka.size)
+        if (kb.numel() if _is_torch(kb) else kb.size) != m or (kd.numel() if _is_torch(kd) else kd.size) != m:
+            raise ValueError("a, b and dist must have one entry per pair")
+        if any(_is_torch(x) and x.is_cuda for x in (ka, kb, kd)):
+            import torch
+
+            torch.cuda.synchronize()  # the producers ran on torch's stream
+        h = GkdHits(pa if m else None, pb if m else None, None, pd if m else None, m, m)
+        out = _merges(lambda mg: self._ck(self._L.gkd_complete_linkage(self._h, int(n), C.byref(h), float(max_dist),
+                                                                      C.byref(mg))), int(n))
+        del ka, kb, kd
+        return out
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -607,3 +641,8 @@ class Group:
         """(a, b, height, size) over all global ids: the single-context Engine.all_vs_all_agglomerate result"""
         return _merges(lambda m: self._ck(self._L.gkd_group_all_vs_all_agglomerate(self._h, int(method), float(max_dist),
                                                                                    C.byref(m))), len(self))
+
+    def all_vs_all_complete_linkage(self, max_dist: float):
+        """(a, b, height, size) over all global ids: the single-context Engine.all_vs_all_complete_linkage result"""
+        return _merges(lambda m: self._ck(self._L.gkd_group_all_vs_all_complete_linkage(self._h, float(max_dist),
+                                                                                        C.byref(m))), len(self))

@@ -329,6 +329,20 @@ int gkd_all_vs_all_agglomerate(gkd_ctx *ctx, uint32_t n, int method, double max_
  * read, not modified), on the context's device.  n is not tied to the context's sets.  One gkd_all_vs_all serves
  * several methods or thresholds this way. */
 int gkd_agglomerate(gkd_ctx *ctx, uint32_t n, const double *dist, int method, double max_dist, gkd_merges *out);
+/* Complete linkage of the first n sets up to max_dist from the pairs within max_dist only; equal, bit for bit, to
+ * gkd_all_vs_all_agglomerate(n, GKD_LINK_COMPLETE, max_dist).  Complete linkage merges A and B at v <= max_dist only
+ * when every pair of A x B is within max_dist, so the pairs beyond it never change a merge.  Every pair i < j is
+ * intersected once; the pairs within max_dist are kept on the device.  Arguments as gkd_all_vs_all_agglomerate (NaN
+ * max_dist or NULL out: GKD_EINVAL; negative max_dist: no merges).
+ * Device memory: O(n) (44 B per set) plus 16 B per pair within max_dist while the pairs are collected, 88 B per pair
+ * while they are sorted into one row per set, and 24 B per pair (both directions of a 4 B neighbour and an 8 B value)
+ * while the clusters merge.  The call fails with GKD_ENOMEM, naming the bytes and the pairs, when an allocation would
+ * exceed the free device memory.  Only the merges leave the device. */
+int gkd_all_vs_all_complete_linkage(gkd_ctx *ctx, uint32_t n, double max_dist, gkd_merges *out);
+/* The same over a caller's pair list (pairs->a, b, dist, n; inter and cap are not read; host or device memory; any
+ * order): ids < n, a != b, each unordered pair at most once, dist on the 2^-53 grid in [0, 2], else GKD_EINVAL.  Pairs
+ * absent from the list are beyond max_dist; listed pairs beyond max_dist take part in no merge. */
+int gkd_complete_linkage(gkd_ctx *ctx, uint32_t n, const gkd_hits *pairs, double max_dist, gkd_merges *out);
 
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
@@ -373,8 +387,14 @@ int gkd_group_all_vs_all_clusters(gkd_group *g, double max_dist, uint32_t *label
 int gkd_group_all_vs_all_linkage(gkd_group *g, double max_dist, gkd_hits *out);
 /* gkd_all_vs_all_agglomerate over all global ids; equal to one context's merges, bit for bit.  The members fill a host
  * triangle of all N(N-1)/2 distances as gkd_group_all_vs_all does (8 B per pair of host memory), then member 0 runs
- * gkd_agglomerate on it (its device needs the matrix of gkd_agglomerate).  The arrays of out are host memory. */
+ * gkd_agglomerate on it (its device needs the matrix of gkd_agglomerate).  Both allocations are checked before any pair
+ * is intersected: the call fails with GKD_ENOMEM, naming the bytes, when either does not fit.  The arrays of out are
+ * host memory. */
 int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, gkd_merges *out);
+/* gkd_all_vs_all_complete_linkage over all global ids; equal to one context's merges, bit for bit.  The members select
+ * the pairs within max_dist as gkd_group_all_vs_all_within does, the host orders them by (a, b) (32 B per pair of host
+ * memory) and member 0 runs gkd_complete_linkage on them.  The arrays of out are host memory. */
+int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_merges *out);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

@@ -273,12 +273,10 @@ JNIEXPORT jint JNICALL FN(allVsAllLinkage)(JNIEnv *env, jclass c, jlong h, jint 
     return rc;
 }
 
-/* the complete- (method 1) or average-linkage (method 2) hierarchy of the first n sets up to maxDist: a, b, height, size
- * hold n - 1 entries (the merges in order); nMerges[0] receives their number */
-JNIEXPORT jint JNICALL FN(allVsAllAgglomerate)(JNIEnv *env, jclass c, jlong h, jint n, jint method, jdouble maxDist,
-                                               jintArray a, jintArray b, jdoubleArray height, jintArray size,
-                                               jintArray nMerges) {
-    (void)c;
+/* one gkd_merges call over the first n sets into Java arrays of n - 1 entries; nMerges[0] receives the merges */
+typedef int (*merges_call)(gkd_ctx *ctx, uint32_t n, int method, double max_dist, gkd_merges *out);
+static jint merges_into(JNIEnv *env, merges_call call, jlong h, jint n, jint method, jdouble maxDist, jintArray a,
+                        jintArray b, jdoubleArray height, jintArray size, jintArray nMerges) {
     if (!a || !b || !height || !size || !nMerges || n < 0 || (*env)->GetArrayLength(env, nMerges) < 1) return GKD_EINVAL;
     const jint cap = n > 0 ? n - 1 : 0;
     if ((*env)->GetArrayLength(env, a) < cap || (*env)->GetArrayLength(env, b) < cap ||
@@ -289,7 +287,7 @@ JNIEXPORT jint JNICALL FN(allVsAllAgglomerate)(JNIEnv *env, jclass c, jlong h, j
     jdouble *ph = (*env)->GetDoubleArrayElements(env, height, NULL);
     jint *ps = (*env)->GetIntArrayElements(env, size, NULL);
     gkd_merges out = {(uint32_t *)pa, (uint32_t *)pb, ph, (uint32_t *)ps, (uint64_t)cap, 0};
-    int rc = (pa && pb && ph && ps) ? gkd_all_vs_all_agglomerate(CTX(h), (uint32_t)n, method, maxDist, &out) : GKD_ENOMEM;
+    int rc = (pa && pb && ph && ps) ? call(CTX(h), (uint32_t)n, method, maxDist, &out) : GKD_ENOMEM;
     if (ps) (*env)->ReleaseIntArrayElements(env, size, ps, 0);
     if (ph) (*env)->ReleaseDoubleArrayElements(env, height, ph, 0);
     if (pb) (*env)->ReleaseIntArrayElements(env, b, pb, 0);
@@ -299,4 +297,25 @@ JNIEXPORT jint JNICALL FN(allVsAllAgglomerate)(JNIEnv *env, jclass c, jlong h, j
         (*env)->SetIntArrayRegion(env, nMerges, 0, 1, &nm);
     }
     return rc;
+}
+
+/* the complete- (method 1) or average-linkage (method 2) hierarchy of the first n sets up to maxDist: a, b, height, size
+ * hold n - 1 entries (the merges in order); nMerges[0] receives their number */
+JNIEXPORT jint JNICALL FN(allVsAllAgglomerate)(JNIEnv *env, jclass c, jlong h, jint n, jint method, jdouble maxDist,
+                                               jintArray a, jintArray b, jdoubleArray height, jintArray size,
+                                               jintArray nMerges) {
+    (void)c;
+    return merges_into(env, gkd_all_vs_all_agglomerate, h, n, method, maxDist, a, b, height, size, nMerges);
+}
+
+static int complete_sparse(gkd_ctx *ctx, uint32_t n, int method, double max_dist, gkd_merges *out) {
+    (void)method;
+    return gkd_all_vs_all_complete_linkage(ctx, n, max_dist, out);
+}
+
+/* the complete-linkage hierarchy of allVsAllAgglomerate(method 1) from the pairs within maxDist only */
+JNIEXPORT jint JNICALL FN(allVsAllCompleteLinkage)(JNIEnv *env, jclass c, jlong h, jint n, jdouble maxDist, jintArray a,
+                                                   jintArray b, jdoubleArray height, jintArray size, jintArray nMerges) {
+    (void)c;
+    return merges_into(env, complete_sparse, h, n, GKD_LINK_COMPLETE, maxDist, a, b, height, size, nMerges);
 }

@@ -58,6 +58,8 @@ final class GkdNative {
      *  cluster's), nMerges[0] their number */
     static native int allVsAllAgglomerate(long ctx, int n, int method, double maxDist, int[] a, int[] b, double[] height,
                                           int[] size, int[] nMerges);
+    static native int allVsAllCompleteLinkage(long ctx, int n, double maxDist, int[] a, int[] b, double[] height, int[] size,
+                                              int[] nMerges);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

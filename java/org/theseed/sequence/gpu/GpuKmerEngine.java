@@ -222,6 +222,16 @@ public class GpuKmerEngine implements AutoCloseable {
         return merges[0];
     }
 
+    /** allVsAllAgglomerate(LINK_COMPLETE, maxDist, ...), equal merge for merge, from the pairs within maxDist only: GPU
+     *  memory grows with those pairs instead of with the square of size(), so it serves collections whose distance
+     *  matrix does not fit on the GPU at dereplication thresholds. */
+    public synchronized int allVsAllCompleteLinkage(double maxDist, int[] a, int[] b, double[] height, int[] size) {
+        this.build();
+        int[] merges = new int[1];
+        check(GkdNative.allVsAllCompleteLinkage(this.ctx, this.size(), maxDist, a, b, height, size, merges));
+        return merges[0];
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
