@@ -1266,6 +1266,29 @@ int run_rect(gkd_ctx *c, const HostPairs &hp, Form &f) {
 }
 
 // ---- selection forms --------------------------------------------------------------------------------------------
+// The pairs of chunk e with dist <= max_dist, compacted in enumeration order: the first cap of them go to the front of
+// the buffers `want` names ({hit_a, hit_b, d_inter, d_dist}), each sized for `room` hits.  *total is the device word
+// that receives the chunk's number of hits; the form reads it back.  `what` names the launches in a profile.
+int select_within(gkd_ctx *c, const Chunk &e, double max_dist, uint32_t a_base, uint64_t cap, uint64_t room,
+                  std::array<bool, 4> want, const char *what, unsigned long long *&total) {
+    const uint64_t nctas = select_within_ctas(e.cnt);
+    int rc;
+    if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
+    if (want[0] && (rc = ensure(c, c->hit_a, room * 4))) return rc;
+    if (want[1] && (rc = ensure(c, c->hit_b, room * 4))) return rc;
+    if (want[2] && (rc = ensure(c, c->d_inter, room * 8))) return rc;
+    if (want[3] && (rc = ensure(c, c->d_dist, room * 8))) return rc;
+    const HitsOut ho{want[0] ? (uint32_t *)c->hit_a.p : nullptr, want[1] ? (uint32_t *)c->hit_b.p : nullptr,
+                     want[2] ? (uint64_t *)c->d_inter.p : nullptr, want[3] ? (double *)c->d_dist.p : nullptr};
+    unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
+    total = cta + nctas;
+    nvtxRangePushA(what);
+    CK(launch_select_within(e.src, e.pc, max_dist, a_base, cap, ho, cta, total, c->stream));
+    nvtxRangePop();
+    c->m.launches += cap ? 3 : 2;
+    return GKD_OK;
+}
+
 // gkd_*_within: the pairs with dist <= max_dist, in enumeration order, to the caller's hits.  hits.n counts every hit so
 // far and is the next write position, so a chunk's hits are read back only once the chunk is kept.
 struct Within : Form {
@@ -1282,22 +1305,12 @@ struct Within : Form {
     int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         const bool any_out = h.a || h.b || h.inter || h.dist;
         wcap = (any_out && h.n < h.cap) ? std::min<uint64_t>(e.cnt, h.cap - h.n) : 0;
-        const uint64_t nctas = select_within_ctas(e.cnt);
-        int rc;
-        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
-        if (h.a && (rc = ensure(c, c->hit_a, wcap * 4))) return rc;
-        if (h.b && (rc = ensure(c, c->hit_b, wcap * 4))) return rc;
-        if (h.inter && (rc = ensure(c, c->d_inter, wcap * 8))) return rc;
-        if (h.dist && (rc = ensure(c, c->d_dist, wcap * 8))) return rc;
-        const HitsOut ho{h.a ? (uint32_t *)c->hit_a.p : nullptr, h.b ? (uint32_t *)c->hit_b.p : nullptr,
-                         h.inter ? (uint64_t *)c->d_inter.p : nullptr, h.dist ? (double *)c->d_dist.p : nullptr};
-        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
-        nvtxRangePushA("gkd kernel 5: within selection");
-        CK(launch_select_within(e.src, e.pc, max_dist, a_base, wcap, ho, cta, cta + nctas, c->stream));
-        nvtxRangePop();
-        c->m.launches += wcap ? 3 : 2;
+        const std::array<bool, 4> want{h.a != nullptr, h.b != nullptr, h.inter != nullptr, h.dist != nullptr};
+        unsigned long long *total;
+        const int rc = select_within(c, e, max_dist, a_base, wcap, wcap, want, "gkd kernel 5: within selection", total);
+        if (rc) return rc;
         CK(cudaEventRecord(c->ev[7], c->stream));
-        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(&chunk_hits, total, 8, cudaMemcpyDeviceToHost, c->stream));
         d2h += 8;
         return GKD_OK;
     }
@@ -1492,19 +1505,11 @@ struct Linkage : Form {
     }
     int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         // every edge of the chunk within max_dist, with room behind them for the forest so far (keep)
-        const uint64_t room = e.cnt + nodes;
-        const uint64_t nctas = select_within_ctas(e.cnt);
-        int rc;
-        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
-        if ((rc = ensure(c, c->hit_a, room * 4)) || (rc = ensure(c, c->hit_b, room * 4))) return rc;
-        if ((rc = ensure(c, c->d_inter, room * 8)) || (rc = ensure(c, c->d_dist, room * 8))) return rc;
-        const HitsOut ho{(uint32_t *)c->hit_a.p, (uint32_t *)c->hit_b.p, (uint64_t *)c->d_inter.p, (double *)c->d_dist.p};
-        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
-        nvtxRangePushA("gkd kernel 5: linkage edges");
-        CK(launch_select_within(e.src, e.pc, max_dist, a_base, e.cnt, ho, cta, cta + nctas, c->stream));
-        nvtxRangePop();
-        c->m.launches += 3;
-        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
+        unsigned long long *total;
+        const int rc = select_within(c, e, max_dist, a_base, e.cnt, e.cnt + nodes, {true, true, true, true},
+                                     "gkd kernel 5: linkage edges", total);
+        if (rc) return rc;
+        CK(cudaMemcpyAsync(&chunk_hits, total, 8, cudaMemcpyDeviceToHost, c->stream));
         d2h += 8;
         return GKD_OK;
     }
@@ -1671,26 +1676,29 @@ int agg_merges(gkd_ctx *c, const char *fn, const AggState &st, gkd_merges *out, 
     return GKD_OK;
 }
 
-// One complete- or average-linkage agglomeration on the context's device (gkd_all_vs_all_agglomerate, gkd_agglomerate):
-// start() checks the free memory and sets up the matrix and state of agglomerate.cu in one buffer of the call; the
-// distances are scattered into it (scatter); finish() runs the rounds, reads the merges back and writes them to out in
-// the sequential order.
-struct Agglomeration {
+// One complete- or average-linkage agglomeration on the context's device: start() checks the free memory and sets up
+// the matrix and state of agglomerate.cu in one buffer of the call; the distances are scattered into it; finish() runs
+// the rounds, reads the merges back and writes them to out in the sequential order.  gkd_all_vs_all_agglomerate: each
+// chunk's distances (the dense epilogue's doubles) go straight into the matrix; a chunk whose join overflowed writes
+// nothing and its redo writes the same entries, so the rounds in finish() see final values.  gkd_agglomerate: start()
+// scatters the caller's triangle dist.
+struct Agglomeration : Form {
     const char *fn;
     uint32_t n;
     int average;
     double max_dist;
+    const double *dist;  // the caller's triangle (host or device memory), or nullptr
     gkd_merges *out;
     void *buf = nullptr;
     cudaStream_t stream = nullptr;
     AggState st{};
-    Agglomeration(const char *fn_, uint32_t n_, int method, double d, gkd_merges *out_)
-        : fn(fn_), n(n_), average(method == GKD_LINK_AVERAGE), max_dist(d), out(out_) {}
+    Agglomeration(const char *fn_, uint32_t n_, int method, double d, const double *dist_, gkd_merges *out_)
+        : fn(fn_), n(n_), average(method == GKD_LINK_AVERAGE), max_dist(d), dist(dist_), out(out_) {}
     ~Agglomeration() {
         if (buf) cudaFreeAsync(buf, stream);
     }
-    std::array<const void *, 8> outputs() const { return {out->a, out->b, out->height, out->size}; }
-    int start(gkd_ctx *c) {
+    std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->height, out->size}; }
+    int start(gkd_ctx *c) override {
         out->n = 0;
         c->m.agglomerate_rounds = 0;
         if (n < 2) return GKD_OK;
@@ -1703,6 +1711,21 @@ struct Agglomeration {
         st = agg_state_at(buf, n, average);
         CK(launch_agg_init(st, c->stream));
         c->m.launches++;
+        if (!dist) return GKD_OK;
+        const uint64_t total = (uint64_t)n * (n - 1) / 2;
+        const bool on_device = classify(dist) == MEM_DEVICE;
+        int rc;
+        for (uint64_t first = 0; first < total; first += PAIR_CHUNK) {
+            const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, total - first);
+            const double *src = dist + first;
+            if (!on_device) {  // staged through the scatter's source buffer, in stream order
+                if ((rc = ensure(c, c->d_dist, cnt * 8))) return rc;
+                CK(cudaMemcpyAsync(c->d_dist.p, src, cnt * 8, cudaMemcpyHostToDevice, c->stream));
+                c->m.h2d_bytes += cnt * 8;
+                src = (const double *)c->d_dist.p;
+            }
+            if ((rc = scatter(c, src, first, cnt, nullptr))) return rc;
+        }
         return GKD_OK;
     }
     // entries [first, first + count) of the triangle, as doubles in device memory
@@ -1711,7 +1734,19 @@ struct Agglomeration {
         c->m.launches++;
         return GKD_OK;
     }
-    int finish(gkd_ctx *c) {
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        int rc = ensure(c, c->d_dist, e.cnt * 8);
+        if (rc) return rc;
+        nvtxRangePushA("gkd kernel 5: agglomerate matrix");
+        CK(launch_epilogue(e.src, e.pc, EpilogueOut{nullptr, (double *)c->d_dist.p, nullptr, nullptr}, c->stream));
+        c->m.launches++;
+        rc = scatter(c, (const double *)c->d_dist.p, e.src.first, e.cnt, e.join_err);
+        nvtxRangePop();
+        if (rc) return rc;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) override {
         if (n < 2) return GKD_OK;
         unsigned long long ctr[AGG_COUNTERS];
         CK(cudaMemcpyAsync(ctr, st.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, c->stream));
@@ -1728,49 +1763,33 @@ struct Agglomeration {
         return agg_merges(c, fn, st, out, [&](uint32_t batch) { return launch_agg_rounds(st, thr, batch, c->n_sms, c->stream); });
     }
 };
-// gkd_all_vs_all_agglomerate: each chunk's distances (the dense epilogue's doubles) go straight into the matrix; a chunk
-// whose join overflowed writes nothing and its redo writes the same entries, so the rounds in finish() see final values.
-struct Agglomerate : Form {
-    Agglomeration g;
-    Agglomerate(uint32_t n, int method, double d, gkd_merges *out) : g("gkd_all_vs_all_agglomerate", n, method, d, out) {}
-    std::array<const void *, 8> outputs() const override { return g.outputs(); }
-    int start(gkd_ctx *c) override { return g.start(c); }
-    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
-        int rc = ensure(c, c->d_dist, e.cnt * 8);
-        if (rc) return rc;
-        nvtxRangePushA("gkd kernel 5: agglomerate matrix");
-        CK(launch_epilogue(e.src, e.pc, EpilogueOut{nullptr, (double *)c->d_dist.p, nullptr, nullptr}, c->stream));
-        c->m.launches++;
-        rc = g.scatter(c, (const double *)c->d_dist.p, e.src.first, e.cnt, e.join_err);
-        nvtxRangePop();
-        if (rc) return rc;
-        CK(cudaEventRecord(c->ev[7], c->stream));
-        return GKD_OK;
-    }
-    int finish(gkd_ctx *c) override { return g.finish(c); }
-};
 
-// One complete-linkage agglomeration from the pairs within max_dist (gkd_all_vs_all_complete_linkage,
-// gkd_complete_linkage): start() sets up the O(n) state of the rounds; append() adds pairs to one device list that grows
-// with them (16 B per pair); finish() builds the rows of agglomerate.cu from the list and runs the rounds on them (24 B
-// per pair).  While the rows are built the list, the sort's buffers (48 B per pair; the list's buffer is the fourth)
-// and the rows are alive at once: 88 B per pair.  Every allocation is checked against the free device memory first.
-struct SparseComplete {
+// One complete-linkage agglomeration from the pairs within max_dist: start() sets up the O(n) state of the rounds;
+// append() adds pairs to one device list that grows with them (16 B per pair); finish() builds the rows of
+// agglomerate.cu from the list and runs the rounds on them (24 B per pair).  While the rows are built the list, the
+// sort's buffers (48 B per pair; the list's buffer is the fourth) and the rows are alive at once: 88 B per pair.  Every
+// allocation is checked against the free device memory first.  gkd_all_vs_all_complete_linkage: each chunk's pairs
+// within max_dist are compacted (as gkd_*_linkage does) and, once the host has seen that the join held, appended to the
+// list.  gkd_complete_linkage: start() appends the caller's list.
+struct SparseComplete : Form {
     const char *fn;
     uint32_t n;
     double max_dist;
+    const gkd_hits *pairs;  // the caller's list (a, b and dist in host or device memory), or nullptr
     gkd_merges *out;
     cudaStream_t stream = nullptr;
     void *state = nullptr, *list_buf = nullptr, *rows_buf = nullptr;
     uint64_t cap = 0, hits = 0;  // pairs the list holds room for, and holds
+    unsigned long long chunk_hits = 0;
     CsList list{};
     AggState st{};
-    SparseComplete(const char *fn_, uint32_t n_, double d, gkd_merges *out_) : fn(fn_), n(n_), max_dist(d), out(out_) {}
+    SparseComplete(const char *fn_, uint32_t n_, double d, const gkd_hits *pairs_, gkd_merges *out_)
+        : fn(fn_), n(n_), max_dist(d), pairs(pairs_), out(out_) {}
     ~SparseComplete() {
         for (void *p : {state, list_buf, rows_buf})
             if (p) cudaFreeAsync(p, stream);
     }
-    std::array<const void *, 8> outputs() const { return {out->a, out->b, out->height, out->size}; }
+    std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->height, out->size}; }
     // bytes more of device memory, or GKD_ENOMEM naming them
     int room(gkd_ctx *c, uint64_t bytes, const char *what) {
         size_t free_b = 0, total_b = 0;
@@ -1780,16 +1799,42 @@ struct SparseComplete {
                         what, (unsigned long long)hits, (unsigned long long)bytes, (unsigned long long)free_b);
         return GKD_OK;
     }
-    int start(gkd_ctx *c) {
+    int start(gkd_ctx *c) override {
         out->n = 0;
         c->m.agglomerate_rounds = 0;
         stream = c->stream;
-        const int rc = room(c, agg_nodes_bytes(n), "the state of the rounds");
+        int rc = room(c, agg_nodes_bytes(n), "the state of the rounds");
         if (rc) return rc;
         CK(cudaMallocAsync(&state, agg_nodes_bytes(n), c->stream));
         st = agg_nodes_at(state, n);
         CK(launch_agg_init(st, c->stream));
         c->m.launches++;
+        if (!pairs || !pairs->n) return GKD_OK;
+        const bool dev_a = classify(pairs->a) == MEM_DEVICE, dev_b = classify(pairs->b) == MEM_DEVICE,
+                   dev_d = classify(pairs->dist) == MEM_DEVICE;
+        for (uint64_t first = 0; first < pairs->n; first += PAIR_CHUNK) {
+            const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, pairs->n - first);
+            const uint32_t *a = pairs->a + first, *b = pairs->b + first;
+            const double *d = pairs->dist + first;
+            // host arrays are staged through the selection buffers, in stream order
+            if (!dev_a) {
+                if ((rc = ensure(c, c->hit_a, cnt * 4))) return rc;
+                CK(cudaMemcpyAsync(c->hit_a.p, a, cnt * 4, cudaMemcpyHostToDevice, c->stream));
+                a = (const uint32_t *)c->hit_a.p;
+            }
+            if (!dev_b) {
+                if ((rc = ensure(c, c->hit_b, cnt * 4))) return rc;
+                CK(cudaMemcpyAsync(c->hit_b.p, b, cnt * 4, cudaMemcpyHostToDevice, c->stream));
+                b = (const uint32_t *)c->hit_b.p;
+            }
+            if (!dev_d) {
+                if ((rc = ensure(c, c->d_dist, cnt * 8))) return rc;
+                CK(cudaMemcpyAsync(c->d_dist.p, d, cnt * 8, cudaMemcpyHostToDevice, c->stream));
+                d = (const double *)c->d_dist.p;
+            }
+            c->m.h2d_bytes += (dev_a ? 0 : cnt * 4) + (dev_b ? 0 : cnt * 4) + (dev_d ? 0 : cnt * 8);
+            if ((rc = append(c, a, b, d, cnt))) return rc;
+        }
         return GKD_OK;
     }
     // count pairs (a, b, dist) in device memory, checked on the device (launch_cs_append)
@@ -1816,7 +1861,24 @@ struct SparseComplete {
         hits += count;
         return GKD_OK;
     }
-    int finish(gkd_ctx *c) {
+    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        unsigned long long *total;
+        const int rc = select_within(c, e, max_dist, a_base, e.cnt, e.cnt, {true, true, false, true},
+                                     "gkd kernel 5: complete linkage pairs", total);
+        if (rc) return rc;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        CK(cudaMemcpyAsync(&chunk_hits, total, 8, cudaMemcpyDeviceToHost, c->stream));
+        d2h += 8;
+        return GKD_OK;
+    }
+    int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
+        const int rc = append(c, (const uint32_t *)c->hit_a.p, (const uint32_t *)c->hit_b.p, (const double *)c->d_dist.p, chunk_hits);
+        if (rc) return rc;
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) override {
         unsigned long long ctr[AGG_COUNTERS];
         CK(cudaMemcpyAsync(ctr, st.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
@@ -1875,41 +1937,6 @@ struct SparseComplete {
         const CsRows r{off, nbr, w};
         return agg_merges(c, fn, st, out, [&](uint32_t batch) { return launch_cs_rounds(st, r, thr, batch, c->n_sms, c->stream); });
     }
-};
-
-// gkd_all_vs_all_complete_linkage: each chunk's pairs within max_dist are compacted (as gkd_*_linkage does) and, once the
-// host has seen that the join held, appended to the call's list; the rows are built and the rounds run in finish().
-struct CompleteLinkage : Form {
-    SparseComplete g;
-    unsigned long long chunk_hits = 0;
-    CompleteLinkage(uint32_t n, double d, gkd_merges *out) : g("gkd_all_vs_all_complete_linkage", n, d, out) {}
-    std::array<const void *, 8> outputs() const override { return g.outputs(); }
-    int start(gkd_ctx *c) override { return g.start(c); }
-    int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
-        const uint64_t nctas = select_within_ctas(e.cnt);
-        int rc;
-        if ((rc = ensure(c, c->sel_cta, (nctas + 1) * 8))) return rc;
-        if ((rc = ensure(c, c->hit_a, e.cnt * 4)) || (rc = ensure(c, c->hit_b, e.cnt * 4)) || (rc = ensure(c, c->d_dist, e.cnt * 8)))
-            return rc;
-        const HitsOut ho{(uint32_t *)c->hit_a.p, (uint32_t *)c->hit_b.p, nullptr, (double *)c->d_dist.p};
-        unsigned long long *cta = (unsigned long long *)c->sel_cta.p;
-        nvtxRangePushA("gkd kernel 5: complete linkage pairs");
-        CK(launch_select_within(e.src, e.pc, g.max_dist, a_base, e.cnt, ho, cta, cta + nctas, c->stream));
-        nvtxRangePop();
-        c->m.launches += 3;
-        CK(cudaEventRecord(c->ev[7], c->stream));
-        CK(cudaMemcpyAsync(&chunk_hits, cta + nctas, 8, cudaMemcpyDeviceToHost, c->stream));
-        d2h += 8;
-        return GKD_OK;
-    }
-    int keep(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
-        const int rc = g.append(c, (const uint32_t *)c->hit_a.p, (const uint32_t *)c->hit_b.p, (const double *)c->d_dist.p, chunk_hits);
-        if (rc) return rc;
-        CK(cudaEventRecord(c->ev[7], c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        return GKD_OK;
-    }
-    int finish(gkd_ctx *c) override { return g.finish(c); }
 };
 
 // the triangle over the first n sets, and the block of queries q x references r
@@ -2768,40 +2795,21 @@ static int agglomerate_args_ok(gkd_ctx *c, const char *fn, int method, double ma
 }
 
 int gkd_all_vs_all_agglomerate(gkd_ctx *c, uint32_t n, int method, double max_dist, gkd_merges *out) {
-    const int rc = agglomerate_args_ok(c, "gkd_all_vs_all_agglomerate", method, max_dist, out);
+    const char *fn = "gkd_all_vs_all_agglomerate";
+    const int rc = agglomerate_args_ok(c, fn, method, max_dist, out);
     if (rc) return rc;
-    Agglomerate f(n, method, max_dist, out);
-    return run_call(c, "gkd_all_vs_all_agglomerate", triangle(n), f);
+    Agglomeration f(fn, n, method, max_dist, nullptr, out);
+    return run_call(c, fn, triangle(n), f);
 }
 
+// the caller's triangle is scattered by the form's start(): a call without pairs to intersect
 int gkd_agglomerate(gkd_ctx *c, uint32_t n, const double *dist, int method, double max_dist, gkd_merges *out) {
     const char *fn = "gkd_agglomerate";
-    int rc = agglomerate_args_ok(c, fn, method, max_dist, out);
+    const int rc = agglomerate_args_ok(c, fn, method, max_dist, out);
     if (rc) return rc;
     if (!dist && n >= 2) return fail(c, GKD_EINVAL, "%s: null dist", fn);
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    Agglomeration g(fn, n, method, max_dist, out);
-    if ((rc = host_outputs_ok(c, fn, g.outputs()))) return rc;
-    c->m.pairs = c->m.intersect_bytes = 0;
-    c->m.intersect_ms = c->m.epilogue_ms = 0;
-    ABI_GUARD_BEGIN
-    if ((rc = g.start(c))) return rc;
-    const uint64_t total = (uint64_t)n * (n - (n > 0)) / 2;
-    const bool on_device = total && classify(dist) == MEM_DEVICE;
-    for (uint64_t first = 0; first < total; first += PAIR_CHUNK) {
-        const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, total - first);
-        const double *src = dist + first;
-        if (!on_device) {  // staged through the scatter's source buffer, in stream order
-            if ((rc = ensure(c, c->d_dist, cnt * 8))) return rc;
-            CK(cudaMemcpyAsync(c->d_dist.p, src, cnt * 8, cudaMemcpyHostToDevice, c->stream));
-            c->m.h2d_bytes += cnt * 8;
-            src = (const double *)c->d_dist.p;
-        }
-        if ((rc = g.scatter(c, src, first, cnt, nullptr))) return rc;
-    }
-    return g.finish(c);
-    ABI_GUARD_END(c)
+    Agglomeration f(fn, n, method, max_dist, dist, out);
+    return run_call(c, fn, triangle(0), f);
 }
 
 // ---- complete linkage from the pairs within max_dist ------------------------------------------------------------
@@ -2809,52 +2817,19 @@ int gkd_all_vs_all_complete_linkage(gkd_ctx *c, uint32_t n, double max_dist, gkd
     const char *fn = "gkd_all_vs_all_complete_linkage";
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "%s: max_dist is NaN", fn);
     if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
-    CompleteLinkage f(n, max_dist, out);
+    SparseComplete f(fn, n, max_dist, nullptr, out);
     return run_call(c, fn, triangle(n), f);
 }
 
+// the caller's list is appended by the form's start(): a call without pairs to intersect
 int gkd_complete_linkage(gkd_ctx *c, uint32_t n, const gkd_hits *pairs, double max_dist, gkd_merges *out) {
     const char *fn = "gkd_complete_linkage";
     if (max_dist != max_dist) return fail(c, GKD_EINVAL, "%s: max_dist is NaN", fn);
     if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
     if (!pairs) return fail(c, GKD_EINVAL, "%s: null pairs", fn);
     if (pairs->n && (!pairs->a || !pairs->b || !pairs->dist)) return fail(c, GKD_EINVAL, "%s: null pair array", fn);
-    CHECK_CTX(c);
-    CK(cudaSetDevice(c->cfg.device));
-    SparseComplete g(fn, n, max_dist, out);
-    int rc = host_outputs_ok(c, fn, g.outputs());
-    if (rc) return rc;
-    c->m.pairs = c->m.intersect_bytes = 0;
-    c->m.intersect_ms = c->m.epilogue_ms = 0;
-    ABI_GUARD_BEGIN
-    if ((rc = g.start(c))) return rc;
-    const bool dev_a = pairs->n && classify(pairs->a) == MEM_DEVICE, dev_b = pairs->n && classify(pairs->b) == MEM_DEVICE,
-               dev_d = pairs->n && classify(pairs->dist) == MEM_DEVICE;
-    for (uint64_t first = 0; first < pairs->n; first += PAIR_CHUNK) {
-        const uint64_t cnt = std::min<uint64_t>(PAIR_CHUNK, pairs->n - first);
-        const uint32_t *a = pairs->a + first, *b = pairs->b + first;
-        const double *d = pairs->dist + first;
-        // host arrays are staged through the selection buffers, in stream order
-        if (!dev_a) {
-            if ((rc = ensure(c, c->hit_a, cnt * 4))) return rc;
-            CK(cudaMemcpyAsync(c->hit_a.p, a, cnt * 4, cudaMemcpyHostToDevice, c->stream));
-            a = (const uint32_t *)c->hit_a.p;
-        }
-        if (!dev_b) {
-            if ((rc = ensure(c, c->hit_b, cnt * 4))) return rc;
-            CK(cudaMemcpyAsync(c->hit_b.p, b, cnt * 4, cudaMemcpyHostToDevice, c->stream));
-            b = (const uint32_t *)c->hit_b.p;
-        }
-        if (!dev_d) {
-            if ((rc = ensure(c, c->d_dist, cnt * 8))) return rc;
-            CK(cudaMemcpyAsync(c->d_dist.p, d, cnt * 8, cudaMemcpyHostToDevice, c->stream));
-            d = (const double *)c->d_dist.p;
-        }
-        c->m.h2d_bytes += (dev_a ? 0 : cnt * 4) + (dev_b ? 0 : cnt * 4) + (dev_d ? 0 : cnt * 8);
-        if ((rc = g.append(c, a, b, d, cnt))) return rc;
-    }
-    return g.finish(c);
-    ABI_GUARD_END(c)
+    SparseComplete f(fn, n, max_dist, pairs, out);
+    return run_call(c, fn, triangle(0), f);
 }
 
 // ---- MinHash sketches ---------------------------------------------------------------------------------------

@@ -519,6 +519,20 @@ int run_members(gkd_group *g, std::vector<Form> &forms) {
     return GKD_OK;
 }
 
+// Every pair of the group within max_dist, in global ids, to all: one RingWithin ring, each member keeping all of its
+// hits.  The members own disjoint pairs, so one sort by (a, b) gives the order of one context's row-major triangle.
+int group_within(gkd_group *g, double max_dist, std::vector<GroupHit> &all) {
+    std::vector<RingWithin> forms(g->members.size(), RingWithin(max_dist));
+    const int rc = run_members(g, forms);
+    if (rc != GKD_OK) return rc;
+    for (auto &f : forms) {
+        all.insert(all.end(), f.hits.begin(), f.hits.end());
+        std::vector<GroupHit>().swap(f.hits);
+    }
+    std::sort(all.begin(), all.end(), [](const GroupHit &p, const GroupHit &q) { return p.a < q.a || (p.a == q.a && p.b < q.b); });
+    return GKD_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -719,16 +733,9 @@ int gkd_group_all_vs_all_within(gkd_group *g, double max_dist, gkd_hits *out) {
     if (!g) return GKD_EINVAL;
     try {
         out->n = 0;
-        std::vector<RingWithin> forms(g->members.size(), RingWithin(max_dist));
-        const int rc = run_members(g, forms);
-        if (rc != GKD_OK) return rc;
-        // the members own disjoint pairs: one sort by (a, b) gives the order of one context's row-major triangle
         std::vector<GroupHit> all;
-        for (auto &f : forms) {
-            all.insert(all.end(), f.hits.begin(), f.hits.end());
-            std::vector<GroupHit>().swap(f.hits);
-        }
-        std::sort(all.begin(), all.end(), [](const GroupHit &p, const GroupHit &q) { return p.a < q.a || (p.a == q.a && p.b < q.b); });
+        const int rc = group_within(g, max_dist, all);
+        if (rc != GKD_OK) return rc;
         out->n = all.size();
         const uint64_t w = std::min<uint64_t>(all.size(), out->cap);
         for (uint64_t t = 0; t < w; t++) {
@@ -873,16 +880,9 @@ int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_mer
     if (!g) return GKD_EINVAL;
     try {
         out->n = 0;
-        // one within pass of the ring, every member keeping all of its hits
-        std::vector<RingWithin> forms(g->members.size(), RingWithin(max_dist));
-        int rc = run_members(g, forms);
-        if (rc != GKD_OK) return rc;
         std::vector<GroupHit> all;
-        for (auto &f : forms) {
-            all.insert(all.end(), f.hits.begin(), f.hits.end());
-            std::vector<GroupHit>().swap(f.hits);
-        }
-        std::sort(all.begin(), all.end(), [](const GroupHit &p, const GroupHit &q) { return p.a < q.a || (p.a == q.a && p.b < q.b); });
+        int rc = group_within(g, max_dist, all);
+        if (rc != GKD_OK) return rc;
         std::vector<uint32_t> a(all.size()), b(all.size());
         std::vector<double> d(all.size());
         for (size_t t = 0; t < all.size(); t++) a[t] = all[t].a, b[t] = all[t].b, d[t] = all[t].dist;

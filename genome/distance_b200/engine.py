@@ -66,6 +66,23 @@ def _is_torch(x) -> bool:
     return type(x).__module__.startswith("torch")
 
 
+def _array(x, dtype, tensor_dtypes: Sequence[str], message: str) -> Tuple[int, int, object]:
+    """(address, count, keep-alive) of a caller's array: anything numpy takes, as a contiguous `dtype` copy where it is
+    not one already, or a contiguous torch tensor of one of `tensor_dtypes` (ValueError(message) otherwise), passed as
+    it is.  A CUDA tensor's device is synchronised first: its producers ran on torch's stream and the library reads it
+    on its own."""
+    if not _is_torch(x):
+        a = np.ascontiguousarray(x, dtype=dtype)
+        return a.ctypes.data, a.size, a
+    import torch
+
+    if x.dtype not in [getattr(torch, t) for t in tensor_dtypes] or not x.is_contiguous():
+        raise ValueError(message)
+    if x.is_cuda:
+        torch.cuda.synchronize(x.device)
+    return x.data_ptr(), x.numel(), x
+
+
 class Engine:
     """One gkd context on one GPU.
 
@@ -225,16 +242,7 @@ class Engine:
 
     def import_set(self, keys) -> int:
         """Add a set from its key array (numpy uint64 on host or torch int64/uint64 on this device); copied."""
-        if isinstance(keys, np.ndarray):
-            a = np.ascontiguousarray(keys, dtype=np.uint64)
-            ptr, n, keep = a.ctypes.data, a.size, a
-        else:
-            import torch
-
-            t = keys.contiguous()
-            if t.is_cuda:
-                torch.cuda.synchronize(self.device)
-            ptr, n, keep = t.data_ptr(), t.numel(), t
+        ptr, n, keep = _array(keys, np.uint64, ("int64", "uint64"), "keys must be a contiguous int64 or uint64 tensor")
         out = C.c_uint32()
         self._ck(self._L.gkd_import_set(self._h, ptr if n else None, n, C.byref(out)))
         del keep
@@ -244,16 +252,7 @@ class Engine:
         """Add many sets from key arrays stored back to back (`keys`: numpy uint64 or torch int64 tensor,
         host or this device; `offsets`: n+1 host integers).  Returns the id of the first new set."""
         offs = np.ascontiguousarray(offsets, dtype=np.uint64)
-        if isinstance(keys, np.ndarray):
-            a = np.ascontiguousarray(keys, dtype=np.uint64)
-            ptr, keep = a.ctypes.data, a
-        else:
-            import torch
-
-            t = keys.contiguous()
-            if t.is_cuda:
-                torch.cuda.synchronize(self.device)
-            ptr, keep = t.data_ptr(), t
+        ptr, _, keep = _array(keys, np.uint64, ("int64", "uint64"), "keys must be a contiguous int64 or uint64 tensor")
         out = C.c_uint32()
         self._ck(self._L.gkd_import_sets(self._h, ptr if int(offs[-1]) else None,
                                          offs.ctypes.data_as(C.POINTER(C.c_uint64)), offs.size - 1, C.byref(out)))
@@ -401,15 +400,7 @@ class Engine:
         n = int(round((1 + (1 + 8 * m) ** 0.5) / 2)) if m else 0
         if n * (n - 1) // 2 != m:
             raise ValueError(f"{m} distances are not a strict upper triangle")
-        if _is_torch(dist):
-            import torch
-
-            if dist.dtype != torch.float64 or not dist.is_contiguous():
-                raise ValueError("dist must be a contiguous float64 tensor")
-            ptr, keep = dist.data_ptr(), dist
-        else:
-            keep = np.ascontiguousarray(dist, dtype=np.float64)
-            ptr = keep.ctypes.data
+        ptr, _, keep = _array(dist, np.float64, ("float64",), "dist must be a contiguous float64 tensor")
         out = _merges(lambda mg: self._ck(self._L.gkd_agglomerate(self._h, n, ptr, int(method), float(max_dist),
                                                                  C.byref(mg))), n)
         del keep
@@ -425,24 +416,11 @@ class Engine:
         """the complete-linkage hierarchy of n records up to max_dist from a caller's pair list: a, b (uint32 ids < n,
         a != b, each unordered pair at most once) and dist (float64 on the 2^-53 grid in [0, 2]), as numpy arrays or
         CUDA tensors, in any order; pairs absent from the list are beyond max_dist"""
-        def arr(x, dt, tdt):
-            if _is_torch(x):
-                import torch
-
-                if x.dtype != getattr(torch, tdt) or not x.is_contiguous():
-                    raise ValueError(f"pair arrays must be contiguous {tdt} tensors")
-                return x.data_ptr(), x
-            keep = np.ascontiguousarray(x, dtype=dt)
-            return keep.ctypes.data, keep
-
-        (pa, ka), (pb, kb), (pd, kd) = arr(a, np.uint32, "int32"), arr(b, np.uint32, "int32"), arr(dist, np.float64, "float64")
-        m = int(ka.numel() if _is_torch(ka) else ka.size)
-        if (kb.numel() if _is_torch(kb) else kb.size) != m or (kd.numel() if _is_torch(kd) else kd.size) != m:
+        pa, m, ka = _array(a, np.uint32, ("int32",), "pair arrays must be contiguous int32 tensors")
+        pb, mb, kb = _array(b, np.uint32, ("int32",), "pair arrays must be contiguous int32 tensors")
+        pd, md, kd = _array(dist, np.float64, ("float64",), "pair arrays must be contiguous float64 tensors")
+        if mb != m or md != m:
             raise ValueError("a, b and dist must have one entry per pair")
-        if any(_is_torch(x) and x.is_cuda for x in (ka, kb, kd)):
-            import torch
-
-            torch.cuda.synchronize()  # the producers ran on torch's stream
         h = GkdHits(pa if m else None, pb if m else None, None, pd if m else None, m, m)
         out = _merges(lambda mg: self._ck(self._L.gkd_complete_linkage(self._h, int(n), C.byref(h), float(max_dist),
                                                                       C.byref(mg))), int(n))

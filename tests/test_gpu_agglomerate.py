@@ -201,6 +201,28 @@ def test_arguments_cap_and_device_outputs():
             e.agglomerate(np.array([0.5, 2.5, 0.25]), gkd.LINK_AVERAGE, 1.0)
 
 
+def test_device_triangle_waits_for_torch(monkeypatch):
+    """the library reads a CUDA triangle on its own stream, so Engine.agglomerate synchronises the tensor's device first:
+    the torch kernel that has just produced it must have finished"""
+    import torch
+
+    seqs = tc._seqs(5, [40_000] * 24)
+    with tc._engine(seqs, 21) as e:
+        _, gd = e.all_vs_all(want_inter=False)
+        want = e.agglomerate(gd, gkd.LINK_COMPLETE, 1.0)
+        dev = torch.from_numpy(gd).to("cuda:0").mul_(1.0)
+        synced = []
+        real = torch.cuda.synchronize
+
+        def synchronize(device=None):
+            synced.append(torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device))
+            real(device)
+
+        monkeypatch.setattr(torch.cuda, "synchronize", synchronize)
+        _eq(e.agglomerate(dev, gkd.LINK_COMPLETE, 1.0), want)
+        assert dev.device in synced
+
+
 def test_more_than_one_chunk():
     """~12,000 gene-sized records: two 64 Mi-pair chunks.  The call equals gkd_agglomerate on the dense triangle."""
     import torch

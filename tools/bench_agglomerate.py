@@ -49,7 +49,7 @@ def scipy_merges(Z, n):
 
 def agglomerate_ms(e, dev, method, repeat):
     """CUDA-event time on gkd_stream of gkd_agglomerate over a triangle in device memory (median of repeat)"""
-    s = torch.cuda.ExternalStream(e.stream_ptr())
+    s = torch.cuda.ExternalStream(e.stream_ptr)
     times = []
     for _ in range(repeat):
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
