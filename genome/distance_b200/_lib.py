@@ -43,6 +43,11 @@ class GkdMerges(C.Structure):
                 ("n", C.c_uint64)]
 
 
+class GkdJoins(C.Structure):
+    _fields_ = [("a", C.c_void_p), ("b", C.c_void_p), ("len_a", C.c_void_p), ("len_b", C.c_void_p), ("cap", C.c_uint64),
+                ("n", C.c_uint64)]
+
+
 class GkdNeighbors(C.Structure):
     _fields_ = [("pos", C.c_void_p), ("inter", C.c_void_p), ("dist", C.c_void_p), ("n_found", C.c_void_p)]
 
@@ -93,6 +98,7 @@ SYMBOLS = {
     "gkd_group_all_vs_all_linkage": (_i32, [_vp, _dbl, C.POINTER(GkdHits)]),
     "gkd_group_all_vs_all_agglomerate": (_i32, [_vp, _i32, _dbl, C.POINTER(GkdMerges)]),
     "gkd_group_all_vs_all_complete_linkage": (_i32, [_vp, _dbl, C.POINTER(GkdMerges)]),
+    "gkd_group_all_vs_all_nj": (_i32, [_vp, C.POINTER(GkdJoins)]),
     "gkd_build_sets": (_i32, [_vp]),
     "gkd_set_size": (_i32, [_vp, _u32, _pu64, _pu64, _pu64]),
     "gkd_export_set": (_i32, [_vp, _u32, _vp, _u64, _pu64]),
@@ -127,6 +133,8 @@ SYMBOLS = {
     "gkd_agglomerate": (_i32, [_vp, _u32, _vp, _i32, _dbl, C.POINTER(GkdMerges)]),
     "gkd_all_vs_all_complete_linkage": (_i32, [_vp, _u32, _dbl, C.POINTER(GkdMerges)]),
     "gkd_complete_linkage": (_i32, [_vp, _u32, C.POINTER(GkdHits), _dbl, C.POINTER(GkdMerges)]),
+    "gkd_all_vs_all_nj": (_i32, [_vp, _u32, C.POINTER(GkdJoins)]),
+    "gkd_nj": (_i32, [_vp, _u32, _vp, C.POINTER(GkdJoins)]),
     "gkd_hash_set": (_i32, [_vp, _u32, _u32, _i32, _vp, _pu32]),
     "gkd_sketch_distances": (_i32, [_vp, _u32, _i32, _vp, _vp, _u64, _vp]),
     "gkd_format_double": (_i32, [_dbl, C.c_char_p, C.c_size_t]),

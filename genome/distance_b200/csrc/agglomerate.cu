@@ -95,22 +95,35 @@ __global__ void __launch_bounds__(AGG_THREADS) k_agg_init(AggState st) {
     }
 }
 
-__global__ void __launch_bounds__(AGG_THREADS) k_agg_scatter(AggState st, const double *__restrict__ src, uint64_t first,
-                                                             uint64_t count, const uint32_t *join_err) {
+// the entry a distance is stored as: d 2^53 (agglomeration; false unless a multiple of 2^-53 in [0, 2]) or d itself
+// (neighbour joining; false unless finite and in [0, 2])
+__device__ __forceinline__ bool square_word(double d, uint64_t &w) {
+    const double x = d * 9007199254740992.0;  // d 2^53, exact
+    if (!(d >= 0.0 && d <= 2.0 && x == floor(x))) return false;
+    w = (uint64_t)x;
+    return true;
+}
+__device__ __forceinline__ bool square_word(double d, double &w) {
+    w = d;
+    return d >= 0.0 && d <= 2.0;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(AGG_THREADS) k_square_scatter(Square<T> sq, const double *__restrict__ src, uint64_t first,
+                                                                uint64_t count, const uint32_t *join_err) {
     if (join_err && *join_err) return;  // the chunk is redone and rewrites these entries
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= count) return;
     uint32_t i, j;
-    upper_pair(first + t, st.n, i, j);
-    const double d = src[t];
-    const double w = d * 9007199254740992.0;  // d 2^53, exact
-    if (!(d >= 0.0 && d <= 2.0 && w == floor(w))) {
-        atomicMin(st.ctr + AGG_BAD, (unsigned long long)(first + t));
+    upper_pair(first + t, sq.n, i, j);
+    T w;
+    if (!square_word(src[t], w)) {
+        atomicMin(sq.bad, (unsigned long long)(first + t));
         return;
     }
-    const uint64_t ij = (uint64_t)i * st.n + j, ji = (uint64_t)j * st.n + i;
-    st.lo[ij] = st.lo[ji] = (uint64_t)w;
-    if (st.average) st.hi[ij] = st.hi[ji] = 0;
+    const uint64_t ij = (uint64_t)i * sq.n + j, ji = (uint64_t)j * sq.n + i;
+    sq.w[ij] = sq.w[ji] = w;
+    if (sq.hi) sq.hi[ij] = sq.hi[ji] = 0;
 }
 
 __global__ void __launch_bounds__(AGG_THREADS) k_agg_scan(AggState st) {
@@ -395,12 +408,19 @@ cudaError_t launch_agg_init(const AggState &st, cudaStream_t s) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_agg_scatter(const AggState &st, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err,
-                               cudaStream_t s) {
+template <typename T>
+cudaError_t launch_square_scatter(const Square<T> &sq, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err,
+                                  cudaStream_t s) {
     if (count == 0) return cudaSuccess;
-    k_agg_scatter<<<(unsigned)((count + AGG_THREADS - 1) / AGG_THREADS), AGG_THREADS, 0, s>>>(st, src, first, count, join_err);
+    k_square_scatter<T><<<(unsigned)((count + AGG_THREADS - 1) / AGG_THREADS), AGG_THREADS, 0, s>>>(sq, src, first, count, join_err);
     return cudaGetLastError();
 }
+template cudaError_t launch_square_scatter<uint64_t>(const Square<uint64_t> &, const double *, uint64_t, uint64_t,
+                                                     const uint32_t *, cudaStream_t);
+template cudaError_t launch_square_scatter<double>(const Square<double> &, const double *, uint64_t, uint64_t,
+                                                   const uint32_t *, cudaStream_t);
+
+Square<uint64_t> agg_square(const AggState &st) { return {st.lo, st.average ? st.hi : nullptr, st.n, st.ctr + AGG_BAD}; }
 
 cudaError_t launch_agg_rounds(const AggState &st, AggThreshold thr, uint32_t rounds, int n_sms, cudaStream_t s) {
     const unsigned node_blocks = (unsigned)(((uint64_t)st.n + AGG_THREADS - 1) / AGG_THREADS);

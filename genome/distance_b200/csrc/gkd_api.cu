@@ -1676,41 +1676,35 @@ int agg_merges(gkd_ctx *c, const char *fn, const AggState &st, gkd_merges *out, 
     return GKD_OK;
 }
 
-// One complete- or average-linkage agglomeration on the context's device: start() checks the free memory and sets up
-// the matrix and state of agglomerate.cu in one buffer of the call; the distances are scattered into it; finish() runs
-// the rounds, reads the merges back and writes them to out in the sequential order.  gkd_all_vs_all_agglomerate: each
-// chunk's distances (the dense epilogue's doubles) go straight into the matrix; a chunk whose join overflowed writes
-// nothing and its redo writes the same entries, so the rounds in finish() see final values.  gkd_agglomerate: start()
-// scatters the caller's triangle dist.
-struct Agglomeration : Form {
+// A form whose engine runs on an n x n matrix of the call's distances in one device buffer (agglomerate.cu, nj.cu).
+// gkd_all_vs_all_*: each chunk's distances (the dense epilogue's doubles) go straight into the matrix; a chunk whose join
+// overflowed writes nothing and its redo writes the same entries, so finish() sees final values.  Over a caller's
+// triangle, start() scatters it.
+struct DenseMatrix : Form {
     const char *fn;
     uint32_t n;
-    int average;
-    double max_dist;
     const double *dist;  // the caller's triangle (host or device memory), or nullptr
-    gkd_merges *out;
+    const char *range;   // the NVTX range of queue()
     void *buf = nullptr;
     cudaStream_t stream = nullptr;
-    AggState st{};
-    Agglomeration(const char *fn_, uint32_t n_, int method, double d, const double *dist_, gkd_merges *out_)
-        : fn(fn_), n(n_), average(method == GKD_LINK_AVERAGE), max_dist(d), dist(dist_), out(out_) {}
-    ~Agglomeration() {
+    DenseMatrix(const char *fn_, uint32_t n_, const double *dist_, const char *range_) : fn(fn_), n(n_), dist(dist_), range(range_) {}
+    ~DenseMatrix() {
         if (buf) cudaFreeAsync(buf, stream);
     }
-    std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->height, out->size}; }
-    int start(gkd_ctx *c) override {
-        out->n = 0;
-        c->m.agglomerate_rounds = 0;
-        if (n < 2) return GKD_OK;
-        const uint64_t need = agg_state_bytes(n, average), room = agg_dense_room();
+    // entries [first, first + count) of the triangle, as doubles in device memory
+    virtual int scatter(gkd_ctx *c, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err) = 0;
+    // buf = need bytes of device memory, or GKD_ENOMEM naming them (what: the engine, for the message)
+    int alloc(gkd_ctx *c, uint64_t need, const char *what) {
+        const uint64_t room = agg_dense_room();
         if (need > room)
-            return fail(c, GKD_ENOMEM, "%s: %s linkage of %u sets needs %llu bytes of device memory; %llu are free", fn,
-                        average ? "average" : "complete", n, (unsigned long long)need, (unsigned long long)room);
+            return fail(c, GKD_ENOMEM, "%s: %s of %u sets needs %llu bytes of device memory; %llu are free", fn, what, n,
+                        (unsigned long long)need, (unsigned long long)room);
         stream = c->stream;
         CK(cudaMallocAsync(&buf, need, c->stream));
-        st = agg_state_at(buf, n, average);
-        CK(launch_agg_init(st, c->stream));
-        c->m.launches++;
+        return GKD_OK;
+    }
+    // the caller's triangle, when there is one, through scatter()
+    int stage(gkd_ctx *c) {
         if (!dist) return GKD_OK;
         const uint64_t total = (uint64_t)n * (n - 1) / 2;
         const bool on_device = classify(dist) == MEM_DEVICE;
@@ -1728,22 +1722,46 @@ struct Agglomeration : Form {
         }
         return GKD_OK;
     }
-    // entries [first, first + count) of the triangle, as doubles in device memory
-    int scatter(gkd_ctx *c, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err) {
-        CK(launch_agg_scatter(st, src, first, count, join_err, c->stream));
-        c->m.launches++;
-        return GKD_OK;
-    }
     int queue(gkd_ctx *c, const Chunk &e, uint64_t &d2h) override {
         int rc = ensure(c, c->d_dist, e.cnt * 8);
         if (rc) return rc;
-        nvtxRangePushA("gkd kernel 5: agglomerate matrix");
+        nvtxRangePushA(range);
         CK(launch_epilogue(e.src, e.pc, EpilogueOut{nullptr, (double *)c->d_dist.p, nullptr, nullptr}, c->stream));
         c->m.launches++;
         rc = scatter(c, (const double *)c->d_dist.p, e.src.first, e.cnt, e.join_err);
         nvtxRangePop();
         if (rc) return rc;
         CK(cudaEventRecord(c->ev[7], c->stream));
+        return GKD_OK;
+    }
+};
+
+// One complete- or average-linkage agglomeration on the context's device: start() checks the free memory and sets up
+// the matrix and state of agglomerate.cu in one buffer of the call; the distances are scattered into it; finish() runs
+// the rounds, reads the merges back and writes them to out in the sequential order.
+struct Agglomeration : DenseMatrix {
+    int average;
+    double max_dist;
+    gkd_merges *out;
+    AggState st{};
+    Agglomeration(const char *fn_, uint32_t n_, int method, double d, const double *dist_, gkd_merges *out_)
+        : DenseMatrix(fn_, n_, dist_, "gkd kernel 5: agglomerate matrix"), average(method == GKD_LINK_AVERAGE), max_dist(d),
+          out(out_) {}
+    std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->height, out->size}; }
+    int start(gkd_ctx *c) override {
+        out->n = 0;
+        c->m.agglomerate_rounds = 0;
+        if (n < 2) return GKD_OK;
+        int rc = alloc(c, agg_state_bytes(n, average), average ? "average linkage" : "complete linkage");
+        if (rc) return rc;
+        st = agg_state_at(buf, n, average);
+        CK(launch_agg_init(st, c->stream));
+        c->m.launches++;
+        return stage(c);
+    }
+    int scatter(gkd_ctx *c, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err) override {
+        CK(launch_square_scatter(agg_square(st), src, first, count, join_err, c->stream));
+        c->m.launches++;
         return GKD_OK;
     }
     int finish(gkd_ctx *c) override {
@@ -1761,6 +1779,62 @@ struct Agglomeration : Form {
         const AggThreshold thr = agg_threshold(max_dist);
         CK(cudaEventRecord(c->ev[6], c->stream));
         return agg_merges(c, fn, st, out, [&](uint32_t batch) { return launch_agg_rounds(st, thr, batch, c->n_sms, c->stream); });
+    }
+};
+
+// One neighbour-joining tree on the context's device: start() checks the free memory and sets up the matrix and state of
+// nj.cu in one buffer of the call; the distances are scattered into it; finish() queues the start sums and all n - 1
+// rounds, then reads the rows back once.
+struct NeighborJoining : DenseMatrix {
+    gkd_joins *out;
+    NjState st{};
+    NeighborJoining(const char *fn_, uint32_t n_, const double *dist_, gkd_joins *out_)
+        : DenseMatrix(fn_, n_, dist_, "gkd kernel 5: neighbour-joining matrix"), out(out_) {}
+    std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->len_a, out->len_b}; }
+    int start(gkd_ctx *c) override {
+        out->n = 0;
+        c->m.agglomerate_rounds = 0;
+        if (n < 2) return GKD_OK;
+        int rc = alloc(c, nj_state_bytes(n), "neighbour joining");
+        if (rc) return rc;
+        st = nj_state_at(buf, n);
+        CK(cudaMemsetAsync(st.bad, 0xFF, 8, c->stream));
+        CK(cudaMemsetAsync(st.ticket, 0, 4, c->stream));
+        return stage(c);
+    }
+    int scatter(gkd_ctx *c, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err) override {
+        CK(launch_square_scatter(nj_square(st), src, first, count, join_err, c->stream));
+        c->m.launches++;
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) override {
+        if (n < 2) return GKD_OK;
+        unsigned long long bad = 0;
+        CK(cudaMemcpyAsync(&bad, st.bad, 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += 8;
+        if (bad != ~0ull) {
+            uint32_t i, j;
+            upper_pair(bad, n, i, j);
+            return fail(c, GKD_EINVAL, "%s: the distance of pair (%u, %u) is not a finite value in [0, 2]", fn, i, j);
+        }
+        CK(cudaEventRecord(c->ev[6], c->stream));
+        CK(launch_nj_rounds(st, c->n_sms, c->stream));
+        c->m.launches += nj_launches(n);
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        const uint64_t rows = n - 1, w = std::min<uint64_t>(rows, out->cap);
+        if (w) {
+            if (out->a) CK(cudaMemcpyAsync(out->a, st.ra, w * 4, cudaMemcpyDefault, c->stream));
+            if (out->b) CK(cudaMemcpyAsync(out->b, st.rb, w * 4, cudaMemcpyDefault, c->stream));
+            if (out->len_a) CK(cudaMemcpyAsync(out->len_a, st.la, w * 8, cudaMemcpyDefault, c->stream));
+            if (out->len_b) CK(cudaMemcpyAsync(out->len_b, st.lb, w * 8, cudaMemcpyDefault, c->stream));
+        }
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += ((out->a ? 4 : 0) + (out->b ? 4 : 0) + (out->len_a ? 8 : 0) + (out->len_b ? 8 : 0)) * w;
+        c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+        c->m.agglomerate_rounds = rows;
+        out->n = rows;
+        return GKD_OK;
     }
 };
 
@@ -2809,6 +2883,31 @@ int gkd_agglomerate(gkd_ctx *c, uint32_t n, const double *dist, int method, doub
     if (rc) return rc;
     if (!dist && n >= 2) return fail(c, GKD_EINVAL, "%s: null dist", fn);
     Agglomeration f(fn, n, method, max_dist, dist, out);
+    return run_call(c, fn, triangle(0), f);
+}
+
+// ---- neighbour joining ------------------------------------------------------------------------------------------
+int gkd_all_vs_all_nj(gkd_ctx *c, uint32_t n, gkd_joins *out) {
+    const char *fn = "gkd_all_vs_all_nj";
+    if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
+    NeighborJoining f(fn, n, nullptr, out);
+    return run_call(c, fn, triangle(n), f);
+}
+
+// the caller's triangle is scattered by the form's start(): a call without pairs to intersect.  A host triangle is
+// checked here, before the context is used; the scatter checks a device one.
+int gkd_nj(gkd_ctx *c, uint32_t n, const double *dist, gkd_joins *out) {
+    const char *fn = "gkd_nj";
+    if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
+    if (!dist && n >= 2) return fail(c, GKD_EINVAL, "%s: null dist", fn);
+    if (n >= 2 && classify(dist) != MEM_DEVICE) {
+        const double *d = dist;
+        for (uint32_t i = 0; i + 1 < n; i++)
+            for (uint32_t j = i + 1; j < n; j++, d++)
+                if (!(*d >= 0.0 && *d <= 2.0))
+                    return fail(c, GKD_EINVAL, "%s: the distance of pair (%u, %u) is not a finite value in [0, 2]", fn, i, j);
+    }
+    NeighborJoining f(fn, n, dist, out);
     return run_call(c, fn, triangle(0), f);
 }
 

@@ -838,6 +838,26 @@ int gkd_group_all_vs_all_linkage(gkd_group *g, double max_dist, gkd_hits *out) {
     }
 }
 
+// The host triangle of all N(N-1)/2 distances, filled through the dense ring, for an engine member 0 then runs on it
+// with `need` bytes of device memory (what: the engine, for the message).  Both allocations are checked before any pair
+// is intersected.
+static int group_triangle(gkd_group *g, const char *fn, const char *what, uint64_t need, std::vector<double> &dist) {
+    const uint64_t N = g->n_genomes;
+    const uint64_t tri = N * (N - (N > 0)) / 2;
+    try {
+        dist.resize(tri);
+    } catch (const std::bad_alloc &) {
+        return gfail(g, GKD_ENOMEM, "%s: the host triangle of %llu sets needs %llu bytes", fn, (unsigned long long)N,
+                     (unsigned long long)(tri * 8));
+    }
+    if (cudaSetDevice(g->members[0].device) != cudaSuccess) return gfail(g, GKD_ECUDA, "%s: cannot select the device of member 0", fn);
+    const uint64_t room = gkd::agg_dense_room();
+    if (N >= 2 && need > room)
+        return gfail(g, GKD_ENOMEM, "%s: %s of %llu sets needs %llu bytes of device memory on member 0; %llu are free", fn, what,
+                     (unsigned long long)N, (unsigned long long)need, (unsigned long long)room);
+    return gkd_group_all_vs_all(g, nullptr, dist.data());
+}
+
 int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, gkd_merges *out) {
     if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_agglomerate: max_dist is NaN");
     if (method != GKD_LINK_COMPLETE && method != GKD_LINK_AVERAGE)
@@ -846,24 +866,10 @@ int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, 
     if (!g) return GKD_EINVAL;
     try {
         out->n = 0;
-        const uint64_t N = g->n_genomes;
-        // both allocations are checked before any pair is intersected: the host triangle, and the matrix of member 0
-        const uint64_t tri = N * (N - (N > 0)) / 2;
         std::vector<double> dist;
-        try {
-            dist.resize(tri);
-        } catch (const std::bad_alloc &) {
-            return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_agglomerate: the host triangle of %llu sets needs %llu bytes",
-                         (unsigned long long)N, (unsigned long long)(tri * 8));
-        }
-        if (cudaSetDevice(g->members[0].device) != cudaSuccess)
-            return gfail(g, GKD_ECUDA, "gkd_group_all_vs_all_agglomerate: cannot select the device of member 0");
-        const uint64_t need = gkd::agg_state_bytes(g->n_genomes, method == GKD_LINK_AVERAGE), room = gkd::agg_dense_room();
-        if (N >= 2 && need > room)
-            return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_agglomerate: %s linkage of %llu sets needs %llu bytes of device "
-                         "memory on member 0; %llu are free", method == GKD_LINK_AVERAGE ? "average" : "complete",
-                         (unsigned long long)N, (unsigned long long)need, (unsigned long long)room);
-        int rc = gkd_group_all_vs_all(g, nullptr, dist.data());
+        int rc = group_triangle(g, "gkd_group_all_vs_all_agglomerate",
+                                method == GKD_LINK_AVERAGE ? "average linkage" : "complete linkage",
+                                gkd::agg_state_bytes(g->n_genomes, method == GKD_LINK_AVERAGE), dist);
         if (rc != GKD_OK) return rc;
         gkd_ctx *c0 = g->members[0].ctx;
         if ((rc = gkd_agglomerate(c0, g->n_genomes, dist.data(), method, max_dist, out)) != GKD_OK)
@@ -871,6 +877,22 @@ int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, 
         return GKD_OK;
     } catch (const std::exception &ex) {
         return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_agglomerate: %s", ex.what());
+    }
+}
+
+int gkd_group_all_vs_all_nj(gkd_group *g, gkd_joins *out) {
+    if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nj: null out");
+    if (!g) return GKD_EINVAL;
+    try {
+        out->n = 0;
+        std::vector<double> dist;
+        int rc = group_triangle(g, "gkd_group_all_vs_all_nj", "neighbour joining", gkd::nj_state_bytes(g->n_genomes), dist);
+        if (rc != GKD_OK) return rc;
+        gkd_ctx *c0 = g->members[0].ctx;
+        if ((rc = gkd_nj(c0, g->n_genomes, dist.data(), out)) != GKD_OK) return gfail(g, rc, "member 0: %s", gkd_last_error(c0));
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_nj: %s", ex.what());
     }
 }
 

@@ -444,11 +444,23 @@ struct AggThreshold {  // v <= max_dist  <=>  S <= (m N) << shift (shift < 0: >>
 uint64_t agg_state_bytes(uint32_t n, int average);  // the matrix and the O(n) state, in one buffer
 AggState agg_state_at(void *base, uint32_t n, int average);
 cudaError_t launch_agg_init(const AggState &st, cudaStream_t s);
+// An n x n matrix the distances of a call are scattered into, entry (i, j) at [i n + j] and [j n + i]: w = d 2^53 (T =
+// uint64_t, agglomeration; hi, when not nullptr, gets the zero high words of the average sums) or w = d (T = double,
+// neighbour joining).
+template <typename T>
+struct Square {
+    T *w;
+    uint64_t *hi;
+    uint32_t n;
+    unsigned long long *bad;  // atomicMin of the pair index of a value that is not a valid entry
+};
+Square<uint64_t> agg_square(const AggState &st);
 // entries [first, first + count) of the row-major strict upper triangle of n, as doubles in src (device), into the
-// matrix; an entry that is not a multiple of 2^-53 in [0, 2] is recorded in AGG_BAD.  Nothing when join_err (may be
-// nullptr) reads nonzero on the stream: the chunk is redone.
-cudaError_t launch_agg_scatter(const AggState &st, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err,
-                               cudaStream_t s);
+// matrix; a value that is not a valid entry (uint64_t: a multiple of 2^-53 in [0, 2]; double: in [0, 2], so not NaN)
+// is recorded in *bad.  Nothing when join_err (may be nullptr) reads nonzero on the stream: the chunk is redone.
+template <typename T>
+cudaError_t launch_square_scatter(const Square<T> &sq, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err,
+                                  cudaStream_t s);
 // `rounds` rounds queued without a host read; a round after one that merged nothing exits at once (AGG_DONE)
 cudaError_t launch_agg_rounds(const AggState &st, AggThreshold thr, uint32_t rounds, int n_sms, cudaStream_t s);
 // the device bytes a dense agglomeration may take on the current device: the free memory, capped by the environment
@@ -504,6 +516,34 @@ __host__ __device__ inline int agg_cmp(uint64_t lo1, uint64_t hi1, uint64_t n1, 
     if (a0 != b0) return a0 < b0 ? -1 : 1;
     return 0;
 }
+// Neighbour joining (nj.cu, gkd_*_nj): the distances of the active clusters in an n x n matrix of doubles in HBM.  The
+// r active clusters of a round hold the slots 0 .. r - 1: when g leaves, the last active slot's row, column, sum and
+// label move into g's slot, so a round reads only the r x r corner.  label[slot] is the cluster's label (its smallest
+// id); Q and its ties are defined on labels, so the layout does not change the result.
+struct NjCand {  // a candidate pair: Q, labels a < b, and the slots of the two clusters
+    double q;
+    uint32_t a, b, sa, sb;
+};
+struct NjState {
+    uint32_t n;
+    double *d;                  // the matrix, entry (x, y) at [x n + y] and [y n + x]
+    double *R;                  // per slot: the row sum of the start, then as the rounds update it
+    uint32_t *label;            // per slot
+    NjCand *part;               // per CTA of the row scan: its best candidate
+    uint32_t *pick;             // the slots of f and g of the current round
+    unsigned int *ticket;       // CTAs of the row scan done (the last one picks)
+    unsigned long long *bad;    // the smallest pair index of an invalid input value (~0: none)
+    uint32_t *ra, *rb;          // the output rows (n - 1 each)
+    double *la, *lb;
+};
+constexpr uint32_t NJ_MAX_CTAS = 2048;  // row-scan CTAs of one round
+uint64_t nj_state_bytes(uint32_t n);    // the matrix and the O(n) state, in one buffer
+NjState nj_state_at(void *base, uint32_t n);
+inline Square<double> nj_square(const NjState &st) { return {st.d, nullptr, st.n, st.bad}; }
+// the start sums and all n - 1 rounds (n >= 2), queued without a host read: 3 (n - 2) + 2 launches; the rows are then in
+// ra, rb, la, lb.  *ticket must be 0 (the scatter's init sets it).
+cudaError_t launch_nj_rounds(const NjState &st, int n_sms, cudaStream_t s);
+inline uint64_t nj_launches(uint32_t n) { return n < 2 ? 0 : 3ull * (n - 2) + 2; }
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless
 // some representative is within max_dist; clears the counts it consumed
 cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *n_reps, uint32_t cand, uint32_t visit,

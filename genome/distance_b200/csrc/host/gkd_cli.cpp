@@ -144,6 +144,8 @@ const std::vector<OptSpec> FASTA_OPTS = {
     {{"--method"}, true, "linkage method of --linkage and --clusters: single (default), complete or average (UPGMA); a "
                          "complete or average merge line holds the two clusters' first records and the merge height "
                          "(additive option)"},
+    {{"--tree"}, false, "write the neighbour-joining tree of all records as one Newick line, rooted at the midpoint of "
+                        "its last edge, instead of the report (additive option)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
@@ -220,6 +222,7 @@ struct DistSource {
         }
         check(rc);
     }
+    void nj(gkd_joins &j) const { check(engine ? gkd_all_vs_all_nj(engine->raw(), n, &j) : gkd_group_all_vs_all_nj(grp, &j)); }
 };
 
 // one report line of fastaDist (:188-192)
@@ -287,6 +290,33 @@ uint32_t writeClusters(std::ostream &writer, const uint32_t *cluster, const Dist
     return clusters;
 }
 
+// a Newick label: single-quoted, with any ' doubled, when it holds whitespace or one of ()[]':;,
+std::string newickLabel(const char *label) {
+    std::string s(label);
+    if (s.find_first_of(" \t\n\v\f\r()[]':;,") == std::string::npos) return s;
+    std::string q = "'";
+    for (char ch : s) {
+        q += ch;
+        if (ch == '\'') q += '\'';
+    }
+    return q + "'";
+}
+
+// `fastaDist --tree`: row t of gkd_joins is the node (A:len_a,B:len_b) of the current subtrees of labels a and b; the
+// last row's node is the root.  One record: its label.  No records: nothing.
+void writeNewick(std::ostream &writer, const gkd_joins &j, const DistSource &src) {
+    if (src.n == 0) return;
+    std::vector<std::string> sub(src.n);
+    for (uint32_t i = 0; i < src.n; i++) sub[i] = newickLabel(src.label(i));
+    for (uint64_t t = 0; t < j.n; t++) {
+        std::string node = "(" + sub[j.a[t]] + ":" + javaDouble(j.len_a[t]) + "," + sub[j.b[t]] + ":" + javaDouble(j.len_b[t]) + ")";
+        sub[j.a[t]].swap(node);
+        std::string().swap(sub[j.b[t]]);
+    }
+    writer << sub[0] << ";\n";
+    writer.flush();
+}
+
 // pairs per gkd_all_vs_all_range_within call of `fastaDist --maxDist`: host memory stays O(range), not O(n^2)
 constexpr uint64_t WITHIN_RANGE = 64ull << 20;
 
@@ -325,6 +355,10 @@ int fastaDist(const std::vector<std::string> &args) {
     if (kmerSize == 0) kmerSize = kmerTypeDefaultK(seqType);
     if (kmerSize < 2) throw ParseFailureException("Kmer size must be at least 2.");
     if (batchSize < 1) throw ParseFailureException("Batch size must be at least 1.");
+    const bool tree = p.values.count("--tree") > 0;
+    if (tree)
+        for (const char *opt : {"--maxDist", "--nearest", "--clusters", "--linkage", "--method"})
+            if (p.values.count(opt)) throw ParseFailureException(std::string("--tree and ") + opt + " cannot be combined.");
     const bool within = p.values.count("--maxDist") > 0;
     const double maxDist = within ? toDouble("--maxDist", p.values["--maxDist"]) : 1.0;
     if (!(maxDist > 0.0 && maxDist <= 1.0)) throw ParseFailureException("Maximum distance must be > 0 and <= 1.");
@@ -383,11 +417,24 @@ int fastaDist(const std::vector<std::string> &args) {
     logInfo(std::to_string(src.n) + " sequences read from input.");
     // runReporter (:134-165): the batch cache and the per-row parallel streams are what the engine
     // replaces; every pair i<j is computed in one batched launch and printed in list order
-    if (!clusters) writer << "seq1\tname1\tseq2\tname2\tdistance\n";
+    if (!clusters && !tree) writer << "seq1\tname1\tseq2\tname2\tdistance\n";
     src.build();
     logInfo(std::to_string(src.n) + " sequences cached" + (src.grp ? " on " + std::to_string(src.gpus) + " GPUs" : "") +
             ". Computing distances.");
     const uint64_t n = src.n, total = n < 2 ? 0 : n * (n - 1) / 2;
+    if (tree) {
+        // each pair i < j is intersected once; the tree is joined on the GPU and only its n - 1 rows leave it
+        const uint64_t cap = n ? n - 1 : 0;
+        std::vector<uint32_t> a(cap), b(cap);
+        std::vector<double> la(cap), lb(cap);
+        gkd_joins j{a.data(), b.data(), la.data(), lb.data(), cap, 0};
+        src.nj(j);
+        writeNewick(writer, j, src);
+        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(j.n) +
+                " joins in the neighbor-joining tree.");
+        writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);
+        return 0;
+    }
     if (method && (clusters || linkage)) {
         // each pair i < j is intersected once; the agglomeration runs on the GPU and only its merges (<= n - 1) leave it
         const uint64_t cap = n ? n - 1 : 0;

@@ -9,7 +9,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (AMBIG_LITERAL, AMBIG_SKIP, DNA, PROT, RNA, STRAND_BOTH, STRAND_CANONICAL, GkdConfig, GkdHits,
-                   GkdMerges, GkdMetrics, GkdNeighbors, GkdOutputs, GkdPackedSet)
+                   GkdJoins, GkdMerges, GkdMetrics, GkdNeighbors, GkdOutputs, GkdPackedSet)
 
 PACKED_DTYPE = np.dtype([("offs_off", "<u8"), ("lows_off", "<u8"), ("pal_offs_off", "<u8"), ("pal_lows_off", "<u8"),
                          ("n", "<u4"), ("n_pal", "<u4"), ("level", "<u4"), ("pal_level", "<u4")])
@@ -53,6 +53,25 @@ def _merges(call, n: int):
     m = GkdMerges(a.ctypes.data, b.ctypes.data, height.ctypes.data, size.ctypes.data, cap, 0)
     call(m)
     return a[:m.n], b[:m.n], height[:m.n], size[:m.n]
+
+
+def _joins(call, n: int):
+    """(a, b, len_a, len_b) numpy arrays of a gkd_joins call `call(joins)`; n - 1 entries always suffice"""
+    cap = max(int(n) - 1, 0)
+    a, b = np.empty(cap, dtype=np.uint32), np.empty(cap, dtype=np.uint32)
+    len_a, len_b = np.empty(cap, dtype=np.float64), np.empty(cap, dtype=np.float64)
+    j = GkdJoins(a.ctypes.data, b.ctypes.data, len_a.ctypes.data, len_b.ctypes.data, cap, 0)
+    call(j)
+    return a[:j.n], b[:j.n], len_a[:j.n], len_b[:j.n]
+
+
+def _triangle_n(dist) -> int:
+    """n of a row-major strict upper triangle of n(n-1)/2 entries (numpy array or tensor); ValueError otherwise"""
+    m = int(dist.numel() if _is_torch(dist) else np.asarray(dist).size)
+    n = int(round((1 + (1 + 8 * m) ** 0.5) / 2)) if m else 0
+    if n * (n - 1) // 2 != m:
+        raise ValueError(f"{m} distances are not a strict upper triangle")
+    return n
 
 
 class GkdError(RuntimeError):
@@ -396,10 +415,7 @@ class Engine:
     def agglomerate(self, dist, method: int, max_dist: float):
         """all_vs_all_agglomerate over a caller's row-major strict upper triangle of distances (a float64 numpy array
         or CUDA tensor of n(n-1)/2 entries, read and not modified), on this context's device"""
-        m = int(dist.numel() if _is_torch(dist) else np.asarray(dist).size)
-        n = int(round((1 + (1 + 8 * m) ** 0.5) / 2)) if m else 0
-        if n * (n - 1) // 2 != m:
-            raise ValueError(f"{m} distances are not a strict upper triangle")
+        n = _triangle_n(dist)
         ptr, _, keep = _array(dist, np.float64, ("float64",), "dist must be a contiguous float64 tensor")
         out = _merges(lambda mg: self._ck(self._L.gkd_agglomerate(self._h, n, ptr, int(method), float(max_dist),
                                                                  C.byref(mg))), n)
@@ -425,6 +441,23 @@ class Engine:
         out = _merges(lambda mg: self._ck(self._L.gkd_complete_linkage(self._h, int(n), C.byref(h), float(max_dist),
                                                                       C.byref(mg))), int(n))
         del ka, kb, kd
+        return out
+
+    def all_vs_all_nj(self, n: int = None):
+        """(a, b, len_a, len_b): the neighbour-joining tree of the first n sets (default: all), one row per join (n - 1
+        rows), rooted at the midpoint of the last edge; row t joins the current subtrees of labels a < b (each the
+        smallest id of its subtree) with branch lengths len_a and len_b.  Every pair is intersected once and its
+        distance stays on the device"""
+        n = len(self) if n is None else int(n)
+        return _joins(lambda j: self._ck(self._L.gkd_all_vs_all_nj(self._h, n, C.byref(j))), n)
+
+    def nj(self, dist):
+        """all_vs_all_nj over a caller's row-major strict upper triangle of distances (a float64 numpy array or CUDA
+        tensor of n(n-1)/2 finite entries in [0, 2], read and not modified), on this context's device"""
+        n = _triangle_n(dist)
+        ptr, _, keep = _array(dist, np.float64, ("float64",), "dist must be a contiguous float64 tensor")
+        out = _joins(lambda j: self._ck(self._L.gkd_nj(self._h, n, ptr, C.byref(j))), n)
+        del keep
         return out
 
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
@@ -624,3 +657,7 @@ class Group:
         """(a, b, height, size) over all global ids: the single-context Engine.all_vs_all_complete_linkage result"""
         return _merges(lambda m: self._ck(self._L.gkd_group_all_vs_all_complete_linkage(self._h, float(max_dist),
                                                                                         C.byref(m))), len(self))
+
+    def all_vs_all_nj(self):
+        """(a, b, len_a, len_b) over all global ids: the single-context Engine.all_vs_all_nj result"""
+        return _joins(lambda j: self._ck(self._L.gkd_group_all_vs_all_nj(self._h, C.byref(j))), len(self))

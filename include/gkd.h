@@ -344,6 +344,38 @@ int gkd_all_vs_all_complete_linkage(gkd_ctx *ctx, uint32_t n, double max_dist, g
  * absent from the list are beyond max_dist; listed pairs beyond max_dist take part in no merge. */
 int gkd_complete_linkage(gkd_ctx *ctx, uint32_t n, const gkd_hits *pairs, double max_dist, gkd_merges *out);
 
+/* Neighbour-joining (NJ) tree of the first n sets.  d(i, j) is the dense call's double; a cluster's label is its
+ * smallest id.  Every operation below is one IEEE double operation rounded to nearest, in the order written (no fused
+ * multiply-add), so the rows are defined bit for bit:
+ *   start:  R_i = (((0 + d(i, 0)) + d(i, 1)) + ... + d(i, n - 1)), ascending k, d(i, i) = 0;
+ *   rounds, while r >= 3 clusters are active: for every pair of active labels a < b,
+ *           Q(a, b) = ((double)(r - 2) d(a, b) - R_a) - R_b; (f, g) is the pair with the smallest (Q, a, b), Q compared
+ *           as doubles (-0.0 == +0.0, ties to the smaller labels); t = (R_f - R_g) / (double)(2 (r - 2));
+ *           len_a = 0.5 d(f, g) + t, len_b = d(f, g) - len_a; for every other active k,
+ *           d(u, k) = 0.5 ((d(f, k) + d(g, k)) - d(f, g)) and R_k = ((R_k - d(f, k)) - d(g, k)) + d(u, k);
+ *           R_u = 0.5 ((R_f + R_g) - (double)r d(f, g)).  The new cluster u takes label f, label g goes inactive, and
+ *           the row (f, g, len_a, len_b) is appended;
+ *   last:   at r = 2 the row (a, b, 0.5 d(a, b), 0.5 d(a, b)), which roots the tree at the midpoint of its last edge.
+ * So the rows form a binary tree as the rows of gkd_merges do: row t joins the current subtrees of labels a and b.
+ * Negative branch lengths are reported as computed.  out->n = n - 1 for n >= 2, else 0; only the first min(n, cap)
+ * entries are written.  Any array may be NULL; host or device memory as for gkd_hits.
+ * Device memory: an n x n matrix of 8 B entries and O(n) state (36 B per set); the call fails with GKD_ENOMEM, naming
+ * the bytes, before any pair is intersected when that exceeds the free device memory.  Only the rows (24 B each) leave
+ * the device. */
+typedef struct gkd_joins {
+    uint32_t *a, *b;        /* labels of the two clusters joined, a < b */
+    double *len_a, *len_b;  /* branch lengths from the new node to a's and to b's cluster */
+    uint64_t cap;           /* entries each non-NULL array can hold */
+    uint64_t n;             /* out: n - 1 for n >= 2, else 0; only min(n, cap) are written */
+} gkd_joins;
+/* Every pair i < j is intersected once and its distance written straight into the matrix on the device. */
+int gkd_all_vs_all_nj(gkd_ctx *ctx, uint32_t n, gkd_joins *out);
+/* The same tree over a caller's row-major strict upper triangle of n(n-1)/2 distances (host or device memory; read, not
+ * modified), on the context's device.  n is not tied to the context's sets.  Every value must be finite and in [0, 2]:
+ * one that is not fails the call with GKD_EINVAL, naming the pair (a host triangle is checked before the context is
+ * used). */
+int gkd_nj(gkd_ctx *ctx, uint32_t n, const double *dist, gkd_joins *out);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -395,6 +427,10 @@ int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, 
  * the pairs within max_dist as gkd_group_all_vs_all_within does, the host orders them by (a, b) (32 B per pair of host
  * memory) and member 0 runs gkd_complete_linkage on them.  The arrays of out are host memory. */
 int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_merges *out);
+/* gkd_all_vs_all_nj over all global ids; equal to one context's rows, bit for bit.  The members fill a host triangle
+ * as gkd_group_all_vs_all_agglomerate does, then member 0 runs gkd_nj on it.  Both allocations are checked before any
+ * pair is intersected (GKD_ENOMEM, naming the bytes).  The arrays of out are host memory. */
+int gkd_group_all_vs_all_nj(gkd_group *g, gkd_joins *out);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

@@ -319,3 +319,30 @@ JNIEXPORT jint JNICALL FN(allVsAllCompleteLinkage)(JNIEnv *env, jclass c, jlong 
     (void)c;
     return merges_into(env, complete_sparse, h, n, GKD_LINK_COMPLETE, maxDist, a, b, height, size, nMerges);
 }
+
+/* the neighbour-joining tree of the first n sets: a, b, lenA, lenB hold n - 1 entries (the joins in order); nJoins[0]
+ * receives their number */
+JNIEXPORT jint JNICALL FN(allVsAllNj)(JNIEnv *env, jclass c, jlong h, jint n, jintArray a, jintArray b, jdoubleArray lenA,
+                                      jdoubleArray lenB, jintArray nJoins) {
+    (void)c;
+    if (!a || !b || !lenA || !lenB || !nJoins || n < 0 || (*env)->GetArrayLength(env, nJoins) < 1) return GKD_EINVAL;
+    const jint cap = n > 0 ? n - 1 : 0;
+    if ((*env)->GetArrayLength(env, a) < cap || (*env)->GetArrayLength(env, b) < cap ||
+        (*env)->GetArrayLength(env, lenA) < cap || (*env)->GetArrayLength(env, lenB) < cap)
+        return GKD_EINVAL;
+    jint *pa = (*env)->GetIntArrayElements(env, a, NULL);
+    jint *pb = (*env)->GetIntArrayElements(env, b, NULL);
+    jdouble *pla = (*env)->GetDoubleArrayElements(env, lenA, NULL);
+    jdouble *plb = (*env)->GetDoubleArrayElements(env, lenB, NULL);
+    gkd_joins out = {(uint32_t *)pa, (uint32_t *)pb, pla, plb, (uint64_t)cap, 0};
+    int rc = (pa && pb && pla && plb) ? gkd_all_vs_all_nj(CTX(h), (uint32_t)n, &out) : GKD_ENOMEM;
+    if (plb) (*env)->ReleaseDoubleArrayElements(env, lenB, plb, 0);
+    if (pla) (*env)->ReleaseDoubleArrayElements(env, lenA, pla, 0);
+    if (pb) (*env)->ReleaseIntArrayElements(env, b, pb, 0);
+    if (pa) (*env)->ReleaseIntArrayElements(env, a, pa, 0);
+    if (rc == GKD_OK) {
+        jint nj = (jint)out.n;
+        (*env)->SetIntArrayRegion(env, nJoins, 0, 1, &nj);
+    }
+    return rc;
+}

@@ -232,6 +232,17 @@ public class GpuKmerEngine implements AutoCloseable {
         return merges[0];
     }
 
+    /** the neighbour-joining tree of every set, rooted at the midpoint of its last edge: join t merges the current
+     *  subtrees whose smallest ids are a[t] &lt; b[t], with branch lengths lenA[t] and lenB[t] from the new node (the
+     *  arrays hold at least size() - 1 entries).  Returns the number of joins, size() - 1 (0 for fewer than two sets).
+     *  Every pair is intersected once; the distances stay on the GPU and only the joins leave it. */
+    public synchronized int allVsAllNj(int[] a, int[] b, double[] lenA, double[] lenB) {
+        this.build();
+        int[] joins = new int[1];
+        check(GkdNative.allVsAllNj(this.ctx, this.size(), a, b, lenA, lenB, joins));
+        return joins[0];
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
