@@ -99,6 +99,7 @@ SYMBOLS = {
     "gkd_group_all_vs_all_agglomerate": (_i32, [_vp, _i32, _dbl, C.POINTER(GkdMerges)]),
     "gkd_group_all_vs_all_complete_linkage": (_i32, [_vp, _dbl, C.POINTER(GkdMerges)]),
     "gkd_group_all_vs_all_nj": (_i32, [_vp, C.POINTER(GkdJoins)]),
+    "gkd_group_all_vs_all_bionj": (_i32, [_vp, C.POINTER(GkdJoins)]),
     "gkd_build_sets": (_i32, [_vp]),
     "gkd_set_size": (_i32, [_vp, _u32, _pu64, _pu64, _pu64]),
     "gkd_export_set": (_i32, [_vp, _u32, _vp, _u64, _pu64]),
@@ -135,6 +136,8 @@ SYMBOLS = {
     "gkd_complete_linkage": (_i32, [_vp, _u32, C.POINTER(GkdHits), _dbl, C.POINTER(GkdMerges)]),
     "gkd_all_vs_all_nj": (_i32, [_vp, _u32, C.POINTER(GkdJoins)]),
     "gkd_nj": (_i32, [_vp, _u32, _vp, C.POINTER(GkdJoins)]),
+    "gkd_all_vs_all_bionj": (_i32, [_vp, _u32, C.POINTER(GkdJoins)]),
+    "gkd_bionj": (_i32, [_vp, _u32, _vp, C.POINTER(GkdJoins)]),
     "gkd_hash_set": (_i32, [_vp, _u32, _u32, _i32, _vp, _pu32]),
     "gkd_sketch_distances": (_i32, [_vp, _u32, _i32, _vp, _vp, _u64, _vp]),
     "gkd_format_double": (_i32, [_dbl, C.c_char_p, C.c_size_t]),

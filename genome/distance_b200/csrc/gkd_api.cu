@@ -1782,22 +1782,24 @@ struct Agglomeration : DenseMatrix {
     }
 };
 
-// One neighbour-joining tree on the context's device: start() checks the free memory and sets up the matrix and state of
-// nj.cu in one buffer of the call; the distances are scattered into it; finish() queues the start sums and all n - 1
-// rounds, then reads the rows back once.
+// One neighbour-joining (bionj: BIONJ) tree on the context's device: start() checks the free memory and sets up the
+// matrix and state of nj.cu in one buffer of the call; the distances are scattered into it; finish() queues the start
+// sums and all n - 1 rounds, then reads the rows back once.
 struct NeighborJoining : DenseMatrix {
+    bool bionj;
     gkd_joins *out;
     NjState st{};
-    NeighborJoining(const char *fn_, uint32_t n_, const double *dist_, gkd_joins *out_)
-        : DenseMatrix(fn_, n_, dist_, "gkd kernel 5: neighbour-joining matrix"), out(out_) {}
+    NeighborJoining(const char *fn_, uint32_t n_, const double *dist_, bool bionj_, gkd_joins *out_)
+        : DenseMatrix(fn_, n_, dist_, bionj_ ? "gkd kernel 5: BIONJ matrix" : "gkd kernel 5: neighbour-joining matrix"),
+          bionj(bionj_), out(out_) {}
     std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->len_a, out->len_b}; }
     int start(gkd_ctx *c) override {
         out->n = 0;
         c->m.agglomerate_rounds = 0;
         if (n < 2) return GKD_OK;
-        int rc = alloc(c, nj_state_bytes(n), "neighbour joining");
+        int rc = bionj ? alloc(c, bionj_state_bytes(n), "BIONJ") : alloc(c, nj_state_bytes(n), "neighbour joining");
         if (rc) return rc;
-        st = nj_state_at(buf, n);
+        st = nj_state_at(buf, n, bionj);
         CK(cudaMemsetAsync(st.bad, 0xFF, 8, c->stream));
         CK(cudaMemsetAsync(st.ticket, 0, 4, c->stream));
         return stage(c);
@@ -2887,17 +2889,15 @@ int gkd_agglomerate(gkd_ctx *c, uint32_t n, const double *dist, int method, doub
 }
 
 // ---- neighbour joining ------------------------------------------------------------------------------------------
-int gkd_all_vs_all_nj(gkd_ctx *c, uint32_t n, gkd_joins *out) {
-    const char *fn = "gkd_all_vs_all_nj";
+static int all_vs_all_joins(gkd_ctx *c, const char *fn, uint32_t n, bool bionj, gkd_joins *out) {
     if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
-    NeighborJoining f(fn, n, nullptr, out);
+    NeighborJoining f(fn, n, nullptr, bionj, out);
     return run_call(c, fn, triangle(n), f);
 }
 
 // the caller's triangle is scattered by the form's start(): a call without pairs to intersect.  A host triangle is
 // checked here, before the context is used; the scatter checks a device one.
-int gkd_nj(gkd_ctx *c, uint32_t n, const double *dist, gkd_joins *out) {
-    const char *fn = "gkd_nj";
+static int joins_of_triangle(gkd_ctx *c, const char *fn, uint32_t n, const double *dist, bool bionj, gkd_joins *out) {
     if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
     if (!dist && n >= 2) return fail(c, GKD_EINVAL, "%s: null dist", fn);
     if (n >= 2 && classify(dist) != MEM_DEVICE) {
@@ -2907,8 +2907,17 @@ int gkd_nj(gkd_ctx *c, uint32_t n, const double *dist, gkd_joins *out) {
                 if (!(*d >= 0.0 && *d <= 2.0))
                     return fail(c, GKD_EINVAL, "%s: the distance of pair (%u, %u) is not a finite value in [0, 2]", fn, i, j);
     }
-    NeighborJoining f(fn, n, dist, out);
+    NeighborJoining f(fn, n, dist, bionj, out);
     return run_call(c, fn, triangle(0), f);
+}
+
+int gkd_all_vs_all_nj(gkd_ctx *c, uint32_t n, gkd_joins *out) { return all_vs_all_joins(c, "gkd_all_vs_all_nj", n, false, out); }
+int gkd_nj(gkd_ctx *c, uint32_t n, const double *dist, gkd_joins *out) { return joins_of_triangle(c, "gkd_nj", n, dist, false, out); }
+int gkd_all_vs_all_bionj(gkd_ctx *c, uint32_t n, gkd_joins *out) {
+    return all_vs_all_joins(c, "gkd_all_vs_all_bionj", n, true, out);
+}
+int gkd_bionj(gkd_ctx *c, uint32_t n, const double *dist, gkd_joins *out) {
+    return joins_of_triangle(c, "gkd_bionj", n, dist, true, out);
 }
 
 // ---- complete linkage from the pairs within max_dist ------------------------------------------------------------

@@ -880,20 +880,31 @@ int gkd_group_all_vs_all_agglomerate(gkd_group *g, int method, double max_dist, 
     }
 }
 
-int gkd_group_all_vs_all_nj(gkd_group *g, gkd_joins *out) {
-    if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_nj: null out");
+// a tree over all global ids: the host triangle through group_triangle, then `call` (gkd_nj or gkd_bionj) on member 0
+// with `need` bytes of its device memory
+static int group_joins(gkd_group *g, const char *fn, const char *what, uint64_t need,
+                       int (*call)(gkd_ctx *, uint32_t, const double *, gkd_joins *), gkd_joins *out) {
+    if (!out) return gfail(g, GKD_EINVAL, "%s: null out", fn);
     if (!g) return GKD_EINVAL;
     try {
         out->n = 0;
         std::vector<double> dist;
-        int rc = group_triangle(g, "gkd_group_all_vs_all_nj", "neighbour joining", gkd::nj_state_bytes(g->n_genomes), dist);
+        int rc = group_triangle(g, fn, what, need, dist);
         if (rc != GKD_OK) return rc;
         gkd_ctx *c0 = g->members[0].ctx;
-        if ((rc = gkd_nj(c0, g->n_genomes, dist.data(), out)) != GKD_OK) return gfail(g, rc, "member 0: %s", gkd_last_error(c0));
+        if ((rc = call(c0, g->n_genomes, dist.data(), out)) != GKD_OK) return gfail(g, rc, "member 0: %s", gkd_last_error(c0));
         return GKD_OK;
     } catch (const std::exception &ex) {
-        return gfail(g, GKD_ENOMEM, "gkd_group_all_vs_all_nj: %s", ex.what());
+        return gfail(g, GKD_ENOMEM, "%s: %s", fn, ex.what());
     }
+}
+
+int gkd_group_all_vs_all_nj(gkd_group *g, gkd_joins *out) {
+    return group_joins(g, "gkd_group_all_vs_all_nj", "neighbour joining", g ? gkd::nj_state_bytes(g->n_genomes) : 0, gkd_nj, out);
+}
+
+int gkd_group_all_vs_all_bionj(gkd_group *g, gkd_joins *out) {
+    return group_joins(g, "gkd_group_all_vs_all_bionj", "BIONJ", g ? gkd::bionj_state_bytes(g->n_genomes) : 0, gkd_bionj, out);
 }
 
 int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_merges *out) {

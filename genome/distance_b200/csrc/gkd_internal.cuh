@@ -520,14 +520,18 @@ __host__ __device__ inline int agg_cmp(uint64_t lo1, uint64_t hi1, uint64_t n1, 
 // r active clusters of a round hold the slots 0 .. r - 1: when g leaves, the last active slot's row, column, sum and
 // label move into g's slot, so a round reads only the r x r corner.  label[slot] is the cluster's label (its smallest
 // id); Q and its ties are defined on labels, so the layout does not change the result.
+// BIONJ (gkd_*_bionj) runs on the same matrix: d(x, y) stays in the upper triangle, [min n + max], and the variance
+// V(x, y) lives in the lower one, [max n + min].  The fill writes d to both, so V starts equal to d.
 struct NjCand {  // a candidate pair: Q, labels a < b, and the slots of the two clusters
     double q;
     uint32_t a, b, sa, sb;
 };
 struct NjState {
     uint32_t n;
-    double *d;                  // the matrix, entry (x, y) at [x n + y] and [y n + x]
+    double *d;                  // the matrix, entry (x, y) at [x n + y] and [y n + x] (BIONJ: d above, V below)
     double *R;                  // per slot: the row sum of the start, then as the rounds update it
+    double *S;                  // BIONJ only (else nullptr): per slot, the row sum of V, kept as R is
+    double *lambda;             // BIONJ only: the current round's weight of f, set by the pick
     uint32_t *label;            // per slot
     NjCand *part;               // per CTA of the row scan: its best candidate
     uint32_t *pick;             // the slots of f and g of the current round
@@ -537,11 +541,12 @@ struct NjState {
     double *la, *lb;
 };
 constexpr uint32_t NJ_MAX_CTAS = 2048;  // row-scan CTAs of one round
-uint64_t nj_state_bytes(uint32_t n);    // the matrix and the O(n) state, in one buffer
-NjState nj_state_at(void *base, uint32_t n);
+uint64_t nj_state_bytes(uint32_t n);     // the matrix and the O(n) state, in one buffer
+uint64_t bionj_state_bytes(uint32_t n);  // nj_state_bytes plus S and lambda
+NjState nj_state_at(void *base, uint32_t n, bool bionj);
 inline Square<double> nj_square(const NjState &st) { return {st.d, nullptr, st.n, st.bad}; }
-// the start sums and all n - 1 rounds (n >= 2), queued without a host read: 3 (n - 2) + 2 launches; the rows are then in
-// ra, rb, la, lb.  *ticket must be 0 (the scatter's init sets it).
+// the start sums and all n - 1 rounds (n >= 2) of NJ, or of BIONJ when st.S is set, queued without a host read:
+// 3 (n - 2) + 2 launches; the rows are then in ra, rb, la, lb.  *ticket must be 0 (the scatter's init sets it).
 cudaError_t launch_nj_rounds(const NjState &st, int n_sms, cudaStream_t s);
 inline uint64_t nj_launches(uint32_t n) { return n < 2 ? 0 : 3ull * (n - 2) + 2; }
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless

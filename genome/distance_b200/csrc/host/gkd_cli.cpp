@@ -146,6 +146,8 @@ const std::vector<OptSpec> FASTA_OPTS = {
                          "(additive option)"},
     {{"--tree"}, false, "write the neighbour-joining tree of all records as one Newick line, rooted at the midpoint of "
                         "its last edge, instead of the report (additive option)"},
+    {{"--treeMethod"}, true, "tree method of --tree: nj (default, neighbour joining) or bionj (BIONJ, which weights each "
+                             "join by the variances of the distances) (additive option)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
@@ -223,6 +225,9 @@ struct DistSource {
         check(rc);
     }
     void nj(gkd_joins &j) const { check(engine ? gkd_all_vs_all_nj(engine->raw(), n, &j) : gkd_group_all_vs_all_nj(grp, &j)); }
+    void bionj(gkd_joins &j) const {
+        check(engine ? gkd_all_vs_all_bionj(engine->raw(), n, &j) : gkd_group_all_vs_all_bionj(grp, &j));
+    }
 };
 
 // one report line of fastaDist (:188-192)
@@ -359,6 +364,13 @@ int fastaDist(const std::vector<std::string> &args) {
     if (tree)
         for (const char *opt : {"--maxDist", "--nearest", "--clusters", "--linkage", "--method"})
             if (p.values.count(opt)) throw ParseFailureException(std::string("--tree and ") + opt + " cannot be combined.");
+    bool bionj = false;
+    if (p.values.count("--treeMethod")) {
+        const std::string &m = p.values["--treeMethod"];
+        if (m == "bionj") bionj = true;
+        else if (m != "nj") throw ParseFailureException("Tree method must be nj or bionj.");
+        if (!tree) throw ParseFailureException("--treeMethod needs --tree.");
+    }
     const bool within = p.values.count("--maxDist") > 0;
     const double maxDist = within ? toDouble("--maxDist", p.values["--maxDist"]) : 1.0;
     if (!(maxDist > 0.0 && maxDist <= 1.0)) throw ParseFailureException("Maximum distance must be > 0 and <= 1.");
@@ -428,10 +440,11 @@ int fastaDist(const std::vector<std::string> &args) {
         std::vector<uint32_t> a(cap), b(cap);
         std::vector<double> la(cap), lb(cap);
         gkd_joins j{a.data(), b.data(), la.data(), lb.data(), cap, 0};
-        src.nj(j);
+        if (bionj) src.bionj(j);
+        else src.nj(j);
         writeNewick(writer, j, src);
-        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(j.n) +
-                " joins in the neighbor-joining tree.");
+        logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(j.n) + " joins in the " +
+                (bionj ? "BIONJ" : "neighbor-joining") + " tree.");
         writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);
         return 0;
     }

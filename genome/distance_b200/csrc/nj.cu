@@ -1,4 +1,4 @@
-// nj.cu -- neighbour joining on the device (kernel-5 form of gkd_*_nj).
+// nj.cu -- neighbour joining and BIONJ on the device (kernel-5 forms of gkd_*_nj and gkd_*_bionj).
 //
 // The distances live in an n x n matrix of doubles in HBM (NjState, gkd_internal.cuh), filled by launch_square_scatter.
 // The r active clusters of a round hold slots 0 .. r - 1.  Every operation of the definition in gkd.h is one IEEE double
@@ -11,6 +11,10 @@
 //            which CTA was last) and appends the round's row; at r = 2 it appends the last row;
 //   update:  one thread per active k: d(u, k) into row and column f, R[k]; the thread of f writes R[u];
 //   move:    slot r - 1 moves into g's slot (row, column, sum, label) unless g held it.
+// BIONJ keeps d in the upper triangle and V in the lower one (gkd_internal.cuh).  The fill, the start and the scan body are
+// NJ's: the fill writes d to both triangles, so the start's column sums are R and S alike, and the scan reads row i from
+// column i + 1 on, which is d.  The pick also fixes lambda from S[f], S[g] and V(f, g); its own update and move then read
+// and write d and V each in its triangle.  No thread of the update reads S[f] or S[g], which the thread of f writes.
 // The host queues every round without reading anything between them.
 #include <cuda_runtime.h>
 
@@ -69,6 +73,7 @@ __global__ void __launch_bounds__(NJ_THREADS) k_nj_start(NjState st) {
         if (k != i) s = __dadd_rn(s, v);
     }
     st.R[i] = s;
+    if (st.S) st.S[i] = s;  // V starts equal to d
     st.label[i] = i;
 }
 
@@ -78,6 +83,7 @@ __device__ __forceinline__ NjCand nj_q(double rm2, double d, double Ri, uint32_t
     return li < lj ? NjCand{__dsub_rn(__dsub_rn(x, Ri), Rj), li, lj, i, j} : NjCand{__dsub_rn(__dsub_rn(x, Rj), Ri), lj, li, j, i};
 }
 
+template <bool BIONJ>
 __global__ void __launch_bounds__(NJ_THREADS) k_nj_scan(NjState st, uint32_t r, uint32_t row) {
     const uint64_t n = st.n;
     if (r == 2) {  // the last row: the midpoint of the last edge
@@ -133,13 +139,23 @@ __global__ void __launch_bounds__(NJ_THREADS) k_nj_scan(NjState st, uint32_t r, 
     best = cta_best(best, part);
     if (threadIdx.x == 0) {
         const uint32_t sf = best.sa, sg = best.sb;
-        const double dfg = st.d[sf * n + sg];
+        const uint64_t lo = min(sf, sg), hi = max(sf, sg);
+        const double dfg = st.d[lo * n + hi];
         const double t = __ddiv_rn(__dsub_rn(st.R[sf], st.R[sg]), (double)(2 * (r - 2)));
         const double df = __dadd_rn(__dmul_rn(0.5, dfg), t);
         st.ra[row] = best.a;
         st.rb[row] = best.b;
         st.la[row] = df;
         st.lb[row] = __dsub_rn(dfg, df);
+        if (BIONJ) {  // lambda = clamp(0.5 + (S_g - S_f) / (2 (r - 2) V(f, g)), 0, 1), or 0.5 when V(f, g) == 0
+            const double vfg = st.d[hi * n + lo];
+            double lam = 0.5;
+            if (vfg != 0.0) {
+                const double x = __dadd_rn(0.5, __ddiv_rn(__dsub_rn(st.S[sg], st.S[sf]), __dmul_rn((double)(2 * (r - 2)), vfg)));
+                lam = x < 0.0 ? 0.0 : x > 1.0 ? 1.0 : x;
+            }
+            *st.lambda = lam;
+        }
         st.pick[0] = sf;
         st.pick[1] = sg;
         *st.ticket = 0;
@@ -180,6 +196,69 @@ __global__ void __launch_bounds__(NJ_THREADS) k_nj_move(NjState st, uint32_t r) 
     }
 }
 
+// BIONJ.  Thread k reads d(f, k), d(g, k), V(f, k), V(g, k) and writes d(u, k), V(u, k) into f's entries, R[k] and S[k];
+// the thread of f writes R[u] and S[u].  lambda was fixed by the pick, so no entry one thread writes is read by another.
+__global__ void __launch_bounds__(NJ_THREADS) k_bionj_update(NjState st, uint32_t r, uint32_t row) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= r) return;
+    const uint64_t n = st.n;
+    const uint32_t sf = st.pick[0], sg = st.pick[1];
+    if (k == sg) return;
+    const double lam = *st.lambda, mu = __dsub_rn(1.0, lam), w = __dmul_rn(lam, mu);
+    const double dfg = st.d[min(sf, sg) * n + max(sf, sg)], vfg = st.d[max(sf, sg) * n + min(sf, sg)];
+    const double la = st.la[row], lb = st.lb[row];
+    if (k == sf) {
+        const double rm2 = (double)(r - 2);
+        st.R[sf] = __dadd_rn(__dmul_rn(lam, __dsub_rn(__dsub_rn(st.R[sf], dfg), __dmul_rn(rm2, la))),
+                             __dmul_rn(mu, __dsub_rn(__dsub_rn(st.R[sg], dfg), __dmul_rn(rm2, lb))));
+        st.S[sf] = __dsub_rn(__dadd_rn(__dmul_rn(lam, __dsub_rn(st.S[sf], vfg)), __dmul_rn(mu, __dsub_rn(st.S[sg], vfg))),
+                             __dmul_rn(rm2, __dmul_rn(w, vfg)));
+        return;
+    }
+    const uint64_t fk = min(sf, k) * n + max(sf, k), kf = max(sf, k) * n + min(sf, k);
+    const uint64_t gk = min(sg, k) * n + max(sg, k), kg = max(sg, k) * n + min(sg, k);
+    const double dfk = st.d[fk], dgk = st.d[gk], vfk = st.d[kf], vgk = st.d[kg];
+    const double duk = __dadd_rn(__dmul_rn(lam, __dsub_rn(dfk, la)), __dmul_rn(mu, __dsub_rn(dgk, lb)));
+    const double vuk = __dsub_rn(__dadd_rn(__dmul_rn(lam, vfk), __dmul_rn(mu, vgk)), __dmul_rn(w, vfg));
+    st.R[k] = __dadd_rn(__dsub_rn(__dsub_rn(st.R[k], dfk), dgk), duk);
+    st.S[k] = __dadd_rn(__dsub_rn(__dsub_rn(st.S[k], vfk), vgk), vuk);
+    st.d[fk] = duk;
+    st.d[kf] = vuk;
+}
+
+// BIONJ: slot r - 1 into g's slot.  Thread k (k < r - 1) copies d(r - 1, k) from [k n + r - 1] into g's upper entry and
+// V(r - 1, k) from [(r - 1) n + k] into g's lower entry; for k < g these are not NJ's row and column
+__global__ void __launch_bounds__(NJ_THREADS) k_bionj_move(NjState st, uint32_t r) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t sg = st.pick[1], last = r - 1;
+    if (sg == last || k >= last || k == sg) return;
+    const uint64_t n = st.n, lo = min(sg, k), hi = max(sg, k);
+    const double d = st.d[k * n + last], v = st.d[last * n + k];
+    st.d[lo * n + hi] = d;
+    st.d[hi * n + lo] = v;
+    if (k == (sg == 0 ? 1u : 0u)) {
+        st.R[sg] = st.R[last];
+        st.S[sg] = st.S[last];
+        st.label[sg] = st.label[last];
+    }
+}
+
+template <bool BIONJ>
+void queue_rounds(const NjState &st, uint32_t max_ctas, cudaStream_t s) {
+    for (uint32_t r = st.n, row = 0; r >= 3; r--, row++) {
+        const unsigned nodes = (r + NJ_THREADS - 1) / NJ_THREADS;
+        k_nj_scan<BIONJ><<<std::min(r - 1, max_ctas), NJ_THREADS, 0, s>>>(st, r, row);
+        if (BIONJ) {
+            k_bionj_update<<<nodes, NJ_THREADS, 0, s>>>(st, r, row);
+            k_bionj_move<<<nodes, NJ_THREADS, 0, s>>>(st, r);
+        } else {
+            k_nj_update<<<nodes, NJ_THREADS, 0, s>>>(st, r);
+            k_nj_move<<<nodes, NJ_THREADS, 0, s>>>(st, r);
+        }
+    }
+    k_nj_scan<BIONJ><<<1, NJ_THREADS, 0, s>>>(st, 2, st.n - 2);
+}
+
 }  // namespace
 
 uint64_t nj_state_bytes(uint32_t n) {
@@ -187,16 +266,26 @@ uint64_t nj_state_bytes(uint32_t n) {
     return N * N * 8 + N * (8 + 4) + N * 24 + NJ_MAX_CTAS * sizeof(NjCand) + 256;
 }
 
-NjState nj_state_at(void *base, uint32_t n) {
+uint64_t bionj_state_bytes(uint32_t n) { return nj_state_bytes(n) + (uint64_t)n * 8 + 8; }
+
+NjState nj_state_at(void *base, uint32_t n, bool bionj) {
     NjState st{};
     const uint64_t N = n;
     st.n = n;
     st.d = (double *)base;
     st.R = st.d + N * N;
     st.la = st.R + N;
+    if (bionj) {
+        st.S = st.la;
+        st.la = st.S + N;
+    }
     st.lb = st.la + N;
     st.part = (NjCand *)(st.lb + N);
     st.bad = (unsigned long long *)(st.part + NJ_MAX_CTAS);
+    if (bionj) {
+        st.lambda = (double *)st.bad;
+        st.bad = (unsigned long long *)(st.lambda + 1);
+    }
     st.ticket = (unsigned int *)(st.bad + 1);
     st.pick = (uint32_t *)(st.ticket + 1);
     st.label = st.pick + 2;
@@ -210,13 +299,10 @@ cudaError_t launch_nj_rounds(const NjState &st, int n_sms, cudaStream_t s) {
     if (n < 2) return cudaSuccess;
     k_nj_start<<<(n + NJ_THREADS - 1) / NJ_THREADS, NJ_THREADS, 0, s>>>(st);
     const uint32_t max_ctas = std::min<uint32_t>(NJ_MAX_CTAS, (uint32_t)n_sms * 4);
-    for (uint32_t r = n, row = 0; r >= 3; r--, row++) {
-        const unsigned nodes = (r + NJ_THREADS - 1) / NJ_THREADS;
-        k_nj_scan<<<std::min(r - 1, max_ctas), NJ_THREADS, 0, s>>>(st, r, row);
-        k_nj_update<<<nodes, NJ_THREADS, 0, s>>>(st, r);
-        k_nj_move<<<nodes, NJ_THREADS, 0, s>>>(st, r);
-    }
-    k_nj_scan<<<1, NJ_THREADS, 0, s>>>(st, 2, n - 2);
+    if (st.S)
+        queue_rounds<true>(st, max_ctas, s);
+    else
+        queue_rounds<false>(st, max_ctas, s);
     return cudaGetLastError();
 }
 

@@ -460,6 +460,21 @@ class Engine:
         del keep
         return out
 
+    def all_vs_all_bionj(self, n: int = None):
+        """(a, b, len_a, len_b): the BIONJ tree of the first n sets (default: all), in the rows of all_vs_all_nj.  BIONJ
+        weights the two clusters of each join by a variance kept for every distance instead of NJ's 1/2 each
+        (include/gkd.h)"""
+        n = len(self) if n is None else int(n)
+        return _joins(lambda j: self._ck(self._L.gkd_all_vs_all_bionj(self._h, n, C.byref(j))), n)
+
+    def bionj(self, dist):
+        """all_vs_all_bionj over a caller's row-major strict upper triangle of distances, as nj()"""
+        n = _triangle_n(dist)
+        ptr, _, keep = _array(dist, np.float64, ("float64",), "dist must be a contiguous float64 tensor")
+        out = _joins(lambda j: self._ck(self._L.gkd_bionj(self._h, n, ptr, C.byref(j))), n)
+        del keep
+        return out
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -661,3 +676,7 @@ class Group:
     def all_vs_all_nj(self):
         """(a, b, len_a, len_b) over all global ids: the single-context Engine.all_vs_all_nj result"""
         return _joins(lambda j: self._ck(self._L.gkd_group_all_vs_all_nj(self._h, C.byref(j))), len(self))
+
+    def all_vs_all_bionj(self):
+        """(a, b, len_a, len_b) over all global ids: the single-context Engine.all_vs_all_bionj result"""
+        return _joins(lambda j: self._ck(self._L.gkd_group_all_vs_all_bionj(self._h, C.byref(j))), len(self))

@@ -376,6 +376,30 @@ int gkd_all_vs_all_nj(gkd_ctx *ctx, uint32_t n, gkd_joins *out);
  * used). */
 int gkd_nj(gkd_ctx *ctx, uint32_t n, const double *dist, gkd_joins *out);
 
+/* BIONJ tree of the first n sets (Gascuel, Mol. Biol. Evol. 14:685-695, 1997): NJ with a variance V for every distance,
+ * which weights the two clusters of each join instead of NJ's fixed 1/2.  The conventions are NJ's above (one IEEE
+ * double operation each, rounded to nearest, in the order written, no fused multiply-add; labels are smallest ids),
+ * and f, g are the clusters of labels a < b:
+ *   start:  R_i as NJ; V(i, j) = d(i, j), so S_i (the row sum of V) = R_i;
+ *   rounds, while r >= 3 clusters are active: Q, the pick (f, g), t, len_a and len_b are NJ's; then
+ *           lambda = 0.5 when V(f, g) == 0 (-0.0 == +0.0), else
+ *           lambda = clamp(0.5 + ((S_g - S_f) / ((double)(2 (r - 2)) V(f, g))), 0, 1);  mu = 1 - lambda;  w = lambda mu;
+ *           for every other active k,
+ *             d(u, k) = (lambda (d(f, k) - len_a)) + (mu (d(g, k) - len_b)),
+ *             V(u, k) = ((lambda V(f, k)) + (mu V(g, k))) - (w V(f, g)),
+ *             R_k = ((R_k - d(f, k)) - d(g, k)) + d(u, k),  S_k = ((S_k - V(f, k)) - V(g, k)) + V(u, k);
+ *           R_u = (lambda ((R_f - d(f, g)) - (double)(r - 2) len_a)) + (mu ((R_g - d(f, g)) - (double)(r - 2) len_b)),
+ *           S_u = ((lambda (S_f - V(f, g))) + (mu (S_g - V(f, g)))) - ((double)(r - 2) (w V(f, g))).
+ *           u takes label f, label g goes inactive, and the row (a, b, len_a, len_b) is appended;
+ *   last:   at r = 2 the row (a, b, 0.5 d(a, b), 0.5 d(a, b)), as NJ.
+ * Gascuel's lambda uses the sum over the other k of V(g, k) - V(f, k), which is S_g - S_f because V is symmetric; the
+ * running sums S are kept as R is, so every round is elementwise and the rows are defined bit for bit.  (The running
+ * sums differ from direct sums by rounding, as R does.)  out, the input checks and the device memory are NJ's, plus
+ * 8 B per set (V is kept in the half of the n x n matrix that NJ stores twice). */
+int gkd_all_vs_all_bionj(gkd_ctx *ctx, uint32_t n, gkd_joins *out);
+/* The BIONJ tree over a caller's triangle, as gkd_nj. */
+int gkd_bionj(gkd_ctx *ctx, uint32_t n, const double *dist, gkd_joins *out);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -431,6 +455,8 @@ int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_mer
  * as gkd_group_all_vs_all_agglomerate does, then member 0 runs gkd_nj on it.  Both allocations are checked before any
  * pair is intersected (GKD_ENOMEM, naming the bytes).  The arrays of out are host memory. */
 int gkd_group_all_vs_all_nj(gkd_group *g, gkd_joins *out);
+/* gkd_all_vs_all_bionj over all global ids, as gkd_group_all_vs_all_nj (member 0 runs gkd_bionj). */
+int gkd_group_all_vs_all_bionj(gkd_group *g, gkd_joins *out);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

@@ -320,11 +320,10 @@ JNIEXPORT jint JNICALL FN(allVsAllCompleteLinkage)(JNIEnv *env, jclass c, jlong 
     return merges_into(env, complete_sparse, h, n, GKD_LINK_COMPLETE, maxDist, a, b, height, size, nMerges);
 }
 
-/* the neighbour-joining tree of the first n sets: a, b, lenA, lenB hold n - 1 entries (the joins in order); nJoins[0]
- * receives their number */
-JNIEXPORT jint JNICALL FN(allVsAllNj)(JNIEnv *env, jclass c, jlong h, jint n, jintArray a, jintArray b, jdoubleArray lenA,
-                                      jdoubleArray lenB, jintArray nJoins) {
-    (void)c;
+/* the tree of `call` (gkd_all_vs_all_nj or gkd_all_vs_all_bionj) over the first n sets: a, b, lenA, lenB hold n - 1
+ * entries (the joins in order); nJoins[0] receives their number */
+static jint joins_into(JNIEnv *env, int (*call)(gkd_ctx *, uint32_t, gkd_joins *), jlong h, jint n, jintArray a,
+                       jintArray b, jdoubleArray lenA, jdoubleArray lenB, jintArray nJoins) {
     if (!a || !b || !lenA || !lenB || !nJoins || n < 0 || (*env)->GetArrayLength(env, nJoins) < 1) return GKD_EINVAL;
     const jint cap = n > 0 ? n - 1 : 0;
     if ((*env)->GetArrayLength(env, a) < cap || (*env)->GetArrayLength(env, b) < cap ||
@@ -335,7 +334,7 @@ JNIEXPORT jint JNICALL FN(allVsAllNj)(JNIEnv *env, jclass c, jlong h, jint n, ji
     jdouble *pla = (*env)->GetDoubleArrayElements(env, lenA, NULL);
     jdouble *plb = (*env)->GetDoubleArrayElements(env, lenB, NULL);
     gkd_joins out = {(uint32_t *)pa, (uint32_t *)pb, pla, plb, (uint64_t)cap, 0};
-    int rc = (pa && pb && pla && plb) ? gkd_all_vs_all_nj(CTX(h), (uint32_t)n, &out) : GKD_ENOMEM;
+    int rc = (pa && pb && pla && plb) ? call(CTX(h), (uint32_t)n, &out) : GKD_ENOMEM;
     if (plb) (*env)->ReleaseDoubleArrayElements(env, lenB, plb, 0);
     if (pla) (*env)->ReleaseDoubleArrayElements(env, lenA, pla, 0);
     if (pb) (*env)->ReleaseIntArrayElements(env, b, pb, 0);
@@ -345,4 +344,18 @@ JNIEXPORT jint JNICALL FN(allVsAllNj)(JNIEnv *env, jclass c, jlong h, jint n, ji
         (*env)->SetIntArrayRegion(env, nJoins, 0, 1, &nj);
     }
     return rc;
+}
+
+/* the neighbour-joining tree of the first n sets */
+JNIEXPORT jint JNICALL FN(allVsAllNj)(JNIEnv *env, jclass c, jlong h, jint n, jintArray a, jintArray b, jdoubleArray lenA,
+                                      jdoubleArray lenB, jintArray nJoins) {
+    (void)c;
+    return joins_into(env, gkd_all_vs_all_nj, h, n, a, b, lenA, lenB, nJoins);
+}
+
+/* the BIONJ tree of the first n sets, in the joins of allVsAllNj */
+JNIEXPORT jint JNICALL FN(allVsAllBionj)(JNIEnv *env, jclass c, jlong h, jint n, jintArray a, jintArray b,
+                                         jdoubleArray lenA, jdoubleArray lenB, jintArray nJoins) {
+    (void)c;
+    return joins_into(env, gkd_all_vs_all_bionj, h, n, a, b, lenA, lenB, nJoins);
 }

@@ -64,6 +64,8 @@ final class GkdNative {
      *  n - 1) receive the joins in order (a &lt; b the joined subtrees' smallest ids, lenA and lenB their branch
      *  lengths), nJoins[0] their number */
     static native int allVsAllNj(long ctx, int n, int[] a, int[] b, double[] lenA, double[] lenB, int[] nJoins);
+    /** the BIONJ tree of the first n sets, in the joins of allVsAllNj */
+    static native int allVsAllBionj(long ctx, int n, int[] a, int[] b, double[] lenA, double[] lenB, int[] nJoins);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

@@ -243,6 +243,16 @@ public class GpuKmerEngine implements AutoCloseable {
         return joins[0];
     }
 
+    /** the BIONJ tree of every set, in the joins of allVsAllNj: BIONJ (Gascuel 1997) weights the two clusters of each
+     *  join by a variance kept for every distance instead of NJ's one half each, which suits distances whose noise
+     *  grows with the distance, such as Mash-style k-mer distances. */
+    public synchronized int allVsAllBionj(int[] a, int[] b, double[] lenA, double[] lenB) {
+        this.build();
+        int[] joins = new int[1];
+        check(GkdNative.allVsAllBionj(this.ctx, this.size(), a, b, lenA, lenB, joins));
+        return joins[0];
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();

@@ -1,19 +1,21 @@
 #!/usr/bin/env python
-"""Neighbour-joining trees on the device (gkd_all_vs_all_nj, gkd_nj) on one GPU, in one command, printing one JSON line.
+"""Neighbour-joining and BIONJ trees on the device (gkd_all_vs_all_nj, gkd_nj, gkd_all_vs_all_bionj, gkd_bionj) on one
+GPU, in one command, printing one JSON line.
 
 Workloads:
 * config 2: 1000 x 5 Mbp from the synthetic generator of tools/bench_rect.py: the dense call (Engine.all_vs_all, the
   triangle copied to the host) and all_vs_all_nj (the triangle stays on the device), whose rows are compared with
-  gkd_nj over the dense triangle in the same run;
-* synthetic: gkd_nj on a triangle already in device memory at n = 5,000 and 20,000: the path sums of a random tree
+  gkd_nj over the dense triangle in the same run, and likewise all_vs_all_bionj against gkd_bionj;
+* synthetic: gkd_nj and gkd_bionj on a triangle already in device memory at n = 5,000 and 20,000: the path sums of a random tree
   (leaves at the ends of 20-bit random paths of a complete binary tree, random pendant edges) plus uniform noise, scaled
   into [0, 1], generated on the device from a seed.
 
-Reported per run: the call time and the rounds time from CUDA events on gkd_stream (the rounds: the library's
-epilogue_ms, which for gkd_nj spans the start sums and all n - 1 rounds), the bytes the row scans must read,
+gkd_nj and gkd_bionj run alternately on the same device triangle, so both see the same card state.  Reported per run
+and per method: the call time and the rounds time from CUDA events on gkd_stream (the rounds: the library's
+epilogue_ms, which spans the start sums and all n - 1 rounds), the bytes the row scans must read (the same for both),
 sum over r = 3 .. n of r (r - 1) / 2 x 8, and that figure over the rounds time, and the launches of the call.  The
 active r x r corner fits the 126 MB L2 once r is below about 4,000, so the last rounds read from L2.  As a CPU reference,
-the numpy oracle (oracle/nj.py) at n = 1,000.  The card's name and power limit are read in the same run.  Writes nothing
+the numpy oracles (oracle/nj.py, oracle/bionj.py) at n = 1,000.  The card's name and power limit are read in the same run.  Writes nothing
 in the tree (--out also writes the JSON line to a file).
 """
 import argparse
@@ -30,7 +32,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 import genome.distance_b200 as gkd  # noqa: E402
 from bench_select import card, measure  # noqa: E402
-from oracle import nj  # noqa: E402
+from oracle import bionj, nj  # noqa: E402
 
 
 def scan_bytes(n):
@@ -64,20 +66,30 @@ def synthetic(n, seed, device="cuda"):
     return out / max(1.0, float(out.max()))
 
 
-def timed_nj(e, dev, repeat):
-    """(rows, call ms, rounds ms, launches of one call): CUDA events on gkd_stream around gkd_nj, median of repeat"""
+def timed_trees(e, dev, repeat):
+    """{"nj": ..., "bionj": ...} of (rows, call ms, rounds ms, launches of one call): CUDA events on gkd_stream around
+    gkd_nj and gkd_bionj, called alternately, median of repeat"""
     s = torch.cuda.ExternalStream(e.stream_ptr)
-    calls, rounds, rows = [], [], None
+    calls = {"nj": e.nj, "bionj": e.bionj}
+    times = {m: ([], [], None, 0) for m in calls}
     for _ in range(repeat):
-        before = e.metrics()["launches"]
-        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        t0.record(s)
-        rows = e.nj(dev)
-        t1.record(s)
-        t1.synchronize()
-        calls.append(t0.elapsed_time(t1))
-        rounds.append(e.metrics()["epilogue_ms"])
-    return rows, float(np.median(calls)), float(np.median(rounds)), int(e.metrics()["launches"] - before)
+        for m, call in calls.items():
+            c, r, _, _ = times[m]
+            before = e.metrics()["launches"]
+            t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            t0.record(s)
+            rows = call(dev)
+            t1.record(s)
+            t1.synchronize()
+            c.append(t0.elapsed_time(t1))
+            r.append(e.metrics()["epilogue_ms"])
+            times[m] = (c, r, rows, int(e.metrics()["launches"] - before))
+    return {m: (rows, float(np.median(c)), float(np.median(r)), launches) for m, (c, r, rows, launches) in times.items()}
+
+
+def same(x, y):
+    return all(np.array_equal(a.view(np.uint64) if a.dtype == np.float64 else a,
+                              b.view(np.uint64) if b.dtype == np.float64 else b) for a, b in zip(x, y))
 
 
 def report(n, rounds_ms, call_ms, launches):
@@ -96,7 +108,8 @@ def main():
     ap.add_argument("--out", default="")
     a = ap.parse_args()
     assert torch.cuda.is_available(), "bench_nj needs a GPU"
-    res = {"what": "neighbour joining on the device: all_vs_all_nj (config 2) and gkd_nj on device triangles", **card()}
+    res = {"what": "neighbour joining and BIONJ on the device: all_vs_all_nj / all_vs_all_bionj (config 2) and gkd_nj / "
+                   "gkd_bionj on device triangles", **card()}
     buf = torch.empty((100, a.length), dtype=torch.uint8, device="cuda")
     with gkd.Engine(k=21) as e:
         for g in range(a.genomes):
@@ -108,17 +121,18 @@ def main():
         e.build()
         _, dense = measure(e, lambda: e.all_vs_all(want_inter=False), a.repeat)
         _, gd = e.all_vs_all(want_inter=False)
-        e.all_vs_all_nj()  # warm-up
-        before = e.metrics()["launches"]
-        got, rd = measure(e, lambda: e.all_vs_all_nj(), a.repeat)
-        rd["launches"] = int(e.metrics()["launches"] - before) // a.repeat
-        rd["rounds"] = int(e.metrics()["agglomerate_rounds"])
-        rows, call_ms, rounds_ms, launches = timed_nj(e, torch.from_numpy(gd).to("cuda"), a.repeat)
-        rd["equal_to_nj_of_dense"] = all(np.array_equal(x.view(np.uint64) if x.dtype == np.float64 else x,
-                                                        y.view(np.uint64) if y.dtype == np.float64 else y)
-                                         for x, y in zip(got, rows))
-        res["config2"] = {"genomes": a.genomes, "length": a.length, "dense_all_vs_all": dense, "all_vs_all_nj": rd,
-                          "nj_of_device_triangle": report(a.genomes, rounds_ms, call_ms, launches)}
+        res["config2"] = {"genomes": a.genomes, "length": a.length, "dense_all_vs_all": dense}
+        got = {}
+        for m, call in (("nj", e.all_vs_all_nj), ("bionj", e.all_vs_all_bionj)):
+            call()  # warm-up
+            before = e.metrics()["launches"]
+            got[m], rd = measure(e, call, a.repeat)
+            rd["launches"] = int(e.metrics()["launches"] - before) // a.repeat
+            rd["rounds"] = int(e.metrics()["agglomerate_rounds"])
+            res["config2"]["all_vs_all_" + m] = rd
+        for m, (rows, call_ms, rounds_ms, launches) in timed_trees(e, torch.from_numpy(gd).to("cuda"), a.repeat).items():
+            res["config2"]["all_vs_all_" + m]["equal_to_%s_of_dense" % m] = same(got[m], rows)
+            res["config2"][m + "_of_device_triangle"] = report(a.genomes, rounds_ms, call_ms, launches)
     del buf
     torch.cuda.empty_cache()
     res["synthetic"] = []
@@ -127,22 +141,25 @@ def main():
             dev = synthetic(n, a.seed + n)
             torch.cuda.synchronize()
             e.nj(dev)  # warm-up of this shape
-            rows, call_ms, rounds_ms, launches = timed_nj(e, dev, a.repeat)
-            r = report(n, rounds_ms, call_ms, launches)
-            r["negative_lengths"] = int((rows[2] < 0).sum() + (rows[3] < 0).sum())
-            res["synthetic"].append(r)
+            e.bionj(dev)
+            for m, (rows, call_ms, rounds_ms, launches) in timed_trees(e, dev, a.repeat).items():
+                r = {"method": m, **report(n, rounds_ms, call_ms, launches)}
+                r["negative_lengths"] = int((rows[2] < 0).sum() + (rows[3] < 0).sum())
+                res["synthetic"].append(r)
             del dev
             torch.cuda.empty_cache()
-    # CPU reference: the numpy oracle at n = 1,000
+    # CPU reference: the numpy oracles at n = 1,000
     ref = synthetic(1000, a.seed).cpu().numpy()
-    t0 = time.perf_counter()
-    want = nj.nj(ref, 1000)
-    cpu_s = time.perf_counter() - t0
     with gkd.Engine(k=21) as e:
-        got = e.nj(ref)
-    same = all(np.array_equal(np.asarray([w[c] for w in want], dtype=x.dtype).view(np.uint8), x.view(np.uint8))
-               for c, x in enumerate(got))
-    res["cpu_oracle_n1000"] = {"seconds": round(cpu_s, 3), "equal_to_device": bool(same)}
+        for m, oracle, call in (("nj", nj.nj, e.nj), ("bionj", lambda d, n: bionj.bionj(d, n)[0], e.bionj)):
+            t0 = time.perf_counter()
+            want = oracle(ref, 1000)
+            cpu_s = time.perf_counter() - t0
+            got = call(ref)
+            eq = all(np.array_equal(np.asarray([w[c] for w in want], dtype=x.dtype).view(np.uint8), x.view(np.uint8))
+                     for c, x in enumerate(got))
+            res["cpu_oracle_n1000" if m == "nj" else "cpu_bionj_oracle_n1000"] = {"seconds": round(cpu_s, 3),
+                                                                                  "equal_to_device": bool(eq)}
     line = json.dumps(res)
     print(line)
     if a.out:
