@@ -14,6 +14,7 @@ STRAND_BOTH, STRAND_CANONICAL = 0, 1
 AMBIG_SKIP, AMBIG_LITERAL = 0, 1
 HASH_JAVA_STRING, HASH_MURMUR3 = 0, 1
 LINK_COMPLETE, LINK_AVERAGE = 1, 2
+TREE_NJ, TREE_BIONJ = 1, 2  # gkd_tree_start: the start tree of gkd_*_bme
 ABI_VERSION = 2
 
 
@@ -100,6 +101,7 @@ SYMBOLS = {
     "gkd_group_all_vs_all_complete_linkage": (_i32, [_vp, _dbl, C.POINTER(GkdMerges)]),
     "gkd_group_all_vs_all_nj": (_i32, [_vp, C.POINTER(GkdJoins)]),
     "gkd_group_all_vs_all_bionj": (_i32, [_vp, C.POINTER(GkdJoins)]),
+    "gkd_group_all_vs_all_bme": (_i32, [_vp, _i32, C.POINTER(GkdJoins), _pu64]),
     "gkd_build_sets": (_i32, [_vp]),
     "gkd_set_size": (_i32, [_vp, _u32, _pu64, _pu64, _pu64]),
     "gkd_export_set": (_i32, [_vp, _u32, _vp, _u64, _pu64]),
@@ -138,6 +140,9 @@ SYMBOLS = {
     "gkd_nj": (_i32, [_vp, _u32, _vp, C.POINTER(GkdJoins)]),
     "gkd_all_vs_all_bionj": (_i32, [_vp, _u32, C.POINTER(GkdJoins)]),
     "gkd_bionj": (_i32, [_vp, _u32, _vp, C.POINTER(GkdJoins)]),
+    "gkd_all_vs_all_bme": (_i32, [_vp, _u32, _i32, C.POINTER(GkdJoins), _pu64]),
+    "gkd_bme": (_i32, [_vp, _u32, _vp, _i32, C.POINTER(GkdJoins), _pu64]),
+    "gkd_bme_nni": (_i32, [_vp, _u32, _vp, C.POINTER(GkdJoins), C.POINTER(GkdJoins), _pu64]),
     "gkd_hash_set": (_i32, [_vp, _u32, _u32, _i32, _vp, _pu32]),
     "gkd_sketch_distances": (_i32, [_vp, _u32, _i32, _vp, _vp, _u64, _vp]),
     "gkd_format_double": (_i32, [_dbl, C.c_char_p, C.c_size_t]),

@@ -1840,6 +1840,81 @@ struct NeighborJoining : DenseMatrix {
     }
 };
 
+// One BME NNI search on the context's device: start() checks the free memory and sets up the table of bme.cu, with the
+// NJ state inside it, in one buffer of the call; the distances are scattered into the NJ matrix; finish() copies them
+// into the table's leaf block, runs the NJ or BIONJ rounds when the call starts from them (their rows are read back:
+// the host holds the topology), then the search, and writes the rows.
+struct BalancedNni : DenseMatrix {
+    int start_tree;                 // GKD_TREE_NJ, GKD_TREE_BIONJ, or 0: the rows in ta, tb
+    std::vector<uint32_t> ta, tb;  // the caller's tree (gkd_bme_nni), checked
+    gkd_joins *out;
+    uint64_t *n_swaps;
+    NjState st{};
+    BalancedNni(const char *fn_, uint32_t n_, const double *dist_, int start_, gkd_joins *out_, uint64_t *n_swaps_)
+        : DenseMatrix(fn_, n_, dist_, "gkd kernel 5: BME table"), start_tree(start_), out(out_), n_swaps(n_swaps_) {}
+    std::array<const void *, 8> outputs() const override { return {out->a, out->b, out->len_a, out->len_b}; }
+    int start(gkd_ctx *c) override {
+        out->n = 0;
+        if (n_swaps) *n_swaps = 0;
+        c->m.agglomerate_rounds = 0;
+        if (n < 2) return GKD_OK;
+        int rc = alloc(c, bme_state_bytes(n), "balanced minimum evolution");
+        if (rc) return rc;
+        st = bme_nj_state_at(buf, n, start_tree == GKD_TREE_BIONJ);
+        CK(cudaMemsetAsync(st.bad, 0xFF, 8, c->stream));
+        CK(cudaMemsetAsync(st.ticket, 0, 4, c->stream));
+        return stage(c);
+    }
+    int scatter(gkd_ctx *c, const double *src, uint64_t first, uint64_t count, const uint32_t *join_err) override {
+        CK(launch_square_scatter(nj_square(st), src, first, count, join_err, c->stream));
+        c->m.launches++;
+        return GKD_OK;
+    }
+    int finish(gkd_ctx *c) override {
+        if (n < 2) return GKD_OK;
+        unsigned long long bad = 0;
+        CK(cudaMemcpyAsync(&bad, st.bad, 8, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.d2h_bytes += 8;
+        if (bad != ~0ull) {
+            uint32_t i, j;
+            upper_pair(bad, n, i, j);
+            return fail(c, GKD_EINVAL, "%s: the distance of pair (%u, %u) is not a finite value in [0, 2]", fn, i, j);
+        }
+        CK(cudaEventRecord(c->ev[6], c->stream));
+        CK(launch_bme_leaves(buf, n, c->stream));
+        c->m.launches++;
+        if (start_tree) {
+            CK(launch_nj_rounds(st, c->n_sms, c->stream));
+            c->m.launches += nj_launches(n);
+            ta.resize(n - 1), tb.resize(n - 1);
+            CK(cudaMemcpyAsync(ta.data(), st.ra, (n - 1) * 4ull, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaMemcpyAsync(tb.data(), st.rb, (n - 1) * 4ull, cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            c->m.d2h_bytes += (n - 1) * 8ull;
+        }
+        BmeRun r;
+        CK(bme_search(buf, n, ta.data(), tb.data(), c->stream, r));
+        CK(cudaEventRecord(c->ev[7], c->stream));
+        c->m.launches += r.launches;
+        c->m.h2d_bytes += r.h2d;
+        c->m.d2h_bytes += r.d2h;
+        const uint64_t rows = n - 1, w = std::min<uint64_t>(rows, out->cap);
+        if (w) {
+            if (out->a) CK(cudaMemcpyAsync(out->a, r.a.data(), w * 4, cudaMemcpyDefault, c->stream));
+            if (out->b) CK(cudaMemcpyAsync(out->b, r.b.data(), w * 4, cudaMemcpyDefault, c->stream));
+            if (out->len_a) CK(cudaMemcpyAsync(out->len_a, r.la.data(), w * 8, cudaMemcpyDefault, c->stream));
+            if (out->len_b) CK(cudaMemcpyAsync(out->len_b, r.lb.data(), w * 8, cudaMemcpyDefault, c->stream));
+        }
+        CK(cudaStreamSynchronize(c->stream));
+        c->m.epilogue_ms += elapsed(c->ev[6], c->ev[7]);
+        c->m.agglomerate_rounds = rows;
+        out->n = rows;
+        if (n_swaps) *n_swaps = r.swaps;
+        return GKD_OK;
+    }
+};
+
 // One complete-linkage agglomeration from the pairs within max_dist: start() sets up the O(n) state of the rounds;
 // append() adds pairs to one device list that grows with them (16 B per pair); finish() builds the rows of
 // agglomerate.cu from the list and runs the rounds on them (24 B per pair).  While the rows are built the list, the
@@ -2918,6 +2993,71 @@ int gkd_all_vs_all_bionj(gkd_ctx *c, uint32_t n, gkd_joins *out) {
 }
 int gkd_bionj(gkd_ctx *c, uint32_t n, const double *dist, gkd_joins *out) {
     return joins_of_triangle(c, "gkd_bionj", n, dist, true, out);
+}
+
+// ---- balanced minimum-evolution NNIs ----------------------------------------------------------------------------
+int gkd_all_vs_all_bme(gkd_ctx *c, uint32_t n, int start, gkd_joins *out, uint64_t *n_swaps) {
+    const char *fn = "gkd_all_vs_all_bme";
+    if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
+    if (start != GKD_TREE_NJ && start != GKD_TREE_BIONJ) return fail(c, GKD_EINVAL, "%s: start %d is not GKD_TREE_NJ or GKD_TREE_BIONJ", fn, start);
+    BalancedNni f(fn, n, nullptr, start, out, n_swaps);
+    return run_call(c, fn, triangle(n), f);
+}
+
+// as joins_of_triangle: a host triangle and a host tree are checked before the context is used
+static int bme_of_triangle(gkd_ctx *c, const char *fn, uint32_t n, const double *dist, int start, const gkd_joins *tree,
+                           gkd_joins *out, uint64_t *n_swaps) {
+    if (!out) return fail(c, GKD_EINVAL, "%s: null out", fn);
+    if (!dist && n >= 2) return fail(c, GKD_EINVAL, "%s: null dist", fn);
+    std::vector<uint32_t> ta, tb;
+    if (!start) {  // the caller's rows: n - 1 joins of current labels a < b
+        if (!tree) return fail(c, GKD_EINVAL, "%s: null tree", fn);
+        const uint64_t rows = n >= 2 ? n - 1 : 0;
+        if (tree->n != rows)
+            return fail(c, GKD_EINVAL, "%s: the tree has %llu rows; a tree of %u sets has %llu", fn, (unsigned long long)tree->n, n,
+                        (unsigned long long)rows);
+        if (rows && (!tree->a || !tree->b)) return fail(c, GKD_EINVAL, "%s: null tree->a or tree->b", fn);
+        ta.resize(rows), tb.resize(rows);
+        if (rows) {
+            if (classify(tree->a) == MEM_DEVICE || classify(tree->b) == MEM_DEVICE) {
+                CK(cudaMemcpy(ta.data(), tree->a, rows * 4, cudaMemcpyDefault));
+                CK(cudaMemcpy(tb.data(), tree->b, rows * 4, cudaMemcpyDefault));
+            } else {
+                std::copy(tree->a, tree->a + rows, ta.begin());
+                std::copy(tree->b, tree->b + rows, tb.begin());
+            }
+        }
+        std::vector<uint8_t> gone(n, 0);
+        for (uint64_t t = 0; t < rows; t++) {
+            const uint32_t a = ta[t], b = tb[t];
+            if (a >= n || b >= n) return fail(c, GKD_EINVAL, "%s: row %llu: label %u is not below n = %u", fn, (unsigned long long)t, std::max(a, b), n);
+            if (a >= b) return fail(c, GKD_EINVAL, "%s: row %llu: labels %u, %u are not a < b", fn, (unsigned long long)t, a, b);
+            if (gone[a] || gone[b])
+                return fail(c, GKD_EINVAL, "%s: row %llu: label %u was joined by an earlier row, so it is not the smallest id of a current subtree",
+                            fn, (unsigned long long)t, gone[a] ? a : b);
+            gone[b] = 1;
+        }
+    }
+    if (n >= 2 && classify(dist) != MEM_DEVICE) {
+        const double *d = dist;
+        for (uint32_t i = 0; i + 1 < n; i++)
+            for (uint32_t j = i + 1; j < n; j++, d++)
+                if (!(*d >= 0.0 && *d <= 2.0))
+                    return fail(c, GKD_EINVAL, "%s: the distance of pair (%u, %u) is not a finite value in [0, 2]", fn, i, j);
+    }
+    BalancedNni f(fn, n, dist, start, out, n_swaps);
+    f.ta = std::move(ta), f.tb = std::move(tb);
+    return run_call(c, fn, triangle(0), f);
+}
+
+int gkd_bme(gkd_ctx *c, uint32_t n, const double *dist, int start, gkd_joins *out, uint64_t *n_swaps) {
+    if (start != GKD_TREE_NJ && start != GKD_TREE_BIONJ)
+        return fail(c, GKD_EINVAL, "gkd_bme: start %d is not GKD_TREE_NJ or GKD_TREE_BIONJ", start);
+    return bme_of_triangle(c, "gkd_bme", n, dist, start, nullptr, out, n_swaps);
+}
+
+int gkd_bme_nni(gkd_ctx *c, uint32_t n, const double *dist, const gkd_joins *tree, gkd_joins *out, uint64_t *n_swaps) {
+    return bme_of_triangle(c, "gkd_bme_nni", n, dist, 0, tree, out, n_swaps);
 }
 
 // ---- complete linkage from the pairs within max_dist ------------------------------------------------------------

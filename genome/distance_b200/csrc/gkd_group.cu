@@ -907,6 +907,26 @@ int gkd_group_all_vs_all_bionj(gkd_group *g, gkd_joins *out) {
     return group_joins(g, "gkd_group_all_vs_all_bionj", "BIONJ", g ? gkd::bionj_state_bytes(g->n_genomes) : 0, gkd_bionj, out);
 }
 
+int gkd_group_all_vs_all_bme(gkd_group *g, int start, gkd_joins *out, uint64_t *n_swaps) {
+    const char *fn = "gkd_group_all_vs_all_bme";
+    if (start != GKD_TREE_NJ && start != GKD_TREE_BIONJ) return gfail(g, GKD_EINVAL, "%s: start %d is not GKD_TREE_NJ or GKD_TREE_BIONJ", fn, start);
+    if (!out) return gfail(g, GKD_EINVAL, "%s: null out", fn);
+    if (!g) return GKD_EINVAL;
+    try {
+        out->n = 0;
+        if (n_swaps) *n_swaps = 0;
+        std::vector<double> dist;
+        int rc = group_triangle(g, fn, "balanced minimum evolution", gkd::bme_state_bytes(g->n_genomes), dist);
+        if (rc != GKD_OK) return rc;
+        gkd_ctx *c0 = g->members[0].ctx;
+        if ((rc = gkd_bme(c0, g->n_genomes, dist.data(), start, out, n_swaps)) != GKD_OK)
+            return gfail(g, rc, "member 0: %s", gkd_last_error(c0));
+        return GKD_OK;
+    } catch (const std::exception &ex) {
+        return gfail(g, GKD_ENOMEM, "%s: %s", fn, ex.what());
+    }
+}
+
 int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_merges *out) {
     if (max_dist != max_dist) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_complete_linkage: max_dist is NaN");
     if (!out) return gfail(g, GKD_EINVAL, "gkd_group_all_vs_all_complete_linkage: null out");

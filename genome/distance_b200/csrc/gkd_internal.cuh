@@ -549,6 +549,22 @@ inline Square<double> nj_square(const NjState &st) { return {st.d, nullptr, st.n
 // 3 (n - 2) + 2 launches; the rows are then in ra, rb, la, lb.  *ticket must be 0 (the scatter's init sets it).
 cudaError_t launch_nj_rounds(const NjState &st, int n_sms, cudaStream_t s);
 inline uint64_t nj_launches(uint32_t n) { return n < 2 ? 0 : 3ull * (n - 2) + 2; }
+// Balanced minimum-evolution NNIs (bme.cu, gkd_*_bme): an M x M table of subtree averages, M = 2n - 2 (n >= 2), whose
+// leaf block is d.  The distances are scattered into the NJ matrix placed in the table's rows n .. (not yet built),
+// copied into the leaf block, and the NJ or BIONJ rounds (when the call starts from them) run there.
+constexpr double BME_EPS = 0x1p-40;  // GKD_BME_EPS
+inline uint64_t bme_max_swaps(uint32_t n) { return 4ull * n; }
+uint64_t bme_table_bytes(uint32_t n);  // the table, with room for the NJ state inside it
+uint64_t bme_state_bytes(uint32_t n);  // the table and the O(n) state, in one buffer
+NjState bme_nj_state_at(void *base, uint32_t n, bool bionj);
+cudaError_t launch_bme_leaves(void *base, uint32_t n, cudaStream_t s);  // the NJ matrix's d into the leaf block
+struct BmeRun {
+    std::vector<uint32_t> a, b;  // the rows, as gkd_joins holds them
+    std::vector<double> la, lb;
+    uint64_t swaps = 0, launches = 0, h2d = 0, d2h = 0;
+};
+// the search from the tree of the rows (a, b) (host, n - 1 each, checked), then the lengths and the rows
+cudaError_t bme_search(void *base, uint32_t n, const uint32_t *a, const uint32_t *b, cudaStream_t s, BmeRun &r);
 // greedy representative pass, decision step: candidate `cand` (visit index `visit`) joins reps[0..*n_reps) unless
 // some representative is within max_dist; clears the counts it consumed
 cudaError_t launch_greedy_decide(const SetDesc *sets, uint32_t *reps, uint32_t *n_reps, uint32_t cand, uint32_t visit,

@@ -148,6 +148,8 @@ const std::vector<OptSpec> FASTA_OPTS = {
                         "its last edge, instead of the report (additive option)"},
     {{"--treeMethod"}, true, "tree method of --tree: nj (default, neighbour joining) or bionj (BIONJ, which weights each "
                              "join by the variances of the distances) (additive option)"},
+    {{"--nni"}, false, "refine the tree of --tree by balanced minimum-evolution nearest-neighbour interchanges and give it "
+                       "BME branch lengths (additive option)"},
     {{"--help", "-h"}, false, "display command-line usage"},
     {{"--verbose", "-v"}, false, "display more frequent log messages"},
 };
@@ -225,6 +227,11 @@ struct DistSource {
         check(rc);
     }
     void nj(gkd_joins &j) const { check(engine ? gkd_all_vs_all_nj(engine->raw(), n, &j) : gkd_group_all_vs_all_nj(grp, &j)); }
+    uint64_t bme(int start, gkd_joins &j) const {
+        uint64_t swaps = 0;
+        check(engine ? gkd_all_vs_all_bme(engine->raw(), n, start, &j, &swaps) : gkd_group_all_vs_all_bme(grp, start, &j, &swaps));
+        return swaps;
+    }
     void bionj(gkd_joins &j) const {
         check(engine ? gkd_all_vs_all_bionj(engine->raw(), n, &j) : gkd_group_all_vs_all_bionj(grp, &j));
     }
@@ -371,6 +378,8 @@ int fastaDist(const std::vector<std::string> &args) {
         else if (m != "nj") throw ParseFailureException("Tree method must be nj or bionj.");
         if (!tree) throw ParseFailureException("--treeMethod needs --tree.");
     }
+    const bool nni = p.values.count("--nni") > 0;
+    if (nni && !tree) throw ParseFailureException("--nni needs --tree.");
     const bool within = p.values.count("--maxDist") > 0;
     const double maxDist = within ? toDouble("--maxDist", p.values["--maxDist"]) : 1.0;
     if (!(maxDist > 0.0 && maxDist <= 1.0)) throw ParseFailureException("Maximum distance must be > 0 and <= 1.");
@@ -440,9 +449,14 @@ int fastaDist(const std::vector<std::string> &args) {
         std::vector<uint32_t> a(cap), b(cap);
         std::vector<double> la(cap), lb(cap);
         gkd_joins j{a.data(), b.data(), la.data(), lb.data(), cap, 0};
-        if (bionj) src.bionj(j);
+        uint64_t swaps = 0;
+        if (nni) swaps = src.bme(bionj ? GKD_TREE_BIONJ : GKD_TREE_NJ, j);
+        else if (bionj) src.bionj(j);
         else src.nj(j);
         writeNewick(writer, j, src);
+        if (nni)
+            logInfo(std::to_string(swaps) + " balanced NNIs applied to the " + (bionj ? "BIONJ" : "neighbor-joining") + " tree" +
+                    (swaps > 0 && swaps == GKD_BME_MAX_SWAPS(n) ? "; the search stopped at its cap of " + std::to_string(swaps) + " swaps." : "."));
         logInfo(std::to_string(total) + " pairs computed in 1 batches, " + std::to_string(j.n) + " joins in the " +
                 (bionj ? "BIONJ" : "neighbor-joining") + " tree.");
         writeMetrics(metricsFile, "fastaDist", src.metricsCtx(), total, src.gpus);

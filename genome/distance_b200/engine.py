@@ -65,6 +65,21 @@ def _joins(call, n: int):
     return a[:j.n], b[:j.n], len_a[:j.n], len_b[:j.n]
 
 
+def _bme_start(start) -> int:
+    """TREE_NJ / TREE_BIONJ of "nj" / "bionj" (or the constant itself); ValueError otherwise"""
+    v = {"nj": _lib.TREE_NJ, "bionj": _lib.TREE_BIONJ}.get(start, start)
+    if v not in (_lib.TREE_NJ, _lib.TREE_BIONJ):
+        raise ValueError(f"start must be 'nj' or 'bionj', not {start!r}")
+    return v
+
+
+def _bme(call, n: int):
+    """((a, b, len_a, len_b), swaps) of a gkd_*_bme call `call(joins, swaps)`"""
+    swaps = C.c_uint64(0)
+    rows = _joins(lambda j: call(j, swaps), n)
+    return rows, int(swaps.value)
+
+
 def _triangle_n(dist) -> int:
     """n of a row-major strict upper triangle of n(n-1)/2 entries (numpy array or tensor); ValueError otherwise"""
     m = int(dist.numel() if _is_torch(dist) else np.asarray(dist).size)
@@ -475,6 +490,36 @@ class Engine:
         del keep
         return out
 
+    def all_vs_all_bme(self, start="bionj", n: int = None):
+        """((a, b, len_a, len_b), swaps): the NJ or BIONJ tree ("nj" / "bionj") of the first n sets (default: all)
+        refined by balanced minimum-evolution NNIs, with BME branch lengths, in the rows of all_vs_all_nj, and the
+        number of swaps taken (include/gkd.h)"""
+        n = len(self) if n is None else int(n)
+        s = _bme_start(start)
+        return _bme(lambda j, w: self._ck(self._L.gkd_all_vs_all_bme(self._h, n, s, C.byref(j), C.byref(w))), n)
+
+    def bme(self, dist, start="bionj"):
+        """all_vs_all_bme over a caller's row-major strict upper triangle of distances, as nj()"""
+        n = _triangle_n(dist)
+        s = _bme_start(start)
+        ptr, _, keep = _array(dist, np.float64, ("float64",), "dist must be a contiguous float64 tensor")
+        out = _bme(lambda j, w: self._ck(self._L.gkd_bme(self._h, n, ptr, s, C.byref(j), C.byref(w))), n)
+        del keep
+        return out
+
+    def bme_nni(self, dist, a, b):
+        """((a, b, len_a, len_b), swaps): the BME NNI search from the caller's tree, the rows (a, b) (n - 1 joins of
+        current labels a < b, as all_vs_all_nj returns them), over a caller's triangle"""
+        n = _triangle_n(dist)
+        ta, tb = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
+        if ta.size != tb.size:
+            raise ValueError("a and b must have the same length")
+        tree = GkdJoins(ta.ctypes.data, tb.ctypes.data, None, None, ta.size, ta.size)
+        ptr, _, keep = _array(dist, np.float64, ("float64",), "dist must be a contiguous float64 tensor")
+        out = _bme(lambda j, w: self._ck(self._L.gkd_bme_nni(self._h, n, ptr, C.byref(tree), C.byref(j), C.byref(w))), n)
+        del keep
+        return out
+
     def pairs(self, a: Sequence[int], b: Sequence[int], inter_out=None, dist_out=None):
         aa, ba = np.ascontiguousarray(a, dtype=np.uint32), np.ascontiguousarray(b, dtype=np.uint32)
         inter, dist, pi, pd = self._outs(aa.size, inter_out, dist_out, True, True)
@@ -680,3 +725,8 @@ class Group:
     def all_vs_all_bionj(self):
         """(a, b, len_a, len_b) over all global ids: the single-context Engine.all_vs_all_bionj result"""
         return _joins(lambda j: self._ck(self._L.gkd_group_all_vs_all_bionj(self._h, C.byref(j))), len(self))
+
+    def all_vs_all_bme(self, start="bionj"):
+        """((a, b, len_a, len_b), swaps) over all global ids: the single-context Engine.all_vs_all_bme result"""
+        s = _bme_start(start)
+        return _bme(lambda j, w: self._ck(self._L.gkd_group_all_vs_all_bme(self._h, s, C.byref(j), C.byref(w))), len(self))

@@ -400,6 +400,49 @@ int gkd_all_vs_all_bionj(gkd_ctx *ctx, uint32_t n, gkd_joins *out);
 /* The BIONJ tree over a caller's triangle, as gkd_nj. */
 int gkd_bionj(gkd_ctx *ctx, uint32_t n, const double *dist, gkd_joins *out);
 
+/* Balanced minimum-evolution (BME) NNI search (Desper & Gascuel, J. Comput. Biol. 9:687-705, 2002): start from the NJ
+ * or BIONJ tree above (or a caller's tree), apply balanced nearest-neighbour interchanges until none shortens the tree
+ * by more than GKD_BME_EPS, then set BME branch lengths.  The conventions are NJ's (one IEEE double operation each,
+ * rounded to nearest, in the order written, no fused multiply-add), so the rows are defined bit for bit and are the
+ * same on every device count.
+ *   tree:    the rows of a gkd_joins read as an unrooted binary tree; the last row's two subtrees are joined by one
+ *            edge, the root edge.  A side is the set of leaves on one side of an edge; its label is its smallest id.  A
+ *            side of more than one leaf has two child sides: the two subtrees it splits into at its nearest node.
+ *   Delta:   for disjoint sides X and Y, Delta(X, Y) = d(x, y) when both are leaves x and y; otherwise let Z be the one
+ *            of X, Y with the larger (size, label), W the other, Z1 and Z2 the children of Z in label order:
+ *            Delta(X, Y) = 0.5 (Delta(Z1, W) + Delta(Z2, W)).  So Delta depends only on the two subtrees.
+ *   gains:   an internal edge has sides A u B and C u D, named so that A holds the smallest label of the four, B is A's
+ *            partner, and label C < label D.  Swapping B and C gains 0.25 ((Delta_AB + Delta_CD) - (Delta_AC + Delta_BD));
+ *            swapping B and D gains 0.25 ((Delta_AB + Delta_CD) - (Delta_AD + Delta_BC)).  The gain is the drop of
+ *            Pauplin's balanced length, the sum over leaf pairs of 2^(1 - edges between them) d.
+ *   search:  each step takes the largest gain over every internal edge and both swaps when it is > GKD_BME_EPS; ties go
+ *            to the smaller edge key, the (label, size) of the edge's side C u D (the side without leaf 0), then to the
+ *            swap of B and C.  The search stops when no gain exceeds GKD_BME_EPS, or after GKD_BME_MAX_SWAPS(n) swaps
+ *            (*n_swaps then equals the cap; not an error).  A swap keeps every edge and changes only splits, so the
+ *            root edge stays an edge (the subtree on the root's side of a swapped edge is the one that stays).
+ *   lengths: internal edge 0.25 (((Delta_AC + Delta_AD) + Delta_BC) + Delta_BD) - 0.5 (Delta_AB + Delta_CD); pendant edge to
+ *            leaf i, whose other side has children A, B in label order, 0.5 ((Delta_iA + Delta_iB) - Delta_AB); the
+ *            root edge between two leaves (n = 2) d.  Both recover the lengths of an additive tree in exact arithmetic.
+ *   output:  rooted at the midpoint of the root edge: the rows in post-order, for every node the child of the smaller
+ *            label first, each row (a, b, len_a, len_b) with a < b the children's labels, the root row last with
+ *            (l/2, l/2) for the root edge's length l.  n <= 3 makes no swap; n = 2 gives the NJ row; n < 2 no row.
+ * out is as NJ's; n_swaps (may be NULL) receives the number of swaps taken.  Device memory: the table of Delta, one
+ * row and column per node but the root, (2n - 2)^2 doubles (about 32 n^2 B), plus O(n) state and an 8 MiB list of the
+ * cells a swap changes (the NJ matrix and the start rounds run inside the table before it is built); the call fails with GKD_ENOMEM, naming the bytes, before any
+ * pair is intersected when that exceeds the free device memory.  Only the rows leave the device. */
+#define GKD_BME_EPS 0x1p-40
+#define GKD_BME_MAX_SWAPS(n) (4ull * (uint64_t)(n))
+typedef enum gkd_tree_start { GKD_TREE_NJ = 1, GKD_TREE_BIONJ = 2 } gkd_tree_start;
+/* Every pair i < j is intersected once and scattered on the device; start is GKD_TREE_NJ or GKD_TREE_BIONJ. */
+int gkd_all_vs_all_bme(gkd_ctx *ctx, uint32_t n, int start, gkd_joins *out, uint64_t *n_swaps);
+/* The same over a caller's triangle, with gkd_nj's checks. */
+int gkd_bme(gkd_ctx *ctx, uint32_t n, const double *dist, int start, gkd_joins *out, uint64_t *n_swaps);
+/* The search from the caller's tree: n - 1 rows (tree->n; a and b read, host or device memory, lengths ignored), each
+ * joining the current subtrees of labels a < b.  A row whose label is not below n, not a < b, or not the smallest id of
+ * a current subtree (joined away by an earlier row), or a row count other than n - 1, fails with GKD_EINVAL naming the
+ * row, before the context is used.  dist as gkd_bme. */
+int gkd_bme_nni(gkd_ctx *ctx, uint32_t n, const double *dist, const gkd_joins *tree, gkd_joins *out, uint64_t *n_swaps);
+
 /* ---- several GPUs in one process ------------------------------------------------------------------------
  * A group is one context per listed device (an ordinal may be listed more than once) driven by one host thread
  * per member.  The pair matrix of FastaDistanceProcessor.runReporter (:141-194) is cut into member blocks, the
@@ -457,6 +500,8 @@ int gkd_group_all_vs_all_complete_linkage(gkd_group *g, double max_dist, gkd_mer
 int gkd_group_all_vs_all_nj(gkd_group *g, gkd_joins *out);
 /* gkd_all_vs_all_bionj over all global ids, as gkd_group_all_vs_all_nj (member 0 runs gkd_bionj). */
 int gkd_group_all_vs_all_bionj(gkd_group *g, gkd_joins *out);
+/* gkd_all_vs_all_bme over all global ids, as gkd_group_all_vs_all_nj (member 0 runs gkd_bme). */
+int gkd_group_all_vs_all_bme(gkd_group *g, int start, gkd_joins *out, uint64_t *n_swaps);
 
 /* ---- MinHash sketches (SURVEY section 8f row 4) ---------------------------------------------------------
  * SequenceKmers.hashSet(width) and Sketch.distance (SketchProcessor.java:91, WidthProcessor.java:177-183,

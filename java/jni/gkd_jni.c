@@ -320,11 +320,14 @@ JNIEXPORT jint JNICALL FN(allVsAllCompleteLinkage)(JNIEnv *env, jclass c, jlong 
     return merges_into(env, complete_sparse, h, n, GKD_LINK_COMPLETE, maxDist, a, b, height, size, nMerges);
 }
 
-/* the tree of `call` (gkd_all_vs_all_nj or gkd_all_vs_all_bionj) over the first n sets: a, b, lenA, lenB hold n - 1
- * entries (the joins in order); nJoins[0] receives their number */
-static jint joins_into(JNIEnv *env, int (*call)(gkd_ctx *, uint32_t, gkd_joins *), jlong h, jint n, jintArray a,
-                       jintArray b, jdoubleArray lenA, jdoubleArray lenB, jintArray nJoins) {
+/* the tree of `call` (gkd_all_vs_all_nj or gkd_all_vs_all_bionj), or with start != 0 of gkd_all_vs_all_bme from that
+ * start tree, over the first n sets: a, b, lenA, lenB hold n - 1 entries (the joins in order); nJoins[0] receives their
+ * number, and nSwaps[0] (BME only) the number of swaps */
+static jint joins_into(JNIEnv *env, int (*call)(gkd_ctx *, uint32_t, gkd_joins *), int start, jlong h, jint n,
+                       jintArray a, jintArray b, jdoubleArray lenA, jdoubleArray lenB, jintArray nJoins,
+                       jlongArray nSwaps) {
     if (!a || !b || !lenA || !lenB || !nJoins || n < 0 || (*env)->GetArrayLength(env, nJoins) < 1) return GKD_EINVAL;
+    if (start && (!nSwaps || (*env)->GetArrayLength(env, nSwaps) < 1)) return GKD_EINVAL;
     const jint cap = n > 0 ? n - 1 : 0;
     if ((*env)->GetArrayLength(env, a) < cap || (*env)->GetArrayLength(env, b) < cap ||
         (*env)->GetArrayLength(env, lenA) < cap || (*env)->GetArrayLength(env, lenB) < cap)
@@ -334,7 +337,10 @@ static jint joins_into(JNIEnv *env, int (*call)(gkd_ctx *, uint32_t, gkd_joins *
     jdouble *pla = (*env)->GetDoubleArrayElements(env, lenA, NULL);
     jdouble *plb = (*env)->GetDoubleArrayElements(env, lenB, NULL);
     gkd_joins out = {(uint32_t *)pa, (uint32_t *)pb, pla, plb, (uint64_t)cap, 0};
-    int rc = (pa && pb && pla && plb) ? call(CTX(h), (uint32_t)n, &out) : GKD_ENOMEM;
+    uint64_t swaps = 0;
+    int rc = !(pa && pb && pla && plb) ? GKD_ENOMEM
+             : start                   ? gkd_all_vs_all_bme(CTX(h), (uint32_t)n, start, &out, &swaps)
+                                       : call(CTX(h), (uint32_t)n, &out);
     if (plb) (*env)->ReleaseDoubleArrayElements(env, lenB, plb, 0);
     if (pla) (*env)->ReleaseDoubleArrayElements(env, lenA, pla, 0);
     if (pb) (*env)->ReleaseIntArrayElements(env, b, pb, 0);
@@ -342,6 +348,10 @@ static jint joins_into(JNIEnv *env, int (*call)(gkd_ctx *, uint32_t, gkd_joins *
     if (rc == GKD_OK) {
         jint nj = (jint)out.n;
         (*env)->SetIntArrayRegion(env, nJoins, 0, 1, &nj);
+        if (start) {
+            jlong ns = (jlong)swaps;
+            (*env)->SetLongArrayRegion(env, nSwaps, 0, 1, &ns);
+        }
     }
     return rc;
 }
@@ -350,12 +360,21 @@ static jint joins_into(JNIEnv *env, int (*call)(gkd_ctx *, uint32_t, gkd_joins *
 JNIEXPORT jint JNICALL FN(allVsAllNj)(JNIEnv *env, jclass c, jlong h, jint n, jintArray a, jintArray b, jdoubleArray lenA,
                                       jdoubleArray lenB, jintArray nJoins) {
     (void)c;
-    return joins_into(env, gkd_all_vs_all_nj, h, n, a, b, lenA, lenB, nJoins);
+    return joins_into(env, gkd_all_vs_all_nj, 0, h, n, a, b, lenA, lenB, nJoins, NULL);
 }
 
 /* the BIONJ tree of the first n sets, in the joins of allVsAllNj */
 JNIEXPORT jint JNICALL FN(allVsAllBionj)(JNIEnv *env, jclass c, jlong h, jint n, jintArray a, jintArray b,
                                          jdoubleArray lenA, jdoubleArray lenB, jintArray nJoins) {
     (void)c;
-    return joins_into(env, gkd_all_vs_all_bionj, h, n, a, b, lenA, lenB, nJoins);
+    return joins_into(env, gkd_all_vs_all_bionj, 0, h, n, a, b, lenA, lenB, nJoins, NULL);
+}
+
+/* the tree of start (GKD_TREE_NJ or GKD_TREE_BIONJ) refined by balanced minimum-evolution NNIs, in the joins of
+ * allVsAllNj; nSwaps[0] receives the number of swaps */
+JNIEXPORT jint JNICALL FN(allVsAllBme)(JNIEnv *env, jclass c, jlong h, jint n, jint start, jintArray a, jintArray b,
+                                       jdoubleArray lenA, jdoubleArray lenB, jintArray nJoins, jlongArray nSwaps) {
+    (void)c;
+    if (start != GKD_TREE_NJ && start != GKD_TREE_BIONJ) return GKD_EINVAL;
+    return joins_into(env, NULL, start, h, n, a, b, lenA, lenB, nJoins, nSwaps);
 }

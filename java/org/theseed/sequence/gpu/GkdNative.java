@@ -66,6 +66,10 @@ final class GkdNative {
     static native int allVsAllNj(long ctx, int n, int[] a, int[] b, double[] lenA, double[] lenB, int[] nJoins);
     /** the BIONJ tree of the first n sets, in the joins of allVsAllNj */
     static native int allVsAllBionj(long ctx, int n, int[] a, int[] b, double[] lenA, double[] lenB, int[] nJoins);
+    /** the NJ (start 1) or BIONJ (start 2) tree of the first n sets refined by balanced minimum-evolution NNIs, in the
+     *  joins of allVsAllNj; nSwaps[0] receives the number of swaps */
+    static native int allVsAllBme(long ctx, int n, int start, int[] a, int[] b, double[] lenA, double[] lenB, int[] nJoins,
+                                  long[] nSwaps);
     /** SequenceKmers.similarity / distance for one pair; either output may be null (length-1 arrays) */
     static native int pair(long ctx, int a, int b, long[] inter, double[] dist);
     /** out[0] = the reference's HashSet size of set id */

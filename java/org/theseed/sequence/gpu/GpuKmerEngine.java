@@ -253,6 +253,16 @@ public class GpuKmerEngine implements AutoCloseable {
         return joins[0];
     }
 
+    /** the NJ (start 1) or BIONJ (start 2) tree of every set refined by balanced minimum-evolution nearest-neighbour
+     *  interchanges (Desper and Gascuel 2002), with BME branch lengths, in the joins of allVsAllNj; returns the number of
+     *  joins, and nSwaps[0] receives the number of swaps taken. */
+    public synchronized int allVsAllBme(int start, int[] a, int[] b, double[] lenA, double[] lenB, long[] nSwaps) {
+        this.build();
+        int[] joins = new int[1];
+        check(GkdNative.allVsAllBme(this.ctx, this.size(), start, a, b, lenA, lenB, joins, nSwaps));
+        return joins[0];
+    }
+
     /** SequenceKmers.distance(other) for the greedy callers (DistanceRepsProcessor, FastaDistanceRepsProcessor) */
     public synchronized double distance(int a, int b) {
         this.build();
